@@ -4,6 +4,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path, rank 0 only
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's outputs, DIR/<name>.npy
 
 Workload (BASELINE.json configs[3], "throughput mode"): 256 scene frames x 5,000 SIFT descriptors
 against 1,000 model objects x 1,000 descriptors, u8 128-d, synthetic (seeded).  Every frame contains
@@ -235,38 +236,10 @@ class CpuReference:
         self.scene = O.Scene(wl["q_xy"], wl["q_angle"], wl["q_octave"], wl["m_xy"], wl["m_angle"], wl["m_octave"],
                              wl["m_image"], wl["img_centroid"], wl["img_size"], int(wl["frame_wh"][0, 0]),
                              int(wl["frame_wh"][0, 1]), np.arange(args.objects, dtype=np.int32))
-        # The Hough / affine leg runs the reference's OWN modules where its checkout exists (the authoring
-        # container); the GPU box has no /root/reference, there the oracle port of the same loops is timed.
-        self.kind, self.refmain = "port", None
+        # The reference itself is not part of this repository: the Hough / affine leg times the oracle's
+        # port of the same single-threaded loops.
+        self.kind = "port"
         self.hough_what = "oracle port of the reference's single-threaded Python Hough/affine loops"
-        if Path("/root/reference/main.py").exists():
-            try:
-                sys.path.insert(0, str(ROOT / "tests" / "golden"))
-                import make_golden
-                self.refmain = make_golden.import_reference()
-                self.kind = "reference"
-                self.hough_what = ("the reference's own Main.apply_hough_transform / get_valid_bins / "
-                                   "apply_affine_parameters (imported from /root/reference, single-threaded Python)")
-            except Exception:
-                self.refmain = None
-
-    def _live_hough_affine(self, mq, mt) -> int:
-        """main.py:89-157 through the unmodified reference modules on the given matches."""
-        cv2, wl = self.cv2, self.wl
-        kp = lambda xy, a, o, i: cv2.KeyPoint(float(xy[i, 0]), float(xy[i, 1]), 1.0, float(a[i]), 0.0, int(o[i]), int(i))  # noqa: E731
-        m = self.refmain.Main()
-        img = wl["m_image"]
-        m.matching_keypoints = [
-            (kp(wl["m_xy"], wl["m_angle"], wl["m_octave"], t), kp(wl["q_xy"], wl["q_angle"], wl["q_octave"], q),
-             tuple(int(v) for v in wl["img_size"][img[t]]), tuple(float(v) for v in wl["img_centroid"][img[t]]))
-            for q, t in zip(mq, mt)]
-        W, H = int(wl["frame_wh"][0, 0]), int(wl["frame_wh"][0, 1])
-        m.rgb_query = np.empty((H, W, 3), np.uint8)      # only .shape is read (main.py:102)
-        m.image_query_size = (W, H)
-        m.apply_hough_transform(15)
-        m.get_valid_bins(5)
-        m.apply_affine_parameters(4)
-        return len(m.valid_bins)
 
     def run(self, q_rows: np.ndarray) -> dict:
         """main.py:180-185 on the given query rows (all from one frame)."""
@@ -282,12 +255,9 @@ class CpuReference:
                 mq.append(int(q_rows[m.queryIdx]))
                 mt.append(int(self.offsets[m.imgIdx] + m.trainIdx))
         t1 = time.perf_counter()
-        if self.refmain is not None:
-            n_live = self._live_hough_affine(mq, mt)
-        else:
-            table = O.hough_vote(self.scene, mq, mt, 15)                    # main.py:89-119
-            vb = O.valid_bins(table, 5)                                     # main.py:121-132
-            n_live = len(O.affine_verify(self.scene, mq, mt, vb, 4))        # main.py:139-157
+        table = O.hough_vote(self.scene, mq, mt, 15)                    # main.py:89-119
+        vb = O.valid_bins(table, 5)                                     # main.py:121-132
+        n_live = len(O.affine_verify(self.scene, mq, mt, vb, 4))        # main.py:139-157
         t2 = time.perf_counter()
         return dict(n=len(q_rows), t_match=t1 - t0, t_hough_affine=t2 - t1, matches=len(mq), live=n_live)
 
@@ -507,6 +477,37 @@ def oracle_spot_check(wl, res, pipe, args, rows=64):
     return out
 
 
+def dump_outputs(res, out_dir, budget=60 << 20):   # below 64 MB with the .npy headers
+    """--dump-outputs: what the last timed step returned to its caller (DetectionPipeline.fetch), one
+    DIR/<name>.npy per array; integers and flags as float64 (exact), floating-point arrays at their own
+    precision, counts as 0-d arrays.  The device appends verified bins in whatever order its atomics
+    resolve, so the per-bin arrays are written in (Hough space, bin code) order and valid_bin, a position
+    in the device's bin table, is left out.  query_rows holds the query row of each entry of the per-query
+    arrays (idx, ok); if they would take the total past `budget` bytes, a fixed seeded sample of rows is
+    written."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+
+    def f(a):
+        a = np.asarray(a)
+        return a if a.dtype.kind == "f" else a.astype(np.float64)
+
+    order = np.lexsort((res["valid_code"], res["valid_group"]))
+    arrays = {k: f(res[k][order]) for k in ("valid_group", "valid_code", "valid_order", "valid_mean", "params",
+                                            "votes", "status")}
+    arrays.update({k: f(v) for k, v in res.items() if k.startswith("n_")})
+    per_query = {"query_rows": f(np.arange(len(res["idx"])) + res["row_lo"]), "idx": f(res["idx"]), "ok": f(res["ok"])}
+    n = len(res["idx"])
+    row_bytes = sum(a[:1].nbytes for a in per_query.values())
+    room = max(budget - sum(a.nbytes for a in arrays.values()), 0) // max(row_bytes, 1)
+    if n > room:
+        keep = np.sort(np.random.default_rng(0).choice(n, room, replace=False))
+        per_query = {k: a[keep] for k, a in per_query.items()}
+    arrays.update(per_query)
+    for k, a in arrays.items():
+        np.save(out / f"{k}.npy", a)
+
+
 def torch_index(rows, like):
     import torch
     return torch.from_numpy(np.asarray(rows, np.int64)).to(like.device)
@@ -616,6 +617,8 @@ def run_ours(args):
     int8_tops = measure_int8_cublas_tops(device) if rank == 0 else None
     m = measure(args, wl, args.shard, rank, world, local, device, barrier)
     pipe, nq, nq_total, res = m["pipe"], m["nq"], m["nq_total"], m["res"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(res, args.dump_outputs)
 
     # ---------------- BASELINE configs[2]: 10k-query latency against the (sharded) 1M database
     c3 = None
@@ -823,7 +826,11 @@ def main():
                     help="--shard db: how the shard-local top-2 are merged (DetectionPipeline)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="CPU work per baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0's result) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -330,6 +330,54 @@ def make_c1(model_wh=(1500, 1000), scene_wh=(2000, 1500), scale=0.5, angle_deg=2
           len(out["live_keys"]), "final", out["final_pose"].round(2).tolist())
 
 
+LIVE_KEYS = ("knn_idx", "knn_dist", "match_q", "match_t", "bin_keys", "bin_votes", "bin_means", "valid_keys",
+             "live_keys", "live_votes", "live_params", "n_pairs_after", "bins", "vote_thr", "affine_thr")
+
+
+def oracle_outputs(sc: scenes.SyntheticScene, bins, vote_thr, affine_thr):
+    """The LIVE_KEYS of run_reference, computed by the oracle (oracle/sod_oracle.py)."""
+    from oracle import sod_oracle as O
+    scene = O.Scene(sc.q_xy, sc.q_angle, sc.q_octave, sc.m_xy, sc.m_angle, sc.m_octave, sc.m_image,
+                    sc.img_centroid, sc.img_size, sc.width, sc.height)
+    idx, d2 = O.knn2(sc.q_des, sc.m_des)
+    ok = O.ratio_pass(d2, idx)
+    match_q, match_t = np.nonzero(ok)[0].astype(np.int32), idx[ok, 0].astype(np.int32)
+    table = O.hough_vote(scene, match_q, match_t, bins)
+    hb = list(table.values())
+    hough = dict(bin_keys=np.array([k[1:] for k in table.keys()], np.int32).reshape(-1, 4),
+                 bin_votes=np.array([b.votes for b in hb], np.int32),
+                 bin_means=np.array([[b.centroid[0], b.centroid[1], b.angle, b.scale, b.img_size[0], b.img_size[1]]
+                                     for b in hb], np.float64).reshape(-1, 6))
+    vb = O.valid_bins(table, vote_thr)
+    valid_keys = np.array([b.pose for b in vb], np.int32).reshape(-1, 4)
+    live = O.affine_verify(scene, match_q, match_t, vb, affine_thr)     # updates the bins of `table` in place
+    return dict(knn_idx=idx.astype(np.int32), knn_dist=O.match_distance(d2), match_q=match_q, match_t=match_t,
+                **hough, valid_keys=valid_keys, live_keys=np.array([b.pose for b in live], np.int32).reshape(-1, 4),
+                live_votes=np.array([b.votes for b in live], np.int32),
+                live_params=np.array([b.affine for b in live], np.float64).reshape(-1, 6),
+                n_pairs_after=np.int64(sum(b.votes for b in live)),
+                bins=np.int32(bins), vote_thr=np.int32(vote_thr), affine_thr=np.int32(affine_thr))
+
+
+def make_live_cases(refmain=None):
+    """tests/golden/live_<seed>.npz for test_oracle_live_reference: the expected outputs of each case,
+    from the reference's Main when `refmain` is given, else from the oracle (`source` records which), and
+    the digest of the inputs: the test regenerates the inputs themselves from the seed."""
+    sys.path.insert(0, str(ROOT))
+    from test_oracle_live_reference import CASES, input_digest
+    for seed, kw, bins, vote_thr, affine_thr in CASES:
+        sc = scenes.make_scene(seed, **kw)
+        if refmain is not None:
+            out = run_reference(refmain, sc, bins=bins, vote_thr=vote_thr, affine_thr=affine_thr)
+            out = {k: out[k] for k in LIVE_KEYS}
+        else:
+            out = oracle_outputs(sc, bins, vote_thr, affine_thr)
+        np.savez_compressed(HERE / f"live_{seed}.npz", **out, input_digest=np.array(input_digest(sc)),
+                            source=np.array("reference" if refmain is not None else "oracle"))
+        print(f"live_{seed}: matches", len(out["match_q"]), "bins", len(out["bin_votes"]), "valid",
+              len(out["valid_keys"]), "live", len(out["live_keys"]))
+
+
 def main():
     if "--c1-only" in sys.argv:
         return make_c1()
@@ -337,6 +385,8 @@ def main():
         return make_postprocess()
     if "--affine-singular-only" in sys.argv:
         return make_affine_singular()
+    if "--live-cases-from-oracle" in sys.argv:
+        return make_live_cases()
     refmain = import_reference()
     import cv2
     for name, kw in SCENES.items():
@@ -351,6 +401,7 @@ def main():
     make_postprocess()
     make_affine_singular()
     make_c1()
+    make_live_cases(refmain)
 
     # known-answer facts (SURVEY.md §4 T4, T5, T8) taken from the reference's own libraries
     import math
