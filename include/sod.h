@@ -392,6 +392,53 @@ int sod_pose_adjacency(const double* cx, const double* cy, const double* reach_x
 int sod_angle_adjacency(const double* angle, const int32_t* segment, int64_t n, double max_degrees,
                         uint32_t* adj, int32_t* label, sod_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * SIFT extraction (in front of the path)
+ * ---------------------------------------------------------------------------------------------- */
+
+/* cv2.SIFT_create() with its default parameters (3 layers per octave, contrast threshold 0.04, edge
+ * threshold 10, sigma 1.6, image doubled first, all features kept) on a u8 gray image (device memory,
+ * rows `pitch` bytes apart, 1..32768 pixels a side).  Keypoints follow cv2's conventions (KeyPoint.pt,
+ * .size, .angle, .response, .octave packed with first octave -1, so unpack_sift_octave applies) and come
+ * sorted and de-duplicated as cv2 returns them; descriptors are u8 rows ready for the matcher.  Not bit-exact:
+ * DESIGN.md 2 states the measured agreement with cv2. */
+#define SOD_SIFT_MAX_OCTAVES 16
+#define SOD_SIFT_MAX_CAP (1 << 24)
+
+typedef struct {
+  float* xy;          /* [cap][2] KeyPoint.pt */
+  float* size;        /* [cap] */
+  float* angle;       /* [cap] degrees in [0,360) */
+  float* response;    /* [cap] */
+  int32_t* octave;    /* [cap] */
+  uint8_t* des;       /* [cap][128] */
+  int32_t* counters;  /* [2] number of keypoints, overflow flag (1 = more than cap keypoints before duplicate
+                         removal: the output is incomplete and must not be used); written by the call */
+  int64_t cap;        /* 1..SOD_SIFT_MAX_CAP */
+} sod_sift_out;
+
+/* Bytes of workspace (256-byte aligned) for an image of this size and max_keypoints = out.cap; 0 if the size or
+ * the capacity is out of range.  max_keypoints = 0 is enough for sod_sift_describe. */
+size_t sod_sift_workspace_bytes(int32_t width, int32_t height, int64_t max_keypoints);
+
+/* Replaces cv2.SIFT_create().detectAndCompute(gray, None) of Main.get_query_features (main.py:43-46) and of
+ * stream.sift_features.  The Gaussian pyramid is left in the workspace (sod_sift_level_offset). */
+int sod_sift_extract(const uint8_t* gray, int32_t width, int32_t height, int64_t pitch, const sod_sift_out* out,
+                     void* workspace, size_t workspace_bytes, sod_stream_t stream);
+
+/* cv2.SIFT.compute(gray, keypoints) for n caller-supplied keypoints (device arrays in the layout of
+ * sod_sift_out): des [n][128].  The pyramid is the one detectAndCompute builds (image doubled, so a keypoint set
+ * that contains octave -1, as every set cv2 detects does).  A keypoint whose octave and layer name no pyramid
+ * level gets a zero row and adds 1 to *n_invalid (device int32, caller zeroes it; may be NULL). */
+int sod_sift_describe(const uint8_t* gray, int32_t width, int32_t height, int64_t pitch, const float* xy,
+                      const float* size, const float* angle, const int32_t* octave, int64_t n, uint8_t* des,
+                      int32_t* n_invalid, void* workspace, size_t workspace_bytes, sod_stream_t stream);
+
+/* Byte offset in the workspace of Gaussian level `level` (0..5) of `octave` (-1 = the doubled image) after
+ * sod_sift_extract / sod_sift_describe, f32 rows of wh_host[0] (HOST, may be NULL) values, wh_host[1] rows.
+ * -1 if the image has no such level.  Lets a caller check the pyramid against cv2. */
+int64_t sod_sift_level_offset(int32_t width, int32_t height, int32_t octave, int32_t level, int32_t* wh_host);
+
 #ifdef __cplusplus
 }
 #endif

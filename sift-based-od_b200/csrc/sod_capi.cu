@@ -59,7 +59,7 @@ int device_sm_count() {
 
 extern "C" {
 
-int sod_version(void) { return 1000; }
+int sod_version(void) { return 1001; }
 
 const char* sod_last_error(void) { return sod::g_err; }
 

@@ -1,0 +1,757 @@
+// SIFT keypoints and descriptors on the device, reproducing cv2.SIFT_create() with its default parameters
+// (3 layers per octave, contrast threshold 0.04, edge threshold 10, sigma 1.6, image doubled first, all
+// features kept).  It replaces the host OpenCV call of Main.get_query_features (main.py:43-46) and of
+// stream.sift_features; the conventions below follow OpenCV's sift.simd.hpp and were checked against cv2
+// as a black box (GaussianBlur = sepFilter2D with getGaussianKernel CV_32F and BORDER_REFLECT_101,
+// resize INTER_LINEAR with half-pixel centres, fastAtan2, the output sort and duplicate rule).
+//
+//   pyramid     u8 -> f32, bilinear x2, Gaussian chain per octave (one fused two-pass launch per level,
+//               the horizontal pass kept in shared memory), octave o+1 starts from every other pixel of
+//               level 3 of octave o.  DoG levels are never stored: every reader takes G[l+1] - G[l].
+//   extrema     one thread per pixel and layer: 26-neighbour test, then OpenCV's Newton refinement,
+//               contrast and edge tests in the same thread; survivors go to a candidate list.
+//   orientation one warp per candidate: 36-bin histogram (per-lane partial histograms summed in a fixed
+//               order, so the result does not depend on scheduling), smoothing, one keypoint per peak.
+//   order       cub radix sort by (x, y), short runs of equal (x, y) ordered by (size, angle, response,
+//               octave), entries equal in (pt, size, angle) dropped: cv2's KeyPointsFilter order.
+//   descriptor  one block per keypoint, 4x4x8 histogram with trilinear spreading, clip 0.2, x512, u8.
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
+
+#include <cfloat>
+#include <climits>
+#include <cmath>
+
+#include "sod_common.cuh"
+
+namespace sod {
+namespace {
+
+constexpr int kLayers = 3;             // nOctaveLayers
+constexpr int kLevels = kLayers + 3;   // Gaussian levels per octave
+constexpr float kSigma = 1.6f;
+constexpr float kContrast = 0.04f;
+constexpr float kEdge = 10.f;
+constexpr int kBorder = 5;             // SIFT_IMG_BORDER
+constexpr int kMaxInterp = 5;          // SIFT_MAX_INTERP_STEPS
+constexpr int kOriBins = 36;
+constexpr int kD = 4, kN = 8;          // descriptor: kD x kD cells of kN orientation bins
+constexpr int kHistLen = (kD + 2) * (kD + 2) * (kN + 2);
+constexpr int kMaxOct = SOD_SIFT_MAX_OCTAVES;
+constexpr int kMaxSide = 32768;        // input side limit: the doubled image stays below 2^16 pixels a side
+constexpr int kTile = 32;              // blur output tile
+constexpr int kMaxRadius = 13;         // largest blur radius of the default parameters (sigma 3.09, 27 taps)
+constexpr int kOriWarps = 4;
+
+struct Pyramid {
+  float* base;
+  int64_t off[kMaxOct];                // element offset of octave o's first level
+  int w[kMaxOct], h[kMaxOct];
+  int n_oct;
+  __host__ __device__ float* level(int o, int l) const { return base + off[o] + (int64_t)l * w[o] * h[o]; }
+};
+
+struct Taps {
+  float k[2 * kMaxRadius + 1];
+  int r;
+};
+
+struct Cand {                          // a refined extremum, before orientation (octave index o is 0-based)
+  float x, y, size, response;
+  int32_t octave, o, layer, r, c;
+};
+
+struct Kp {                            // a finished keypoint in cv2's conventions (first octave -1)
+  float x, y, size, angle, response;
+  int32_t octave;
+};
+
+// Workspace layout (byte offsets from the workspace start, every block 256-byte aligned).  The pyramid comes
+// first so that sod_sift_level_offset does not depend on the keypoint capacity.
+struct Plan {
+  Pyramid pyr;
+  size_t cand, raw, keys_in, keys_out, vals_in, vals_out, keep, pos, counters, cub_tmp, cub_bytes, total;
+};
+
+size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
+
+int octave_count(int width, int height) {
+  // cvRound(log2(min side of the doubled image) - 2) - firstOctave, firstOctave = -1
+  const double m = 2.0 * (width < height ? width : height);
+  return (int)std::lrint(std::log(m) / std::log(2.0) - 2.0) + 1;
+}
+
+// Pyramid geometry and workspace offsets; cap = 0 plans the pyramid alone (sod_sift_describe).
+bool make_plan(int width, int height, int64_t cap, Plan* p) {
+  int n_oct = octave_count(width, height);
+  if (n_oct < 0) n_oct = 0;
+  if (n_oct > kMaxOct) return false;
+  p->pyr.base = nullptr;
+  p->pyr.n_oct = n_oct;
+  int64_t off = 0;
+  int w = 2 * width, h = 2 * height;
+  for (int o = 0; o < kMaxOct; ++o) {
+    p->pyr.off[o] = off;
+    p->pyr.w[o] = o < n_oct ? w : 0;
+    p->pyr.h[o] = o < n_oct ? h : 0;
+    if (o < n_oct) {
+      off += (int64_t)kLevels * w * h;
+      w /= 2;
+      h /= 2;
+    }
+  }
+  size_t at = align256((size_t)off * sizeof(float));
+  auto take = [&](size_t bytes) { size_t r = at; at += align256(bytes); return r; };
+  p->cand = take(sizeof(Cand) * cap);
+  p->raw = take(sizeof(Kp) * cap);
+  p->keys_in = take(sizeof(uint64_t) * cap);
+  p->keys_out = take(sizeof(uint64_t) * cap);
+  p->vals_in = take(sizeof(int32_t) * cap);
+  p->vals_out = take(sizeof(int32_t) * cap);
+  p->keep = take(sizeof(int32_t) * cap);
+  p->pos = take(sizeof(int32_t) * cap);
+  p->counters = take(sizeof(int32_t) * 4);
+  size_t sort_bytes = 0, scan_bytes = 0;
+  if (cap > 0) {
+    cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, (const uint64_t*)nullptr, (uint64_t*)nullptr,
+                                    (const int32_t*)nullptr, (int32_t*)nullptr, (int)cap);
+    cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const int32_t*)nullptr, (int32_t*)nullptr, (int)cap);
+  }
+  p->cub_bytes = sort_bytes > scan_bytes ? sort_bytes : scan_bytes;
+  p->cub_tmp = take(p->cub_bytes);
+  p->total = at;
+  return true;
+}
+
+// cv::getGaussianKernel(round(8 sigma + 1) | 1, sigma, CV_32F): exp in double, stored as float, normalised
+// by the double sum of the stored values.
+bool gaussian_taps(double sigma, Taps* t) {
+  const int n = (int)std::lrint(sigma * 8 + 1) | 1;
+  t->r = n / 2;
+  if (t->r > kMaxRadius) return false;
+  const double scale2 = -0.5 / (sigma * sigma);
+  double sum = 0;
+  for (int i = 0; i < n; ++i) {
+    const double x = i - (n - 1) * 0.5;
+    t->k[i] = (float)std::exp(scale2 * x * x);
+    sum += t->k[i];
+  }
+  sum = 1. / sum;
+  for (int i = 0; i < n; ++i) t->k[i] = (float)(t->k[i] * sum);
+  return true;
+}
+
+// ---------------------------------------------------------------------------------------------- device
+
+__device__ __forceinline__ int reflect101(int p, int len) {   // cv::borderInterpolate, BORDER_REFLECT_101
+  if (len == 1) return 0;
+  while ((unsigned)p >= (unsigned)len) p = p < 0 ? -p : 2 * len - 2 - p;
+  return p;
+}
+
+// cv::fastAtan2 (degrees in [0, 360)), the polynomial OpenCV uses in its SIFT, not atan2.
+__device__ __forceinline__ float fast_atan2(float y, float x) {
+  constexpr float s = (float)(180 / 3.14159265358979323846);
+  const float p1 = 0.9997878412794807f * s, p3 = -0.3258083974640975f * s, p5 = 0.1555786518463281f * s,
+              p7 = -0.04432655554792128f * s;
+  const float ax = fabsf(x), ay = fabsf(y);
+  float a, c, c2;
+  if (ax >= ay) {
+    c = ay / (ax + (float)DBL_EPSILON);
+    c2 = c * c;
+    a = (((p7 * c2 + p5) * c2 + p3) * c2 + p1) * c;
+  } else {
+    c = ax / (ay + (float)DBL_EPSILON);
+    c2 = c * c;
+    a = 90.f - (((p7 * c2 + p5) * c2 + p3) * c2 + p1) * c;
+  }
+  if (x < 0) a = 180.f - a;
+  if (y < 0) a = 360.f - a;
+  return a;
+}
+
+// cv::resize(INTER_LINEAR) to exactly twice the size: source coordinate (d + 0.5) / 2 - 0.5, clamped.
+__global__ void sift_upsample_kernel(const uint8_t* __restrict__ src, int sw, int sh, int64_t pitch,
+                                     float* __restrict__ dst) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
+  const int dw = 2 * sw, dh = 2 * sh;
+  if (x >= dw || y >= dh) return;
+  float fx = (float)((x + 0.5) * 0.5 - 0.5), fy = (float)((y + 0.5) * 0.5 - 0.5);
+  int sx = (int)floorf(fx), sy = (int)floorf(fy);
+  fx -= sx;
+  fy -= sy;
+  if (sx < 0) fx = 0.f, sx = 0;
+  if (sy < 0) fy = 0.f, sy = 0;
+  if (sx >= sw - 1) fx = 0.f, sx = sw - 1;
+  if (sy >= sh - 1) fy = 0.f, sy = sh - 1;
+  const int sx1 = min(sx + 1, sw - 1), sy1 = min(sy + 1, sh - 1);
+  const uint8_t* r0 = src + (int64_t)sy * pitch;
+  const uint8_t* r1 = src + (int64_t)sy1 * pitch;
+  const float a0 = (float)r0[sx] * (1.f - fx) + (float)r0[sx1] * fx;
+  const float a1 = (float)r1[sx] * (1.f - fx) + (float)r1[sx1] * fx;
+  dst[(int64_t)y * dw + x] = a0 * (1.f - fy) + a1 * fy;
+}
+
+// cv::GaussianBlur on a float image: horizontal pass into shared memory, then the vertical pass, both in the
+// symmetric form of OpenCV's row / column filters (centre tap, then pairs outwards), BORDER_REFLECT_101.
+__global__ void __launch_bounds__(256) sift_blur_kernel(const float* __restrict__ src, float* __restrict__ dst,
+                                                       int w, int h, Taps t) {
+  __shared__ float in[kTile + 2 * kMaxRadius][kTile + 2 * kMaxRadius + 1];
+  __shared__ float mid[kTile + 2 * kMaxRadius][kTile + 1];
+  __shared__ float k[2 * kMaxRadius + 1];
+  const int r = t.r, x0 = blockIdx.x * kTile, y0 = blockIdx.y * kTile, span = kTile + 2 * r;
+  if (threadIdx.x < 2 * r + 1) k[threadIdx.x] = t.k[threadIdx.x];
+  for (int i = threadIdx.x; i < span * span; i += blockDim.x) {
+    const int ty = i / span, tx = i - ty * span;
+    const int gy = reflect101(y0 - r + ty, h), gx = reflect101(x0 - r + tx, w);
+    SOD_DCHECK(gy >= 0 && gy < h && gx >= 0 && gx < w);
+    in[ty][tx] = src[(int64_t)gy * w + gx];
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < span * kTile; i += blockDim.x) {
+    const int ty = i / kTile, tx = i - ty * kTile;
+    const float* s = &in[ty][tx + r];
+    float acc = k[r] * s[0];
+    for (int j = 1; j <= r; ++j) acc += k[r + j] * (s[j] + s[-j]);
+    mid[ty][tx] = acc;
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < kTile * kTile; i += blockDim.x) {
+    const int ty = i / kTile, tx = i - ty * kTile, gx = x0 + tx, gy = y0 + ty;
+    if (gx >= w || gy >= h) continue;
+    float acc = k[r] * mid[ty + r][tx];
+    for (int j = 1; j <= r; ++j) acc += k[r + j] * (mid[ty + r + j][tx] + mid[ty + r - j][tx]);
+    dst[(int64_t)gy * w + gx] = acc;
+  }
+}
+
+// cv::resize(INTER_NEAREST) to half size: every other pixel.
+__global__ void sift_halve_kernel(const float* __restrict__ src, int sw, float* __restrict__ dst, int dw, int dh) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
+  if (x >= dw || y >= dh) return;
+  dst[(int64_t)y * dw + x] = src[(int64_t)(2 * y) * sw + 2 * x];
+}
+
+// DoG level l of octave o at (r, c): G[l+1] - G[l], the value cv::subtract stores.
+__device__ __forceinline__ float dog(const Pyramid& P, int o, int l, int r, int c) {
+  const int64_t i = (int64_t)r * P.w[o] + c;
+  return P.level(o, l + 1)[i] - P.level(o, l)[i];
+}
+
+// OpenCV's adjustLocalExtrema: Newton steps on the 3x3 Hessian of the DoG (derivatives scaled by 1/255),
+// contrast and edge tests, keypoint fields in the octave numbering of the doubled image.
+__device__ bool refine(const Pyramid& P, int o, int& layer, int& r, int& c, Cand* kp) {
+  constexpr float img_scale = 1.f / 255.f, deriv_scale = img_scale * 0.5f, second_scale = img_scale,
+                  cross_scale = img_scale * 0.25f;
+  const int w = P.w[o], h = P.h[o];
+  float xi = 0, xr = 0, xc = 0;
+  int i = 0;
+  for (; i < kMaxInterp; ++i) {
+    auto D = [&](int dl, int dr, int dc) { return dog(P, o, layer + dl, r + dr, c + dc); };
+    const float dx = (D(0, 0, 1) - D(0, 0, -1)) * deriv_scale, dy = (D(0, 1, 0) - D(0, -1, 0)) * deriv_scale,
+                ds = (D(1, 0, 0) - D(-1, 0, 0)) * deriv_scale;
+    const float v2 = D(0, 0, 0) * 2;
+    const float dxx = (D(0, 0, 1) + D(0, 0, -1) - v2) * second_scale;
+    const float dyy = (D(0, 1, 0) + D(0, -1, 0) - v2) * second_scale;
+    const float dss = (D(1, 0, 0) + D(-1, 0, 0) - v2) * second_scale;
+    const float dxy = (D(0, 1, 1) - D(0, 1, -1) - D(0, -1, 1) + D(0, -1, -1)) * cross_scale;
+    const float dxs = (D(1, 0, 1) - D(1, 0, -1) - D(-1, 0, 1) + D(-1, 0, -1)) * cross_scale;
+    const float dys = (D(1, 1, 0) - D(1, -1, 0) - D(-1, 1, 0) + D(-1, -1, 0)) * cross_scale;
+    // Matx33f::solve(DECOMP_LU) of a 3x3 system: Cramer's rule; a singular matrix leaves X = 0
+    const float a00 = dxx, a01 = dxy, a02 = dxs, a10 = dxy, a11 = dyy, a12 = dys, a20 = dxs, a21 = dys, a22 = dss;
+    float det = a00 * (a11 * a22 - a21 * a12) - a01 * (a10 * a22 - a20 * a12) + a02 * (a10 * a21 - a20 * a11);
+    float X0 = 0, X1 = 0, X2 = 0;
+    if (det != 0) {
+      det = 1 / det;
+      X0 = det * (dx * (a11 * a22 - a12 * a21) - a01 * (dy * a22 - a12 * ds) + a02 * (dy * a21 - a11 * ds));
+      X1 = det * (a00 * (dy * a22 - a12 * ds) - dx * (a10 * a22 - a12 * a20) + a02 * (a10 * ds - dy * a20));
+      X2 = det * (a00 * (a11 * ds - dy * a21) - a01 * (a10 * ds - dy * a20) + dx * (a10 * a21 - a11 * a20));
+    }
+    xi = -X2;
+    xr = -X1;
+    xc = -X0;
+    if (fabsf(xi) < 0.5f && fabsf(xr) < 0.5f && fabsf(xc) < 0.5f) break;
+    constexpr float far = (float)(INT_MAX / 3);
+    if (fabsf(xi) > far || fabsf(xr) > far || fabsf(xc) > far) return false;
+    c += __float2int_rn(xc);
+    r += __float2int_rn(xr);
+    layer += __float2int_rn(xi);
+    if (layer < 1 || layer > kLayers || c < kBorder || c >= w - kBorder || r < kBorder || r >= h - kBorder)
+      return false;
+  }
+  if (i >= kMaxInterp) return false;
+  auto D = [&](int dl, int dr, int dc) { return dog(P, o, layer + dl, r + dr, c + dc); };
+  const float dx = (D(0, 0, 1) - D(0, 0, -1)) * deriv_scale, dy = (D(0, 1, 0) - D(0, -1, 0)) * deriv_scale,
+              ds = (D(1, 0, 0) - D(-1, 0, 0)) * deriv_scale;
+  const float t = dx * xc + dy * xr + ds * xi;
+  const float contr = D(0, 0, 0) * img_scale + t * 0.5f;
+  if (fabsf(contr) * kLayers < kContrast) return false;
+  const float v2 = D(0, 0, 0) * 2.f;
+  const float dxx = (D(0, 0, 1) + D(0, 0, -1) - v2) * second_scale;
+  const float dyy = (D(0, 1, 0) + D(0, -1, 0) - v2) * second_scale;
+  const float dxy = (D(0, 1, 1) - D(0, 1, -1) - D(0, -1, 1) + D(0, -1, -1)) * cross_scale;
+  const float tr = dxx + dyy, det = dxx * dyy - dxy * dxy;
+  if (det <= 0 || tr * tr * kEdge >= (kEdge + 1) * (kEdge + 1) * det) return false;
+  const float scale = (float)(1 << o);
+  kp->x = ((float)c + xc) * scale;
+  kp->y = ((float)r + xr) * scale;
+  kp->octave = o + (layer << 8) + (__double2int_rn(((double)xi + 0.5) * 255) << 16);
+  kp->size = kSigma * powf(2.f, ((float)layer + xi) / kLayers) * scale * 2;
+  kp->response = fabsf(contr);
+  return true;
+}
+
+// Scale-space extrema of octave o: |DoG| > floor(0.5 * 0.04 / 3 * 255) = 1, not smaller (or not larger)
+// than all 26 neighbours, outside the 5-pixel border; refined survivors are appended to cand.
+__global__ void sift_extrema_kernel(Pyramid P, int o, Cand* __restrict__ cand, int cap, int* __restrict__ counters) {
+  const int c = kBorder + blockIdx.x * blockDim.x + threadIdx.x;
+  const int r = kBorder + blockIdx.y * blockDim.y + threadIdx.y;
+  const int layer = 1 + blockIdx.z;
+  if (c >= P.w[o] - kBorder || r >= P.h[o] - kBorder) return;
+  const float val = dog(P, o, layer, r, c);
+  if (!(fabsf(val) > 1.f)) return;
+  bool ext = true;
+  if (val > 0) {
+    for (int dl = -1; dl <= 1 && ext; ++dl)
+      for (int dr = -1; dr <= 1 && ext; ++dr)
+        for (int dc = -1; dc <= 1; ++dc)
+          if ((dl | dr | dc) && !(val >= dog(P, o, layer + dl, r + dr, c + dc))) { ext = false; break; }
+  } else {
+    for (int dl = -1; dl <= 1 && ext; ++dl)
+      for (int dr = -1; dr <= 1 && ext; ++dr)
+        for (int dc = -1; dc <= 1; ++dc)
+          if ((dl | dr | dc) && !(val <= dog(P, o, layer + dl, r + dr, c + dc))) { ext = false; break; }
+  }
+  if (!ext) return;
+  int l1 = layer, r1 = r, c1 = c;
+  Cand kp;
+  if (!refine(P, o, l1, r1, c1, &kp)) return;
+  kp.o = o;
+  kp.layer = l1;
+  kp.r = r1;
+  kp.c = c1;
+  const int slot = atomicAdd(&counters[0], 1);
+  if (slot >= cap) {
+    atomicExch(&counters[2], 1);
+    return;
+  }
+  SOD_DCHECK(slot >= 0 && slot < cap);
+  cand[slot] = kp;
+}
+
+// OpenCV's calcOrientationHist + the peak loop of findScaleSpaceExtrema, one warp per candidate.  Every
+// keypoint is written already moved to the first octave -1 (octave byte - 1, pt and size halved).
+__global__ void __launch_bounds__(32 * kOriWarps) sift_orient_kernel(Pyramid P, const Cand* __restrict__ cand,
+                                                                     int cap, int* __restrict__ counters,
+                                                                     Kp* __restrict__ raw) {
+  __shared__ float part[kOriWarps][32][kOriBins + 1];
+  __shared__ float hist[kOriWarps][kOriBins + 4];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int n = min(counters[0], cap);
+  for (int ci = blockIdx.x * kOriWarps + wib; ci < n; ci += gridDim.x * kOriWarps) {
+    const Cand k = cand[ci];
+    SOD_DCHECK(k.o >= 0 && k.o < P.n_oct && k.layer >= 1 && k.layer <= kLayers);
+    const float* img = P.level(k.o, k.layer);
+    const int w = P.w[k.o], h = P.h[k.o];
+    const float scl = k.size * 0.5f / (float)(1 << k.o);
+    const int radius = __float2int_rn(4.5f * scl);
+    const float sigma = 1.5f * scl, expf_scale = -1.f / (2.f * sigma * sigma);
+    for (int b = 0; b < kOriBins; ++b) part[wib][lane][b] = 0.f;
+    const int side = 2 * radius + 1;
+    for (int s = lane; s < side * side; s += 32) {
+      const int i = s / side - radius, j = s % side - radius;
+      const int y = k.r + i, x = k.c + j;
+      if (y <= 0 || y >= h - 1 || x <= 0 || x >= w - 1) continue;
+      const float dx = img[(int64_t)y * w + x + 1] - img[(int64_t)y * w + x - 1];
+      const float dy = img[(int64_t)(y - 1) * w + x] - img[(int64_t)(y + 1) * w + x];
+      const float wt = expf((float)(i * i + j * j) * expf_scale);
+      const float ori = fast_atan2(dy, dx), mag = sqrtf(dx * dx + dy * dy);
+      int bin = __float2int_rn((kOriBins / 360.f) * ori);
+      if (bin >= kOriBins) bin -= kOriBins;
+      if (bin < 0) bin += kOriBins;
+      SOD_DCHECK(bin >= 0 && bin < kOriBins);
+      part[wib][lane][bin] += wt * mag;
+    }
+    __syncwarp();
+    for (int b = lane; b < kOriBins; b += 32) {
+      float acc = 0.f;
+      for (int l = 0; l < 32; ++l) acc += part[wib][l][b];
+      hist[wib][b + 2] = acc;
+    }
+    __syncwarp();
+    if (lane == 0) {
+      float* t = &hist[wib][2];
+      t[-1] = t[kOriBins - 1];
+      t[-2] = t[kOriBins - 2];
+      t[kOriBins] = t[0];
+      t[kOriBins + 1] = t[1];
+      float sm[kOriBins];
+      float omax = 0.f;
+      for (int b = 0; b < kOriBins; ++b) {
+        sm[b] = (t[b - 2] + t[b + 2]) * (1.f / 16.f) + (t[b - 1] + t[b + 1]) * (4.f / 16.f) + t[b] * (6.f / 16.f);
+        omax = b ? fmaxf(omax, sm[b]) : sm[b];
+      }
+      const float mag_thr = omax * 0.8f;
+      for (int j = 0; j < kOriBins; ++j) {
+        const int l = j > 0 ? j - 1 : kOriBins - 1, r2 = j < kOriBins - 1 ? j + 1 : 0;
+        if (sm[j] > sm[l] && sm[j] > sm[r2] && sm[j] >= mag_thr) {
+          float bin = j + 0.5f * (sm[l] - sm[r2]) / (sm[l] - 2 * sm[j] + sm[r2]);
+          bin = bin < 0 ? kOriBins + bin : bin >= kOriBins ? bin - kOriBins : bin;
+          float angle = 360.f - (float)((360.f / kOriBins) * bin);
+          if (fabsf(angle - 360.f) < FLT_EPSILON) angle = 0.f;
+          const int slot = atomicAdd(&counters[1], 1);
+          if (slot >= cap) {
+            atomicExch(&counters[2], 1);
+            continue;
+          }
+          SOD_DCHECK(slot >= 0 && slot < cap);
+          Kp& o = raw[slot];
+          o.x = k.x * 0.5f;
+          o.y = k.y * 0.5f;
+          o.size = k.size * 0.5f;
+          o.angle = angle;
+          o.response = k.response;
+          o.octave = (k.octave & ~255) | ((k.octave - 1) & 255);
+        }
+      }
+    }
+    __syncwarp();
+  }
+}
+
+// Sort keys: (x bits, y bits) of the non-negative coordinates order as (x, y); unused slots sort last.
+__global__ void sift_sort_keys_kernel(const Kp* __restrict__ raw, const int* __restrict__ counters, int cap,
+                                      uint64_t* __restrict__ keys, int32_t* __restrict__ vals) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= cap) return;
+  const int n = min(counters[1], cap);
+  keys[i] = i < n ? ((uint64_t)__float_as_uint(raw[i].x) << 32) | __float_as_uint(raw[i].y) : ~0ull;
+  vals[i] = i;
+}
+
+__device__ __forceinline__ bool kp_less(const Kp& a, const Kp& b) {   // cv2's order after equal (x, y)
+  if (a.size != b.size) return a.size < b.size;
+  if (a.angle != b.angle) return a.angle < b.angle;
+  if (a.response != b.response) return a.response < b.response;
+  return a.octave < b.octave;
+}
+
+// Orders every run of equal (x, y) by (size, angle, response, octave); runs are a few keypoints long (the
+// orientations of one location), so the first thread of a run sorts it by insertion.
+__global__ void sift_sort_runs_kernel(const Kp* __restrict__ raw, const int* __restrict__ counters, int cap,
+                                      const uint64_t* __restrict__ keys, int32_t* __restrict__ vals) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const int n = min(counters[1], cap);
+  if (i >= n || (i > 0 && keys[i - 1] == keys[i]) || i + 1 >= n || keys[i + 1] != keys[i]) return;
+  int e = i + 1;
+  while (e < n && keys[e] == keys[i]) ++e;
+  for (int a = i + 1; a < e; ++a) {
+    const int v = vals[a];
+    SOD_DCHECK(v >= 0 && v < cap);
+    int b = a - 1;
+    while (b >= i && kp_less(raw[v], raw[vals[b]])) {
+      vals[b + 1] = vals[b];
+      --b;
+    }
+    vals[b + 1] = v;
+  }
+}
+
+// KeyPointsFilter::removeDuplicatedSorted: keep an entry unless it equals its predecessor in pt, size and
+// angle (equal entries are adjacent in this order).
+__global__ void sift_keep_kernel(const Kp* __restrict__ raw, const int* __restrict__ counters, int cap,
+                                 const int32_t* __restrict__ vals, int32_t* __restrict__ keep) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= cap) return;
+  const int n = min(counters[1], cap);
+  int k = 0;
+  if (i < n) {
+    k = 1;
+    if (i > 0) {
+      SOD_DCHECK(vals[i] >= 0 && vals[i] < cap && vals[i - 1] >= 0 && vals[i - 1] < cap);
+      const Kp a = raw[vals[i - 1]], b = raw[vals[i]];
+      k = !(a.x == b.x && a.y == b.y && a.size == b.size && a.angle == b.angle);
+    }
+  }
+  keep[i] = k;
+}
+
+__global__ void sift_emit_kernel(const Kp* __restrict__ raw, const int* __restrict__ counters, int cap,
+                                 const int32_t* __restrict__ vals, const int32_t* __restrict__ keep,
+                                 const int32_t* __restrict__ pos, sod_sift_out out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= cap) return;
+  if (i == cap - 1) {
+    out.counters[0] = pos[i] + keep[i];
+    out.counters[1] = counters[2];
+  }
+  if (!keep[i]) return;
+  const int p = pos[i], v = vals[i];
+  SOD_DCHECK(p >= 0 && p < cap && v >= 0 && v < cap);
+  const Kp k = raw[v];
+  out.xy[2 * p] = k.x;
+  out.xy[2 * p + 1] = k.y;
+  out.size[p] = k.size;
+  out.angle[p] = k.angle;
+  out.response[p] = k.response;
+  out.octave[p] = k.octave;
+}
+
+// OpenCV's calcDescriptors + calcSIFTDescriptor, one 128-thread block per keypoint.  n_dev (device, may be
+// NULL) overrides n.  A keypoint whose octave / layer names no level of the pyramid gets a zero row and is
+// counted in n_invalid (cv2 refuses such a keypoint).
+__global__ void __launch_bounds__(128) sift_descriptor_kernel(Pyramid P, const float* __restrict__ xy,
+                                                              const float* __restrict__ size,
+                                                              const float* __restrict__ angle,
+                                                              const int32_t* __restrict__ octave, int64_t n,
+                                                              const int32_t* __restrict__ n_dev,
+                                                              uint8_t* __restrict__ des, int32_t* n_invalid) {
+  __shared__ float hist[kHistLen];
+  __shared__ float red[4];
+  const int tid = threadIdx.x;
+  if (n_dev && n_dev[0] < n) n = n_dev[0];
+  for (int64_t q = blockIdx.x; q < n; q += gridDim.x) {
+    const int packed = octave[q];
+    int oct = packed & 255;
+    const int layer = (packed >> 8) & 255;
+    oct = oct < 128 ? oct : (-128 | oct);
+    const int o = oct + 1;
+    if (o < 0 || o >= P.n_oct || layer > kLayers + 2) {
+      des[q * 128 + tid] = 0;
+      if (tid == 0 && n_invalid) atomicAdd(n_invalid, 1);
+      continue;
+    }
+    const float scale = oct >= 0 ? 1.f / (float)(1 << oct) : (float)(1 << -oct);
+    const float scl = size[q] * scale * 0.5f;
+    const float ptx = xy[2 * q] * scale, pty = xy[2 * q + 1] * scale;
+    float ori = 360.f - angle[q];
+    if (fabsf(ori - 360.f) < FLT_EPSILON) ori = 0.f;
+    const float* img = P.level(o, layer);
+    const int cols = P.w[o], rows = P.h[o];
+    const int px = __float2int_rn(ptx), py = __float2int_rn(pty);
+    float cos_t = cosf(ori * (float)(3.14159265358979323846 / 180)),
+          sin_t = sinf(ori * (float)(3.14159265358979323846 / 180));
+    const float bins_per_deg = kN / 360.f, exp_scale = -1.f / (kD * kD * 0.5f);
+    const float hist_width = 3.f * scl;
+    int radius = __float2int_rn(hist_width * 1.4142135623730951f * (kD + 1) * 0.5f);
+    radius = min(radius, (int)sqrt((double)cols * cols + (double)rows * rows));
+    cos_t /= hist_width;
+    sin_t /= hist_width;
+    for (int i = tid; i < kHistLen; i += blockDim.x) hist[i] = 0.f;
+    __syncthreads();
+    const int side = 2 * radius + 1;
+    for (int s = tid; s < side * side; s += blockDim.x) {
+      const int i = s / side - radius, j = s % side - radius;
+      const float c_rot = j * cos_t - i * sin_t, r_rot = j * sin_t + i * cos_t;
+      float rbin = r_rot + kD / 2 - 0.5f, cbin = c_rot + kD / 2 - 0.5f;
+      const int r = py + i, c = px + j;
+      if (!(rbin > -1 && rbin < kD && cbin > -1 && cbin < kD && r > 0 && r < rows - 1 && c > 0 && c < cols - 1))
+        continue;
+      const float dx = img[(int64_t)r * cols + c + 1] - img[(int64_t)r * cols + c - 1];
+      const float dy = img[(int64_t)(r - 1) * cols + c] - img[(int64_t)(r + 1) * cols + c];
+      const float wt = expf((c_rot * c_rot + r_rot * r_rot) * exp_scale);
+      float obin = (fast_atan2(dy, dx) - ori) * bins_per_deg;
+      const float mag = sqrtf(dx * dx + dy * dy) * wt;
+      const int r0 = (int)floorf(rbin), c0 = (int)floorf(cbin);
+      int o0 = (int)floorf(obin);
+      rbin -= r0;
+      cbin -= c0;
+      obin -= o0;
+      if (o0 < 0) o0 += kN;
+      if (o0 >= kN) o0 -= kN;
+      const float v_r1 = mag * rbin, v_r0 = mag - v_r1;
+      const float v_rc11 = v_r1 * cbin, v_rc10 = v_r1 - v_rc11;
+      const float v_rc01 = v_r0 * cbin, v_rc00 = v_r0 - v_rc01;
+      const float v_rco111 = v_rc11 * obin, v_rco110 = v_rc11 - v_rco111;
+      const float v_rco101 = v_rc10 * obin, v_rco100 = v_rc10 - v_rco101;
+      const float v_rco011 = v_rc01 * obin, v_rco010 = v_rc01 - v_rco011;
+      const float v_rco001 = v_rc00 * obin, v_rco000 = v_rc00 - v_rco001;
+      const int idx = ((r0 + 1) * (kD + 2) + c0 + 1) * (kN + 2) + o0;
+      SOD_DCHECK(idx >= 0 && idx + (kD + 3) * (kN + 2) + 1 < kHistLen);
+      atomicAdd(&hist[idx], v_rco000);
+      atomicAdd(&hist[idx + 1], v_rco001);
+      atomicAdd(&hist[idx + (kN + 2)], v_rco010);
+      atomicAdd(&hist[idx + (kN + 3)], v_rco011);
+      atomicAdd(&hist[idx + (kD + 2) * (kN + 2)], v_rco100);
+      atomicAdd(&hist[idx + (kD + 2) * (kN + 2) + 1], v_rco101);
+      atomicAdd(&hist[idx + (kD + 3) * (kN + 2)], v_rco110);
+      atomicAdd(&hist[idx + (kD + 3) * (kN + 2) + 1], v_rco111);
+    }
+    __syncthreads();
+    // the orientation histograms are circular: bins n and n+1 fold onto 0 and 1
+    const int cell = tid / kN, k = tid % kN;
+    const int hidx = ((cell / kD + 1) * (kD + 2) + (cell % kD + 1)) * (kN + 2);
+    float v = hist[hidx + k] + (k < 2 ? hist[hidx + kN + k] : 0.f);
+    auto block_sum = [&](float x) {
+      for (int m = 16; m; m >>= 1) x += __shfl_xor_sync(0xffffffffu, x, m);
+      if ((tid & 31) == 0) red[tid >> 5] = x;
+      __syncthreads();
+      const float s = red[0] + red[1] + red[2] + red[3];
+      __syncthreads();
+      return s;
+    };
+    const float thr = sqrtf(block_sum(v * v)) * 0.2f;
+    v = fminf(v, thr);
+    const float nrm = 512.f / fmaxf(sqrtf(block_sum(v * v)), FLT_EPSILON);
+    des[q * 128 + tid] = (uint8_t)min(255, max(0, __float2int_rn(v * nrm)));
+  }
+}
+
+// The Gaussian pyramid of one image into the workspace.
+int build_pyramid(const uint8_t* gray, int width, int height, int64_t pitch, const Pyramid& P, cudaStream_t st) {
+  double sig[kLevels];
+  const double k = std::pow(2., 1. / kLayers);
+  for (int i = 1; i < kLevels; ++i) {
+    const double prev = std::pow(k, (double)(i - 1)) * kSigma, total = prev * k;
+    sig[i] = std::sqrt(total * total - prev * prev);
+  }
+  Taps taps[kLevels];
+  const float sig_diff = sqrtf(fmaxf(kSigma * kSigma - 0.5f * 0.5f * 4, 0.01f));
+  if (!gaussian_taps(sig_diff, &taps[0])) return SOD_ERR_UNSUPPORTED;
+  for (int i = 1; i < kLevels; ++i)
+    if (!gaussian_taps(sig[i], &taps[i])) return SOD_ERR_UNSUPPORTED;
+  const dim3 pb(32, 8);
+  auto pgrid = [&](int w, int h) { return dim3((w + 31) / 32, (h + 7) / 8); };
+  auto tgrid = [&](int w, int h) { return dim3((w + kTile - 1) / kTile, (h + kTile - 1) / kTile); };
+  // the doubled image goes to level 1's slot, blurred into level 0, and level 1 is then computed over it
+  sift_upsample_kernel<<<pgrid(P.w[0], P.h[0]), pb, 0, st>>>(gray, width, height, pitch, P.level(0, 1));
+  sift_blur_kernel<<<tgrid(P.w[0], P.h[0]), 256, 0, st>>>(P.level(0, 1), P.level(0, 0), P.w[0], P.h[0], taps[0]);
+  for (int o = 0; o < P.n_oct; ++o) {
+    if (o > 0)
+      sift_halve_kernel<<<pgrid(P.w[o], P.h[o]), pb, 0, st>>>(P.level(o - 1, kLayers), P.w[o - 1], P.level(o, 0),
+                                                            P.w[o], P.h[o]);
+    for (int l = 1; l < kLevels; ++l)
+      sift_blur_kernel<<<tgrid(P.w[o], P.h[o]), 256, 0, st>>>(P.level(o, l - 1), P.level(o, l), P.w[o], P.h[o],
+                                                              taps[l]);
+  }
+  SOD_CHECK_LAUNCH("sift pyramid");
+  return SOD_OK;
+}
+
+int check_image(const uint8_t* gray, int32_t width, int32_t height, int64_t pitch, const char* fn) {
+  SOD_CHECK_ARG(width >= 1 && height >= 1 && width <= kMaxSide && height <= kMaxSide,
+                "%s: image size %dx%d out of range (1..%d a side)", fn, width, height, kMaxSide);
+  SOD_CHECK_ARG(pitch >= width, "%s: pitch %lld < width %d", fn, (long long)pitch, width);
+  SOD_CHECK_ARG(gray != nullptr, "%s: null image", fn);
+  return SOD_OK;
+}
+
+}  // namespace
+}  // namespace sod
+
+using namespace sod;
+
+extern "C" {
+
+size_t sod_sift_workspace_bytes(int32_t width, int32_t height, int64_t max_keypoints) {
+  Plan p;
+  if (width < 1 || height < 1 || width > kMaxSide || height > kMaxSide || max_keypoints < 0 ||
+      max_keypoints > SOD_SIFT_MAX_CAP || !make_plan(width, height, max_keypoints, &p))
+    return 0;
+  return p.total;
+}
+
+int64_t sod_sift_level_offset(int32_t width, int32_t height, int32_t octave, int32_t level, int32_t* wh_host) {
+  Plan p;
+  if (width < 1 || height < 1 || width > kMaxSide || height > kMaxSide || !make_plan(width, height, 0, &p) ||
+      octave < -1 || octave + 1 >= p.pyr.n_oct || level < 0 || level >= kLevels) {
+    set_error("sod_sift_level_offset: no level %d of octave %d for a %dx%d image", level, octave, width, height);
+    return -1;
+  }
+  if (wh_host) {
+    wh_host[0] = p.pyr.w[octave + 1];
+    wh_host[1] = p.pyr.h[octave + 1];
+  }
+  const int o = octave + 1;
+  return (p.pyr.off[o] + (int64_t)level * p.pyr.w[o] * p.pyr.h[o]) * (int64_t)sizeof(float);
+}
+
+int sod_sift_extract(const uint8_t* gray, int32_t width, int32_t height, int64_t pitch, const sod_sift_out* out,
+                     void* workspace, size_t workspace_bytes, sod_stream_t stream) {
+  if (int rc = check_image(gray, width, height, pitch, "sod_sift_extract")) return rc;
+  SOD_CHECK_ARG(out != nullptr, "sod_sift_extract: null out");
+  SOD_CHECK_ARG(out->cap >= 1 && out->cap <= SOD_SIFT_MAX_CAP, "sod_sift_extract: cap %lld out of range (1..%d)",
+                (long long)out->cap, SOD_SIFT_MAX_CAP);
+  SOD_CHECK_ARG(out->xy && out->size && out->angle && out->response && out->octave && out->des && out->counters,
+                "sod_sift_extract: null output array");
+  Plan p;
+  SOD_CHECK_ARG(make_plan(width, height, out->cap, &p), "sod_sift_extract: too many octaves");
+  SOD_CHECK_ARG(workspace != nullptr && workspace_bytes >= p.total && ((uintptr_t)workspace & 255) == 0,
+                "sod_sift_extract: workspace of %zu bytes at %p; need %zu bytes, 256-byte aligned", workspace_bytes,
+                workspace, p.total);
+  cudaStream_t st = (cudaStream_t)stream;
+  char* ws = (char*)workspace;
+  p.pyr.base = (float*)ws;
+  const int cap = (int)out->cap;
+  int32_t* counters = (int32_t*)(ws + p.counters);
+  Cand* cand = (Cand*)(ws + p.cand);
+  Kp* raw = (Kp*)(ws + p.raw);
+  uint64_t* keys_in = (uint64_t*)(ws + p.keys_in);
+  uint64_t* keys_out = (uint64_t*)(ws + p.keys_out);
+  int32_t* vals_in = (int32_t*)(ws + p.vals_in);
+  int32_t* vals_out = (int32_t*)(ws + p.vals_out);
+  int32_t* keep = (int32_t*)(ws + p.keep);
+  int32_t* pos = (int32_t*)(ws + p.pos);
+  SOD_CHECK_CUDA(cudaMemsetAsync(counters, 0, 4 * sizeof(int32_t), st));
+  if (p.pyr.n_oct > 0) {
+    if (int rc = build_pyramid(gray, width, height, pitch, p.pyr, st)) return rc;
+    for (int o = 0; o < p.pyr.n_oct; ++o) {
+      const int iw = p.pyr.w[o] - 2 * kBorder, ih = p.pyr.h[o] - 2 * kBorder;
+      if (iw <= 0 || ih <= 0) continue;
+      sift_extrema_kernel<<<dim3((iw + 31) / 32, (ih + 7) / 8, kLayers), dim3(32, 8), 0, st>>>(p.pyr, o, cand, cap,
+                                                                                            counters);
+    }
+    SOD_CHECK_LAUNCH("sift_extrema_kernel");
+    const int sms = device_sm_count();
+    if (sms < 0) return SOD_ERR_CUDA;
+    sift_orient_kernel<<<sms * 8, 32 * kOriWarps, 0, st>>>(p.pyr, cand, cap, counters, raw);
+    SOD_CHECK_LAUNCH("sift_orient_kernel");
+  }
+  const int blocks = (cap + 255) / 256;
+  sift_sort_keys_kernel<<<blocks, 256, 0, st>>>(raw, counters, cap, keys_in, vals_in);
+  SOD_CHECK_LAUNCH("sift_sort_keys_kernel");
+  size_t tmp = p.cub_bytes;
+  SOD_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(ws + p.cub_tmp, tmp, keys_in, keys_out, vals_in, vals_out, cap, 0,
+                                                 64, st));
+  sift_sort_runs_kernel<<<blocks, 256, 0, st>>>(raw, counters, cap, keys_out, vals_out);
+  sift_keep_kernel<<<blocks, 256, 0, st>>>(raw, counters, cap, vals_out, keep);
+  SOD_CHECK_LAUNCH("sift_keep_kernel");
+  tmp = p.cub_bytes;
+  SOD_CHECK_CUDA(cub::DeviceScan::ExclusiveSum(ws + p.cub_tmp, tmp, keep, pos, cap, st));
+  sift_emit_kernel<<<blocks, 256, 0, st>>>(raw, counters, cap, vals_out, keep, pos, *out);
+  SOD_CHECK_LAUNCH("sift_emit_kernel");
+  if (p.pyr.n_oct > 0) {
+    const int sms = device_sm_count();
+    if (sms < 0) return SOD_ERR_CUDA;
+    sift_descriptor_kernel<<<sms * 16, 128, 0, st>>>(p.pyr, out->xy, out->size, out->angle, out->octave, cap,
+                                                     out->counters, out->des, nullptr);
+    SOD_CHECK_LAUNCH("sift_descriptor_kernel");
+  }
+  return SOD_OK;
+}
+
+int sod_sift_describe(const uint8_t* gray, int32_t width, int32_t height, int64_t pitch, const float* xy,
+                      const float* size, const float* angle, const int32_t* octave, int64_t n, uint8_t* des,
+                      int32_t* n_invalid, void* workspace, size_t workspace_bytes, sod_stream_t stream) {
+  if (int rc = check_image(gray, width, height, pitch, "sod_sift_describe")) return rc;
+  SOD_CHECK_ARG(n >= 0 && n <= SOD_SIFT_MAX_CAP, "sod_sift_describe: n %lld out of range (0..%d)", (long long)n,
+                SOD_SIFT_MAX_CAP);
+  if (n == 0) return SOD_OK;
+  SOD_CHECK_ARG(xy && size && angle && octave && des, "sod_sift_describe: null keypoint or descriptor array");
+  Plan p;
+  SOD_CHECK_ARG(make_plan(width, height, 0, &p), "sod_sift_describe: too many octaves");
+  SOD_CHECK_ARG(workspace != nullptr && workspace_bytes >= p.total && ((uintptr_t)workspace & 255) == 0,
+                "sod_sift_describe: workspace of %zu bytes at %p; need %zu bytes, 256-byte aligned", workspace_bytes,
+                workspace, p.total);
+  cudaStream_t st = (cudaStream_t)stream;
+  p.pyr.base = (float*)workspace;
+  if (p.pyr.n_oct > 0)
+    if (int rc = build_pyramid(gray, width, height, pitch, p.pyr, st)) return rc;
+  const int sms = device_sm_count();
+  if (sms < 0) return SOD_ERR_CUDA;
+  sift_descriptor_kernel<<<sms * 16, 128, 0, st>>>(p.pyr, xy, size, angle, octave, n, nullptr, des, n_invalid);
+  SOD_CHECK_LAUNCH("sift_descriptor_kernel");
+  return SOD_OK;
+}
+
+}  // extern "C"

@@ -57,6 +57,11 @@ class AffineOut(C.Structure):
                 ("member_keep", _p), ("cap_valid", _i64), ("cap_votes", _i64)]
 
 
+class SiftOut(C.Structure):
+    _fields_ = [("xy", _p), ("size", _p), ("angle", _p), ("response", _p), ("octave", _p), ("des", _p),
+                ("counters", _p), ("cap", _i64)]
+
+
 STAGES = {"match": 0, "hough_prep": 1, "hough_vote": 2, "hough_finish": 3, "affine": 4}
 
 
@@ -139,6 +144,10 @@ _PROTOS = {
     "sod_valid_bin_records": (C.c_int, [C.POINTER(HoughOut), C.POINTER(AffineOut), _p, _p, _p, _p, _p]),
     "sod_affine_verify": (C.c_int, [C.POINTER(Scene), _p, _p, C.POINTER(HoughOut), _i32, _i32, _i32,
                                     C.c_double, C.c_double, _i32, C.POINTER(AffineOut), _p]),
+    "sod_sift_workspace_bytes": (C.c_size_t, [_i32, _i32, _i64]),
+    "sod_sift_extract": (C.c_int, [_p, _i32, _i32, _i64, C.POINTER(SiftOut), _p, C.c_size_t, _p]),
+    "sod_sift_describe": (C.c_int, [_p, _i32, _i32, _i64, _p, _p, _p, _p, _i64, _p, _p, _p, C.c_size_t, _p]),
+    "sod_sift_level_offset": (_i64, [_i32, _i32, _i32, _i32, _p]),
 }
 
 
