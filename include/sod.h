@@ -41,12 +41,6 @@ const char* sod_last_error(void);
 /* Number of SMs of the current device (grid sizing; 148 on B200). Negative on error. */
 int sod_device_sm_count(void);
 
-/* Process-wide tuning options (nothing in the reference).  "match_cta_pair": 1 = sod_match_top2* runs
- * on CTA pairs (tcgen05.mma.cta_group::2: the two SMs of a TPC share every database tile), 0 = one CTA per
- * SM; the results are identical.  Unknown names return SOD_ERR_INVALID_ARGUMENT. */
-int sod_set_option(const char* name, int32_t value);
-int32_t sod_get_option(const char* name);
-
 /* Measurement hook (bench.py's roofline figures; nothing in the reference): while enabled on the
  * calling thread, every entry point brackets the launches of the stages below with CUDA events on the
  * caller's stream (up to 128 calls per stage between reads; no synchronisation, two event records per

@@ -59,7 +59,7 @@ int device_sm_count() {
 
 extern "C" {
 
-int sod_version(void) { return 1001; }
+int sod_version(void) { return 2000; }
 
 const char* sod_last_error(void) { return sod::g_err; }
 

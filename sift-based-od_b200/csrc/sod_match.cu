@@ -5,12 +5,14 @@
 // contraction q.t runs on the 5th-gen tensor cores (tcgen05.mma kind::i8, u8 x u8 -> s32 in TMEM)
 // and the top-2 selection happens in the TMEM epilogue without ever writing distances to HBM.
 //
-// Kernel anatomy (one persistent CTA per SM, 640 threads):
-//   warp 0      TMA producer: query block (2 x 128 rows, double buffered) + database tiles
-//               (128 rows = 16 KB, kStages-deep ring) + the tile's 1040 B slice of per-row constants
-//               (|t|^2 << 8 | column, chunk minima, original rows) in its own, deeper ring.
-//   warps 1, 3  MMA issuers, one per query half: per database tile 4 UTCIMMA (M=128,N=128,K=32)
-//               each into four independent 128-column TMEM accumulator slots (2 halves x 2 buffers).
+// Kernel anatomy (persistent CTA pairs: a cluster of 2 CTAs on the two SMs of a TPC, 640 threads each):
+//   warp 0      TMA producer: the CTA's query block (2 x 128 rows, double buffered) + its half of each
+//               database tile (64 of the tile's 128 rows = 8 KB, 8-deep ring) + the whole tile's 1040 B
+//               slice of per-row constants (|t|^2 << 8 | column, chunk minima, original rows) in its own,
+//               deeper ring.
+//   warps 1, 3  MMA issuers of the leader CTA, one per query half: per database tile 4 UTCIMMA.2CTA
+//               (M=256 over both CTAs, N=128, K=32) each into four independent 128-column TMEM
+//               accumulator slots per CTA (2 halves x 2 buffers).
 //   warp 2      TMEM allocator.
 //   warps 4-19  epilogue: thread <-> query row (TMEM lane), 16 warps = 4 lane quadrants x 2 query
 //               halves x 2 tile parities (even / odd tiles).  A warp pulls the 128 columns of its
@@ -26,8 +28,6 @@
 // by original index and a permutation maps back, so results (incl. ties -> lowest original index,
 // as cv2) do not depend on the reordering.
 #include <climits>
-#include <cstdlib>
-#include <cstring>
 #include <cub/device/device_radix_sort.cuh>
 
 #include "sod_common.cuh"
@@ -38,16 +38,11 @@
 namespace sod {
 namespace {
 
-#ifndef SOD_MATCH_CTA_PAIR_DEFAULT
-#define SOD_MATCH_CTA_PAIR_DEFAULT 1
-#endif
-
 constexpr int kTileM = 128;                 // query rows per MMA (TMEM lanes)
 constexpr int kHalves = 2;                  // query tiles per CTA sharing one database tile
 constexpr int kBlockQ = kTileM * kHalves;   // 256 query rows per unit
 constexpr int kTileN = SOD_TILE_ROWS;       // database rows per MMA
 constexpr int kTileBytes = kTileN * SOD_DESC_DIM;  // 16 KB (A half-tile has the same size)
-constexpr int kStages = 6;
 constexpr int kChunk = 32;                  // accumulator columns per tcgen05.ld
 constexpr int kCqTile = SOD_CQ_TILE_INTS;   // 128 x |t|^2 + 4 per-chunk minima + 128 x original row
 constexpr int kCqPerm = kTileN + 4;         // offset of the permutation inside a tile's slice
@@ -70,23 +65,19 @@ static_assert(128 * kRegsLight + kEpiWarps * 32 * kRegsEpilogue <= kThreads * kR
 constexpr int kBarGroups = kParity;  // accumulator barriers are indexed by step % kBarGroups: every barrier is
                                      // then waited on by ONE set of epilogue warps for consecutive phases (a
                                      // parity wait must never skip a phase)
-// Shared-memory layout.  kPair = the CTA-pair form (cta_group::2): a CTA holds HALF of every database tile
-// (64 rows, 8 KB), so its ring is deeper for the same bytes in flight.
-template <bool kPair>
-struct Layout {
-  static constexpr int kStagesL = kPair ? 8 : kStages;
-  static constexpr int kBStageBytes = kPair ? kTileBytes / 2 : kTileBytes;
-  static constexpr int kCqSlotsL = 16;                      // >= kStagesL + 3 (slot-reuse argument in the producer);
-                                                            // a power of two keeps `step % slots` a mask
-  static constexpr int kOffA = 0;                                     // [2 buffers][2 halves][16 KB]
-  static constexpr int kOffB = kOffA + 2 * kHalves * kTileBytes;      // [stages][16 KB | 8 KB]
-  static constexpr int kOffCq = kOffB + kStagesL * kBStageBytes;      // [cq slots][260] int32
-  static constexpr int kOffBar = kOffCq + kCqSlotsL * kCqTileBytes;
-  static constexpr int kNumBars = 2 * kStagesL + 4 + 4 * kBarGroups + kCqSlotsL;
-  static constexpr int kOffTmemPtr = kOffBar + kNumBars * 8;
-  static constexpr int kSmemBytes = kOffTmemPtr + 16 + 1024;          // +1024: manual 1 KB alignment
-  static_assert(kCqSlotsL >= kStagesL + 3 && (kCqSlotsL & (kCqSlotsL - 1)) == 0, "cq ring too shallow");
-};
+// Shared-memory layout.  A CTA holds HALF of every database tile (64 rows, 8 KB).
+constexpr int kStages = 8;                   // database ring depth
+constexpr int kBStageBytes = kTileBytes / 2;
+constexpr int kCqSlots = 16;                 // >= kStages + 3 (slot-reuse argument in the producer);
+                                             // a power of two keeps `step % slots` a mask
+constexpr int kOffA = 0;                                     // [2 buffers][2 halves][16 KB]
+constexpr int kOffB = kOffA + 2 * kHalves * kTileBytes;      // [stages][8 KB]
+constexpr int kOffCq = kOffB + kStages * kBStageBytes;       // [cq slots][260] int32
+constexpr int kOffBar = kOffCq + kCqSlots * kCqTileBytes;
+constexpr int kNumBars = 2 * kStages + 4 + 4 * kBarGroups + kCqSlots;
+constexpr int kOffTmemPtr = kOffBar + kNumBars * 8;
+constexpr int kSmemBytes = kOffTmemPtr + 16 + 1024;          // +1024: manual 1 KB alignment
+static_assert(kCqSlots >= kStages + 3 && (kCqSlots & (kCqSlots - 1)) == 0, "cq ring too shallow");
 
 struct MatchArgs {
   const int32_t* qn;   // [nq] |q|^2
@@ -99,7 +90,7 @@ struct MatchArgs {
   int n_tiles;         // tiles swept by this launch: [tile_begin, tile_begin + n_tiles)
   int tile_begin;
   int n_qblocks;
-  int n_qunits;        // query blocks per unit row: n_qblocks, or ceil(n_qblocks / 2) CTA pairs
+  int n_qunits;        // units per segment: ceil(n_qblocks / 2), a CTA pair sweeps two query blocks
   int n_seg;
   int idx_base;
   // Threshold publishing over peer memory (database sharded over several GPUs, kSeeded sweeps): when a unit
@@ -194,20 +185,17 @@ __device__ __forceinline__ void top2_chunk(const uint32_t* v, const int4* __rest
 // run), which have nobody to share with inside the launch and must not pay the per-tile load and
 // atomicMin of the sharing code (B200, 1.28 M queries x 125k-row shard: 15.27 ms against 16.21 ms
 // with the sharing instance and 16.44 ms unseeded; profiles/r02_threshold_seeding.txt).
-// kPair: two CTAs of a cluster (the two SMs of a TPC) run ONE tcgen05.mma.cta_group::2 per query half over
+// The two CTAs of a cluster (the two SMs of a TPC) run ONE tcgen05.mma.cta_group::2 per query half over
 // M = 256 rows - 128 query rows of each CTA - and N = 128 database rows, of which each CTA stages 64: the
-// database stream from L2 and the shared-memory operand reads per MAC drop (B: 8 KB instead of 16 KB per
-// CTA and tile), the accumulators and the whole epilogue stay per CTA exactly as in the single-CTA form.
-// The leader CTA (cluster rank 0) issues the MMAs; TMA loads of both CTAs report to the leader's "full"
-// barriers, tcgen05.commit multicasts "free" / "accumulator ready" to both CTAs, and the epilogue warps of
-// both CTAs release accumulator slots on the leader's barriers.
-template <bool kShare, bool kSeeded = false, bool kPair = false>
+// database stream from L2 and the shared-memory operand reads per MAC are half of what one CTA per tile
+// would need (B: 8 KB instead of 16 KB per CTA and tile).  The accumulators and the whole epilogue are per
+// CTA.  The leader CTA (cluster rank 0) issues the MMAs; TMA loads of both CTAs report to the leader's
+// "full" barriers, tcgen05.commit multicasts "free" / "accumulator ready" to both CTAs, and the epilogue
+// warps of both CTAs release accumulator slots on the leader's barriers.
+template <bool kShare, bool kSeeded = false>
 __global__ void __launch_bounds__(kThreads, 1)
 match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
                   const __grid_constant__ CUtensorMap tmap_db, const MatchArgs a) {
-  using L = Layout<kPair>;
-  constexpr int kSt = L::kStagesL;
-  constexpr int kCqS = L::kCqSlotsL;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw_addr = smem_u32(smem_raw);
   const uint32_t base = (raw_addr + 1023u) & ~1023u;  // SWIZZLE_128B tiles need 1 KB alignment
@@ -215,27 +203,27 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  const uint32_t cta_rank = kPair ? cluster_ctarank() : 0u;   // 0 = leader of the pair
-  const int unit0 = kPair ? static_cast<int>(cluster_id_x()) : static_cast<int>(blockIdx.x);
-  const int unit_step = kPair ? static_cast<int>(cluster_count_x()) : static_cast<int>(gridDim.x);
+  const uint32_t cta_rank = cluster_ctarank();   // 0 = leader of the pair
+  const int unit0 = static_cast<int>(cluster_id_x());
+  const int unit_step = static_cast<int>(cluster_count_x());
 
-  const uint32_t bar0 = base + L::kOffBar;
+  const uint32_t bar0 = base + kOffBar;
   auto bar_full = [&](int s) { return bar0 + 8u * s; };
-  auto bar_empty = [&](int s) { return bar0 + 8u * (kSt + s); };
-  auto bar_afull = [&](int b) { return bar0 + 8u * (2 * kSt + b); };
-  auto bar_aempty = [&](int b) { return bar0 + 8u * (2 * kSt + 2 + b); };
+  auto bar_empty = [&](int s) { return bar0 + 8u * (kStages + s); };
+  auto bar_afull = [&](int b) { return bar0 + 8u * (2 * kStages + b); };
+  auto bar_aempty = [&](int b) { return bar0 + 8u * (2 * kStages + 2 + b); };
   // accumulator hand-off barriers per (step % kBarGroups, half); the TMEM slot itself is step & 1
-  auto bar_tfull = [&](int g, int h) { return bar0 + 8u * (2 * kSt + 4 + 2 * g + h); };
-  auto bar_tempty = [&](int g, int h) { return bar0 + 8u * (2 * kSt + 4 + 2 * kBarGroups + 2 * g + h); };
-  auto bar_cqfull = [&](int s) { return bar0 + 8u * (2 * kSt + 4 + 4 * kBarGroups + s); };
-  volatile uint32_t* tmem_ptr_smem = reinterpret_cast<volatile uint32_t*>(smem + L::kOffTmemPtr);
+  auto bar_tfull = [&](int g, int h) { return bar0 + 8u * (2 * kStages + 4 + 2 * g + h); };
+  auto bar_tempty = [&](int g, int h) { return bar0 + 8u * (2 * kStages + 4 + 2 * kBarGroups + 2 * g + h); };
+  auto bar_cqfull = [&](int s) { return bar0 + 8u * (2 * kStages + 4 + 4 * kBarGroups + s); };
+  volatile uint32_t* tmem_ptr_smem = reinterpret_cast<volatile uint32_t*>(smem + kOffTmemPtr);
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmap_q);
     tma_prefetch_desc(&tmap_db);
   }
   if (warp == 1 && lane == 0) {
-    for (int s = 0; s < kSt; ++s) {
+    for (int s = 0; s < kStages; ++s) {
       mbar_init(bar_full(s), 1);
       mbar_init(bar_empty(s), kHalves);  // one tcgen05.commit per issuing warp
     }
@@ -246,22 +234,17 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
     for (int g = 0; g < kBarGroups; ++g)
       for (int h = 0; h < kHalves; ++h) {
         mbar_init(bar_tfull(g, h), 1);
-        mbar_init(bar_tempty(g, h), kPair ? 8 : 4);  // the four quadrant warps that read one slot (of each CTA)
+        mbar_init(bar_tempty(g, h), 8);  // the four quadrant warps that read one slot, of each CTA
       }
-    for (int s = 0; s < kCqS; ++s) mbar_init(bar_cqfull(s), 1);
+    for (int s = 0; s < kCqSlots; ++s) mbar_init(bar_cqfull(s), 1);
     fence_mbar_init();
   }
   if (warp == 2) {
-    if constexpr (kPair) {
-      tmem_alloc_pair(smem_u32(const_cast<uint32_t*>(tmem_ptr_smem)), kTmemCols);
-      tmem_relinquish_pair();
-    } else {
-      tmem_alloc(smem_u32(const_cast<uint32_t*>(tmem_ptr_smem)), kTmemCols);
-      tmem_relinquish();
-    }
+    tmem_alloc_pair(smem_u32(const_cast<uint32_t*>(tmem_ptr_smem)), kTmemCols);
+    tmem_relinquish_pair();
   }
   tc_fence_before();
-  if constexpr (kPair) cluster_sync_all(); else __syncthreads();
+  cluster_sync_all();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr_smem;
 
@@ -278,46 +261,34 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
         const int seg = u / a.n_qunits;
         int qu = u - seg * a.n_qunits + a.unit_rot;   // unit_rot < n_qunits (0 unless n_seg == 1)
         if (qu >= a.n_qunits) qu -= a.n_qunits;
-        const int qb = kPair ? qu * 2 + static_cast<int>(cta_rank) : qu;
+        const int qb = qu * 2 + static_cast<int>(cta_rank);
         const int t0 = a.tile_begin + static_cast<int>(static_cast<int64_t>(seg) * a.n_tiles / a.n_seg);
         const int t1 = a.tile_begin + static_cast<int>(static_cast<int64_t>(seg + 1) * a.n_tiles / a.n_seg);
         const uint32_t ab = ucount & 1u, aph = (ucount >> 1) & 1u;
         mbar_wait(bar_aempty(ab), aph ^ 1u);
-        if constexpr (kPair) {
-          // both CTAs' query blocks report to the leader's barrier, which expects the bytes of both
-          if (cta_rank == 0) mbar_arrive_expect_tx(bar_afull(ab), 2 * kHalves * kTileBytes);
-          const uint32_t afull_leader = mapa_shared(bar_afull(ab), 0);
-          for (int h = 0; h < kHalves; ++h)
-            tma_load_2d_pair(base + L::kOffA + (ab * kHalves + h) * kTileBytes, &tmap_q, afull_leader, 0,
-                             qb * kBlockQ + h * kTileM);
-        } else {
-          mbar_arrive_expect_tx(bar_afull(ab), kHalves * kTileBytes);
-          for (int h = 0; h < kHalves; ++h)
-            tma_load_2d(base + L::kOffA + (ab * kHalves + h) * kTileBytes, &tmap_q, bar_afull(ab), 0,
-                        qb * kBlockQ + h * kTileM);
-        }
+        // both CTAs' query blocks report to the leader's barrier, which expects the bytes of both
+        if (cta_rank == 0) mbar_arrive_expect_tx(bar_afull(ab), 2 * kHalves * kTileBytes);
+        const uint32_t afull_leader = mapa_shared(bar_afull(ab), 0);
+        for (int h = 0; h < kHalves; ++h)
+          tma_load_2d_pair(base + kOffA + (ab * kHalves + h) * kTileBytes, &tmap_q, afull_leader, 0,
+                           qb * kBlockQ + h * kTileM);
         for (int t = t0; t < t1; ++t, ++step) {
-          const uint32_t s = step % kSt, ph = (step / kSt) & 1u;
+          const uint32_t s = step % kStages, ph = (step / kStages) & 1u;
           mbar_wait(bar_empty(s), ph ^ 1u);
-          if constexpr (kPair) {
-            // this CTA stages rows [64 * rank, 64 * rank + 64) of the tile
-            if (cta_rank == 0) mbar_arrive_expect_tx(bar_full(s), 2 * L::kBStageBytes);
-            tma_load_2d_pair(base + L::kOffB + s * L::kBStageBytes, &tmap_db, mapa_shared(bar_full(s), 0), 0,
-                             t * kTileN + static_cast<int>(cta_rank) * (kTileN / 2));
-          } else {
-            mbar_arrive_expect_tx(bar_full(s), kTileBytes);
-            tma_load_2d(base + L::kOffB + s * kTileBytes, &tmap_db, bar_full(s), 0, t * kTileN);
-          }
+          // this CTA stages rows [64 * rank, 64 * rank + 64) of the tile
+          if (cta_rank == 0) mbar_arrive_expect_tx(bar_full(s), 2 * kBStageBytes);
+          tma_load_2d_pair(base + kOffB + s * kBStageBytes, &tmap_db, mapa_shared(bar_full(s), 0), 0,
+                           t * kTileN + static_cast<int>(cta_rank) * (kTileN / 2));
           // cq slice rides in its own, deeper ring: stage s is released when the MMAs that read it
           // retire, but the epilogue still reads cq after it has handed the accumulator back.
           // The write for step j happens after MMA(j-kStages) retired; that MMA was issued after
           // every epilogue warp RELEASED step j-kStages-2, i.e. finished its arithmetic on step
-          // j-kStages-3.  Steps j-kStages-2 .. j-1 may still be live -> kStages+3 slots are needed.
-          // (Pair form: every CTA needs the constants of the WHOLE tile - its accumulators span all 128
-          // database rows - and loads them itself; the argument holds per CTA because the MMAs are joint.)
-          const uint32_t slot = step % kCqS;
+          // j-kStages-3.  Steps j-kStages-2 .. j-1 may still be live -> kStages+3 = 11 of the 16 slots
+          // are needed.  Every CTA needs the constants of the WHOLE tile - its accumulators span all 128
+          // database rows - and loads them itself; the argument holds per CTA because the MMAs are joint.
+          const uint32_t slot = step % kCqSlots;
           mbar_arrive_expect_tx(bar_cqfull(slot), kCqTileBytes);
-          bulk_load_1d(base + L::kOffCq + slot * kCqTileBytes, a.cq + static_cast<int64_t>(t) * kCqTile,
+          bulk_load_1d(base + kOffCq + slot * kCqTileBytes, a.cq + static_cast<int64_t>(t) * kCqTile,
                        kCqTileBytes, bar_cqfull(slot));
         }
       }
@@ -331,7 +302,7 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
     // tcgen05 instructions are issued by one elected lane.  (Inside a divergent `if (lane == 0)`
     // every UTCIMMA operand needs an R2UR move.)
     const int h = warp >> 1;
-    constexpr uint32_t idesc = umma_idesc_u8(kPair ? 2 * kTileM : kTileM, kTileN);
+    constexpr uint32_t idesc = umma_idesc_u8(2 * kTileM, kTileN);
     uint32_t step = 0, ucount = 0;
     for (int u = unit0; u < total_units; u += unit_step, ++ucount) {
       const int seg = u / a.n_qunits;
@@ -339,11 +310,11 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
       const int t1 = a.tile_begin + static_cast<int>(static_cast<int64_t>(seg + 1) * a.n_tiles / a.n_seg);
       const uint32_t ab = ucount & 1u, aph = (ucount >> 1) & 1u;
       mbar_wait(bar_afull(ab), aph);
-      const uint64_t adesc = umma_desc_k128(base + L::kOffA + (ab * kHalves + h) * kTileBytes);
+      const uint64_t adesc = umma_desc_k128(base + kOffA + (ab * kHalves + h) * kTileBytes);
       for (int t = t0; t < t1; ++t, ++step) {
-        const uint32_t s = step % kSt, ph = (step / kSt) & 1u;
+        const uint32_t s = step % kStages, ph = (step / kStages) & 1u;
         const uint32_t acc = step & 1u;
-        const uint64_t bdesc = umma_desc_k128(base + L::kOffB + s * L::kBStageBytes);
+        const uint64_t bdesc = umma_desc_k128(base + kOffB + s * kBStageBytes);
         const uint32_t d = tmem_base + acc * (kHalves * kTileN) + h * kTileN;
         mbar_wait(bar_full(s), ph);
         if (step >= 2)  // slot step & 1 was last used by step - 2: wait for its epilogue warps' release
@@ -351,24 +322,14 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
         tc_fence_after();
         if (elect_one()) {
 #pragma unroll
-          for (int k = 0; k < SOD_DESC_DIM / 32; ++k) {  // K = 32 bytes per UTCIMMA: +2 x 16 B
-            if constexpr (kPair) umma_i8_pair(d, adesc + 2 * k, bdesc + 2 * k, idesc, k > 0);
-            else umma_i8(d, adesc + 2 * k, bdesc + 2 * k, idesc, k > 0);
-          }
-          if constexpr (kPair) {
-            umma_commit_pair(bar_tfull(step % kBarGroups, h), 3);  // this half is ready in both CTAs
-            umma_commit_pair(bar_empty(s), 3);   // (count 2) stage free in both CTAs once both halves retire
-          } else {
-            umma_commit(bar_tfull(step % kBarGroups, h));  // this half is ready for its epilogue warps
-            umma_commit(bar_empty(s));       // (count 2) database stage free once both halves retire
-          }
+          for (int k = 0; k < SOD_DESC_DIM / 32; ++k)  // K = 32 bytes per UTCIMMA: +2 x 16 B
+            umma_i8_pair(d, adesc + 2 * k, bdesc + 2 * k, idesc, k > 0);
+          umma_commit_pair(bar_tfull(step % kBarGroups, h), 3);  // this half is ready in both CTAs
+          umma_commit_pair(bar_empty(s), 3);   // (count 2) stage free in both CTAs once both halves retire
         }
         __syncwarp();
       }
-      if (elect_one()) {  // (count 2) query block buffer free
-        if constexpr (kPair) umma_commit_pair(bar_aempty(ab), 3);
-        else umma_commit(bar_aempty(ab));
-      }
+      if (elect_one()) umma_commit_pair(bar_aempty(ab), 3);  // (count 2) query block buffer free
       __syncwarp();
     }
   }
@@ -385,24 +346,22 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
     // launch - tens of cycles each, in front of the barrier waits): keep them in registers.
     uint32_t tfull_h = bar_tfull(0, h);      // + 16 * (step % kBarGroups)
     uint32_t cqfull_0 = bar_cqfull(0);       // + 8 * slot
-    uint32_t cq_0 = base + L::kOffCq;        // + slot * kCqTileBytes (shared-memory window address)
+    uint32_t cq_0 = base + kOffCq;           // + slot * kCqTileBytes (shared-memory window address)
     uint32_t taddr_h = tmem_base + lane_sel + h * kTileN;   // + (step & 1) * (kHalves * kTileN)
     asm volatile("" : "+r"(par), "+r"(tfull_h), "+r"(cqfull_0), "+r"(taddr_h));
-    if constexpr (kPair) asm volatile("" : "+r"(cq_0));  // (the single-CTA form has no register to spare for it)
-    // pair form: accumulator slots are released on the LEADER's barriers (the leader issues the MMAs)
-    uint32_t tempty_rel0 = kPair ? mapa_shared(bar_tempty(0, h), 0) : bar_tempty(0, h);
-    uint32_t tempty_rel1 = kPair ? mapa_shared(bar_tempty(1, h), 0) : bar_tempty(1, h);
-    if constexpr (kPair) {
-      // keep the two cluster addresses in registers: rematerialised, each release would re-read the cluster
-      // rank (S2R, tens of cycles) on the critical path between the TMEM load and the slot's release
-      asm volatile("" : "+r"(tempty_rel0), "+r"(tempty_rel1));
-    }
+    asm volatile("" : "+r"(cq_0));
+    // accumulator slots are released on the LEADER's barriers (the leader issues the MMAs)
+    uint32_t tempty_rel0 = mapa_shared(bar_tempty(0, h), 0);
+    uint32_t tempty_rel1 = mapa_shared(bar_tempty(1, h), 0);
+    // keep the two cluster addresses in registers: rematerialised, each release would re-read the cluster
+    // rank (S2R, tens of cycles) on the critical path between the TMEM load and the slot's release
+    asm volatile("" : "+r"(tempty_rel0), "+r"(tempty_rel1));
     uint32_t step = 0, ucount = 1;
     for (int u = unit0; u < total_units; u += unit_step, ++ucount) {
       const int seg = u / a.n_qunits;
       int qu = u - seg * a.n_qunits + a.unit_rot;
       if (qu >= a.n_qunits) qu -= a.n_qunits;
-      const int qb = kPair ? qu * 2 + static_cast<int>(cta_rank) : qu;
+      const int qb = qu * 2 + static_cast<int>(cta_rank);
       const int t0 = a.tile_begin + static_cast<int>(static_cast<int64_t>(seg) * a.n_tiles / a.n_seg);
       const int t1 = a.tile_begin + static_cast<int>(static_cast<int64_t>(seg + 1) * a.n_tiles / a.n_seg);
       const int row = qb * kBlockQ + h * kTileM + quad * 32 + lane;
@@ -421,7 +380,7 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
       const uint32_t step_end = step + static_cast<uint32_t>(t1 - t0);
       for (step += (par ^ step) & 1u; step < step_end; step += 2) {
         const uint32_t acc = step & 1u, bg = step % kBarGroups, bgph = (step / kBarGroups) & 1u;
-        const uint32_t slot = step % kCqS, cqph = (step / kCqS) & 1u;
+        const uint32_t slot = step % kCqSlots, cqph = (step / kCqSlots) & 1u;
         mbar_wait(cqfull_0 + 8u * slot, cqph);  // landed long ago: returns at the first poll
         mbar_wait(tfull_h + 16u * bg, bgph);
         tc_fence_after();
@@ -439,10 +398,7 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
         tmem_ld64_wait(taddr + 2 * kChunk, v);
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) {
-          if constexpr (kPair) mbar_arrive_cluster(bg ? tempty_rel1 : tempty_rel0);
-          else mbar_arrive(bg ? tempty_rel1 : tempty_rel0);
-        }
+        if (lane == 0) mbar_arrive_cluster(bg ? tempty_rel1 : tempty_rel0);
         top2_chunk(v, c4 + 16, cmin.z, perm_s, a.idx_base, best, thr);
         top2_chunk(v + kChunk, c4 + 24, cmin.w, perm_s, a.idx_base, best, thr);
         if (kShare && thr_row) {
@@ -477,13 +433,8 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
   }
 
   tc_fence_before();
-  if constexpr (kPair) {
-    cluster_sync_all();  // the peer's shared memory and barriers stay alive until both CTAs are done
-    if (warp == 2) tmem_dealloc_pair(tmem_base, kTmemCols);
-  } else {
-    __syncthreads();
-    if (warp == 2) tmem_dealloc(tmem_base, kTmemCols);
-  }
+  cluster_sync_all();  // the peer's shared memory and barriers stay alive until both CTAs are done
+  if (warp == 2) tmem_dealloc_pair(tmem_base, kTmemCols);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -715,21 +666,21 @@ struct Plan {
 };
 
 // Split every query block's database sweep into n_seg contiguous segments so that
-// n_qunits*n_seg units fill the persistent grid evenly (cost = makespan in tile steps).  pair: a unit is
-// swept by a CTA pair (two query blocks side by side), the grid holds sms / 2 pairs.
-Plan make_plan(int64_t nq, int64_t ndb, int sms, bool pair = false) {
+// n_qunits*n_seg units fill the persistent grid evenly (cost = makespan in tile steps).  A unit is swept
+// by a CTA pair (two query blocks side by side); the grid holds sms / 2 pairs (sms >= 2).
+Plan make_plan(int64_t nq, int64_t ndb, int sms) {
   Plan p;
   p.n_tiles = static_cast<int>((ndb + kTileN - 1) / kTileN);
   p.n_qblocks = static_cast<int>((nq + kBlockQ - 1) / kBlockQ);
-  p.n_qunits = pair ? (p.n_qblocks + 1) / 2 : p.n_qblocks;
-  if (pair) sms /= 2;
+  p.n_qunits = (p.n_qblocks + 1) / 2;
+  const int pairs = sms / 2;
   p.n_seg = 1;
   if (p.n_tiles > 0 && p.n_qblocks > 0) {
     const int max_seg = p.n_tiles < 512 ? p.n_tiles : 512;
     int64_t best = -1;
     for (int s = 1; s <= max_seg; ++s) {
       const int64_t units = static_cast<int64_t>(p.n_qunits) * s;
-      const int64_t waves = (units + sms - 1) / sms;
+      const int64_t waves = (units + pairs - 1) / pairs;
       // +12: pipeline fill and the slow-path chunks of a unit's first columns (measured; units of one
       // query block share their thresholds, so a later segment does not start from scratch)
       const int64_t cost = waves * ((p.n_tiles + s - 1) / s + 12);
@@ -740,7 +691,7 @@ Plan make_plan(int64_t nq, int64_t ndb, int sms, bool pair = false) {
     }
   }
   const int64_t units = static_cast<int64_t>(p.n_qunits) * p.n_seg;
-  p.grid = static_cast<int>(units < sms ? units : sms) * (pair ? 2 : 1);
+  p.grid = static_cast<int>(units < pairs ? units : pairs) * 2;
   return p;
 }
 
@@ -748,18 +699,6 @@ Plan make_plan(int64_t nq, int64_t ndb, int sms, bool pair = false) {
 int make_desc_map(CUtensorMap* m, const uint8_t* ptr, int64_t n_rows, int box_rows = kTileN) {
   return make_rowmajor_map(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, ptr, n_rows, SOD_DESC_DIM, SOD_DESC_DIM,
                            box_rows);
-}
-
-// Which form of the matcher sod_match_top2* launches: 0 = one CTA per SM (tcgen05.mma.cta_group::1),
-// 1 = CTA pairs (cta_group::2).  Process-wide; sod_set_option("match_cta_pair", v) or the environment
-// variable SOD_MATCH_CTA_PAIR at the first launch.
-int g_match_pair = -1;
-bool match_pair_enabled() {
-  if (g_match_pair < 0) {
-    const char* e = getenv("SOD_MATCH_CTA_PAIR");
-    g_match_pair = e ? (atoi(e) != 0) : SOD_MATCH_CTA_PAIR_DEFAULT;
-  }
-  return g_match_pair != 0;
 }
 
 }  // namespace
@@ -848,26 +787,8 @@ int64_t sod_row_thr_ints(int64_t n_query) {
 size_t sod_match_workspace_bytes(int64_t n_query, int64_t n_db) {
   if (n_query <= 0 || n_db <= 0) return 16;
   const int sms = device_sm_count();
-  // enough for either form of the kernel: the option may change between this query and the launch
-  const size_t single = match_workspace_need(make_plan(n_query, n_db, sms > 0 ? sms : 148, false), n_query);
-  const size_t pair = match_workspace_need(make_plan(n_query, n_db, sms > 0 ? sms : 148, true), n_query);
-  return (single > pair ? single : pair) + 16;
-}
-
-int sod_set_option(const char* name, int32_t value) {
-  SOD_CHECK_ARG(name, "null option name");
-  if (strcmp(name, "match_cta_pair") == 0) {
-    g_match_pair = value != 0;
-    return SOD_OK;
-  }
-  set_error("unknown option '%s'", name);
-  return SOD_ERR_INVALID_ARGUMENT;
-}
-
-int32_t sod_get_option(const char* name) {
-  if (name && strcmp(name, "match_cta_pair") == 0) return match_pair_enabled() ? 1 : 0;
-  set_error("unknown option '%s'", name ? name : "(null)");
-  return SOD_ERR_INVALID_ARGUMENT;
+  // (a device with fewer than two SMs is rejected by the match itself)
+  return match_workspace_need(make_plan(n_query, n_db, sms >= 2 ? sms : 148), n_query) + 16;
 }
 
 int sod_match_top2(const uint8_t* q, const int32_t* qn, int64_t n_query, const uint8_t* db_sorted,
@@ -920,8 +841,11 @@ int sod_match_top2_peer(const uint8_t* q, const int32_t* qn, int64_t n_query, co
                 "q, db, cq and workspace must be 16-byte aligned");
   const int sms = device_sm_count();
   if (sms <= 0) return SOD_ERR_CUDA;
-  const bool pair = match_pair_enabled() && sms >= 2;
-  const Plan p = make_plan(n_query, (tile_end - tile_begin) * kTileN, sms, pair);
+  if (sms < 2) {
+    set_error("sod_match_top2: the matcher runs on CTA pairs and needs at least 2 SMs, the device has %d", sms);
+    return SOD_ERR_UNSUPPORTED;
+  }
+  const Plan p = make_plan(n_query, (tile_end - tile_begin) * kTileN, sms);
   const size_t need = match_workspace_need(p, n_query);
   SOD_CHECK_ARG(workspace_bytes >= need, "workspace too small: %zu < %zu", workspace_bytes, need);
 
@@ -929,7 +853,7 @@ int sod_match_top2_peer(const uint8_t* q, const int32_t* qn, int64_t n_query, co
   int rc = make_desc_map(&map_q, q, n_query);
   if (rc != SOD_OK) return rc;
   // stored padded to whole tiles; a CTA of a pair stages half a tile (64 rows) per step
-  rc = make_desc_map(&map_db, db, (n_db + kTileN - 1) / kTileN * kTileN, pair ? kTileN / 2 : kTileN);
+  rc = make_desc_map(&map_db, db, (n_db + kTileN - 1) / kTileN * kTileN, kTileN / 2);
   if (rc != SOD_OK) return rc;
 
   MatchArgs a;
@@ -955,32 +879,29 @@ int sod_match_top2_peer(const uint8_t* q, const int32_t* qn, int64_t n_query, co
   // peer publishing and the rotated visiting order belong to single-segment sweeps (the seeded instance)
   const bool peer_mode = n_peers > 0 && row_thr && p.n_seg == 1;
   a.n_peers = peer_mode ? n_peers : 0;
-  a.unit_rot = peer_mode ? static_cast<int>((block_rotation / (pair ? 2 : 1)) % p.n_qunits) : 0;
+  a.unit_rot = peer_mode ? static_cast<int>((block_rotation / 2) % p.n_qunits) : 0;
   for (int i = 0; i < SOD_EXCHANGE_MAX_RANKS; ++i) a.peer_thr[i] = (peer_mode && i < n_peers) ? peer_thr_host[i] : nullptr;
   for (int i = 0; i < a.n_peers; ++i) SOD_CHECK_ARG(a.peer_thr[i], "null threshold array of rank %d", i);
 
   // The attribute is per device (a process may drive several), so it is set at every launch: ~1 us.
   const bool seeded = row_thr && p.n_seg == 1, share = a.row_thr && !seeded;
-  auto* kernel = pair ? (seeded ? match_top2_kernel<false, true, true>
-                                : share ? match_top2_kernel<true, false, true> : match_top2_kernel<false, false, true>)
-                      : (seeded ? match_top2_kernel<false, true, false>
-                                : share ? match_top2_kernel<true, false, false> : match_top2_kernel<false, false, false>);
-  const int smem_bytes = pair ? Layout<true>::kSmemBytes : Layout<false>::kSmemBytes;
-  SOD_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+  auto* kernel = seeded ? match_top2_kernel<false, true>
+                        : share ? match_top2_kernel<true, false> : match_top2_kernel<false, false>;
+  SOD_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
   {
     StageScope timed(SOD_STAGE_MATCH, st);
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(static_cast<unsigned>(p.grid));
     cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = static_cast<size_t>(smem_bytes);
+    cfg.dynamicSmemBytes = static_cast<size_t>(kSmemBytes);
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = pair ? 2 : 1;
+    attr[0].val.clusterDim.x = 2;
     attr[0].val.clusterDim.y = 1;
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = pair ? 1 : 0;
+    cfg.numAttrs = 1;
     SOD_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kernel, map_q, map_db, a));
   }
   SOD_CHECK_LAUNCH("match_top2_kernel");

@@ -37,20 +37,8 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t byt
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
-#ifndef SOD_WAIT_HINT_NS
-#define SOD_WAIT_HINT_NS 0  // 0: default hardware time limit for one try_wait
-#endif
 __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
   uint32_t ok;
-#if SOD_WAIT_HINT_NS > 0
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}\n"
-      : "=r"(ok)
-      : "r"(bar), "r"(parity), "r"(static_cast<uint32_t>(SOD_WAIT_HINT_NS))
-      : "memory");
-#else
   asm volatile(
       "{\n\t.reg .pred p;\n\t"
       "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
@@ -58,7 +46,6 @@ __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
       : "=r"(ok)
       : "r"(bar), "r"(parity)
       : "memory");
-#endif
   return ok != 0;
 }
 // Spin with a watchdog: a protocol bug traps (launch error) instead of hanging the GPU.  The clock
@@ -119,17 +106,6 @@ __device__ __forceinline__ void tc_fence_before() {
 }
 __device__ __forceinline__ void tc_fence_after() {
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-}
-// D[tmem] (+)= A[smem] * B[smem], u8 x u8 -> s32 (SASS: UTCIMMA). One thread issues.
-__device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b,
-                                        uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}\n"
-      :
-      : "r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
 }
 // D[tmem] (+)= A[smem] * B[smem], bf16 x bf16 -> f32 (SASS: UTCHMMA), K = 16 per instruction.
 __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b,

@@ -65,17 +65,6 @@ class SiftOut(C.Structure):
 STAGES = {"match": 0, "hough_prep": 1, "hough_vote": 2, "hough_finish": 3, "affine": 4}
 
 
-def set_option(name: str, value: int) -> None:
-    check(lib.sod_set_option(name.encode(), int(value)), "sod_set_option")
-
-
-def get_option(name: str) -> int:
-    v = int(lib.sod_get_option(name.encode()))
-    if v < 0:
-        check(v, "sod_get_option")
-    return v
-
-
 def timing_enable(on: bool = True) -> None:
     check(lib.sod_timing_enable(int(on)), "sod_timing_enable")
 
@@ -97,8 +86,6 @@ _PROTOS = {
     "sod_version": (C.c_int, []),
     "sod_last_error": (C.c_char_p, []),
     "sod_device_sm_count": (C.c_int, []),
-    "sod_set_option": (C.c_int, [C.c_char_p, _i32]),
-    "sod_get_option": (_i32, [C.c_char_p]),
     "sod_timing_enable": (C.c_int, [_i32]),
     "sod_timing_read": (_i32, [_i32, _p, _i32]),
     "sod_cq_ints": (_i64, [_i64]),

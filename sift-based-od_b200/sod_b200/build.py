@@ -93,7 +93,7 @@ def build_variant(name: str, defines: list[str]) -> Path:
 
 
 if __name__ == "__main__":
-    if "--variant" in sys.argv:    # python -m sod_b200.build --variant initonly -DSOD_THR_INIT_ONLY
+    if "--variant" in sys.argv:    # python -m sod_b200.build --variant checked -DSOD_DEVICE_CHECKS
         i = sys.argv.index("--variant")
         print(build_variant(sys.argv[i + 1], [a for a in sys.argv[i + 2:] if a.startswith("-D")]))
     else:
