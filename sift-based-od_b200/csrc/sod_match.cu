@@ -6,19 +6,18 @@
 // and the top-2 selection happens in the TMEM epilogue without ever writing distances to HBM.
 //
 // Kernel anatomy (persistent CTA pairs: a cluster of 2 CTAs on the two SMs of a TPC, 640 threads each):
-//   warp 0      TMA producer: the CTA's query block (2 x 128 rows, double buffered) + its half of each
+//   warp 0      TMA producer: the CTA's query block (4 x 128 rows, double buffered) + its half of each
 //               database tile (64 of the tile's 128 rows = 8 KB, 8-deep ring) + the whole tile's 1040 B
 //               slice of per-row constants (|t|^2 << 8 | column, chunk minima, original rows) in its own,
 //               deeper ring.
-//   warps 1, 3  MMA issuers of the leader CTA, one per query half: per database tile 4 UTCIMMA.2CTA
-//               (M=256 over both CTAs, N=128, K=32) each into four independent 128-column TMEM
-//               accumulator slots per CTA (2 halves x 2 buffers).
+//   warps 1, 3  MMA issuers of the leader CTA, two query tiles each (warp 1 -> tiles 0 and 2, warp 3 ->
+//               tiles 1 and 3): per database tile and query tile 4 UTCIMMA.2CTA (M=256 over both CTAs,
+//               N=128, K=32) into that query tile's 128-column TMEM accumulator slot (4 slots per CTA).
 //   warp 2      TMEM allocator.
-//   warps 4-19  epilogue: thread <-> query row (TMEM lane), 16 warps = 4 lane quadrants x 2 query
-//               halves x 2 tile parities (even / odd tiles).  A warp pulls the 128 columns of its
-//               slot into registers in two loads, releases the slot, and prunes: a column can only
-//               enter the row's top-2 if |t|^2 - 2 q.t <= current 2nd best.  (Two threads per row:
-//               two candidate lists, merged by K3.)
+//   warps 4-19  epilogue: thread <-> query row (TMEM lane), 16 warps = 4 lane quadrants x 4 query tiles,
+//               one thread per query row that sees every database tile.  A warp pulls the 128 columns of
+//               its slot into registers in two loads, releases the slot, and prunes: a column can only
+//               enter the row's top-2 if |t|^2 - 2 q.t <= current 2nd best.
 //
 // Pruning needs a bound that is tight PER ROW: a warp takes the slow path as soon as one of its 32
 // rows does.  sod_db_prepare therefore stores the database sorted by |t|^2, so that the smallest
@@ -39,8 +38,10 @@ namespace sod {
 namespace {
 
 constexpr int kTileM = 128;                 // query rows per MMA (TMEM lanes)
-constexpr int kHalves = 2;                  // query tiles per CTA sharing one database tile
-constexpr int kBlockQ = kTileM * kHalves;   // 256 query rows per unit
+constexpr int kQTiles = 4;                  // query tiles per CTA sharing one database tile
+constexpr int kBlockQ = kTileM * kQTiles;   // 512 query rows per CTA (a pair unit sweeps 1024)
+constexpr int kAbiBlockQ = 256;             // query block of the C ABI: row_thr is padded to it and
+                                            // block_rotation counts it
 constexpr int kTileN = SOD_TILE_ROWS;       // database rows per MMA
 constexpr int kTileBytes = kTileN * SOD_DESC_DIM;  // 16 KB (A half-tile has the same size)
 constexpr int kChunk = 32;                  // accumulator columns per tcgen05.ld
@@ -49,9 +50,9 @@ constexpr int kCqPerm = kTileN + 4;         // offset of the permutation inside 
 constexpr int kCqTileBytes = kCqTile * 4;   // 1040 B, a multiple of 16 for the bulk copy
 constexpr int kNoKey = 0x7FFFFF;            // |t|^2 of padding rows / "no candidate yet" (> 128*255^2,
                                             // and (kNoKey << 8 | 127) still fits int32)
-constexpr int kParity = 2;                  // epilogue warps per (quadrant, half): even / odd tiles; one
-                                            // candidate list per row, segment and parity
-constexpr int kEpiWarps = 4 * kHalves * kParity;    // (TMEM lane quadrant) x (query half) x (tile parity)
+constexpr int kEpiWarps = 4 * kQTiles;      // (TMEM lane quadrant) x (query tile); one candidate list per
+                                            // row and segment
+constexpr int kIssuers = 2;                 // MMA-issuing warps (1 and 3), kQTiles / kIssuers tiles each
 constexpr int kThreads = (4 + kEpiWarps) * 32;
 constexpr int kTmemCols = 512;
 constexpr int kRegsLight = 56;      // producer / MMA / allocator warpgroup after setmaxnreg.dec
@@ -62,35 +63,35 @@ constexpr int kRegsLaunch = 65536 / kThreads / 8 * 8;
 static_assert(128 * kRegsLight + kEpiWarps * 32 * kRegsEpilogue <= kThreads * kRegsLaunch,
               "setmaxnreg budget exceeds the CTA's register pool");
 
-constexpr int kBarGroups = kParity;  // accumulator barriers are indexed by step % kBarGroups: every barrier is
-                                     // then waited on by ONE set of epilogue warps for consecutive phases (a
-                                     // parity wait must never skip a phase)
+static_assert(kQTiles * kTileN == kTmemCols, "one 128-column accumulator slot per query tile fills TMEM");
+
 // Shared-memory layout.  A CTA holds HALF of every database tile (64 rows, 8 KB).
 constexpr int kStages = 8;                   // database ring depth
 constexpr int kBStageBytes = kTileBytes / 2;
-constexpr int kCqSlots = 16;                 // >= kStages + 3 (slot-reuse argument in the producer);
+constexpr int kCqSlots = 16;                 // >= kStages + 2 (slot-reuse argument in the producer);
                                              // a power of two keeps `step % slots` a mask
-constexpr int kOffA = 0;                                     // [2 buffers][2 halves][16 KB]
-constexpr int kOffB = kOffA + 2 * kHalves * kTileBytes;      // [stages][8 KB]
+constexpr int kOffA = 0;                                     // [2 buffers][4 query tiles][16 KB]
+constexpr int kOffB = kOffA + 2 * kQTiles * kTileBytes;      // [stages][8 KB]
 constexpr int kOffCq = kOffB + kStages * kBStageBytes;       // [cq slots][260] int32
 constexpr int kOffBar = kOffCq + kCqSlots * kCqTileBytes;
-constexpr int kNumBars = 2 * kStages + 4 + 4 * kBarGroups + kCqSlots;
+constexpr int kNumBars = 2 * kStages + 4 + 2 * kQTiles + kCqSlots;
 constexpr int kOffTmemPtr = kOffBar + kNumBars * 8;
 constexpr int kSmemBytes = kOffTmemPtr + 16 + 1024;          // +1024: manual 1 KB alignment
-static_assert(kCqSlots >= kStages + 3 && (kCqSlots & (kCqSlots - 1)) == 0, "cq ring too shallow");
+static_assert(kCqSlots >= kStages + 2 && (kCqSlots & (kCqSlots - 1)) == 0, "cq ring too shallow");
+static_assert(kSmemBytes <= 227 * 1024, "shared memory exceeds the 227 KB a block may use");
 
 struct MatchArgs {
   const int32_t* qn;   // [nq] |q|^2
   const int32_t* cq;   // [n_tiles][260] per stored row: |t|^2 << 8 | column, chunk minima of |t|^2,
                        // original row (-1 = padding)
-  uint32_t* part_d2;   // [n_seg * 2][nq][2]  (one list per segment and column half)
-  int32_t* part_idx;   // [n_seg * 2][nq][2]
-  int32_t* row_thr;    // [n_qblocks * 256] shared pruning thresholds (memset to 0x7F..), or nullptr
+  uint32_t* part_d2;   // [n_seg][nq][2]  (one list per segment)
+  int32_t* part_idx;   // [n_seg][nq][2]
+  int32_t* row_thr;    // [thr_rows] shared pruning thresholds (memset to 0x7F..), or nullptr
   int nq;
+  int thr_rows;        // nq rounded up to kAbiBlockQ (sod_row_thr_ints): rows past it have no threshold
   int n_tiles;         // tiles swept by this launch: [tile_begin, tile_begin + n_tiles)
   int tile_begin;
-  int n_qblocks;
-  int n_qunits;        // units per segment: ceil(n_qblocks / 2), a CTA pair sweeps two query blocks
+  int n_qunits;        // units per segment: ceil(n_qblocks / 2), a CTA pair sweeps two query blocks (1024 rows)
   int n_seg;
   int idx_base;
   // Threshold publishing over peer memory (database sharded over several GPUs, kSeeded sweeps): when a unit
@@ -136,8 +137,9 @@ constexpr long long kNoKey64 = (static_cast<long long>(kNoKey) << 32) | 0x7FFFFF
 // The epilogue is bound by ALU issue slots, so the instruction count of this rare path matters: a
 // branch-free 32-key tournament (+53 instructions) cost 5 %, finer sub-trees (more branches) 10 %.
 // All tests are exact; pruning never changes the result.
-// `thr` is the pruning threshold: the row's 2nd best over everything either of its two threads has
-// seen (an element above it cannot be in the merged top-2; ties go through).
+// `thr` is the pruning threshold: the row's 2nd best over everything its thread has seen, and over what
+// other units sweeping the row have published (an element above it cannot be in the merged top-2; ties
+// go through).
 __device__ __forceinline__ void top2_chunk(const uint32_t* v, const int4* __restrict__ cp4,
                                            int cmin, const int32_t* __restrict__ perm_s,
                                            int idx_base, Top2& best, int& thr) {
@@ -185,7 +187,7 @@ __device__ __forceinline__ void top2_chunk(const uint32_t* v, const int4* __rest
 // run), which have nobody to share with inside the launch and must not pay the per-tile load and
 // atomicMin of the sharing code (B200, 1.28 M queries x 125k-row shard: 15.27 ms against 16.21 ms
 // with the sharing instance and 16.44 ms unseeded; profiles/r02_threshold_seeding.txt).
-// The two CTAs of a cluster (the two SMs of a TPC) run ONE tcgen05.mma.cta_group::2 per query half over
+// The two CTAs of a cluster (the two SMs of a TPC) run ONE tcgen05.mma.cta_group::2 per query tile over
 // M = 256 rows - 128 query rows of each CTA - and N = 128 database rows, of which each CTA stages 64: the
 // database stream from L2 and the shared-memory operand reads per MAC are half of what one CTA per tile
 // would need (B: 8 KB instead of 16 KB per CTA and tile).  The accumulators and the whole epilogue are per
@@ -212,10 +214,10 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
   auto bar_empty = [&](int s) { return bar0 + 8u * (kStages + s); };
   auto bar_afull = [&](int b) { return bar0 + 8u * (2 * kStages + b); };
   auto bar_aempty = [&](int b) { return bar0 + 8u * (2 * kStages + 2 + b); };
-  // accumulator hand-off barriers per (step % kBarGroups, half); the TMEM slot itself is step & 1
-  auto bar_tfull = [&](int g, int h) { return bar0 + 8u * (2 * kStages + 4 + 2 * g + h); };
-  auto bar_tempty = [&](int g, int h) { return bar0 + 8u * (2 * kStages + 4 + 2 * kBarGroups + 2 * g + h); };
-  auto bar_cqfull = [&](int s) { return bar0 + 8u * (2 * kStages + 4 + 4 * kBarGroups + s); };
+  // accumulator hand-off barriers of query tile h's TMEM slot: one phase per tile step
+  auto bar_tfull = [&](int h) { return bar0 + 8u * (2 * kStages + 4 + h); };
+  auto bar_tempty = [&](int h) { return bar0 + 8u * (2 * kStages + 4 + kQTiles + h); };
+  auto bar_cqfull = [&](int s) { return bar0 + 8u * (2 * kStages + 4 + 2 * kQTiles + s); };
   volatile uint32_t* tmem_ptr_smem = reinterpret_cast<volatile uint32_t*>(smem + kOffTmemPtr);
 
   if (warp == 0 && lane == 0) {
@@ -225,17 +227,16 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < kStages; ++s) {
       mbar_init(bar_full(s), 1);
-      mbar_init(bar_empty(s), kHalves);  // one tcgen05.commit per issuing warp
+      mbar_init(bar_empty(s), kIssuers);  // one tcgen05.commit per issuing warp
     }
     for (int b = 0; b < 2; ++b) {
       mbar_init(bar_afull(b), 1);
-      mbar_init(bar_aempty(b), kHalves);
+      mbar_init(bar_aempty(b), kIssuers);
     }
-    for (int g = 0; g < kBarGroups; ++g)
-      for (int h = 0; h < kHalves; ++h) {
-        mbar_init(bar_tfull(g, h), 1);
-        mbar_init(bar_tempty(g, h), 8);  // the four quadrant warps that read one slot, of each CTA
-      }
+    for (int h = 0; h < kQTiles; ++h) {
+      mbar_init(bar_tfull(h), 1);
+      mbar_init(bar_tempty(h), 8);  // the four quadrant warps that read one slot, of each CTA
+    }
     for (int s = 0; s < kCqSlots; ++s) mbar_init(bar_cqfull(s), 1);
     fence_mbar_init();
   }
@@ -267,10 +268,10 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
         const uint32_t ab = ucount & 1u, aph = (ucount >> 1) & 1u;
         mbar_wait(bar_aempty(ab), aph ^ 1u);
         // both CTAs' query blocks report to the leader's barrier, which expects the bytes of both
-        if (cta_rank == 0) mbar_arrive_expect_tx(bar_afull(ab), 2 * kHalves * kTileBytes);
+        if (cta_rank == 0) mbar_arrive_expect_tx(bar_afull(ab), 2 * kQTiles * kTileBytes);
         const uint32_t afull_leader = mapa_shared(bar_afull(ab), 0);
-        for (int h = 0; h < kHalves; ++h)
-          tma_load_2d_pair(base + kOffA + (ab * kHalves + h) * kTileBytes, &tmap_q, afull_leader, 0,
+        for (int h = 0; h < kQTiles; ++h)
+          tma_load_2d_pair(base + kOffA + (ab * kQTiles + h) * kTileBytes, &tmap_q, afull_leader, 0,
                            qb * kBlockQ + h * kTileM);
         for (int t = t0; t < t1; ++t, ++step) {
           const uint32_t s = step % kStages, ph = (step / kStages) & 1u;
@@ -281,11 +282,12 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
                            t * kTileN + static_cast<int>(cta_rank) * (kTileN / 2));
           // cq slice rides in its own, deeper ring: stage s is released when the MMAs that read it
           // retire, but the epilogue still reads cq after it has handed the accumulator back.
-          // The write for step j happens after MMA(j-kStages) retired; that MMA was issued after
-          // every epilogue warp RELEASED step j-kStages-2, i.e. finished its arithmetic on step
-          // j-kStages-3.  Steps j-kStages-2 .. j-1 may still be live -> kStages+3 = 11 of the 16 slots
-          // are needed.  Every CTA needs the constants of the WHOLE tile - its accumulators span all 128
-          // database rows - and loads them itself; the argument holds per CTA because the MMAs are joint.
+          // The write for step j happens after the MMAs of step j-kStages (all four query tiles)
+          // retired; each of them was issued after the epilogue warps of its tile RELEASED step
+          // j-kStages-1, so every epilogue warp has finished its arithmetic on step j-kStages-2.
+          // Steps j-kStages-1 .. j-1 may still be live -> kStages+2 = 10 of the 16 slots are needed.
+          // Every CTA needs the constants of the WHOLE tile - its accumulators span all 128 database
+          // rows - and loads them itself; the argument holds per CTA because the MMAs are joint.
           const uint32_t slot = step % kCqSlots;
           mbar_arrive_expect_tx(bar_cqfull(slot), kCqTileBytes);
           bulk_load_1d(base + kOffCq + slot * kCqTileBytes, a.cq + static_cast<int64_t>(t) * kCqTile,
@@ -295,13 +297,15 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
     }
   } else if ((warp == 1 || warp == 3) && cta_rank == 0) {
     // ------------------------------------------------------------------ MMA issuers
-    // Two issuing warps, one per query half (warp 1 -> half 0, warp 3 -> half 1): with K = 128 an
-    // accumulator slot holds only 256 clk of tensor work, so the issuing warp's own instruction
-    // stream and barrier round trips must stay well below that per slot.  Each warp runs its loop
-    // convergently so that addresses, phases and descriptors live in uniform registers; only the
-    // tcgen05 instructions are issued by one elected lane.  (Inside a divergent `if (lane == 0)`
-    // every UTCIMMA operand needs an R2UR move.)
-    const int h = warp >> 1;
+    // Two issuing warps with two query tiles each (warp 1 -> tiles 0 and 2, warp 3 -> tiles 1 and 3, so
+    // that the tensor pipe sees the tiles of a stage roughly in the order 0, 1, 2, 3): with K = 128 an
+    // accumulator slot holds only 256 clk of tensor work, so the issuing warp's own instruction stream
+    // and barrier round trips must stay well below that per slot.  Slot h is reused at the next tile
+    // step, after the MMAs of the three other query tiles (768 clk): that is the epilogue's window to
+    // pull it into registers.  Each warp runs its loop convergently so that addresses, phases and
+    // descriptors live in uniform registers; only the tcgen05 instructions are issued by one elected
+    // lane.  (Inside a divergent `if (lane == 0)` every UTCIMMA operand needs an R2UR move.)
+    const int h0 = warp >> 1;
     constexpr uint32_t idesc = umma_idesc_u8(2 * kTileM, kTileN);
     uint32_t step = 0, ucount = 0;
     for (int u = unit0; u < total_units; u += unit_step, ++ucount) {
@@ -310,24 +314,28 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
       const int t1 = a.tile_begin + static_cast<int>(static_cast<int64_t>(seg + 1) * a.n_tiles / a.n_seg);
       const uint32_t ab = ucount & 1u, aph = (ucount >> 1) & 1u;
       mbar_wait(bar_afull(ab), aph);
-      const uint64_t adesc = umma_desc_k128(base + kOffA + (ab * kHalves + h) * kTileBytes);
+      const uint32_t a_buf = base + kOffA + ab * (kQTiles * kTileBytes);
       for (int t = t0; t < t1; ++t, ++step) {
         const uint32_t s = step % kStages, ph = (step / kStages) & 1u;
-        const uint32_t acc = step & 1u;
         const uint64_t bdesc = umma_desc_k128(base + kOffB + s * kBStageBytes);
-        const uint32_t d = tmem_base + acc * (kHalves * kTileN) + h * kTileN;
         mbar_wait(bar_full(s), ph);
-        if (step >= 2)  // slot step & 1 was last used by step - 2: wait for its epilogue warps' release
-          mbar_wait(bar_tempty((step - 2) % kBarGroups, h), ((step - 2) / kBarGroups) & 1u);
-        tc_fence_after();
-        if (elect_one()) {
 #pragma unroll
-          for (int k = 0; k < SOD_DESC_DIM / 32; ++k)  // K = 32 bytes per UTCIMMA: +2 x 16 B
-            umma_i8_pair(d, adesc + 2 * k, bdesc + 2 * k, idesc, k > 0);
-          umma_commit_pair(bar_tfull(step % kBarGroups, h), 3);  // this half is ready in both CTAs
-          umma_commit_pair(bar_empty(s), 3);   // (count 2) stage free in both CTAs once both halves retire
+        for (int i = 0; i < kQTiles / kIssuers; ++i) {
+          const int h = h0 + kIssuers * i;
+          const uint64_t adesc = umma_desc_k128(a_buf + h * kTileBytes);
+          if (step >= 1)  // slot h was last used by step - 1: wait for its epilogue warps' release
+            mbar_wait(bar_tempty(h), (step - 1) & 1u);
+          tc_fence_after();
+          if (elect_one()) {
+#pragma unroll
+            for (int k = 0; k < SOD_DESC_DIM / 32; ++k)  // K = 32 bytes per UTCIMMA: +2 x 16 B
+              umma_i8_pair(tmem_base + h * kTileN, adesc + 2 * k, bdesc + 2 * k, idesc, k > 0);
+            umma_commit_pair(bar_tfull(h), 3);  // this query tile is ready in both CTAs
+            // (count 2) stage free in both CTAs once both warps' tiles retire
+            if (i == kQTiles / kIssuers - 1) umma_commit_pair(bar_empty(s), 3);
+          }
+          __syncwarp();
         }
-        __syncwarp();
       }
       if (elect_one()) umma_commit_pair(bar_aempty(ab), 3);  // (count 2) query block buffer free
       __syncwarp();
@@ -338,24 +346,21 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
     if constexpr (kRegsEpilogue > kRegsLaunch) setmaxnreg_inc<kRegsEpilogue>();
     const int e = warp - 4;
     const int quad = warp & 3;          // TMEM lane quadrant this warp may read
-    const int h = (e >> 2) & 1;         // which query half-tile
-    uint32_t par = e >> 3;              // this warp takes the tiles with (step & 1) == par
+    const int h = e >> 2;               // which query tile
     const uint32_t lane_sel = static_cast<uint32_t>(quad * 32) << 16;
     // Loop invariants the compiler would otherwise rebuild at the top of EVERY tile step from special
-    // registers (S2R SR_TID.X for the parity, S2R SR_CgaCtaId for the shared-memory window of a cluster
+    // registers (S2R SR_TID.X for the query tile, S2R SR_CgaCtaId for the shared-memory window of a cluster
     // launch - tens of cycles each, in front of the barrier waits): keep them in registers.
-    uint32_t tfull_h = bar_tfull(0, h);      // + 16 * (step % kBarGroups)
+    uint32_t tfull_h = bar_tfull(h);
     uint32_t cqfull_0 = bar_cqfull(0);       // + 8 * slot
     uint32_t cq_0 = base + kOffCq;           // + slot * kCqTileBytes (shared-memory window address)
-    uint32_t taddr_h = tmem_base + lane_sel + h * kTileN;   // + (step & 1) * (kHalves * kTileN)
-    asm volatile("" : "+r"(par), "+r"(tfull_h), "+r"(cqfull_0), "+r"(taddr_h));
-    asm volatile("" : "+r"(cq_0));
-    // accumulator slots are released on the LEADER's barriers (the leader issues the MMAs)
-    uint32_t tempty_rel0 = mapa_shared(bar_tempty(0, h), 0);
-    uint32_t tempty_rel1 = mapa_shared(bar_tempty(1, h), 0);
-    // keep the two cluster addresses in registers: rematerialised, each release would re-read the cluster
-    // rank (S2R, tens of cycles) on the critical path between the TMEM load and the slot's release
-    asm volatile("" : "+r"(tempty_rel0), "+r"(tempty_rel1));
+    uint32_t taddr = tmem_base + lane_sel + h * kTileN;     // this warp's lanes of slot h
+    asm volatile("" : "+r"(tfull_h), "+r"(cqfull_0), "+r"(taddr), "+r"(cq_0));
+    // accumulator slots are released on the LEADER's barriers (the leader issues the MMAs); kept in a
+    // register: rematerialised, each release would re-read the cluster rank (S2R, tens of cycles) on the
+    // critical path between the TMEM load and the slot's release
+    uint32_t tempty_rel = mapa_shared(bar_tempty(h), 0);
+    asm volatile("" : "+r"(tempty_rel));
     uint32_t step = 0, ucount = 1;
     for (int u = unit0; u < total_units; u += unit_step, ++ucount) {
       const int seg = u / a.n_qunits;
@@ -367,28 +372,24 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
       const int row = qb * kBlockQ + h * kTileM + quad * 32 + lane;
       Top2 best{kNoKey64, kNoKey64, kNoKey};
       // Threshold sharing between the units that sweep different database segments for the same
-      // query rows (and between the row's two threads): every holder of the row publishes its 2nd
-      // best with atomicMin, everyone prunes with the minimum.  Any unit's 2nd best is an upper
-      // bound of the row's final 2nd best, so this stays exact; without it every segment pays the
-      // ~2 ln(n) threshold-establishing updates again.  (row_thr is padded to whole query blocks; the
-      // phantom block of an odd pair lies past it and is never read or written.)
-      const bool thr_row = (kShare || kSeeded) && qb < a.n_qblocks;
-      int* const gthr = (kShare || kSeeded) ? a.row_thr + (qb * kBlockQ + h * kTileM + quad * 32 + lane) : nullptr;
+      // query rows: every holder of the row publishes its 2nd best with atomicMin, everyone prunes
+      // with the minimum.  Any unit's 2nd best is an upper bound of the row's final 2nd best, so this
+      // stays exact; without it every segment pays the ~2 ln(n) threshold-establishing updates again.  (row_thr is padded to 256 rows; the rest of the
+      // last query block, and the phantom block of an odd pair, lie past it and are never read or written.)
+      const bool thr_row = (kShare || kSeeded) && row < a.thr_rows;
+      int* const gthr = (kShare || kSeeded) ? a.row_thr + row : nullptr;
       int published = kNoKey;
       int thr = thr_row ? min(kNoKey, __ldcg(gthr)) : kNoKey;
-      // this warp takes every other tile of the unit: the ones whose global step has its parity
       const uint32_t step_end = step + static_cast<uint32_t>(t1 - t0);
-      for (step += (par ^ step) & 1u; step < step_end; step += 2) {
-        const uint32_t acc = step & 1u, bg = step % kBarGroups, bgph = (step / kBarGroups) & 1u;
+      for (; step < step_end; ++step) {
         const uint32_t slot = step % kCqSlots, cqph = (step / kCqSlots) & 1u;
         mbar_wait(cqfull_0 + 8u * slot, cqph);  // landed long ago: returns at the first poll
-        mbar_wait(tfull_h + 16u * bg, bgph);
+        mbar_wait(tfull_h, step & 1u);
         tc_fence_after();
         const int32_t* cs = reinterpret_cast<const int32_t*>(__cvta_shared_to_generic(cq_0 + slot * kCqTileBytes));
         const int32_t* perm_s = cs + kCqPerm;
         // fetched now, folded in after this tile: the L2 round trip hides behind the tile's work
         const int g_next = (kShare && thr_row) ? __ldcg(gthr) : kNoKey;
-        const uint32_t taddr = taddr_h + acc * (kHalves * kTileN);
         const int4* c4 = reinterpret_cast<const int4*>(cs);
         const int4 cmin = c4[kTileN / 4];
         uint32_t v[2 * kChunk];
@@ -398,7 +399,7 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
         tmem_ld64_wait(taddr + 2 * kChunk, v);
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(bg ? tempty_rel1 : tempty_rel0);
+        if (lane == 0) mbar_arrive_cluster(tempty_rel);
         top2_chunk(v, c4 + 16, cmin.z, perm_s, a.idx_base, best, thr);
         top2_chunk(v + kChunk, c4 + 24, cmin.w, perm_s, a.idx_base, best, thr);
         if (kShare && thr_row) {
@@ -409,7 +410,6 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
           thr = min(thr, g_next);
         }
       }
-      step = step_end;
       if (kSeeded && thr_row && best.d2 < kNoKey) {
         if (a.n_peers > 0) {
           // reductions over NVLink into every rank's array (no return value: fire and forget)
@@ -421,7 +421,7 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap_q,
       }
       if (row < a.nq) {
         const int qn = a.qn[row];
-        const int64_t o = ((static_cast<int64_t>(seg) * kParity + par) * a.nq + row) * 2;
+        const int64_t o = (static_cast<int64_t>(seg) * a.nq + row) * 2;
         SOD_DCHECK(seg < a.n_seg && (best.k1 == kNoKey64 || static_cast<int>(best.k1 & 0xFFFFFFFFll) >= a.idx_base));
         const int d1 = static_cast<int>(best.k1 >> 32), d2 = static_cast<int>(best.k2 >> 32);
         a.part_d2[o + 0] = d1 != kNoKey ? static_cast<uint32_t>(d1 + qn) : 0xFFFFFFFFu;
@@ -665,9 +665,15 @@ struct Plan {
   int n_tiles, n_qblocks, n_qunits, n_seg, grid;
 };
 
+// Per-unit cost outside its tile steps, in tile steps: the 12 steps of 2 query tiles measured for the earlier
+// two-tile form, as time, in the twice-as-long steps of 4 query tiles (B200: 0.65 us against 0.36 us per step).
+// A one-wave sweep timed at 64 .. 2048 tiles does not isolate it (the slow path is front-loaded, so the cost
+// per step falls along the sweep); profiles/r04_match_four_tiles.txt.
+constexpr int kUnitFillSteps = 6;
+
 // Split every query block's database sweep into n_seg contiguous segments so that
 // n_qunits*n_seg units fill the persistent grid evenly (cost = makespan in tile steps).  A unit is swept
-// by a CTA pair (two query blocks side by side); the grid holds sms / 2 pairs (sms >= 2).
+// by a CTA pair (two query blocks of 512 rows side by side); the grid holds sms / 2 pairs (sms >= 2).
 Plan make_plan(int64_t nq, int64_t ndb, int sms) {
   Plan p;
   p.n_tiles = static_cast<int>((ndb + kTileN - 1) / kTileN);
@@ -681,9 +687,9 @@ Plan make_plan(int64_t nq, int64_t ndb, int sms) {
     for (int s = 1; s <= max_seg; ++s) {
       const int64_t units = static_cast<int64_t>(p.n_qunits) * s;
       const int64_t waves = (units + pairs - 1) / pairs;
-      // +12: pipeline fill and the slow-path chunks of a unit's first columns (measured; units of one
+      // + kUnitFillSteps: pipeline fill and the slow-path chunks of a unit's first columns (units of one
       // query block share their thresholds, so a later segment does not start from scratch)
-      const int64_t cost = waves * ((p.n_tiles + s - 1) / s + 12);
+      const int64_t cost = waves * ((p.n_tiles + s - 1) / s + kUnitFillSteps);
       if (best < 0 || cost < best) {
         best = cost;
         p.n_seg = s;
@@ -772,17 +778,18 @@ int sod_query_prepare(const uint8_t* q, int64_t n_rows, int32_t* qn, sod_stream_
   return SOD_OK;
 }
 
-// partial lists [n_seg * kParity][nq][2] (d2 + idx), then the shared thresholds [n_qblocks * 256]
+static int64_t thr_rows(int64_t n_query) {
+  return n_query <= 0 ? 0 : (n_query + kAbiBlockQ - 1) / kAbiBlockQ * kAbiBlockQ;
+}
+// partial lists [n_seg][nq][2] (d2 + idx), then the shared thresholds [thr_rows(nq)]
 static size_t match_lists_bytes(const Plan& p, int64_t n_query) {
-  return static_cast<size_t>(p.n_seg) * kParity * static_cast<size_t>(n_query) * 2 * 8;
+  return static_cast<size_t>(p.n_seg) * static_cast<size_t>(n_query) * 2 * 8;
 }
 static size_t match_workspace_need(const Plan& p, int64_t n_query) {
-  return match_lists_bytes(p, n_query) + static_cast<size_t>(p.n_qblocks) * kBlockQ * 4;
+  return match_lists_bytes(p, n_query) + static_cast<size_t>(thr_rows(n_query)) * 4;
 }
 
-int64_t sod_row_thr_ints(int64_t n_query) {
-  return n_query <= 0 ? 0 : (n_query + kBlockQ - 1) / kBlockQ * kBlockQ;
-}
+int64_t sod_row_thr_ints(int64_t n_query) { return thr_rows(n_query); }
 
 size_t sod_match_workspace_bytes(int64_t n_query, int64_t n_db) {
   if (n_query <= 0 || n_db <= 0) return 16;
@@ -815,7 +822,7 @@ int sod_match_top2_peer(const uint8_t* q, const int32_t* qn, int64_t n_query, co
                 "bad peer threshold table");
   SOD_CHECK_ARG(block_rotation >= 0, "negative block rotation");
   SOD_CHECK_ARG(n_query >= 0 && n_db >= 0, "negative size");
-  SOD_CHECK_ARG(n_query < (int64_t(1) << 31) - kBlockQ && n_db < (int64_t(1) << 31) - kTileN,
+  SOD_CHECK_ARG(n_query < (int64_t(1) << 31) - 2 * kBlockQ && n_db < (int64_t(1) << 31) - kTileN,
                 "size out of range");
   SOD_CHECK_ARG(static_cast<int64_t>(db_index_base) + n_db < (int64_t(1) << 31),
                 "db_index_base + n_db overflows int32");
@@ -860,26 +867,27 @@ int sod_match_top2_peer(const uint8_t* q, const int32_t* qn, int64_t n_query, co
   a.qn = qn;
   a.cq = cq;
   a.part_d2 = static_cast<uint32_t*>(workspace);
-  a.part_idx = reinterpret_cast<int32_t*>(a.part_d2 + static_cast<size_t>(p.n_seg) * kParity * n_query * 2);
+  a.part_idx = reinterpret_cast<int32_t*>(a.part_d2 + static_cast<size_t>(p.n_seg) * n_query * 2);
   // Thresholds are shared whenever a query row is swept by more than one unit; 0x7F7F7F7F = none yet
   // A caller-held array additionally carries thresholds across launches (and, after a min-reduce, across
   // the shards of several GPUs): it is read at the start and holds min(input, this sweep's 2nd best) after.
   a.row_thr = row_thr;
   if (!row_thr && p.n_seg > 1) {
     a.row_thr = reinterpret_cast<int32_t*>(static_cast<uint8_t*>(workspace) + match_lists_bytes(p, n_query));
-    SOD_CHECK_CUDA(cudaMemsetAsync(a.row_thr, 0x7F, static_cast<size_t>(p.n_qblocks) * kBlockQ * 4, st));
+    SOD_CHECK_CUDA(cudaMemsetAsync(a.row_thr, 0x7F, static_cast<size_t>(thr_rows(n_query)) * 4, st));
   }
   a.nq = static_cast<int>(n_query);
+  a.thr_rows = static_cast<int>(thr_rows(n_query));
   a.n_tiles = p.n_tiles;
   a.tile_begin = static_cast<int>(tile_begin);
-  a.n_qblocks = p.n_qblocks;
   a.n_qunits = p.n_qunits;
   a.n_seg = p.n_seg;
   a.idx_base = db_index_base;
   // peer publishing and the rotated visiting order belong to single-segment sweeps (the seeded instance)
   const bool peer_mode = n_peers > 0 && row_thr && p.n_seg == 1;
   a.n_peers = peer_mode ? n_peers : 0;
-  a.unit_rot = peer_mode ? static_cast<int>((block_rotation / 2) % p.n_qunits) : 0;
+  // block_rotation counts blocks of 256 query rows; a unit holds 2 * kBlockQ = 1024
+  a.unit_rot = peer_mode ? static_cast<int>((block_rotation / (2 * kBlockQ / kAbiBlockQ)) % p.n_qunits) : 0;
   for (int i = 0; i < SOD_EXCHANGE_MAX_RANKS; ++i) a.peer_thr[i] = (peer_mode && i < n_peers) ? peer_thr_host[i] : nullptr;
   for (int i = 0; i < a.n_peers; ++i) SOD_CHECK_ARG(a.peer_thr[i], "null threshold array of rank %d", i);
 
@@ -905,7 +913,7 @@ int sod_match_top2_peer(const uint8_t* q, const int32_t* qn, int64_t n_query, co
     SOD_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kernel, map_q, map_db, a));
   }
   SOD_CHECK_LAUNCH("match_top2_kernel");
-  top2_merge_kernel<<<mblocks, mthreads, 0, st>>>(a.part_idx, a.part_d2, p.n_seg * kParity, n_query,
+  top2_merge_kernel<<<mblocks, mthreads, 0, st>>>(a.part_idx, a.part_d2, p.n_seg, n_query,
                                                   out_idx, out_d2, nullptr, nullptr, 0.0);
   SOD_CHECK_LAUNCH("top2_merge_kernel");
   return SOD_OK;
