@@ -131,6 +131,59 @@ __device__ __forceinline__ bool residual_on_edge(double du, double dv, double x_
   return fabs(du - x_ref) <= 1e-9 * x_ref + 1e-7 || fabs(dv - y_ref) <= 1e-9 * y_ref + 1e-7;
 }
 
+// Residual limits (x_ref, y_ref) of a bin: remove_outliers thresholds use pose[3], the sigma BIN INDEX
+// (AffineParameters.py:120-121).  A factor <= 0 disables its limit.
+__device__ __forceinline__ double2 residual_limits(const AffineArgs& a, int rec) {
+  const int frame = a.bin_group[rec] / a.sc.groups_per_frame;
+  SOD_DCHECK(frame >= 0 && frame < a.sc.n_frames);
+  const int isigma = a.bin_code[rec] % a.bins;
+  const double inf = __longlong_as_double(0x7ff0000000000000ll);
+  return make_double2(
+      a.factor_x > 0 ? __ddiv_rn(static_cast<double>(a.sc.frame_wh[2 * frame] * isigma), a.factor_x) : inf,
+      a.factor_y > 0 ? __ddiv_rn(static_cast<double>(a.sc.frame_wh[2 * frame + 1] * isigma), a.factor_y) : inf);
+}
+
+// A bin whose members lie past cap_votes (member_keep was sized for another Hough result) is not verified:
+// reject_bin flags the overflow and gives the bin no votes.
+__device__ __forceinline__ bool members_past_capacity(const AffineArgs& a, int off, int cnt) {
+  return static_cast<int64_t>(off) + cnt > a.out.cap_votes;
+}
+__device__ __forceinline__ void reject_bin(const AffineArgs& a, int64_t v) {
+  a.out.counters[1] = 1;
+  a.out.votes[v] = 0;
+  a.out.status[v] = 0;
+}
+
+// (x, y) of the model point and (u, v) of the query point of member j: three dependent gathers
+// (member -> match -> keypoint).
+__device__ __forceinline__ float4 pair_coords(const AffineArgs& a, const int32_t* mem, int j) {
+  const int m = mem[j];
+  SOD_DCHECK(m >= 0 && a.match_t[m] >= 0 && a.match_t[m] < a.sc.model.n && a.match_q[m] >= 0 &&
+             a.match_q[m] < a.sc.query.n);
+  const float2 pm = reinterpret_cast<const float2*>(a.sc.model.xy)[a.match_t[m]];
+  const float2 pq = reinterpret_cast<const float2*>(a.sc.query.xy)[a.match_q[m]];
+  return make_float4(pm.x, pm.y, pq.x, pq.y);
+}
+
+// |u_AP - u| of a pair for the fitted coordinate u_AP = ma * x + mb * y + t, in the reference's operation
+// order (AffineParameters.py:128-155): (m1, m2, tx) against the query's u, (m3, m4, ty) against its v.
+__device__ __forceinline__ double fit_residual(double ma, double mb, double t, double x, double y, float u) {
+  return fabs(__dadd_rn(__dadd_rn(__dmul_rn(ma, x), __dmul_rn(mb, y)), t) - static_cast<double>(u));
+}
+
+// One bin's result: parameters in the order m1 m2 m3 m4 tx ty, votes, status word (bit 0 live, 1 singular,
+// 2 residual on edge, 8.. passes) and the singular / on-edge counters.
+__device__ __forceinline__ void write_bin_result(const AffineArgs& a, int64_t v, const double (&pu)[3],
+                                                 const double (&pv)[3], int votes, int live, int singular,
+                                                 int on_edge, int passes) {
+  double* p = a.out.params + v * 6;
+  p[0] = pu[0]; p[1] = pu[1]; p[2] = pv[0]; p[3] = pv[1]; p[4] = pu[2]; p[5] = pv[2];
+  a.out.votes[v] = votes;
+  a.out.status[v] = live | (singular << 1) | ((on_edge ? 1 : 0) << 2) | (passes << 8);
+  if (singular) atomicAdd(&a.out.counters[2], 1);
+  if (on_edge) atomicAdd(&a.out.counters[3], on_edge);
+}
+
 // One THREAD per small valid bin (the vast majority: random bins with 5-10 votes): the alive set is
 // a 32-bit mask, every pass re-gathers the coordinates of the alive pairs.
 constexpr int kSmallThreads = 128;
@@ -142,9 +195,6 @@ __global__ void __launch_bounds__(kSmallThreads) affine_verify_small_kernel(cons
   __shared__ float4 s_pairs[kSmallStage][kSmallThreads];
   int64_t n_valid = a.out.counters[0];
   if (n_valid > a.out.cap_valid) n_valid = a.out.cap_valid;
-  const float2* mxy = reinterpret_cast<const float2*>(a.sc.model.xy);
-  const float2* qxy = reinterpret_cast<const float2*>(a.sc.query.xy);
-  const double inf = __longlong_as_double(0x7ff0000000000000ll);
   for (int64_t v = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; v < n_valid;
        v += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     const int rec = a.out.valid_bin[v];
@@ -152,28 +202,16 @@ __global__ void __launch_bounds__(kSmallThreads) affine_verify_small_kernel(cons
     const int cnt = a.bin_count[rec];
     if (cnt > kSmallAffine) continue;
     const int off = a.bin_offset[rec];
-    if (static_cast<int64_t>(off) + cnt > a.out.cap_votes) {  // member_keep was sized for another Hough result
-      a.out.counters[1] = 1;
-      a.out.votes[v] = 0;
-      a.out.status[v] = 0;
+    if (members_past_capacity(a, off, cnt)) {
+      reject_bin(a, v);
       continue;
     }
-    const int frame = a.bin_group[rec] / a.sc.groups_per_frame;
-    const int isigma = a.bin_code[rec] % a.bins;
-    const double x_ref = a.factor_x > 0 ? __ddiv_rn(static_cast<double>(a.sc.frame_wh[2 * frame] * isigma), a.factor_x) : inf;
-    const double y_ref = a.factor_y > 0 ? __ddiv_rn(static_cast<double>(a.sc.frame_wh[2 * frame + 1] * isigma), a.factor_y) : inf;
+    const double2 lim = residual_limits(a, rec);
     const int32_t* mem = a.members + off;
-    auto gather = [&](int j) -> float4 {
-      const int m = mem[j];
-      SOD_DCHECK(m >= 0 && a.match_t[m] >= 0 && a.match_t[m] < a.sc.model.n && a.match_q[m] >= 0 &&
-                 a.match_q[m] < a.sc.query.n);
-      const float2 pm = mxy[a.match_t[m]], pq = qxy[a.match_q[m]];
-      return make_float4(pm.x, pm.y, pq.x, pq.y);
-    };
     const int n_stage = cnt < kSmallStage ? cnt : kSmallStage;
 #pragma unroll 4
-    for (int j = 0; j < n_stage; ++j) s_pairs[j][threadIdx.x] = gather(j);
-    auto pair_of = [&](int j) -> float4 { return j < kSmallStage ? s_pairs[j][threadIdx.x] : gather(j); };
+    for (int j = 0; j < n_stage; ++j) s_pairs[j][threadIdx.x] = pair_coords(a, mem, j);
+    auto pair_of = [&](int j) -> float4 { return j < kSmallStage ? s_pairs[j][threadIdx.x] : pair_coords(a, mem, j); };
     unsigned alive = cnt >= 32 ? 0xffffffffu : ((1u << cnt) - 1u);
     int n_alive = cnt, passes = 0, live = 0, singular = 0, on_edge = 0;
     double pu[3] = {0, 0, 0}, pv[3] = {0, 0, 0};
@@ -192,12 +230,10 @@ __global__ void __launch_bounds__(kSmallThreads) affine_verify_small_kernel(cons
       for (int j = 0; j < cnt; ++j) {
         if (!(alive >> j & 1u)) continue;
         const float4 c = pair_of(j);
-        const double x = c.x, y = c.y;
-        const double ua = __dadd_rn(__dadd_rn(__dmul_rn(pu[0], x), __dmul_rn(pu[1], y)), pu[2]);
-        const double va = __dadd_rn(__dadd_rn(__dmul_rn(pv[0], x), __dmul_rn(pv[1], y)), pv[2]);
-        const double du = fabs(ua - static_cast<double>(c.z)), dv = fabs(va - static_cast<double>(c.w));
-        on_edge += residual_on_edge(du, dv, x_ref, y_ref) ? 1 : 0;
-        if (du > x_ref || dv > y_ref) {
+        const double du = fit_residual(pu[0], pu[1], pu[2], c.x, c.y, c.z);
+        const double dv = fit_residual(pv[0], pv[1], pv[2], c.x, c.y, c.w);
+        on_edge += residual_on_edge(du, dv, lim.x, lim.y) ? 1 : 0;
+        if (du > lim.x || dv > lim.y) {
           alive &= ~(1u << j);
           ++removed;
         }
@@ -210,12 +246,7 @@ __global__ void __launch_bounds__(kSmallThreads) affine_verify_small_kernel(cons
     }
     uint8_t* keep = a.out.member_keep + off;
     for (int j = 0; j < cnt; ++j) keep[j] = (alive >> j) & 1u;
-    double* p = a.out.params + v * 6;
-    p[0] = pu[0]; p[1] = pu[1]; p[2] = pv[0]; p[3] = pv[1]; p[4] = pu[2]; p[5] = pv[2];
-    a.out.votes[v] = n_alive;
-    a.out.status[v] = live | (singular << 1) | ((on_edge ? 1 : 0) << 2) | (passes << 8);
-    if (singular) atomicAdd(&a.out.counters[2], 1);
-    if (on_edge) atomicAdd(&a.out.counters[3], on_edge);
+    write_bin_result(a, v, pu, pv, n_alive, live, singular, on_edge, passes);
   }
 }
 
@@ -239,8 +270,6 @@ __global__ void __launch_bounds__(kAffineWarps * 32) affine_verify_kernel(const 
   const int64_t n_warps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
   int64_t n_valid = a.out.counters[0];
   if (n_valid > a.out.cap_valid) n_valid = a.out.cap_valid;
-  const float2* mxy = reinterpret_cast<const float2*>(a.sc.model.xy);
-  const float2* qxy = reinterpret_cast<const float2*>(a.sc.query.xy);
   // Almost every selected bin is a small one (affine_verify_small_kernel's): the lanes look at a window of up
   // to 32 list entries at a time and the warp then takes the big bins among them in turn.  (One entry per warp and step meant
   // 1.6 M dependent look-ups spread over 3,000 warps at C5: 0.66 ms for 9,000 big bins.)
@@ -263,39 +292,21 @@ __global__ void __launch_bounds__(kAffineWarps * 32) affine_verify_kernel(const 
     const int rec = __shfl_sync(0xffffffffu, rec_l, src);
     const int cnt = __shfl_sync(0xffffffffu, cnt_l, src);
     const int off = a.bin_offset[rec];
-    if (static_cast<int64_t>(off) + cnt > a.out.cap_votes) {
-      if (lane == 0) {
-        a.out.counters[1] = 1;
-        a.out.votes[v] = 0;
-        a.out.status[v] = 0;
-      }
+    if (members_past_capacity(a, off, cnt)) {
+      if (lane == 0) reject_bin(a, v);
       continue;
     }
-    const int frame = a.bin_group[rec] / a.sc.groups_per_frame;
-    const int isigma = a.bin_code[rec] % a.bins;
-    // remove_outliers thresholds use pose[3], the sigma BIN INDEX (AffineParameters.py:120-121)
-    const double inf = __longlong_as_double(0x7ff0000000000000ll);
-    const double x_ref = a.factor_x > 0 ? __ddiv_rn(static_cast<double>(a.sc.frame_wh[2 * frame] * isigma), a.factor_x) : inf;
-    const double y_ref = a.factor_y > 0 ? __ddiv_rn(static_cast<double>(a.sc.frame_wh[2 * frame + 1] * isigma), a.factor_y) : inf;
+    const double2 lim = residual_limits(a, rec);
     uint8_t* keep = a.out.member_keep + off;
     const int32_t* mem = a.members + off;
     __syncwarp();  // the previous bin's readers of the stage are done
 #pragma unroll 4
     for (int j = lane; j < cnt; j += 32) {
       keep[j] = 1;
-      if (j < kAffineStage) {
-        const int m = mem[j];
-        const float2 pm = mxy[a.match_t[m]], pq = qxy[a.match_q[m]];
-        stage[j] = make_float4(pm.x, pm.y, pq.x, pq.y);
-      }
+      if (j < kAffineStage) stage[j] = pair_coords(a, mem, j);
     }
     __syncwarp();
-    auto pair_of = [&](int j) -> float4 {
-      if (j < kAffineStage) return stage[j];
-      const int m = mem[j];
-      const float2 pm = mxy[a.match_t[m]], pq = qxy[a.match_q[m]];
-      return make_float4(pm.x, pm.y, pq.x, pq.y);
-    };
+    auto pair_of = [&](int j) -> float4 { return j < kAffineStage ? stage[j] : pair_coords(a, mem, j); };
     int alive = cnt, passes = 0, live = 0, singular = 0, on_edge = 0;
     double pu[3] = {0, 0, 0}, pv[3] = {0, 0, 0};
     while (true) {
@@ -317,12 +328,10 @@ __global__ void __launch_bounds__(kAffineWarps * 32) affine_verify_kernel(const 
       for (int j = lane; j < cnt; j += 32) {
         if (!keep[j]) continue;
         const float4 c = pair_of(j);
-        const double x = c.x, y = c.y;
-        const double ua = __dadd_rn(__dadd_rn(__dmul_rn(pu[0], x), __dmul_rn(pu[1], y)), pu[2]);
-        const double va = __dadd_rn(__dadd_rn(__dmul_rn(pv[0], x), __dmul_rn(pv[1], y)), pv[2]);
-        const double du = fabs(ua - static_cast<double>(c.z)), dv = fabs(va - static_cast<double>(c.w));
-        on_edge += residual_on_edge(du, dv, x_ref, y_ref) ? 1 : 0;
-        if (du > x_ref || dv > y_ref) {
+        const double du = fit_residual(pu[0], pu[1], pu[2], c.x, c.y, c.z);
+        const double dv = fit_residual(pv[0], pv[1], pv[2], c.x, c.y, c.w);
+        on_edge += residual_on_edge(du, dv, lim.x, lim.y) ? 1 : 0;
+        if (du > lim.x || dv > lim.y) {
           keep[j] = 0;
           ++removed;
         }
@@ -338,14 +347,7 @@ __global__ void __launch_bounds__(kAffineWarps * 32) affine_verify_kernel(const 
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) on_edge += __shfl_xor_sync(0xffffffffu, on_edge, o);
-    if (lane == 0) {
-      double* p = a.out.params + v * 6;
-      p[0] = pu[0]; p[1] = pu[1]; p[2] = pv[0]; p[3] = pv[1]; p[4] = pu[2]; p[5] = pv[2];
-      a.out.votes[v] = alive;
-      a.out.status[v] = live | (singular << 1) | ((on_edge ? 1 : 0) << 2) | (passes << 8);
-      if (singular) atomicAdd(&a.out.counters[2], 1);
-      if (on_edge) atomicAdd(&a.out.counters[3], on_edge);
-    }
+    if (lane == 0) write_bin_result(a, v, pu, pv, alive, live, singular, on_edge, passes);
    }
   }
 }

@@ -218,6 +218,34 @@ __global__ void pose_bin_index_kernel(const double* __restrict__ pose, int64_t n
                 (static_cast<uint32_t>(it) << 16) | (static_cast<uint32_t>(is) << 24);
 }
 
+// Inclusive prefix sum of v over the lanes of a warp.
+__device__ __forceinline__ int warp_inclusive_scan(int v) {
+  const int lane = threadIdx.x & 31;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int t = __shfl_up_sync(0xffffffffu, v, o);
+    if (lane >= o) v += t;
+  }
+  return v;
+}
+
+// Exclusive prefix sum of v over a CTA of 32 warps: the warps' totals meet in warp_sums[32] (shared memory),
+// warp 0 turns them into the warps' exclusive prefixes, every thread adds its own warp's.  Every thread must
+// call it.  The CTA's total is the last thread's result + v.
+__device__ __forceinline__ int cta_exclusive_scan(int v, int* warp_sums) {
+  SOD_DCHECK(blockDim.x == 1024);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int incl = warp_inclusive_scan(v);
+  if (lane == 31) warp_sums[warp] = incl;
+  __syncthreads();
+  if (warp == 0) {
+    const int w = warp_sums[lane];
+    warp_sums[lane] = warp_inclusive_scan(w) - w;
+  }
+  __syncthreads();
+  return warp_sums[warp] + incl - v;
+}
+
 // Exclusive scan of n ints.  One CTA scans rounds of 8,192 elements (8 consecutive per thread) and carries
 // the running total; `seed` (may be NULL) holds the value the first element starts from and `n_end` (may be
 // < 0) is where the grand total is written.  Small inputs (compaction blocks) take one launch of one CTA.
@@ -228,12 +256,10 @@ constexpr int kScanItems = 8;
 constexpr int kScanTile = 1024 * kScanItems;
 __global__ void __launch_bounds__(1024) exclusive_scan_kernel(const int32_t* __restrict__ in,
                                                               int64_t n, int32_t* __restrict__ out,
-                                                              int32_t* __restrict__ out_copy,
                                                               int32_t* __restrict__ total,
                                                               const int32_t* __restrict__ tile_seed) {
   __shared__ int32_t warp_sums[32];
   __shared__ int32_t carry;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   // grid form: this CTA owns tile blockIdx.x only and starts from the scanned sum of the tiles before it
   const int64_t first = tile_seed ? static_cast<int64_t>(blockIdx.x) * kScanTile : 0;
   const int64_t last = tile_seed ? (first + kScanTile < n ? first + kScanTile : n) : n;
@@ -248,35 +274,14 @@ __global__ void __launch_bounds__(1024) exclusive_scan_kernel(const int32_t* __r
       v[k] = i0 + k < n ? in[i0 + k] : 0;
       sum += v[k];
     }
-    int32_t incl = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= o) incl += t;
-    }
-    if (lane == 31) warp_sums[warp] = incl;
-    __syncthreads();
-    if (warp == 0) {
-      int32_t w = warp_sums[lane];
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const int32_t t = __shfl_up_sync(0xffffffffu, w, o);
-        if (lane >= o) w += t;
-      }
-      warp_sums[lane] = w;
-    }
-    __syncthreads();
-    int32_t excl = carry + (warp ? warp_sums[warp - 1] : 0) + incl - sum;
+    int32_t excl = carry + cta_exclusive_scan(sum, warp_sums);
 #pragma unroll
     for (int k = 0; k < kScanItems; ++k) {
-      if (i0 + k < n) {
-        out[i0 + k] = excl;
-        if (out_copy) out_copy[i0 + k] = excl;
-      }
+      if (i0 + k < n) out[i0 + k] = excl;
       excl += v[k];
     }
     __syncthreads();
-    if (threadIdx.x == 0) carry += warp_sums[31];
+    if (threadIdx.x == blockDim.x - 1) carry = excl;  // the last thread's end = the running total
     __syncthreads();
   }
   if (threadIdx.x == 0 && last == n) {
@@ -309,14 +314,14 @@ __global__ void __launch_bounds__(1024) scan_tile_sums_kernel(const int32_t* __r
 cudaError_t device_exclusive_scan(const int32_t* in, int64_t n, int32_t* out, int32_t* tile_ws, cudaStream_t st) {
   const int64_t tiles = (n + kScanTile - 1) / kScanTile;
   if (tiles <= 2 || !tile_ws) {
-    exclusive_scan_kernel<<<1, 1024, 0, st>>>(in, n, out, nullptr, nullptr, nullptr);
+    exclusive_scan_kernel<<<1, 1024, 0, st>>>(in, n, out, nullptr, nullptr);
     return cudaGetLastError();
   }
   int32_t* sums = tile_ws;
   int32_t* seeds = tile_ws + tiles + 1;
   scan_tile_sums_kernel<<<static_cast<unsigned>(tiles), 1024, 0, st>>>(in, n, sums);
-  exclusive_scan_kernel<<<1, 1024, 0, st>>>(sums, tiles, seeds, nullptr, nullptr, nullptr);
-  exclusive_scan_kernel<<<static_cast<unsigned>(tiles), 1024, 0, st>>>(in, n, out, nullptr, nullptr, seeds);
+  exclusive_scan_kernel<<<1, 1024, 0, st>>>(sums, tiles, seeds, nullptr, nullptr);
+  exclusive_scan_kernel<<<static_cast<unsigned>(tiles), 1024, 0, st>>>(in, n, out, nullptr, seeds);
   return cudaGetLastError();
 }
 
@@ -369,6 +374,65 @@ __device__ __forceinline__ void for_each_vote(uint32_t base, const Bins4& bins, 
   }
 }
 
+// The steps both forms of a space's vote share.  s_counts: [0] n_bins, [1] n_votes, [2] rec_base,
+// [3] vote_base, [4] rec_cur, [5] vote_cur, [6] ok.
+//
+// After phase A: the CTA's bins and votes (each thread's my_bins / my_votes) reserve one range of records and
+// one of members.  False (and counters[3] set) if either would pass its capacity.
+__device__ __forceinline__ bool reserve_space(const VoteArgs& a, int my_bins, int my_votes, int* s_counts) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    my_bins += __shfl_xor_sync(0xffffffffu, my_bins, o);
+    my_votes += __shfl_xor_sync(0xffffffffu, my_votes, o);
+  }
+  if ((threadIdx.x & 31) == 0 && my_votes) {
+    atomicAdd(&s_counts[0], my_bins);
+    atomicAdd(&s_counts[1], my_votes);
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    s_counts[2] = atomicAdd(&a.counters[0], s_counts[0]);
+    s_counts[3] = atomicAdd(&a.counters[1], s_counts[1]);
+    s_counts[6] = (static_cast<int64_t>(s_counts[2]) + s_counts[0] <= a.cap_bins) &&
+                  (static_cast<int64_t>(s_counts[3]) + s_counts[1] <= a.cap_votes);
+    if (!s_counts[6]) a.counters[3] = 1;
+  }
+  __syncthreads();
+  return s_counts[6] != 0;
+}
+
+// Phase B for one match: each vote that created its bin emits the bin record and turns the bin's counter
+// into the offset of its members.
+__device__ __forceinline__ void emit_created_bins(const VoteArgs& a, uint32_t* hist, int64_t g, uint32_t base,
+                                                  const Bins4& bins, unsigned created, const int& rec_base,
+                                                  const int& vote_base, int* s_counts) {
+  for_each_vote(base, bins, [&](int o, int code) {
+    if (!(created >> o & 1u)) return;
+    const int cnt = static_cast<int>(hist[code]);
+    const int rec = rec_base + atomicAdd(&s_counts[4], 1);
+    const int off = vote_base + atomicAdd(&s_counts[5], cnt);
+    SOD_DCHECK(rec < a.cap_bins && static_cast<int64_t>(off) + cnt <= a.cap_votes);
+    a.bin_group[rec] = static_cast<int32_t>(g);
+    a.bin_code[rec] = code;
+    a.bin_count[rec] = cnt;
+    a.bin_offset[rec] = off;
+    hist[code] = static_cast<uint32_t>(off);
+  });
+}
+
+// Phase C for one vote: match m at the bin's offset + the vote's arrival rank r.
+__device__ __forceinline__ void store_member(const VoteArgs& a, const uint32_t* hist, int code, uint32_t r, int m) {
+  SOD_DCHECK(static_cast<int64_t>(hist[code]) + r < a.cap_votes);
+  a.members_raw[hist[code] + r] = m;
+}
+
+// Phase D for one match: the bins it created get their counters back to zero.
+__device__ __forceinline__ void clear_created_bins(uint32_t* hist, uint32_t base, const Bins4& bins, unsigned created) {
+  for_each_vote(base, bins, [&](int o, int code) {
+    if (created >> o & 1u) hist[code] = 0u;
+  });
+}
+
 // One Hough space: the four phases over the matches [beg, end) of the space.  kWide: arrival ranks as
 // 32-bit values (spaces of more than 65,535 matches), else packed 16-bit pairs (half the traffic).
 //  A  every vote takes the next rank of its bin: ONE shared-memory atomic per vote; rank 0 created the bin.
@@ -380,10 +444,9 @@ __device__ __forceinline__ void for_each_vote(uint32_t base, const Bins4& bins, 
 template <bool kWide>
 __device__ __forceinline__ void vote_space(const VoteArgs& a, uint32_t* hist, int64_t g, int beg, int end,
                                            int* s_counts) {
-  // s_counts: [0] n_bins, [1] n_votes, [2] rec_base, [3] vote_base, [4] rec_cur, [5] vote_cur, [6] ok
   constexpr int kWords = kWide ? 16 : 8;  // 32-bit words of rank storage per match
   const Bins4 bins = a.bins;
-  const int tid = threadIdx.x, lane = tid & 31;
+  const int tid = threadIdx.x;
   if (tid == 0) s_counts[0] = s_counts[1] = s_counts[4] = s_counts[5] = 0;
   __syncthreads();
   int my_bins = 0, my_votes = 0;
@@ -407,42 +470,13 @@ __device__ __forceinline__ void vote_space(const VoteArgs& a, uint32_t* hist, in
     a.creator[p] = static_cast<uint16_t>(created);
     my_bins += __popc(created);
   }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    my_bins += __shfl_xor_sync(0xffffffffu, my_bins, o);
-    my_votes += __shfl_xor_sync(0xffffffffu, my_votes, o);
-  }
-  if (lane == 0 && my_votes) {
-    atomicAdd(&s_counts[0], my_bins);
-    atomicAdd(&s_counts[1], my_votes);
-  }
-  __syncthreads();
-  if (tid == 0) {
-    s_counts[2] = atomicAdd(&a.counters[0], s_counts[0]);
-    s_counts[3] = atomicAdd(&a.counters[1], s_counts[1]);
-    s_counts[6] = (static_cast<int64_t>(s_counts[2]) + s_counts[0] <= a.cap_bins) &&
-                  (static_cast<int64_t>(s_counts[3]) + s_counts[1] <= a.cap_votes);
-    if (!s_counts[6]) a.counters[3] = 1;
-  }
-  __syncthreads();
-  const bool ok = s_counts[6] != 0;
+  const bool ok = reserve_space(a, my_bins, my_votes, s_counts);
   const int rec_base = s_counts[2], vote_base = s_counts[3];
   if (ok) {
     for (int p = beg + tid; p < end; p += kVoteThreads) {
       const unsigned created = a.creator[p];
       if (!created) continue;
-      for_each_vote(a.base_bin[p], bins, [&](int o, int code) {
-        if (!(created >> o & 1u)) return;
-        const int cnt = static_cast<int>(hist[code]);
-        const int rec = rec_base + atomicAdd(&s_counts[4], 1);
-        const int off = vote_base + atomicAdd(&s_counts[5], cnt);
-        SOD_DCHECK(rec < a.cap_bins && static_cast<int64_t>(off) + cnt <= a.cap_votes);
-        a.bin_group[rec] = static_cast<int32_t>(g);
-        a.bin_code[rec] = code;
-        a.bin_count[rec] = cnt;
-        a.bin_offset[rec] = off;
-        hist[code] = static_cast<uint32_t>(off);
-      });
+      emit_created_bins(a, hist, g, a.base_bin[p], bins, created, rec_base, vote_base, s_counts);
     }
   }
   __syncthreads();
@@ -457,9 +491,7 @@ __device__ __forceinline__ void vote_space(const VoteArgs& a, uint32_t* hist, in
         rk[4 * i] = v.x; rk[4 * i + 1] = v.y; rk[4 * i + 2] = v.z; rk[4 * i + 3] = v.w;
       }
       for_each_vote(a.base_bin[p], bins, [&](int o, int code) {
-        const uint32_t r = kWide ? rk[o] : (rk[o >> 1] >> ((o & 1) * 16)) & 0xFFFFu;
-        SOD_DCHECK(static_cast<int64_t>(hist[code]) + r < a.cap_votes);
-        a.members_raw[hist[code] + r] = m;
+        store_member(a, hist, code, kWide ? rk[o] : (rk[o >> 1] >> ((o & 1) * 16)) & 0xFFFFu, m);
       });
     }
   }
@@ -467,9 +499,7 @@ __device__ __forceinline__ void vote_space(const VoteArgs& a, uint32_t* hist, in
   for (int p = beg + tid; p < end; p += kVoteThreads) {
     const unsigned created = a.creator[p];
     if (!created) continue;
-    for_each_vote(a.base_bin[p], bins, [&](int o, int code) {
-      if (created >> o & 1u) hist[code] = 0u;
-    });
+    clear_created_bins(hist, a.base_bin[p], bins, created);
   }
   __syncthreads();
 }
@@ -481,7 +511,7 @@ __device__ __forceinline__ void vote_space(const VoteArgs& a, uint32_t* hist, in
 __device__ __forceinline__ void vote_space_small(const VoteArgs& a, uint32_t* hist, int64_t g, int beg, int end,
                                                  int* s_counts) {
   const Bins4 bins = a.bins;
-  const int tid = threadIdx.x, lane = tid & 31;
+  const int tid = threadIdx.x;
   const int p = beg + tid;
   const bool have = p < end;
   if (tid == 0) s_counts[0] = s_counts[1] = s_counts[4] = s_counts[5] = 0;
@@ -502,55 +532,17 @@ __device__ __forceinline__ void vote_space_small(const VoteArgs& a, uint32_t* hi
       ++my_votes;
     });
   }
-  int my_bins = __popc(created);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    my_bins += __shfl_xor_sync(0xffffffffu, my_bins, o);
-    my_votes += __shfl_xor_sync(0xffffffffu, my_votes, o);
-  }
-  if (lane == 0 && my_votes) {
-    atomicAdd(&s_counts[0], my_bins);
-    atomicAdd(&s_counts[1], my_votes);
-  }
-  __syncthreads();
-  if (tid == 0) {
-    s_counts[2] = atomicAdd(&a.counters[0], s_counts[0]);
-    s_counts[3] = atomicAdd(&a.counters[1], s_counts[1]);
-    s_counts[6] = (static_cast<int64_t>(s_counts[2]) + s_counts[0] <= a.cap_bins) &&
-                  (static_cast<int64_t>(s_counts[3]) + s_counts[1] <= a.cap_votes);
-    if (!s_counts[6]) a.counters[3] = 1;
-  }
-  __syncthreads();
-  const bool ok = s_counts[6] != 0;
+  const bool ok = reserve_space(a, __popc(created), my_votes, s_counts);
   const int rec_base = s_counts[2], vote_base = s_counts[3];
-  if (ok && created) {
-    for_each_vote(base, bins, [&](int o, int code) {
-      if (!(created >> o & 1u)) return;
-      const int cnt = static_cast<int>(hist[code]);
-      const int rec = rec_base + atomicAdd(&s_counts[4], 1);
-      const int off = vote_base + atomicAdd(&s_counts[5], cnt);
-      SOD_DCHECK(rec < a.cap_bins && static_cast<int64_t>(off) + cnt <= a.cap_votes);
-      a.bin_group[rec] = static_cast<int32_t>(g);
-      a.bin_code[rec] = code;
-      a.bin_count[rec] = cnt;
-      a.bin_offset[rec] = off;
-      hist[code] = static_cast<uint32_t>(off);
-    });
-  }
+  if (ok && created) emit_created_bins(a, hist, g, base, bins, created, rec_base, vote_base, s_counts);
   __syncthreads();
   if (ok && have) {
     for_each_vote(base, bins, [&](int o, int code) {
-      const uint32_t r = (rk[o >> 1] >> ((o & 1) * 16)) & 0xFFFFu;
-      SOD_DCHECK(static_cast<int64_t>(hist[code]) + r < a.cap_votes);
-      a.members_raw[hist[code] + r] = m;
+      store_member(a, hist, code, (rk[o >> 1] >> ((o & 1) * 16)) & 0xFFFFu, m);
     });
   }
   __syncthreads();
-  if (created) {
-    for_each_vote(base, bins, [&](int o, int code) {
-      if (created >> o & 1u) hist[code] = 0u;
-    });
-  }
+  if (created) clear_created_bins(hist, base, bins, created);
   __syncthreads();
 }
 
@@ -853,25 +845,7 @@ __global__ void __launch_bounds__(kHugeThreads, 1) hough_finish_huge_kernel(cons
       int mine = 0;
 #pragma unroll 4
       for (int k = 0; k < kPer; ++k) mine += __popc(bitmap[tid * kPer + k]);
-      int incl = mine;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const int v = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += v;
-      }
-      if (lane == 31) s_warp_tot[warp] = incl;
-      __syncthreads();
-      if (warp == 0) {
-        int wv = s_warp_tot[lane], wi = wv;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-          const int v = __shfl_up_sync(0xffffffffu, wi, o);
-          if (lane >= o) wi += v;
-        }
-        s_warp_tot[lane] = wi - wv;  // exclusive
-      }
-      __syncthreads();
-      int pos = s_base + s_warp_tot[warp] + incl - mine;
+      int pos = s_base + cta_exclusive_scan(mine, s_warp_tot);
       for (int k = 0; k < kPer; ++k) {
         uint32_t word = bitmap[tid * kPer + k];
         while (word) {
@@ -935,13 +909,8 @@ compact_write_kernel(const int32_t* __restrict__ idx, const uint8_t* __restrict_
   if (lane == 0) warp_base[warp] = __popc(b);
   __syncthreads();
   if (warp == 0) {
-    int v = warp_base[lane], incl = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int t = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= o) incl += t;
-    }
-    warp_base[lane] = incl - v;
+    const int v = warp_base[lane];
+    warp_base[lane] = warp_inclusive_scan(v) - v;
   }
   __syncthreads();
   if (keep) {
@@ -1029,7 +998,7 @@ int sod_compact_matches(const int32_t* idx, const uint8_t* pass, int64_t n_query
   compact_count_kernel<<<static_cast<unsigned>(blocks), kCompactThreads, 0, st>>>(idx, pass, n_query, t_lo,
                                                                                   t_hi, counts);
   SOD_CHECK_LAUNCH("compact_count_kernel");
-  exclusive_scan_kernel<<<1, 1024, 0, st>>>(counts, blocks, offs, nullptr, n_out, nullptr);
+  exclusive_scan_kernel<<<1, 1024, 0, st>>>(counts, blocks, offs, n_out, nullptr);
   SOD_CHECK_LAUNCH("exclusive_scan_kernel");
   compact_write_kernel<<<static_cast<unsigned>(blocks), kCompactThreads, 0, st>>>(
       idx, pass, n_query, t_lo, t_hi, offs, match_q, match_t);

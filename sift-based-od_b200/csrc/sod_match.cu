@@ -611,20 +611,15 @@ __global__ void top2_merge_kernel(const int32_t* __restrict__ parts_idx,
   write_top2_row(row, i1, d1, i2, d2, out_idx, out_d2, out_dist, out_pass, ratio);
 }
 
-// K3, exchange form.  A candidate as one signed 64-bit key (d2 << 32 | global row): signed order is the
-// (distance, index) order of the merge.  No entry: kNoneKey.  Keys travel as [row][2] pairs, so a
+// K3, exchange form: candidate lists as packed keys (sod_top2.cuh).  Keys travel as [row][2] pairs, so a
 // contiguous range of query rows is a contiguous message.
 __global__ void top2_keys_kernel(const int32_t* __restrict__ idx, const uint32_t* __restrict__ d2, int64_t nq,
                                  int64_t n_rows, longlong2* __restrict__ keys) {
   const int64_t row = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (row >= n_rows) return;
   longlong2 k = make_longlong2(kNoneKey, kNoneKey);  // rows past nq: padding up to a whole number of slices
-  if (row < nq) {
-    const int2 ci = *reinterpret_cast<const int2*>(idx + row * 2);
-    const uint2 cd = *reinterpret_cast<const uint2*>(d2 + row * 2);
-    if (ci.x >= 0) k.x = (static_cast<long long>(cd.x) << 32) | static_cast<uint32_t>(ci.x);
-    if (ci.y >= 0) k.y = (static_cast<long long>(cd.y) << 32) | static_cast<uint32_t>(ci.y);
-  }
+  if (row < nq)
+    k = top2_pack_keys(*reinterpret_cast<const int2*>(idx + row * 2), *reinterpret_cast<const uint2*>(d2 + row * 2));
   keys[row] = k;
 }
 
@@ -635,16 +630,7 @@ __global__ void top2_merge_keys_kernel(const longlong2* __restrict__ parts, int 
   const int64_t row = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (row >= n_rows) return;
   long long k1 = kNoneKey, k2 = kNoneKey;
-  for (int p = 0; p < n_parts; ++p) {
-    const longlong2 c = parts[static_cast<int64_t>(p) * n_rows + row];
-    // c.x <= c.y: at most c.x and c.y enter, in this order
-    if (c.x < k1) {
-      k2 = min(k1, c.y);
-      k1 = c.x;
-    } else if (c.x < k2) {
-      k2 = c.x;
-    }
-  }
+  for (int p = 0; p < n_parts; ++p) top2_fold_keys(k1, k2, parts[static_cast<int64_t>(p) * n_rows + row]);
   out[row] = make_longlong2(k1, k2);
 }
 
@@ -654,11 +640,7 @@ __global__ void top2_from_keys_kernel(const longlong2* __restrict__ keys, int64_
   const int64_t row = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (row >= nq) return;
   const longlong2 k = keys[row];
-  const bool h1 = k.x != kNoneKey, h2 = k.y != kNoneKey;
-  write_top2_row(row, h1 ? static_cast<int32_t>(k.x & 0xFFFFFFFFll) : -1,
-                 h1 ? static_cast<uint32_t>(k.x >> 32) : 0xFFFFFFFFu,
-                 h2 ? static_cast<int32_t>(k.y & 0xFFFFFFFFll) : -1,
-                 h2 ? static_cast<uint32_t>(k.y >> 32) : 0xFFFFFFFFu, out_idx, out_d2, out_dist, out_pass, ratio);
+  write_top2_keys_row(row, k.x, k.y, out_idx, out_d2, out_dist, out_pass, ratio);
 }
 
 struct Plan {
