@@ -430,8 +430,46 @@ int sod_sift_describe(const uint8_t* gray, int32_t width, int32_t height, int64_
 
 /* Byte offset in the workspace of Gaussian level `level` (0..5) of `octave` (-1 = the doubled image) after
  * sod_sift_extract / sod_sift_describe, f32 rows of wh_host[0] (HOST, may be NULL) values, wh_host[1] rows.
- * -1 if the image has no such level.  Lets a caller check the pyramid against cv2. */
+ * -1 if the image has no such level.  Lets a caller check the pyramid against cv2.  After
+ * sod_sift_extract_batch the same level of frame f lies f x sod_sift_batch_workspace_bytes(w, h, 1, 0) bytes
+ * further on (one frame's pyramid, 256-byte aligned). */
 int64_t sod_sift_level_offset(int32_t width, int32_t height, int32_t octave, int32_t level, int32_t* wh_host);
+
+/* ---- SIFT over a batch of same-size frames in one pass.  Every stage runs once for all frames (one launch per
+ * pyramid level), and the rows come out packed frame after frame, already in the layout the detection path
+ * takes (des, xy, angle, octave and the frame of each row). */
+#define SOD_SIFT_MAX_FRAMES 4096
+
+typedef struct {
+  float* xy;              /* [cap_rows][2] KeyPoint.pt */
+  float* size;            /* [cap_rows] */
+  float* angle;           /* [cap_rows] degrees in [0,360) */
+  float* response;        /* [cap_rows] */
+  int32_t* octave;        /* [cap_rows] */
+  uint8_t* des;           /* [cap_rows][128] */
+  int32_t* frame;         /* [cap_rows] frame (0..frames-1) of each row */
+  int32_t* count;         /* [frames] keypoints of each frame (after max_per_frame) */
+  int32_t* offset;        /* [frames] first row of each frame: frame f is rows [offset[f], offset[f] + count[f]) */
+  int32_t* overflow;      /* [frames] 1 = the frame had more than cap_per_frame keypoints before duplicate removal:
+                             its rows are incomplete and must not be used */
+  int32_t* rows_overflow; /* [1] 1 = the packed rows exceed cap_rows: rows from cap_rows on were dropped */
+  int64_t cap_rows;       /* 1..SOD_SIFT_MAX_CAP */
+  int64_t cap_per_frame;  /* keypoints one frame may produce before duplicate removal; frames x cap_per_frame
+                             <= SOD_SIFT_MAX_CAP */
+} sod_sift_batch_out;
+
+/* Bytes of workspace (256-byte aligned) for `frames` images of this size and cap_per_frame = out.cap_per_frame;
+ * 0 if an argument is out of range.  At least frames x the pyramid of one frame. */
+size_t sod_sift_batch_workspace_bytes(int32_t width, int32_t height, int32_t frames, int64_t cap_per_frame);
+
+/* sod_sift_extract of `frames` u8 gray images of one size (image f at gray + f x frame_stride, rows `pitch`
+ * bytes apart, frame_stride >= pitch x height).  Frame f's rows are the first max_per_frame (0 = all) keypoints
+ * sod_sift_extract gives for that image alone, in the same order; count, offset and every row are written on
+ * the device, so the call never synchronises and can be captured in a CUDA graph.  Nothing is truncated
+ * silently: overflow[f] and rows_overflow say when rows are missing. */
+int sod_sift_extract_batch(const uint8_t* gray, int32_t width, int32_t height, int64_t pitch, int64_t frame_stride,
+                           int32_t frames, int64_t max_per_frame, const sod_sift_batch_out* out, void* workspace,
+                           size_t workspace_bytes, sod_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -15,6 +15,13 @@
 //   order       cub radix sort by (x, y), short runs of equal (x, y) ordered by (size, angle, response,
 //               octave), entries equal in (pt, size, angle) dropped: cv2's KeyPointsFilter order.
 //   descriptor  one block per keypoint, 4x4x8 histogram with trilinear spreading, clip 0.2, x512, u8.
+//
+// Every kernel has a frame dimension: a batch of B same-size images is one launch per pyramid level and one per
+// stage.  Frame f has its own pyramid (at f x the pyramid of one frame in the workspace), its own counters and
+// its own candidate / keypoint slabs of cap entries.  The order is per frame: the (x, y) sort over all slabs is
+// followed, for B > 1, by a stable sort by frame, so each frame's slab ends up in the order one frame alone
+// gets.  sod_sift_extract is the batch of one.
+#include <cub/block/block_scan.cuh>
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
@@ -46,9 +53,12 @@ constexpr int kOriWarps = 4;
 struct Pyramid {
   float* base;
   int64_t off[kMaxOct];                // element offset of octave o's first level
+  int64_t fstride;                     // elements from one frame's pyramid to the next
   int w[kMaxOct], h[kMaxOct];
   int n_oct;
-  __host__ __device__ float* level(int o, int l) const { return base + off[o] + (int64_t)l * w[o] * h[o]; }
+  __host__ __device__ float* level(int o, int l, int f = 0) const {
+    return base + f * fstride + off[o] + (int64_t)l * w[o] * h[o];
+  }
 };
 
 struct Taps {
@@ -58,7 +68,7 @@ struct Taps {
 
 struct Cand {                          // a refined extremum, before orientation (octave index o is 0-based)
   float x, y, size, response;
-  int32_t octave, o, layer, r, c;
+  int32_t octave, o, layer, r, c, frame;
 };
 
 struct Kp {                            // a finished keypoint in cv2's conventions (first octave -1)
@@ -66,11 +76,19 @@ struct Kp {                            // a finished keypoint in cv2's conventio
   int32_t octave;
 };
 
-// Workspace layout (byte offsets from the workspace start, every block 256-byte aligned).  The pyramid comes
-// first so that sod_sift_level_offset does not depend on the keypoint capacity.
+// Per-frame counters: candidates, keypoints, overflow flag, unused.  After them, kBatchInts ints of the batch:
+// [0] rows written (the descriptor count).
+constexpr int kFrameInts = 4;
+constexpr int kBatchInts = 4;
+
+// Workspace layout (byte offsets from the workspace start, every block 256-byte aligned).  The pyramids come
+// first so that sod_sift_level_offset (frame 0) does not depend on the keypoint capacity or the batch.  Slabs
+// hold frames x cap entries, frame f's at f x cap.
 struct Plan {
   Pyramid pyr;
-  size_t cand, raw, keys_in, keys_out, vals_in, vals_out, keep, pos, counters, cub_tmp, cub_bytes, total;
+  int frames;
+  int64_t cap;
+  size_t cand, raw, keys_in, keys_out, vals_in, vals_out, keep, pos, counters, offset, cub_tmp, cub_bytes, total;
 };
 
 size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
@@ -81,8 +99,9 @@ int octave_count(int width, int height) {
   return (int)std::lrint(std::log(m) / std::log(2.0) - 2.0) + 1;
 }
 
-// Pyramid geometry and workspace offsets; cap = 0 plans the pyramid alone (sod_sift_describe).
-bool make_plan(int width, int height, int64_t cap, Plan* p) {
+// Pyramid geometry and workspace offsets for `frames` images and cap keypoints a frame; cap = 0 plans the
+// pyramids alone (sod_sift_describe).  frames x cap <= SOD_SIFT_MAX_CAP is the caller's check.
+bool make_plan(int width, int height, int frames, int64_t cap, Plan* p) {
   int n_oct = octave_count(width, height);
   if (n_oct < 0) n_oct = 0;
   if (n_oct > kMaxOct) return false;
@@ -100,24 +119,34 @@ bool make_plan(int width, int height, int64_t cap, Plan* p) {
       h /= 2;
     }
   }
-  size_t at = align256((size_t)off * sizeof(float));
+  const size_t pyr_bytes = align256((size_t)off * sizeof(float));
+  p->pyr.fstride = (int64_t)(pyr_bytes / sizeof(float));
+  p->frames = frames;
+  p->cap = cap;
+  const int64_t slots = frames * cap;
+  size_t at = pyr_bytes * frames;
   auto take = [&](size_t bytes) { size_t r = at; at += align256(bytes); return r; };
-  p->cand = take(sizeof(Cand) * cap);
-  p->raw = take(sizeof(Kp) * cap);
-  p->keys_in = take(sizeof(uint64_t) * cap);
-  p->keys_out = take(sizeof(uint64_t) * cap);
-  p->vals_in = take(sizeof(int32_t) * cap);
-  p->vals_out = take(sizeof(int32_t) * cap);
-  p->keep = take(sizeof(int32_t) * cap);
-  p->pos = take(sizeof(int32_t) * cap);
-  p->counters = take(sizeof(int32_t) * 4);
-  size_t sort_bytes = 0, scan_bytes = 0;
-  if (cap > 0) {
+  p->cand = take(sizeof(Cand) * slots);
+  p->raw = take(sizeof(Kp) * slots);
+  p->keys_in = take(sizeof(uint64_t) * slots);      // for B > 1 also the frame keys of the second sort (2 x u32)
+  p->keys_out = take(sizeof(uint64_t) * slots);
+  p->vals_in = take(sizeof(int32_t) * slots);
+  p->vals_out = take(sizeof(int32_t) * slots);
+  p->keep = take(sizeof(int32_t) * slots);
+  p->pos = take(sizeof(int32_t) * slots);
+  p->counters = take(slots > 0 ? sizeof(int32_t) * (kFrameInts * frames + kBatchInts) : 0);
+  p->offset = take(slots > 0 ? sizeof(int32_t) * frames : 0);
+  size_t sort_bytes = 0, frame_sort_bytes = 0, scan_bytes = 0;
+  if (slots > 0) {
     cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, (const uint64_t*)nullptr, (uint64_t*)nullptr,
-                                    (const int32_t*)nullptr, (int32_t*)nullptr, (int)cap);
-    cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const int32_t*)nullptr, (int32_t*)nullptr, (int)cap);
+                                    (const int32_t*)nullptr, (int32_t*)nullptr, (int)slots);
+    if (frames > 1)
+      cub::DeviceRadixSort::SortPairs(nullptr, frame_sort_bytes, (const uint32_t*)nullptr, (uint32_t*)nullptr,
+                                      (const int32_t*)nullptr, (int32_t*)nullptr, (int)slots);
+    cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const int32_t*)nullptr, (int32_t*)nullptr, (int)slots);
   }
   p->cub_bytes = sort_bytes > scan_bytes ? sort_bytes : scan_bytes;
+  if (frame_sort_bytes > p->cub_bytes) p->cub_bytes = frame_sort_bytes;
   p->cub_tmp = take(p->cub_bytes);
   p->total = at;
   return true;
@@ -171,11 +200,14 @@ __device__ __forceinline__ float fast_atan2(float y, float x) {
 }
 
 // cv::resize(INTER_LINEAR) to exactly twice the size: source coordinate (d + 0.5) / 2 - 0.5, clamped.
+// blockIdx.z = frame: its image at z x frame_stride bytes, its output at z x dst_stride elements.
 __global__ void sift_upsample_kernel(const uint8_t* __restrict__ src, int sw, int sh, int64_t pitch,
-                                     float* __restrict__ dst) {
+                                     int64_t frame_stride, float* __restrict__ dst, int64_t dst_stride) {
   const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
   const int dw = 2 * sw, dh = 2 * sh;
   if (x >= dw || y >= dh) return;
+  src += blockIdx.z * frame_stride;
+  dst += blockIdx.z * dst_stride;
   float fx = (float)((x + 0.5) * 0.5 - 0.5), fy = (float)((y + 0.5) * 0.5 - 0.5);
   int sx = (int)floorf(fx), sy = (int)floorf(fy);
   fx -= sx;
@@ -194,12 +226,15 @@ __global__ void sift_upsample_kernel(const uint8_t* __restrict__ src, int sw, in
 
 // cv::GaussianBlur on a float image: horizontal pass into shared memory, then the vertical pass, both in the
 // symmetric form of OpenCV's row / column filters (centre tap, then pairs outwards), BORDER_REFLECT_101.
+// blockIdx.z = frame, fstride elements apart.
 __global__ void __launch_bounds__(256) sift_blur_kernel(const float* __restrict__ src, float* __restrict__ dst,
-                                                       int w, int h, Taps t) {
+                                                       int w, int h, Taps t, int64_t fstride) {
   __shared__ float in[kTile + 2 * kMaxRadius][kTile + 2 * kMaxRadius + 1];
   __shared__ float mid[kTile + 2 * kMaxRadius][kTile + 1];
   __shared__ float k[2 * kMaxRadius + 1];
   const int r = t.r, x0 = blockIdx.x * kTile, y0 = blockIdx.y * kTile, span = kTile + 2 * r;
+  src += blockIdx.z * fstride;
+  dst += blockIdx.z * fstride;
   if (threadIdx.x < 2 * r + 1) k[threadIdx.x] = t.k[threadIdx.x];
   for (int i = threadIdx.x; i < span * span; i += blockDim.x) {
     const int ty = i / span, tx = i - ty * span;
@@ -225,29 +260,30 @@ __global__ void __launch_bounds__(256) sift_blur_kernel(const float* __restrict_
   }
 }
 
-// cv::resize(INTER_NEAREST) to half size: every other pixel.
-__global__ void sift_halve_kernel(const float* __restrict__ src, int sw, float* __restrict__ dst, int dw, int dh) {
+// cv::resize(INTER_NEAREST) to half size: every other pixel.  blockIdx.z = frame, fstride elements apart.
+__global__ void sift_halve_kernel(const float* __restrict__ src, int sw, float* __restrict__ dst, int dw, int dh,
+                                  int64_t fstride) {
   const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
   if (x >= dw || y >= dh) return;
-  dst[(int64_t)y * dw + x] = src[(int64_t)(2 * y) * sw + 2 * x];
+  dst[blockIdx.z * fstride + (int64_t)y * dw + x] = src[blockIdx.z * fstride + (int64_t)(2 * y) * sw + 2 * x];
 }
 
-// DoG level l of octave o at (r, c): G[l+1] - G[l], the value cv::subtract stores.
-__device__ __forceinline__ float dog(const Pyramid& P, int o, int l, int r, int c) {
+// DoG level l of octave o of frame f at (r, c): G[l+1] - G[l], the value cv::subtract stores.
+__device__ __forceinline__ float dog(const Pyramid& P, int f, int o, int l, int r, int c) {
   const int64_t i = (int64_t)r * P.w[o] + c;
-  return P.level(o, l + 1)[i] - P.level(o, l)[i];
+  return P.level(o, l + 1, f)[i] - P.level(o, l, f)[i];
 }
 
 // OpenCV's adjustLocalExtrema: Newton steps on the 3x3 Hessian of the DoG (derivatives scaled by 1/255),
 // contrast and edge tests, keypoint fields in the octave numbering of the doubled image.
-__device__ bool refine(const Pyramid& P, int o, int& layer, int& r, int& c, Cand* kp) {
+__device__ bool refine(const Pyramid& P, int f, int o, int& layer, int& r, int& c, Cand* kp) {
   constexpr float img_scale = 1.f / 255.f, deriv_scale = img_scale * 0.5f, second_scale = img_scale,
                   cross_scale = img_scale * 0.25f;
   const int w = P.w[o], h = P.h[o];
   float xi = 0, xr = 0, xc = 0;
   int i = 0;
   for (; i < kMaxInterp; ++i) {
-    auto D = [&](int dl, int dr, int dc) { return dog(P, o, layer + dl, r + dr, c + dc); };
+    auto D = [&](int dl, int dr, int dc) { return dog(P, f, o, layer + dl, r + dr, c + dc); };
     const float dx = (D(0, 0, 1) - D(0, 0, -1)) * deriv_scale, dy = (D(0, 1, 0) - D(0, -1, 0)) * deriv_scale,
                 ds = (D(1, 0, 0) - D(-1, 0, 0)) * deriv_scale;
     const float v2 = D(0, 0, 0) * 2;
@@ -280,7 +316,7 @@ __device__ bool refine(const Pyramid& P, int o, int& layer, int& r, int& c, Cand
       return false;
   }
   if (i >= kMaxInterp) return false;
-  auto D = [&](int dl, int dr, int dc) { return dog(P, o, layer + dl, r + dr, c + dc); };
+  auto D = [&](int dl, int dr, int dc) { return dog(P, f, o, layer + dl, r + dr, c + dc); };
   const float dx = (D(0, 0, 1) - D(0, 0, -1)) * deriv_scale, dy = (D(0, 1, 0) - D(0, -1, 0)) * deriv_scale,
               ds = (D(1, 0, 0) - D(-1, 0, 0)) * deriv_scale;
   const float t = dx * xc + dy * xr + ds * xi;
@@ -302,56 +338,61 @@ __device__ bool refine(const Pyramid& P, int o, int& layer, int& r, int& c, Cand
 }
 
 // Scale-space extrema of octave o: |DoG| > floor(0.5 * 0.04 / 3 * 255) = 1, not smaller (or not larger)
-// than all 26 neighbours, outside the 5-pixel border; refined survivors are appended to cand.
+// than all 26 neighbours, outside the 5-pixel border; refined survivors are appended to their frame's slab of
+// cand.  blockIdx.z = frame * kLayers + layer - 1.
 __global__ void sift_extrema_kernel(Pyramid P, int o, Cand* __restrict__ cand, int cap, int* __restrict__ counters) {
   const int c = kBorder + blockIdx.x * blockDim.x + threadIdx.x;
   const int r = kBorder + blockIdx.y * blockDim.y + threadIdx.y;
-  const int layer = 1 + blockIdx.z;
+  const int f = blockIdx.z / kLayers, layer = 1 + blockIdx.z % kLayers;
   if (c >= P.w[o] - kBorder || r >= P.h[o] - kBorder) return;
-  const float val = dog(P, o, layer, r, c);
+  const float val = dog(P, f, o, layer, r, c);
   if (!(fabsf(val) > 1.f)) return;
   bool ext = true;
   if (val > 0) {
     for (int dl = -1; dl <= 1 && ext; ++dl)
       for (int dr = -1; dr <= 1 && ext; ++dr)
         for (int dc = -1; dc <= 1; ++dc)
-          if ((dl | dr | dc) && !(val >= dog(P, o, layer + dl, r + dr, c + dc))) { ext = false; break; }
+          if ((dl | dr | dc) && !(val >= dog(P, f, o, layer + dl, r + dr, c + dc))) { ext = false; break; }
   } else {
     for (int dl = -1; dl <= 1 && ext; ++dl)
       for (int dr = -1; dr <= 1 && ext; ++dr)
         for (int dc = -1; dc <= 1; ++dc)
-          if ((dl | dr | dc) && !(val <= dog(P, o, layer + dl, r + dr, c + dc))) { ext = false; break; }
+          if ((dl | dr | dc) && !(val <= dog(P, f, o, layer + dl, r + dr, c + dc))) { ext = false; break; }
   }
   if (!ext) return;
   int l1 = layer, r1 = r, c1 = c;
   Cand kp;
-  if (!refine(P, o, l1, r1, c1, &kp)) return;
+  if (!refine(P, f, o, l1, r1, c1, &kp)) return;
   kp.o = o;
   kp.layer = l1;
   kp.r = r1;
   kp.c = c1;
-  const int slot = atomicAdd(&counters[0], 1);
+  kp.frame = f;
+  int* fc = counters + f * kFrameInts;
+  const int slot = atomicAdd(&fc[0], 1);
   if (slot >= cap) {
-    atomicExch(&counters[2], 1);
+    atomicExch(&fc[2], 1);
     return;
   }
   SOD_DCHECK(slot >= 0 && slot < cap);
-  cand[slot] = kp;
+  cand[(int64_t)f * cap + slot] = kp;
 }
 
-// OpenCV's calcOrientationHist + the peak loop of findScaleSpaceExtrema, one warp per candidate.  Every
-// keypoint is written already moved to the first octave -1 (octave byte - 1, pt and size halved).
+// OpenCV's calcOrientationHist + the peak loop of findScaleSpaceExtrema, one warp per candidate; blockIdx.y is
+// the frame whose slab the blocks walk.  Every keypoint is written to its frame's raw slab already moved to the
+// first octave -1 (octave byte - 1, pt and size halved).
 __global__ void __launch_bounds__(32 * kOriWarps) sift_orient_kernel(Pyramid P, const Cand* __restrict__ cand,
                                                                      int cap, int* __restrict__ counters,
                                                                      Kp* __restrict__ raw) {
   __shared__ float part[kOriWarps][32][kOriBins + 1];
   __shared__ float hist[kOriWarps][kOriBins + 4];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-  const int n = min(counters[0], cap);
+  int* fc = counters + blockIdx.y * kFrameInts;
+  const int n = min(fc[0], cap);
   for (int ci = blockIdx.x * kOriWarps + wib; ci < n; ci += gridDim.x * kOriWarps) {
-    const Cand k = cand[ci];
-    SOD_DCHECK(k.o >= 0 && k.o < P.n_oct && k.layer >= 1 && k.layer <= kLayers);
-    const float* img = P.level(k.o, k.layer);
+    const Cand k = cand[(int64_t)blockIdx.y * cap + ci];
+    SOD_DCHECK(k.o >= 0 && k.o < P.n_oct && k.layer >= 1 && k.layer <= kLayers && k.frame == (int)blockIdx.y);
+    const float* img = P.level(k.o, k.layer, k.frame);
     const int w = P.w[k.o], h = P.h[k.o];
     const float scl = k.size * 0.5f / (float)(1 << k.o);
     const int radius = __float2int_rn(4.5f * scl);
@@ -399,13 +440,13 @@ __global__ void __launch_bounds__(32 * kOriWarps) sift_orient_kernel(Pyramid P, 
           bin = bin < 0 ? kOriBins + bin : bin >= kOriBins ? bin - kOriBins : bin;
           float angle = 360.f - (float)((360.f / kOriBins) * bin);
           if (fabsf(angle - 360.f) < FLT_EPSILON) angle = 0.f;
-          const int slot = atomicAdd(&counters[1], 1);
+          const int slot = atomicAdd(&fc[1], 1);
           if (slot >= cap) {
-            atomicExch(&counters[2], 1);
+            atomicExch(&fc[2], 1);
             continue;
           }
           SOD_DCHECK(slot >= 0 && slot < cap);
-          Kp& o = raw[slot];
+          Kp& o = raw[(int64_t)k.frame * cap + slot];
           o.x = k.x * 0.5f;
           o.y = k.y * 0.5f;
           o.size = k.size * 0.5f;
@@ -419,14 +460,29 @@ __global__ void __launch_bounds__(32 * kOriWarps) sift_orient_kernel(Pyramid P, 
   }
 }
 
-// Sort keys: (x bits, y bits) of the non-negative coordinates order as (x, y); unused slots sort last.
+// Sort key: (x bits, y bits) of the non-negative coordinates order as (x, y).
+__device__ __forceinline__ uint64_t xy_key(const Kp& k) {
+  return ((uint64_t)__float_as_uint(k.x) << 32) | __float_as_uint(k.y);
+}
+
+// Keys of every slot of every frame's raw slab; unused slots sort last.
 __global__ void sift_sort_keys_kernel(const Kp* __restrict__ raw, const int* __restrict__ counters, int cap,
-                                      uint64_t* __restrict__ keys, int32_t* __restrict__ vals) {
+                                      int slots, uint64_t* __restrict__ keys, int32_t* __restrict__ vals) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= cap) return;
-  const int n = min(counters[1], cap);
-  keys[i] = i < n ? ((uint64_t)__float_as_uint(raw[i].x) << 32) | __float_as_uint(raw[i].y) : ~0ull;
+  if (i >= slots) return;
+  const int f = i / cap, n = min(counters[f * kFrameInts + 1], cap);
+  keys[i] = i - f * cap < n ? xy_key(raw[i]) : ~0ull;
   vals[i] = i;
+}
+
+// B > 1: the frame of each slot in (x, y) order, the key of the stable sort that gathers each frame's slots
+// into its slab again (in (x, y) order, unused slots last).
+__global__ void sift_frame_keys_kernel(const int32_t* __restrict__ vals, int cap, int slots,
+                                       uint32_t* __restrict__ fkeys) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= slots) return;
+  SOD_DCHECK(vals[i] >= 0 && vals[i] < slots);
+  fkeys[i] = (uint32_t)(vals[i] / cap);
 }
 
 __device__ __forceinline__ bool kp_less(const Kp& a, const Kp& b) {   // cv2's order after equal (x, y)
@@ -436,18 +492,23 @@ __device__ __forceinline__ bool kp_less(const Kp& a, const Kp& b) {   // cv2's o
   return a.octave < b.octave;
 }
 
-// Orders every run of equal (x, y) by (size, angle, response, octave); runs are a few keypoints long (the
-// orientations of one location), so the first thread of a run sorts it by insertion.
+// Orders every run of equal (x, y) inside a frame's slab by (size, angle, response, octave); runs are a few
+// keypoints long (the orientations of one location), so the first thread of a run sorts it by insertion.  The
+// other threads of a run only compare keys, which every entry of the run shares.
 __global__ void sift_sort_runs_kernel(const Kp* __restrict__ raw, const int* __restrict__ counters, int cap,
-                                      const uint64_t* __restrict__ keys, int32_t* __restrict__ vals) {
+                                      int slots, int32_t* __restrict__ vals) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  const int n = min(counters[1], cap);
-  if (i >= n || (i > 0 && keys[i - 1] == keys[i]) || i + 1 >= n || keys[i + 1] != keys[i]) return;
+  if (i >= slots) return;
+  const int f = i / cap, j = i - f * cap, n = min(counters[f * kFrameInts + 1], cap);
+  if (j + 1 >= n) return;
+  const uint64_t key = xy_key(raw[vals[i]]);
+  if ((j > 0 && xy_key(raw[vals[i - 1]]) == key) || xy_key(raw[vals[i + 1]]) != key) return;
+  const int end = f * cap + n;
   int e = i + 1;
-  while (e < n && keys[e] == keys[i]) ++e;
+  while (e < end && xy_key(raw[vals[e]]) == key) ++e;
   for (int a = i + 1; a < e; ++a) {
     const int v = vals[a];
-    SOD_DCHECK(v >= 0 && v < cap);
+    SOD_DCHECK(v >= f * cap && v < end);
     int b = a - 1;
     while (b >= i && kp_less(raw[v], raw[vals[b]])) {
       vals[b + 1] = vals[b];
@@ -459,16 +520,16 @@ __global__ void sift_sort_runs_kernel(const Kp* __restrict__ raw, const int* __r
 
 // KeyPointsFilter::removeDuplicatedSorted: keep an entry unless it equals its predecessor in pt, size and
 // angle (equal entries are adjacent in this order).
-__global__ void sift_keep_kernel(const Kp* __restrict__ raw, const int* __restrict__ counters, int cap,
+__global__ void sift_keep_kernel(const Kp* __restrict__ raw, const int* __restrict__ counters, int cap, int slots,
                                  const int32_t* __restrict__ vals, int32_t* __restrict__ keep) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= cap) return;
-  const int n = min(counters[1], cap);
+  if (i >= slots) return;
+  const int f = i / cap, j = i - f * cap, n = min(counters[f * kFrameInts + 1], cap);
   int k = 0;
-  if (i < n) {
+  if (j < n) {
     k = 1;
-    if (i > 0) {
-      SOD_DCHECK(vals[i] >= 0 && vals[i] < cap && vals[i - 1] >= 0 && vals[i - 1] < cap);
+    if (j > 0) {
+      SOD_DCHECK(vals[i] >= 0 && vals[i] < slots && vals[i - 1] >= 0 && vals[i - 1] < slots);
       const Kp a = raw[vals[i - 1]], b = raw[vals[i]];
       k = !(a.x == b.x && a.y == b.y && a.size == b.size && a.angle == b.angle);
     }
@@ -476,18 +537,63 @@ __global__ void sift_keep_kernel(const Kp* __restrict__ raw, const int* __restri
   keep[i] = k;
 }
 
-__global__ void sift_emit_kernel(const Kp* __restrict__ raw, const int* __restrict__ counters, int cap,
-                                 const int32_t* __restrict__ vals, const int32_t* __restrict__ keep,
-                                 const int32_t* __restrict__ pos, sod_sift_out out) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= cap) return;
-  if (i == cap - 1) {
-    out.counters[0] = pos[i] + keep[i];
-    out.counters[1] = counters[2];
+// Where the rows go.  count / offset / overflow have one entry per frame; frame and rows_overflow may be NULL.
+struct Rows {
+  float *xy, *size, *angle, *response;
+  int32_t* octave;
+  uint8_t* des;
+  int32_t *frame, *count, *offset, *overflow, *rows_overflow;
+  int64_t cap_rows;
+};
+
+// Per frame: the keypoints left after duplicate removal, capped at max_per_frame (0 = all), and where they start
+// when the frames are packed in batch order; the overflow flags; batch[0] = rows written.  One block.
+__global__ void __launch_bounds__(256) sift_frame_rows_kernel(const int32_t* __restrict__ keep,
+                                                              const int32_t* __restrict__ pos,
+                                                              const int* __restrict__ counters, int cap, int frames,
+                                                              int64_t max_per_frame, Rows out,
+                                                              int* __restrict__ batch) {
+  using Scan = cub::BlockScan<int, 256>;
+  __shared__ typename Scan::TempStorage tmp;
+  __shared__ int carry;
+  if (threadIdx.x == 0) carry = 0;
+  __syncthreads();
+  for (int f0 = 0; f0 < frames; f0 += 256) {
+    const int f = f0 + threadIdx.x;
+    int n = 0;
+    if (f < frames) {
+      const int last = (f + 1) * cap - 1;
+      n = pos[last] + keep[last] - pos[f * cap];
+      if (max_per_frame > 0 && n > max_per_frame) n = (int)max_per_frame;
+    }
+    int excl, total;
+    Scan(tmp).ExclusiveSum(n, excl, total);
+    if (f < frames) {
+      out.count[f] = n;
+      out.offset[f] = carry + excl;
+      out.overflow[f] = counters[f * kFrameInts + 2];
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) carry += total;
+    __syncthreads();
   }
-  if (!keep[i]) return;
-  const int p = pos[i], v = vals[i];
-  SOD_DCHECK(p >= 0 && p < cap && v >= 0 && v < cap);
+  if (threadIdx.x == 0) {
+    batch[0] = (int)min((int64_t)carry, out.cap_rows);
+    if (out.rows_overflow) out.rows_overflow[0] = carry > out.cap_rows;
+  }
+}
+
+// The first count[f] kept entries of each frame, at rows offset[f].. (rows past cap_rows are dropped and flagged).
+__global__ void sift_emit_kernel(const Kp* __restrict__ raw, int cap, int slots, const int32_t* __restrict__ vals,
+                                 const int32_t* __restrict__ keep, const int32_t* __restrict__ pos, Rows out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= slots || !keep[i]) return;
+  const int f = i / cap, local = pos[i] - pos[f * cap];
+  if (local >= out.count[f]) return;
+  const int64_t p = (int64_t)out.offset[f] + local;
+  if (p >= out.cap_rows) return;
+  const int v = vals[i];
+  SOD_DCHECK(p >= 0 && v >= f * cap && v < (f + 1) * cap);
   const Kp k = raw[v];
   out.xy[2 * p] = k.x;
   out.xy[2 * p + 1] = k.y;
@@ -495,15 +601,18 @@ __global__ void sift_emit_kernel(const Kp* __restrict__ raw, const int* __restri
   out.angle[p] = k.angle;
   out.response[p] = k.response;
   out.octave[p] = k.octave;
+  if (out.frame) out.frame[p] = f;
 }
 
 // OpenCV's calcDescriptors + calcSIFTDescriptor, one 128-thread block per keypoint.  n_dev (device, may be
-// NULL) overrides n.  A keypoint whose octave / layer names no level of the pyramid gets a zero row and is
-// counted in n_invalid (cv2 refuses such a keypoint).
-__global__ void __launch_bounds__(128) sift_descriptor_kernel(Pyramid P, const float* __restrict__ xy,
+// NULL) overrides n; frame (may be NULL = all 0) names each keypoint's pyramid.  A keypoint whose octave / layer
+// names no level of the pyramid gets a zero row and is counted in n_invalid (cv2 refuses such a keypoint).
+// 16 blocks an SM (32 registers): the grid below is 16 blocks an SM, one wave.
+__global__ void __launch_bounds__(128, 16) sift_descriptor_kernel(Pyramid P, const float* __restrict__ xy,
                                                               const float* __restrict__ size,
                                                               const float* __restrict__ angle,
-                                                              const int32_t* __restrict__ octave, int64_t n,
+                                                              const int32_t* __restrict__ octave,
+                                                              const int32_t* __restrict__ frame, int64_t n,
                                                               const int32_t* __restrict__ n_dev,
                                                               uint8_t* __restrict__ des, int32_t* n_invalid) {
   __shared__ float hist[kHistLen];
@@ -526,7 +635,9 @@ __global__ void __launch_bounds__(128) sift_descriptor_kernel(Pyramid P, const f
     const float ptx = xy[2 * q] * scale, pty = xy[2 * q + 1] * scale;
     float ori = 360.f - angle[q];
     if (fabsf(ori - 360.f) < FLT_EPSILON) ori = 0.f;
-    const float* img = P.level(o, layer);
+    const int f = frame ? frame[q] : 0;
+    SOD_DCHECK(f >= 0);
+    const float* img = P.level(o, layer, f);
     const int cols = P.w[o], rows = P.h[o];
     const int px = __float2int_rn(ptx), py = __float2int_rn(pty);
     float cos_t = cosf(ori * (float)(3.14159265358979323846 / 180)),
@@ -597,8 +708,9 @@ __global__ void __launch_bounds__(128) sift_descriptor_kernel(Pyramid P, const f
   }
 }
 
-// The Gaussian pyramid of one image into the workspace.
-int build_pyramid(const uint8_t* gray, int width, int height, int64_t pitch, const Pyramid& P, cudaStream_t st) {
+// The Gaussian pyramids of `frames` images (frame_stride bytes apart) into the workspace, one launch per level.
+int build_pyramid(const uint8_t* gray, int width, int height, int64_t pitch, int64_t frame_stride, int frames,
+                  const Pyramid& P, cudaStream_t st) {
   double sig[kLevels];
   const double k = std::pow(2., 1. / kLayers);
   for (int i = 1; i < kLevels; ++i) {
@@ -611,20 +723,91 @@ int build_pyramid(const uint8_t* gray, int width, int height, int64_t pitch, con
   for (int i = 1; i < kLevels; ++i)
     if (!gaussian_taps(sig[i], &taps[i])) return SOD_ERR_UNSUPPORTED;
   const dim3 pb(32, 8);
-  auto pgrid = [&](int w, int h) { return dim3((w + 31) / 32, (h + 7) / 8); };
-  auto tgrid = [&](int w, int h) { return dim3((w + kTile - 1) / kTile, (h + kTile - 1) / kTile); };
+  auto pgrid = [&](int w, int h) { return dim3((w + 31) / 32, (h + 7) / 8, frames); };
+  auto tgrid = [&](int w, int h) { return dim3((w + kTile - 1) / kTile, (h + kTile - 1) / kTile, frames); };
+  const int64_t fs = P.fstride;
   // the doubled image goes to level 1's slot, blurred into level 0, and level 1 is then computed over it
-  sift_upsample_kernel<<<pgrid(P.w[0], P.h[0]), pb, 0, st>>>(gray, width, height, pitch, P.level(0, 1));
-  sift_blur_kernel<<<tgrid(P.w[0], P.h[0]), 256, 0, st>>>(P.level(0, 1), P.level(0, 0), P.w[0], P.h[0], taps[0]);
+  sift_upsample_kernel<<<pgrid(P.w[0], P.h[0]), pb, 0, st>>>(gray, width, height, pitch, frame_stride, P.level(0, 1),
+                                                             fs);
+  sift_blur_kernel<<<tgrid(P.w[0], P.h[0]), 256, 0, st>>>(P.level(0, 1), P.level(0, 0), P.w[0], P.h[0], taps[0], fs);
   for (int o = 0; o < P.n_oct; ++o) {
     if (o > 0)
       sift_halve_kernel<<<pgrid(P.w[o], P.h[o]), pb, 0, st>>>(P.level(o - 1, kLayers), P.w[o - 1], P.level(o, 0),
-                                                            P.w[o], P.h[o]);
+                                                            P.w[o], P.h[o], fs);
     for (int l = 1; l < kLevels; ++l)
       sift_blur_kernel<<<tgrid(P.w[o], P.h[o]), 256, 0, st>>>(P.level(o, l - 1), P.level(o, l), P.w[o], P.h[o],
-                                                              taps[l]);
+                                                              taps[l], fs);
   }
   SOD_CHECK_LAUNCH("sift pyramid");
+  return SOD_OK;
+}
+
+// Detection, order, duplicate removal, rows and descriptors of p.frames images: the whole of sod_sift_extract and
+// sod_sift_extract_batch after their argument checks.  Never synchronises.
+int extract_frames(const uint8_t* gray, int width, int height, int64_t pitch, int64_t frame_stride, Plan& p,
+                   int64_t max_per_frame, const Rows& out, void* workspace, cudaStream_t st) {
+  char* ws = (char*)workspace;
+  p.pyr.base = (float*)ws;
+  const int cap = (int)p.cap, frames = p.frames, slots = frames * cap;
+  int32_t* counters = (int32_t*)(ws + p.counters);
+  int32_t* batch = counters + kFrameInts * frames;
+  Cand* cand = (Cand*)(ws + p.cand);
+  Kp* raw = (Kp*)(ws + p.raw);
+  uint64_t* keys_in = (uint64_t*)(ws + p.keys_in);
+  uint64_t* keys_out = (uint64_t*)(ws + p.keys_out);
+  int32_t* vals_in = (int32_t*)(ws + p.vals_in);
+  int32_t* vals_out = (int32_t*)(ws + p.vals_out);
+  int32_t* keep = (int32_t*)(ws + p.keep);
+  int32_t* pos = (int32_t*)(ws + p.pos);
+  SOD_CHECK_CUDA(cudaMemsetAsync(counters, 0, (kFrameInts * frames + kBatchInts) * sizeof(int32_t), st));
+  const int sms = device_sm_count();
+  if (sms < 0) return SOD_ERR_CUDA;
+  if (p.pyr.n_oct > 0) {
+    if (int rc = build_pyramid(gray, width, height, pitch, frame_stride, frames, p.pyr, st)) return rc;
+    for (int o = 0; o < p.pyr.n_oct; ++o) {
+      const int iw = p.pyr.w[o] - 2 * kBorder, ih = p.pyr.h[o] - 2 * kBorder;
+      if (iw <= 0 || ih <= 0) continue;
+      sift_extrema_kernel<<<dim3((iw + 31) / 32, (ih + 7) / 8, kLayers * frames), dim3(32, 8), 0, st>>>(
+          p.pyr, o, cand, cap, counters);
+    }
+    SOD_CHECK_LAUNCH("sift_extrema_kernel");
+    // sms * 8 blocks in all, as for one frame, split over the frames' slabs
+    sift_orient_kernel<<<dim3((sms * 8 + frames - 1) / frames, frames), 32 * kOriWarps, 0, st>>>(p.pyr, cand, cap,
+                                                                                             counters, raw);
+    SOD_CHECK_LAUNCH("sift_orient_kernel");
+  }
+  const int blocks = (slots + 255) / 256;
+  sift_sort_keys_kernel<<<blocks, 256, 0, st>>>(raw, counters, cap, slots, keys_in, vals_in);
+  SOD_CHECK_LAUNCH("sift_sort_keys_kernel");
+  size_t tmp = p.cub_bytes;
+  SOD_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(ws + p.cub_tmp, tmp, keys_in, keys_out, vals_in, vals_out, slots, 0,
+                                                 64, st));
+  int32_t* vals = vals_out;
+  if (frames > 1) {
+    uint32_t* fkeys_in = (uint32_t*)keys_in;      // keys_in is free after the first sort: 2 x slots u32
+    uint32_t* fkeys_out = fkeys_in + slots;
+    sift_frame_keys_kernel<<<blocks, 256, 0, st>>>(vals_out, cap, slots, fkeys_in);
+    SOD_CHECK_LAUNCH("sift_frame_keys_kernel");
+    int bits = 0;
+    while ((1 << bits) < frames) ++bits;
+    tmp = p.cub_bytes;
+    SOD_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(ws + p.cub_tmp, tmp, fkeys_in, fkeys_out, vals_out, vals_in, slots,
+                                                   0, bits, st));
+    vals = vals_in;
+  }
+  sift_sort_runs_kernel<<<blocks, 256, 0, st>>>(raw, counters, cap, slots, vals);
+  sift_keep_kernel<<<blocks, 256, 0, st>>>(raw, counters, cap, slots, vals, keep);
+  SOD_CHECK_LAUNCH("sift_keep_kernel");
+  tmp = p.cub_bytes;
+  SOD_CHECK_CUDA(cub::DeviceScan::ExclusiveSum(ws + p.cub_tmp, tmp, keep, pos, slots, st));
+  sift_frame_rows_kernel<<<1, 256, 0, st>>>(keep, pos, counters, cap, frames, max_per_frame, out, batch);
+  sift_emit_kernel<<<blocks, 256, 0, st>>>(raw, cap, slots, vals, keep, pos, out);
+  SOD_CHECK_LAUNCH("sift_emit_kernel");
+  if (p.pyr.n_oct > 0) {
+    sift_descriptor_kernel<<<sms * 16, 128, 0, st>>>(p.pyr, out.xy, out.size, out.angle, out.octave, out.frame,
+                                                     out.cap_rows, batch, out.des, nullptr);
+    SOD_CHECK_LAUNCH("sift_descriptor_kernel");
+  }
   return SOD_OK;
 }
 
@@ -643,17 +826,22 @@ using namespace sod;
 
 extern "C" {
 
-size_t sod_sift_workspace_bytes(int32_t width, int32_t height, int64_t max_keypoints) {
+size_t sod_sift_batch_workspace_bytes(int32_t width, int32_t height, int32_t frames, int64_t cap_per_frame) {
   Plan p;
-  if (width < 1 || height < 1 || width > kMaxSide || height > kMaxSide || max_keypoints < 0 ||
-      max_keypoints > SOD_SIFT_MAX_CAP || !make_plan(width, height, max_keypoints, &p))
+  if (width < 1 || height < 1 || width > kMaxSide || height > kMaxSide || frames < 1 ||
+      frames > SOD_SIFT_MAX_FRAMES || cap_per_frame < 0 || cap_per_frame > SOD_SIFT_MAX_CAP ||
+      frames * cap_per_frame > SOD_SIFT_MAX_CAP || !make_plan(width, height, frames, cap_per_frame, &p))
     return 0;
   return p.total;
 }
 
+size_t sod_sift_workspace_bytes(int32_t width, int32_t height, int64_t max_keypoints) {
+  return sod_sift_batch_workspace_bytes(width, height, 1, max_keypoints);
+}
+
 int64_t sod_sift_level_offset(int32_t width, int32_t height, int32_t octave, int32_t level, int32_t* wh_host) {
   Plan p;
-  if (width < 1 || height < 1 || width > kMaxSide || height > kMaxSide || !make_plan(width, height, 0, &p) ||
+  if (width < 1 || height < 1 || width > kMaxSide || height > kMaxSide || !make_plan(width, height, 1, 0, &p) ||
       octave < -1 || octave + 1 >= p.pyr.n_oct || level < 0 || level >= kLevels) {
     set_error("sod_sift_level_offset: no level %d of octave %d for a %dx%d image", level, octave, width, height);
     return -1;
@@ -675,59 +863,47 @@ int sod_sift_extract(const uint8_t* gray, int32_t width, int32_t height, int64_t
   SOD_CHECK_ARG(out->xy && out->size && out->angle && out->response && out->octave && out->des && out->counters,
                 "sod_sift_extract: null output array");
   Plan p;
-  SOD_CHECK_ARG(make_plan(width, height, out->cap, &p), "sod_sift_extract: too many octaves");
+  SOD_CHECK_ARG(make_plan(width, height, 1, out->cap, &p), "sod_sift_extract: too many octaves");
   SOD_CHECK_ARG(workspace != nullptr && workspace_bytes >= p.total && ((uintptr_t)workspace & 255) == 0,
                 "sod_sift_extract: workspace of %zu bytes at %p; need %zu bytes, 256-byte aligned", workspace_bytes,
                 workspace, p.total);
-  cudaStream_t st = (cudaStream_t)stream;
-  char* ws = (char*)workspace;
-  p.pyr.base = (float*)ws;
-  const int cap = (int)out->cap;
-  int32_t* counters = (int32_t*)(ws + p.counters);
-  Cand* cand = (Cand*)(ws + p.cand);
-  Kp* raw = (Kp*)(ws + p.raw);
-  uint64_t* keys_in = (uint64_t*)(ws + p.keys_in);
-  uint64_t* keys_out = (uint64_t*)(ws + p.keys_out);
-  int32_t* vals_in = (int32_t*)(ws + p.vals_in);
-  int32_t* vals_out = (int32_t*)(ws + p.vals_out);
-  int32_t* keep = (int32_t*)(ws + p.keep);
-  int32_t* pos = (int32_t*)(ws + p.pos);
-  SOD_CHECK_CUDA(cudaMemsetAsync(counters, 0, 4 * sizeof(int32_t), st));
-  if (p.pyr.n_oct > 0) {
-    if (int rc = build_pyramid(gray, width, height, pitch, p.pyr, st)) return rc;
-    for (int o = 0; o < p.pyr.n_oct; ++o) {
-      const int iw = p.pyr.w[o] - 2 * kBorder, ih = p.pyr.h[o] - 2 * kBorder;
-      if (iw <= 0 || ih <= 0) continue;
-      sift_extrema_kernel<<<dim3((iw + 31) / 32, (ih + 7) / 8, kLayers), dim3(32, 8), 0, st>>>(p.pyr, o, cand, cap,
-                                                                                            counters);
-    }
-    SOD_CHECK_LAUNCH("sift_extrema_kernel");
-    const int sms = device_sm_count();
-    if (sms < 0) return SOD_ERR_CUDA;
-    sift_orient_kernel<<<sms * 8, 32 * kOriWarps, 0, st>>>(p.pyr, cand, cap, counters, raw);
-    SOD_CHECK_LAUNCH("sift_orient_kernel");
-  }
-  const int blocks = (cap + 255) / 256;
-  sift_sort_keys_kernel<<<blocks, 256, 0, st>>>(raw, counters, cap, keys_in, vals_in);
-  SOD_CHECK_LAUNCH("sift_sort_keys_kernel");
-  size_t tmp = p.cub_bytes;
-  SOD_CHECK_CUDA(cub::DeviceRadixSort::SortPairs(ws + p.cub_tmp, tmp, keys_in, keys_out, vals_in, vals_out, cap, 0,
-                                                 64, st));
-  sift_sort_runs_kernel<<<blocks, 256, 0, st>>>(raw, counters, cap, keys_out, vals_out);
-  sift_keep_kernel<<<blocks, 256, 0, st>>>(raw, counters, cap, vals_out, keep);
-  SOD_CHECK_LAUNCH("sift_keep_kernel");
-  tmp = p.cub_bytes;
-  SOD_CHECK_CUDA(cub::DeviceScan::ExclusiveSum(ws + p.cub_tmp, tmp, keep, pos, cap, st));
-  sift_emit_kernel<<<blocks, 256, 0, st>>>(raw, counters, cap, vals_out, keep, pos, *out);
-  SOD_CHECK_LAUNCH("sift_emit_kernel");
-  if (p.pyr.n_oct > 0) {
-    const int sms = device_sm_count();
-    if (sms < 0) return SOD_ERR_CUDA;
-    sift_descriptor_kernel<<<sms * 16, 128, 0, st>>>(p.pyr, out->xy, out->size, out->angle, out->octave, cap,
-                                                     out->counters, out->des, nullptr);
-    SOD_CHECK_LAUNCH("sift_descriptor_kernel");
-  }
-  return SOD_OK;
+  // the batch of one: count and overflow land in out->counters, the frame's offset (0) in the workspace
+  const Rows rows{out->xy,       out->size,         out->angle,  out->response,
+                  out->octave,   out->des,          nullptr,     out->counters,
+                  (int32_t*)((char*)workspace + p.offset), out->counters + 1, nullptr, out->cap};
+  return extract_frames(gray, width, height, pitch, (int64_t)pitch * height, p, 0, rows, workspace,
+                        (cudaStream_t)stream);
+}
+
+int sod_sift_extract_batch(const uint8_t* gray, int32_t width, int32_t height, int64_t pitch, int64_t frame_stride,
+                           int32_t frames, int64_t max_per_frame, const sod_sift_batch_out* out, void* workspace,
+                           size_t workspace_bytes, sod_stream_t stream) {
+  const char* fn = "sod_sift_extract_batch";
+  if (int rc = check_image(gray, width, height, pitch, fn)) return rc;
+  SOD_CHECK_ARG(frames >= 1 && frames <= SOD_SIFT_MAX_FRAMES, "%s: frames %d out of range (1..%d)", fn, frames,
+                SOD_SIFT_MAX_FRAMES);
+  SOD_CHECK_ARG(frame_stride >= pitch * height, "%s: frame_stride %lld < pitch x height %lld", fn,
+                (long long)frame_stride, (long long)(pitch * height));
+  SOD_CHECK_ARG(max_per_frame >= 0, "%s: max_per_frame %lld < 0", fn, (long long)max_per_frame);
+  SOD_CHECK_ARG(out != nullptr, "%s: null out", fn);
+  SOD_CHECK_ARG(out->cap_per_frame >= 1 && out->cap_per_frame <= SOD_SIFT_MAX_CAP &&
+                    frames * out->cap_per_frame <= SOD_SIFT_MAX_CAP,
+                "%s: cap_per_frame %lld out of range (1..%d / frames)", fn, (long long)out->cap_per_frame,
+                SOD_SIFT_MAX_CAP);
+  SOD_CHECK_ARG(out->cap_rows >= 1 && out->cap_rows <= SOD_SIFT_MAX_CAP, "%s: cap_rows %lld out of range (1..%d)",
+                fn, (long long)out->cap_rows, SOD_SIFT_MAX_CAP);
+  SOD_CHECK_ARG(out->xy && out->size && out->angle && out->response && out->octave && out->des && out->frame &&
+                    out->count && out->offset && out->overflow && out->rows_overflow,
+                "%s: null output array", fn);
+  Plan p;
+  SOD_CHECK_ARG(make_plan(width, height, frames, out->cap_per_frame, &p), "%s: too many octaves", fn);
+  SOD_CHECK_ARG(workspace != nullptr && workspace_bytes >= p.total && ((uintptr_t)workspace & 255) == 0,
+                "%s: workspace of %zu bytes at %p; need %zu bytes, 256-byte aligned", fn, workspace_bytes, workspace,
+                p.total);
+  const Rows rows{out->xy,    out->size,  out->angle,  out->response,   out->octave, out->des,
+                  out->frame, out->count, out->offset, out->overflow, out->rows_overflow, out->cap_rows};
+  return extract_frames(gray, width, height, pitch, frame_stride, p, max_per_frame, rows, workspace,
+                        (cudaStream_t)stream);
 }
 
 int sod_sift_describe(const uint8_t* gray, int32_t width, int32_t height, int64_t pitch, const float* xy,
@@ -739,17 +915,18 @@ int sod_sift_describe(const uint8_t* gray, int32_t width, int32_t height, int64_
   if (n == 0) return SOD_OK;
   SOD_CHECK_ARG(xy && size && angle && octave && des, "sod_sift_describe: null keypoint or descriptor array");
   Plan p;
-  SOD_CHECK_ARG(make_plan(width, height, 0, &p), "sod_sift_describe: too many octaves");
+  SOD_CHECK_ARG(make_plan(width, height, 1, 0, &p), "sod_sift_describe: too many octaves");
   SOD_CHECK_ARG(workspace != nullptr && workspace_bytes >= p.total && ((uintptr_t)workspace & 255) == 0,
                 "sod_sift_describe: workspace of %zu bytes at %p; need %zu bytes, 256-byte aligned", workspace_bytes,
                 workspace, p.total);
   cudaStream_t st = (cudaStream_t)stream;
   p.pyr.base = (float*)workspace;
   if (p.pyr.n_oct > 0)
-    if (int rc = build_pyramid(gray, width, height, pitch, p.pyr, st)) return rc;
+    if (int rc = build_pyramid(gray, width, height, pitch, (int64_t)pitch * height, 1, p.pyr, st)) return rc;
   const int sms = device_sm_count();
   if (sms < 0) return SOD_ERR_CUDA;
-  sift_descriptor_kernel<<<sms * 16, 128, 0, st>>>(p.pyr, xy, size, angle, octave, n, nullptr, des, n_invalid);
+  sift_descriptor_kernel<<<sms * 16, 128, 0, st>>>(p.pyr, xy, size, angle, octave, nullptr, n, nullptr, des,
+                                                   n_invalid);
   SOD_CHECK_LAUNCH("sift_descriptor_kernel");
   return SOD_OK;
 }

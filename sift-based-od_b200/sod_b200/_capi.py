@@ -62,6 +62,12 @@ class SiftOut(C.Structure):
                 ("counters", _p), ("cap", _i64)]
 
 
+class SiftBatchOut(C.Structure):
+    _fields_ = [("xy", _p), ("size", _p), ("angle", _p), ("response", _p), ("octave", _p), ("des", _p),
+                ("frame", _p), ("count", _p), ("offset", _p), ("overflow", _p), ("rows_overflow", _p),
+                ("cap_rows", _i64), ("cap_per_frame", _i64)]
+
+
 STAGES = {"match": 0, "hough_prep": 1, "hough_vote": 2, "hough_finish": 3, "affine": 4}
 
 
@@ -135,6 +141,9 @@ _PROTOS = {
     "sod_sift_extract": (C.c_int, [_p, _i32, _i32, _i64, C.POINTER(SiftOut), _p, C.c_size_t, _p]),
     "sod_sift_describe": (C.c_int, [_p, _i32, _i32, _i64, _p, _p, _p, _p, _i64, _p, _p, _p, C.c_size_t, _p]),
     "sod_sift_level_offset": (_i64, [_i32, _i32, _i32, _i32, _p]),
+    "sod_sift_batch_workspace_bytes": (C.c_size_t, [_i32, _i32, _i32, _i64]),
+    "sod_sift_extract_batch": (C.c_int, [_p, _i32, _i32, _i64, _i64, _i32, _i64, C.POINTER(SiftBatchOut), _p,
+                                         C.c_size_t, _p]),
 }
 
 

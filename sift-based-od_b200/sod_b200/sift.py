@@ -4,11 +4,15 @@ pose, the u8 matcher, the drop-in Main) reads them unchanged.  Opt-in: OpenCV SI
 and the reference; DESIGN.md 2 states how closely this one agrees with it.
 
     stream = FrameStream(pipeline, extractor=GpuSift())
+
+GpuSift.extract_batch runs many same-size frames in one pass (sod_sift_extract_batch) and leaves the result on the
+device, in the layout DetectionPipeline.load_queries takes; FrameStream uses it when the extractor has it.
 """
 from __future__ import annotations
 
 import ctypes as C
 import threading
+from dataclasses import dataclass
 
 import numpy as np
 
@@ -30,6 +34,83 @@ def _gray(image) -> np.ndarray:
     if gray.dtype != np.uint8 or gray.ndim != 2:
         raise ValueError(f"expected an 8-bit gray or BGR image, got {gray.dtype} {gray.shape}")
     return np.ascontiguousarray(gray)
+
+
+def _is_cuda(x) -> bool:
+    return getattr(x, "is_cuda", False)
+
+
+@dataclass
+class SiftBatch:
+    """The keypoints of a batch of same-size frames, packed frame after frame on the device.
+
+    des u8 [rows, 128], xy f32 [rows, 2], angle, size, response f32 [rows], octave, frame i32 [rows]: frame k's
+    keypoints are rows offset[k]:offset[k] + count[k] (host arrays), in the order GpuSift.extract gives for that
+    frame alone.  The tensors are GpuSift's buffers: the next extract_batch of the same size, batch and slot
+    overwrites them."""
+    des: object
+    xy: object
+    angle: object
+    octave: object
+    size: object
+    response: object
+    frame: object
+    count: np.ndarray
+    offset: np.ndarray
+    frame_size: tuple
+
+    def __len__(self) -> int:
+        return len(self.count)
+
+    @property
+    def rows(self) -> int:
+        return int(self.count.sum())
+
+    def arrays(self, k: int) -> dict:
+        """Frame k's keypoints as host arrays, in the format of GpuSift.extract."""
+        lo, hi = int(self.offset[k]), int(self.offset[k] + self.count[k])
+        out = {name: getattr(self, name)[lo:hi].cpu().numpy()
+               for name in ("xy", "size", "angle", "response", "octave", "des")}
+        out["frame_size"] = self.frame_size
+        return out
+
+    def features(self, k: int) -> FrameFeatures:
+        r = self.arrays(k)
+        return FrameFeatures(r["des"], r["xy"], r["angle"], r["octave"], r["frame_size"])
+
+
+class _BatchBuffers:
+    """Device workspace, pinned host staging, device input and packed output rows for one (size, frames)."""
+
+    def __init__(self, width: int, height: int, frames: int, capacity: int, max_keypoints: int | None, device):
+        import torch
+        self.bytes = int(_capi.lib.sod_sift_batch_workspace_bytes(width, height, frames, capacity))
+        if self.bytes == 0:
+            raise ValueError(f"sod_sift: {frames} frames of {width}x{height} with capacity {capacity} out of range")
+        rows = frames * (capacity if max_keypoints is None else min(capacity, max(1, int(max_keypoints))))
+        mk = lambda shape, dt: torch.empty(shape, dtype=dt, device=device)  # noqa: E731
+        self.ws = mk(self.bytes, torch.uint8)
+        self.img = mk((frames, height, width), torch.uint8)
+        self.host = None                       # pinned [frames, h, w], made on the first host upload
+        self.outs = [None, None]               # output rows per slot, made on first use
+        self.frames, self.rows, self.capacity, self.device = frames, rows, capacity, device
+        self.flags = torch.empty((3 * frames + 1,), dtype=torch.int32, pin_memory=True)
+
+    def out(self, slot: int):
+        import torch
+        if self.outs[slot] is None:
+            f, r = self.frames, self.rows
+            mk = lambda shape, dt: torch.empty(shape, dtype=dt, device=self.device)  # noqa: E731
+            t = dict(xy=mk((r, 2), torch.float32), size=mk(r, torch.float32), angle=mk(r, torch.float32),
+                     response=mk(r, torch.float32), octave=mk(r, torch.int32), des=mk((r, 128), torch.uint8),
+                     frame=mk(r, torch.int32), flags=mk(3 * f + 1, torch.int32))
+            fl = t["flags"]
+            st = _capi.SiftBatchOut(*(t[k].data_ptr() for k in ("xy", "size", "angle", "response", "octave", "des",
+                                                                  "frame")),
+                                    fl[:f].data_ptr(), fl[f:2 * f].data_ptr(), fl[2 * f:3 * f].data_ptr(),
+                                    fl[3 * f:].data_ptr(), r, self.capacity)
+            self.outs[slot] = (t, st)
+        return self.outs[slot]
 
 
 class _Buffers:
@@ -75,13 +156,17 @@ class GpuSift:
         self._lock = threading.Lock()
         self._stream = None
         self._buffers: dict[tuple[int, int], _Buffers] = {}
+        self._batch_buffers: dict[tuple[int, int, int], _BatchBuffers] = {}
 
-    def _setup(self, width: int, height: int) -> _Buffers:
+    def _setup_stream(self) -> None:
         import torch
         if self._stream is None:
             self._device = torch.device("cuda", torch.cuda.current_device()) if self._device is None \
                 else torch.device(self._device)
             self._stream = torch.cuda.Stream(self._device)
+
+    def _setup(self, width: int, height: int) -> _Buffers:
+        self._setup_stream()
         b = self._buffers.get((width, height))
         if b is None:
             b = self._buffers[(width, height)] = _Buffers(width, height, self.capacity, self._device)
@@ -116,6 +201,86 @@ class GpuSift:
         out["frame_size"] = (w, h)
         return out
 
+    @staticmethod
+    def prepare(image):
+        """What extract_batch takes of one frame: a CUDA u8 [H, W] tensor as it is, anything else as _gray makes
+        it (decoded and converted on the host).  FrameStream's worker threads call this."""
+        return image if _is_cuda(image) else _gray(image)
+
+    def extract_batch(self, images, slot: int = 0) -> SiftBatch:
+        """SIFT of a batch of same-size frames in one pass, the result left on the device.
+
+        images  a CUDA u8 tensor [B, H, W], or a list of CUDA u8 [H, W] tensors and / or host images / paths
+                (decoded and converted as extract does; an all-host list is uploaded as one pinned [B, H, W] copy)
+        slot    0 or 1: which of two output sets to fill, so that a caller can read one batch while the next is
+                extracted
+
+        Waits for the batch (counts are read on the host); a frame with more than `capacity` keypoints raises
+        SodError naming it."""
+        import torch
+        if slot not in (0, 1):
+            raise ValueError("slot must be 0 or 1")
+        dev_in = _is_cuda(images)
+        frames = images if dev_in else [self.prepare(im) for im in images]
+        if len(frames) == 0:
+            raise ValueError("extract_batch needs at least one frame")
+        shapes = {tuple(f.shape[-2:]) for f in frames} if not dev_in else {tuple(images.shape[-2:])}
+        if len(shapes) != 1:
+            raise ValueError(f"extract_batch needs frames of one size, got {sorted(shapes)}")
+        (h, w), n = shapes.pop(), len(frames)
+        if dev_in and (images.dim() != 3 or images.dtype != torch.uint8):
+            raise ValueError(f"expected a u8 [B, H, W] tensor, got {images.dtype} {tuple(images.shape)}")
+        with self._lock, torch.cuda.device(self._device or torch.cuda.current_device()):
+            self._setup_stream()
+            b = self._batch_buffers.get((w, h, n))
+            if b is None:
+                b = self._batch_buffers[(w, h, n)] = _BatchBuffers(w, h, n, self.capacity, self.max_keypoints,
+                                                                   self._device)
+            t, out = b.out(slot)
+            src, pitch, fstride = b.img, w, w * h
+            if dev_in or any(_is_cuda(f) for f in frames):
+                # CUDA inputs come from the caller's current stream; host inputs need no wait, so the SIFT can
+                # run beside the caller's other work (FrameStream's previous detection pass)
+                self._stream.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(self._stream):
+                if dev_in:
+                    if images.device != b.img.device:
+                        raise ValueError(f"images are on {images.device}, GpuSift on {b.img.device}")
+                    if images.stride(2) == 1 and images.stride(1) >= w and images.stride(0) >= images.stride(1) * h:
+                        src, pitch, fstride = images, images.stride(1), images.stride(0)
+                    else:
+                        b.img.copy_(images)
+                else:
+                    on_host = [k for k, f in enumerate(frames) if not _is_cuda(f)]
+                    if on_host and b.host is None:
+                        b.host = torch.empty((n, h, w), dtype=torch.uint8, pin_memory=True)
+                    for k in on_host:
+                        b.host[k].copy_(torch.from_numpy(frames[k]))
+                    if len(on_host) == n:
+                        b.img.copy_(b.host, non_blocking=True)
+                    else:
+                        for k, f in enumerate(frames):
+                            b.img[k].copy_(f if _is_cuda(f) else b.host[k], non_blocking=True)
+                mk = 0 if self.max_keypoints is None else max(1, int(self.max_keypoints))
+                _capi.check(_capi.lib.sod_sift_extract_batch(src.data_ptr(), w, h, pitch, fstride, n, mk,
+                                                             C.byref(out), b.ws.data_ptr(), b.bytes,
+                                                             self._stream.cuda_stream), "sod_sift_extract_batch")
+                b.flags.copy_(t["flags"], non_blocking=True)
+            # the whole batch is done once this returns: its rows may be read on any stream, and the pinned
+            # staging and the workspace are free for the next call
+            self._stream.synchronize()
+            fl = b.flags.numpy()
+            count, offset, overflow = fl[:n].astype(np.int64), fl[n:2 * n].astype(np.int64), fl[2 * n:3 * n]
+        bad = np.nonzero(overflow)[0]
+        if len(bad):
+            raise _capi.SodError(f"sod_sift_extract_batch: more than capacity={self.capacity} keypoints in frame "
+                                 f"{int(bad[0])} ({w}x{h}) of the batch; use a larger GpuSift(capacity=...)")
+        if fl[3 * n]:
+            raise _capi.SodError("sod_sift_extract_batch: the packed rows exceed the output buffers")
+        rows = int(count.sum())
+        return SiftBatch(t["des"][:rows], t["xy"][:rows], t["angle"][:rows], t["octave"][:rows], t["size"][:rows],
+                         t["response"][:rows], t["frame"][:rows], count, offset, (w, h))
+
     def __call__(self, image) -> FrameFeatures:
         r = self.extract(image)
         return FrameFeatures(r["des"], r["xy"], r["angle"], r["octave"], r["frame_size"])
@@ -144,9 +309,11 @@ class GpuSift:
                     raise ValueError(f"{bad} keypoints name no octave / layer of the {w}x{h} image's pyramid")
                 return des.cpu().numpy()
 
-    def gaussian_level(self, frame_size: tuple[int, int], octave: int, level: int) -> np.ndarray:
+    def gaussian_level(self, frame_size: tuple[int, int], octave: int, level: int,
+                       batch: tuple[int, int] | None = None) -> np.ndarray:
         """Gaussian level `level` (0..5) of `octave` (-1 = the doubled image) of the last frame of this size
-        extracted or described, f32 [h, w]."""
+        extracted or described, f32 [h, w].  batch = (frames, k): frame k of the last extract_batch of `frames`
+        frames of this size."""
         import torch
         w, h = frame_size
         wh = (C.c_int32 * 2)()
@@ -154,7 +321,11 @@ class GpuSift:
         if off < 0:
             _capi.check(-1, "sod_sift_level_offset")
         with self._lock:
-            b = self._buffers[(w, h)]
+            if batch is None:
+                ws = self._buffers[(w, h)].ws
+            else:
+                ws = self._batch_buffers[(w, h, batch[0])].ws
+                off += batch[1] * int(_capi.lib.sod_sift_batch_workspace_bytes(w, h, 1, 0))
             self._stream.synchronize()
             n = wh[0] * wh[1]
-            return b.ws[off:off + 4 * n].view(torch.float32).reshape(wh[1], wh[0]).cpu().numpy()
+            return ws[off:off + 4 * n].view(torch.float32).reshape(wh[1], wh[0]).cpu().numpy()

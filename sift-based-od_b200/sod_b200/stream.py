@@ -6,8 +6,11 @@ SIFT is the slow stage, so FrameStream extracts features of upcoming frames on a
 threads (OpenCV releases the GIL) while the GPU runs match -> ratio -> Hough -> affine on the
 previous batch; batches are packed into pinned, double-buffered staging while the GPU is busy, their
 host->device copies run on the pipeline's copy stream under the previous batch's kernels, and
-results are handed to the caller while the next batch runs.  OpenCV SIFT itself stays the extractor (input
-stage, out of scope for the GPU path).
+results are handed to the caller while the next batch runs.  OpenCV SIFT itself stays the default extractor.
+
+With an extractor that has extract_batch (sod_b200.sift.GpuSift) the stream runs on the device instead: worker
+threads only decode and convert frames, runs of same-size frames are extracted in one SIFT pass, and the rows go
+from the SIFT output to the pipeline's query buffers by device-to-device copies.
 """
 from __future__ import annotations
 
@@ -115,19 +118,26 @@ class FrameStream:
     batch_frames  frames per GPU pass
     workers       host threads running the extractor
     prefetch      frames whose extraction may be in flight ahead of the GPU
+    features      add each frame's FrameFeatures to its result (result["features"])
 
     run(frames) yields (frame_index, result) in input order; result holds the frame's matches and
-    verified bins (see _split) and, with poses=True, the final poses of the frame."""
+    verified bins (see _split) and, with poses=True, the final poses of the frame.
+
+    An extractor with extract_batch and prepare (GpuSift) selects the device path: workers run prepare (decode,
+    colour conversion; CUDA tensors pass as they are), consecutive frames of one size form a SIFT batch of up to
+    batch_frames frames, and each detection pass takes the longest prefix of a batch's frames whose rows fit
+    max_queries.  The SIFT of the next batch is enqueued before the host waits for the current pass.  The device
+    path needs a pipeline whose ranks do not share one batch (shard="frames" or one rank)."""
 
     def __init__(self, pipeline, extractor: Callable[[object], FrameFeatures] = sift_features, batch_frames: int = 8,
-                 workers: int = 8, prefetch: int | None = None, poses: bool = True):
+                 workers: int = 8, prefetch: int | None = None, poses: bool = True, features: bool = False):
         self.pipeline, self.extractor = pipeline, extractor
         self.batch_frames = int(batch_frames)
         if pipeline.scene.n_frames < self.batch_frames:
             raise ValueError("pipeline.frame_wh must have one row per frame of a batch")
         self.workers = int(workers)
         self.prefetch = int(prefetch) if prefetch is not None else 2 * self.batch_frames + self.workers
-        self.poses = poses
+        self.poses, self.features = poses, bool(features)
         self._staging: list[_Staging] = []
 
     # -------------------------------------------------------------------------------- GPU side
@@ -152,32 +162,40 @@ class FrameStream:
         self._copied[slot] = getattr(p, "_loaded", [None, None])[slot]
         return p.detect_device(n, slot)
 
-    def _finish(self, r, feats: list[FrameFeatures], first_index: int):
-        """Device->host read of a batch (synchronises) + final poses, split per frame."""
-        if r is None:                                # no descriptors in the whole batch
+    def _fetch(self, r):
+        """Device->host read of a pass (synchronises) + final poses."""
+        if r is None:                                # no descriptors in the whole pass
             z = np.zeros(0, np.int32)
-            out = dict(ok=np.zeros(0, np.uint8), idx=np.zeros((0, 2), np.int32), valid_group=z, valid_code=z, votes=z,
-                       status=z, params=np.zeros((0, 6)))
-            return [(first_index + k, self._split(out, {}, k, feats)) for k in range(len(feats))]
+            return dict(ok=np.zeros(0, np.uint8), idx=np.zeros((0, 2), np.int32), valid_group=z, valid_code=z, votes=z,
+                        status=z, params=np.zeros((0, 6))), {}
         out = self.pipeline.fetch(r)
-        poses = self.pipeline.final_poses(out) if self.poses else {}
-        return [(first_index + k, self._split(out, poses, k, feats)) for k in range(len(feats))]
+        return out, (self.pipeline.final_poses(out) if self.poses else {})
 
-    def _split(self, out: dict, poses: dict, slot: int, feats: list[FrameFeatures]) -> dict:
-        """The part of a batch result that belongs to frame `slot`: match pairs as (query keypoint
-        index within the frame, database row), verified bins, final poses."""
-        lo = sum(len(f) for f in feats[:slot])
-        hi = lo + len(feats[slot])
+    def _finish(self, r, feats: list[FrameFeatures], first_index: int):
+        """Device->host read of a batch + final poses, split per frame."""
+        out, poses = self._fetch(r)
+        starts = np.cumsum([0] + [len(f) for f in feats])
+        return [(first_index + k, self._split(out, poses, k, starts[k], starts[k + 1], feats[k]))
+                for k in range(len(feats))]
+
+    def _split(self, out: dict, poses: dict, slot: int, lo: int, hi: int, feats: FrameFeatures | None) -> dict:
+        """The part of a batch result that belongs to frame `slot`, whose query rows are [lo, hi): match pairs as
+        (query keypoint index within the frame, database row), verified bins, final poses."""
         ok = out["ok"][lo:hi].astype(bool)
         gpf = self.pipeline.spaces_per_frame
         mine = (out["valid_group"] // gpf) == slot
         return dict(match_q=np.nonzero(ok)[0].astype(np.int32), match_t=out["idx"][lo:hi, 0][ok],
                     n_descriptors=hi - lo, valid_group=out["valid_group"][mine] % gpf, valid_code=out["valid_code"][mine],
                     votes=out["votes"][mine], live=(out["status"][mine] & 1).astype(bool), params=out["params"][mine],
-                    final_pose=poses.get(slot, []))
+                    final_pose=poses.get(slot, []), **({"features": feats} if self.features else {}))
 
     # -------------------------------------------------------------------------------- driver
     def run(self, frames: Iterable) -> Iterator[tuple[int, dict]]:
+        if hasattr(self.extractor, "extract_batch"):
+            return self._run_device(frames)
+        return self._run_host(frames)
+
+    def _run_host(self, frames: Iterable) -> Iterator[tuple[int, dict]]:
         p = self.pipeline
         with ThreadPoolExecutor(self.workers) as pool:
             pending: deque = deque()          # futures of extracted frames, input order
@@ -222,3 +240,95 @@ class FrameStream:
                     break
                 index += len(feats)
                 slot ^= 1
+
+    # -------------------------------------------------------------------------------- device path
+    def _prepared(self, pool, frames: Iterable) -> Iterator[list]:
+        """Runs of consecutive same-size prepared frames, at most batch_frames long, in input order; preparation
+        runs up to `prefetch` frames ahead on the worker threads."""
+        pending: deque = deque()
+        it = iter(frames)
+        exhausted = False
+        while True:
+            while not exhausted and len(pending) < self.prefetch:
+                try:
+                    pending.append(pool.submit(self.extractor.prepare, next(it)))
+                except StopIteration:
+                    exhausted = True
+            if not pending:
+                return
+            run = [pending.popleft().result()]
+            shape = tuple(run[0].shape[-2:])
+            while len(run) < self.batch_frames:
+                if not pending:
+                    if exhausted:
+                        break
+                    try:
+                        pending.append(pool.submit(self.extractor.prepare, next(it)))
+                    except StopIteration:
+                        exhausted = True
+                        break
+                if tuple(pending[0].result().shape[-2:]) != shape:
+                    break
+                run.append(pending.popleft().result())
+            yield run
+
+    def _passes(self, pool, frames: Iterable) -> Iterator[tuple]:
+        """(SIFT batch, first frame, end frame, input index of the batch's frame 0, host features or None) per
+        detection pass: the longest prefix of the batch's remaining frames whose rows fit max_queries.  SIFT
+        batches alternate between the extractor's two output sets."""
+        index, slot = 0, 0
+        for run in self._prepared(pool, frames):
+            sb = self.extractor.extract_batch(run, slot=slot)
+            feats = [sb.features(k) for k in range(len(sb))] if self.features else None
+            count, a = np.asarray(sb.count), 0
+            while a < len(count):
+                b, rows = a, 0
+                while b < len(count) and rows + count[b] <= self.pipeline.max_queries:
+                    rows += count[b]
+                    b += 1
+                if b == a:
+                    raise ValueError(f"a frame has {int(count[a])} descriptors, more than max_queries "
+                                     f"{self.pipeline.max_queries}")
+                yield sb, a, b, index, feats
+                a = b
+            index += len(count)
+            slot ^= 1
+
+    def _enqueue_device(self, sb, a: int, b: int, slot: int):
+        """Frame size, device-to-device copies of frames [a, b) of SIFT batch sb into query-buffer set `slot`,
+        and the pass's kernels.  The pass keeps the frames' indices within the SIFT batch, so frame k's Hough
+        spaces are k * spaces_per_frame + object."""
+        p = self.pipeline
+        lo, hi = int(sb.offset[a]), int(sb.offset[b - 1] + sb.count[b - 1])
+        if hi == lo:
+            return None
+        p.scene.frame_wh[:, 0].fill_(sb.frame_size[0])
+        p.scene.frame_wh[:, 1].fill_(sb.frame_size[1])
+        p.load_queries(sb.des[lo:hi], sb.xy[lo:hi], sb.angle[lo:hi], sb.octave[lo:hi], sb.frame[lo:hi], slot=slot,
+                       overlap=p.device.type == "cuda")
+        return p.detect_device(hi - lo, slot)
+
+    def _finish_device(self, r, sb, a: int, b: int, index: int, feats) -> list:
+        out, poses = self._fetch(r)
+        base = int(sb.offset[a])
+        return [(index + k, self._split(out, poses, k, int(sb.offset[k]) - base,
+                                        int(sb.offset[k] + sb.count[k]) - base, feats[k] if feats else None))
+                for k in range(a, b)]
+
+    def _run_device(self, frames: Iterable) -> Iterator[tuple[int, dict]]:
+        p = self.pipeline
+        if getattr(p, "world", 1) > 1 and getattr(p, "shard_mode", "db") == "db":
+            raise ValueError("FrameStream's device path needs the whole batch on one rank: every rank of a "
+                             "database-sharded pipeline would need the same query rows, and GPU SIFT descriptors "
+                             "may differ by 1 between runs; use DetectionPipeline(shard='frames')")
+        with ThreadPoolExecutor(self.workers) as pool:
+            # Per pass: take the next pass (which may run the next SIFT batch, while the GPU still runs the
+            # previous pass), read back the previous pass, enqueue this one, hand the previous frames over.
+            prev, slot = None, 0
+            for sb, a, b, index, feats in self._passes(pool, frames):
+                results = self._finish_device(*prev) if prev is not None else []
+                prev = (self._enqueue_device(sb, a, b, slot), sb, a, b, index, feats)
+                yield from results
+                slot ^= 1
+            if prev is not None:
+                yield from self._finish_device(*prev)
