@@ -471,6 +471,25 @@ int sod_sift_extract_batch(const uint8_t* gray, int32_t width, int32_t height, i
                            int32_t frames, int64_t max_per_frame, const sod_sift_batch_out* out, void* workspace,
                            size_t workspace_bytes, sod_stream_t stream);
 
+/* ---- SIFT over a batch of frames of different sizes in one pass (training images of one width and many heights,
+ * say).  Each (octave, level) is still one launch for all frames, sized for the largest frame that has it. */
+#define SOD_SIFT_MAX_MIXED_FRAMES 64
+
+/* Bytes of workspace (256-byte aligned) for `frames` images of the sizes wh_host[2f], wh_host[2f+1] (HOST) and
+ * cap_per_frame; 0 if an argument is out of range.  Frame f's pyramid lies at the sum of
+ * sod_sift_batch_workspace_bytes(w, h, 1, 0) of frames 0..f-1, so sod_sift_level_offset reads any frame's levels;
+ * after the pyramids come the slabs of sod_sift_batch_workspace_bytes and a 160-byte geometry record a frame. */
+size_t sod_sift_mixed_workspace_bytes(const int32_t* wh_host, int32_t frames, int64_t cap_per_frame);
+
+/* sod_sift_extract_batch of `frames` u8 gray images of any sizes: image f at images_host[f] (a HOST array of
+ * device pointers), wh_host[2f] x wh_host[2f+1] pixels (1..32768 a side), rows pitch_host[f] >= width bytes apart.
+ * Frame f's rows are the first max_per_frame (0 = all) keypoints sod_sift_extract gives for that image alone, in
+ * the same order, with out as in sod_sift_extract_batch.  The geometry reaches the device as a kernel argument, so
+ * the call never synchronises and can be captured in a CUDA graph. */
+int sod_sift_extract_mixed(const uint8_t* const* images_host, const int32_t* wh_host, const int64_t* pitch_host,
+                           int32_t frames, int64_t max_per_frame, const sod_sift_batch_out* out, void* workspace,
+                           size_t workspace_bytes, sod_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

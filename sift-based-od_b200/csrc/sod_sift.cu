@@ -20,13 +20,16 @@
 // stage.  Frame f has its own pyramid (at f x the pyramid of one frame in the workspace), its own counters and
 // its own candidate / keypoint slabs of cap entries.  The order is per frame: the (x, y) sort over all slabs is
 // followed, for B > 1, by a stable sort by frame, so each frame's slab ends up in the order one frame alone
-// gets.  sod_sift_extract is the batch of one.
+// gets.  sod_sift_extract is the batch of one.  sod_sift_extract_mixed runs frames of different sizes through the
+// same kernels: each reads a frame's geometry through the layout it is instantiated for (Pyramid or Mixed, below).
 #include <cub/block/block_scan.cuh>
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
+#include <algorithm>
 #include <cfloat>
 #include <climits>
+#include <cstdio>
 #include <cmath>
 
 #include "sod_common.cuh"
@@ -50,6 +53,10 @@ constexpr int kTile = 32;              // blur output tile
 constexpr int kMaxRadius = 13;         // largest blur radius of the default parameters (sigma 3.09, 27 taps)
 constexpr int kOriWarps = 4;
 
+// The kernels read a frame's geometry through one accessor, templated on the layout: Pyramid (frames of one size,
+// fstride elements apart) or Mixed (a per-frame table, frames of any size).  Both give level(o, l, f), the size
+// width / height(o, f) of octave o of frame f and octaves(f); the pyramid kernels take a step view of either
+// (UniformUpsample / UniformStep or MixedStep: where frame f reads and writes one level).
 struct Pyramid {
   float* base;
   int64_t off[kMaxOct];                // element offset of octave o's first level
@@ -59,6 +66,89 @@ struct Pyramid {
   __host__ __device__ float* level(int o, int l, int f = 0) const {
     return base + f * fstride + off[o] + (int64_t)l * w[o] * h[o];
   }
+  __device__ int width(int o, int) const { return w[o]; }
+  __device__ int height(int o, int) const { return h[o]; }
+  __device__ int octaves(int) const { return n_oct; }
+};
+
+// One frame of a mixed batch, written into the workspace by sift_mixed_setup_kernel.  Octave o of the frame is
+// (2 width) >> o by (2 height) >> o pixels for o < n_oct, its first level at element off[o] of the workspace.
+struct FrameGeom {
+  const uint8_t* img;
+  int64_t pitch;
+  int64_t off[kMaxOct];
+  int32_t width, height, n_oct, pad;
+};
+
+struct MixedTable {                    // the kernel parameter that carries the table to the device
+  FrameGeom f[SOD_SIFT_MAX_MIXED_FRAMES];
+};
+
+struct Mixed {
+  float* base;
+  const FrameGeom* g;
+  int frames;
+  __device__ int octaves(int f) const {
+    SOD_DCHECK(f >= 0 && f < frames);
+    return g[f].n_oct;
+  }
+  __device__ int width(int o, int f) const { return o < octaves(f) ? (2 * g[f].width) >> o : 0; }
+  __device__ int height(int o, int f) const { return o < octaves(f) ? (2 * g[f].height) >> o : 0; }
+  __device__ float* level(int o, int l, int f) const {
+    SOD_DCHECK(f >= 0 && f < frames && o >= 0 && o < g[f].n_oct && l >= 0 && l < kLevels);
+    return base + g[f].off[o] + (int64_t)l * width(o, f) * height(o, f);
+  }
+};
+
+struct Plane {                         // one level of one frame; w = h = 0 when the frame has no such octave
+  float* p;
+  int w, h;
+};
+
+struct Image {
+  const uint8_t* p;
+  int w, h;
+  int64_t pitch;
+};
+
+// Frames of one size: every pointer is frame 0's, frame f's lies f strides further on.
+struct UniformUpsample {
+  const uint8_t* src;
+  int sw, sh;
+  int64_t pitch, frame_stride;
+  float* dst;
+  int64_t dst_stride;
+  __device__ Image image(int f) const { return {src + f * frame_stride, sw, sh, pitch}; }
+  __device__ Plane out(int f) const { return {dst + f * dst_stride, 2 * sw, 2 * sh}; }
+};
+
+struct UniformStep {
+  static constexpr bool kRagged = false;
+  const float* src;
+  float* dst;
+  int sw, sh, dw, dh;
+  int64_t fstride;
+  __device__ Plane in(int f) const { return {const_cast<float*>(src) + f * fstride, sw, sh}; }
+  __device__ Plane out(int f) const { return {dst + f * fstride, dw, dh}; }
+};
+
+// Frames of any size: level (oi, li) -> level (oo, lo) of each frame (oi = -1: its u8 image).  Grids cover the
+// largest frame; blocks outside their frame's level return at once.
+struct MixedStep {
+  static constexpr bool kRagged = true;
+  Mixed P;
+  int oi, li, oo, lo;
+  __device__ Image image(int f) const {
+    SOD_DCHECK(f >= 0 && f < P.frames);
+    const FrameGeom& g = P.g[f];
+    return {g.img, g.width, g.height, g.pitch};
+  }
+  __device__ Plane plane(int o, int l, int f) const {
+    const int w = P.width(o, f), h = P.height(o, f);
+    return {w ? P.level(o, l, f) : nullptr, w, h};
+  }
+  __device__ Plane in(int f) const { return plane(oi, li, f); }
+  __device__ Plane out(int f) const { return plane(oo, lo, f); }
 };
 
 struct Taps {
@@ -89,6 +179,7 @@ struct Plan {
   int frames;
   int64_t cap;
   size_t cand, raw, keys_in, keys_out, vals_in, vals_out, keep, pos, counters, offset, cub_tmp, cub_bytes, total;
+  size_t geom = 0;                     // mixed batches: the FrameGeom table
 };
 
 size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
@@ -99,32 +190,47 @@ int octave_count(int width, int height) {
   return (int)std::lrint(std::log(m) / std::log(2.0) - 2.0) + 1;
 }
 
-// Pyramid geometry and workspace offsets for `frames` images and cap keypoints a frame; cap = 0 plans the
-// pyramids alone (sod_sift_describe).  frames x cap <= SOD_SIFT_MAX_CAP is the caller's check.
-bool make_plan(int width, int height, int frames, int64_t cap, Plan* p) {
+// The pyramid of one image of this size (base and fstride left to the caller) and its bytes, 256-byte aligned;
+// false if it has too many octaves.
+bool plan_pyramid(int width, int height, Pyramid* P, size_t* bytes) {
   int n_oct = octave_count(width, height);
   if (n_oct < 0) n_oct = 0;
   if (n_oct > kMaxOct) return false;
-  p->pyr.base = nullptr;
-  p->pyr.n_oct = n_oct;
+  P->base = nullptr;
+  P->n_oct = n_oct;
   int64_t off = 0;
   int w = 2 * width, h = 2 * height;
   for (int o = 0; o < kMaxOct; ++o) {
-    p->pyr.off[o] = off;
-    p->pyr.w[o] = o < n_oct ? w : 0;
-    p->pyr.h[o] = o < n_oct ? h : 0;
+    P->off[o] = off;
+    P->w[o] = o < n_oct ? w : 0;
+    P->h[o] = o < n_oct ? h : 0;
     if (o < n_oct) {
       off += (int64_t)kLevels * w * h;
       w /= 2;
       h /= 2;
     }
   }
-  const size_t pyr_bytes = align256((size_t)off * sizeof(float));
+  *bytes = align256((size_t)off * sizeof(float));
+  return true;
+}
+
+// The slabs of `frames` x cap keypoints from byte `at` of the workspace on, and the total.
+void plan_slabs(int frames, int64_t cap, size_t at, Plan* p);
+
+// Pyramid geometry and workspace offsets for `frames` images and cap keypoints a frame; cap = 0 plans the
+// pyramids alone (sod_sift_describe).  frames x cap <= SOD_SIFT_MAX_CAP is the caller's check.
+bool make_plan(int width, int height, int frames, int64_t cap, Plan* p) {
+  size_t pyr_bytes;
+  if (!plan_pyramid(width, height, &p->pyr, &pyr_bytes)) return false;
   p->pyr.fstride = (int64_t)(pyr_bytes / sizeof(float));
+  plan_slabs(frames, cap, pyr_bytes * frames, p);
+  return true;
+}
+
+void plan_slabs(int frames, int64_t cap, size_t at, Plan* p) {
   p->frames = frames;
   p->cap = cap;
   const int64_t slots = frames * cap;
-  size_t at = pyr_bytes * frames;
   auto take = [&](size_t bytes) { size_t r = at; at += align256(bytes); return r; };
   p->cand = take(sizeof(Cand) * slots);
   p->raw = take(sizeof(Kp) * slots);
@@ -149,6 +255,36 @@ bool make_plan(int width, int height, int frames, int64_t cap, Plan* p) {
   if (frame_sort_bytes > p->cub_bytes) p->cub_bytes = frame_sort_bytes;
   p->cub_tmp = take(p->cub_bytes);
   p->total = at;
+}
+
+// A mixed batch: frame f's pyramid at the sum of the pyramids of frames 0..f-1 (each as plan_pyramid sizes it),
+// then the slabs as for a uniform batch, then the geometry table (p->geom, frames x FrameGeom).  p->pyr holds the
+// launch grids: per octave the largest size any frame has, and the largest octave count.  Sizes are the caller's
+// check (1..kMaxSide a side).
+bool make_mixed_plan(const int32_t* wh, int frames, int64_t cap, Plan* p, MixedTable* t) {
+  Pyramid& grid = p->pyr;
+  grid = Pyramid{};
+  size_t at = 0;
+  for (int f = 0; f < frames; ++f) {
+    Pyramid one;
+    size_t bytes;
+    if (!plan_pyramid(wh[2 * f], wh[2 * f + 1], &one, &bytes)) return false;
+    FrameGeom& g = t->f[f];
+    g = FrameGeom{};
+    g.width = wh[2 * f];
+    g.height = wh[2 * f + 1];
+    g.n_oct = one.n_oct;
+    for (int o = 0; o < kMaxOct; ++o) {
+      g.off[o] = (int64_t)(at / sizeof(float)) + one.off[o];
+      grid.w[o] = std::max(grid.w[o], one.w[o]);
+      grid.h[o] = std::max(grid.h[o], one.h[o]);
+    }
+    grid.n_oct = std::max(grid.n_oct, one.n_oct);
+    at += bytes;
+  }
+  plan_slabs(frames, cap, at, p);
+  p->geom = p->total;
+  p->total += align256(sizeof(FrameGeom) * frames);
   return true;
 }
 
@@ -200,14 +336,17 @@ __device__ __forceinline__ float fast_atan2(float y, float x) {
 }
 
 // cv::resize(INTER_LINEAR) to exactly twice the size: source coordinate (d + 0.5) / 2 - 0.5, clamped.
-// blockIdx.z = frame: its image at z x frame_stride bytes, its output at z x dst_stride elements.
-__global__ void sift_upsample_kernel(const uint8_t* __restrict__ src, int sw, int sh, int64_t pitch,
-                                     int64_t frame_stride, float* __restrict__ dst, int64_t dst_stride) {
+// blockIdx.z = frame.
+template <class S>
+__global__ void sift_upsample_kernel(S s) {
   const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
-  const int dw = 2 * sw, dh = 2 * sh;
+  const Image im = s.image(blockIdx.z);
+  const Plane d = s.out(blockIdx.z);
+  const int sw = im.w, sh = im.h, dw = d.w, dh = d.h;
+  const int64_t pitch = im.pitch;
   if (x >= dw || y >= dh) return;
-  src += blockIdx.z * frame_stride;
-  dst += blockIdx.z * dst_stride;
+  const uint8_t* __restrict__ src = im.p;
+  float* __restrict__ dst = d.p;
   float fx = (float)((x + 0.5) * 0.5 - 0.5), fy = (float)((y + 0.5) * 0.5 - 0.5);
   int sx = (int)floorf(fx), sy = (int)floorf(fy);
   fx -= sx;
@@ -226,15 +365,17 @@ __global__ void sift_upsample_kernel(const uint8_t* __restrict__ src, int sw, in
 
 // cv::GaussianBlur on a float image: horizontal pass into shared memory, then the vertical pass, both in the
 // symmetric form of OpenCV's row / column filters (centre tap, then pairs outwards), BORDER_REFLECT_101.
-// blockIdx.z = frame, fstride elements apart.
-__global__ void __launch_bounds__(256) sift_blur_kernel(const float* __restrict__ src, float* __restrict__ dst,
-                                                       int w, int h, Taps t, int64_t fstride) {
+// blockIdx.z = frame; source and destination have the same size.
+template <class S>
+__global__ void __launch_bounds__(256) sift_blur_kernel(S s, Taps t) {
   __shared__ float in[kTile + 2 * kMaxRadius][kTile + 2 * kMaxRadius + 1];
   __shared__ float mid[kTile + 2 * kMaxRadius][kTile + 1];
   __shared__ float k[2 * kMaxRadius + 1];
-  const int r = t.r, x0 = blockIdx.x * kTile, y0 = blockIdx.y * kTile, span = kTile + 2 * r;
-  src += blockIdx.z * fstride;
-  dst += blockIdx.z * fstride;
+  const Plane a = s.in(blockIdx.z);
+  const int w = a.w, h = a.h, r = t.r, x0 = blockIdx.x * kTile, y0 = blockIdx.y * kTile, span = kTile + 2 * r;
+  if (S::kRagged && (x0 >= w || y0 >= h)) return;
+  const float* __restrict__ src = a.p;
+  float* __restrict__ dst = s.out(blockIdx.z).p;
   if (threadIdx.x < 2 * r + 1) k[threadIdx.x] = t.k[threadIdx.x];
   for (int i = threadIdx.x; i < span * span; i += blockDim.x) {
     const int ty = i / span, tx = i - ty * span;
@@ -260,26 +401,30 @@ __global__ void __launch_bounds__(256) sift_blur_kernel(const float* __restrict_
   }
 }
 
-// cv::resize(INTER_NEAREST) to half size: every other pixel.  blockIdx.z = frame, fstride elements apart.
-__global__ void sift_halve_kernel(const float* __restrict__ src, int sw, float* __restrict__ dst, int dw, int dh,
-                                  int64_t fstride) {
+// cv::resize(INTER_NEAREST) to half size: every other pixel.  blockIdx.z = frame.
+template <class S>
+__global__ void sift_halve_kernel(S s) {
   const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
-  if (x >= dw || y >= dh) return;
-  dst[blockIdx.z * fstride + (int64_t)y * dw + x] = src[blockIdx.z * fstride + (int64_t)(2 * y) * sw + 2 * x];
+  const Plane d = s.out(blockIdx.z);
+  if (x >= d.w || y >= d.h) return;
+  const Plane a = s.in(blockIdx.z);
+  d.p[(int64_t)y * d.w + x] = a.p[(int64_t)(2 * y) * a.w + 2 * x];
 }
 
 // DoG level l of octave o of frame f at (r, c): G[l+1] - G[l], the value cv::subtract stores.
-__device__ __forceinline__ float dog(const Pyramid& P, int f, int o, int l, int r, int c) {
-  const int64_t i = (int64_t)r * P.w[o] + c;
+template <class L>
+__device__ __forceinline__ float dog(const L& P, int f, int o, int l, int r, int c) {
+  const int64_t i = (int64_t)r * P.width(o, f) + c;
   return P.level(o, l + 1, f)[i] - P.level(o, l, f)[i];
 }
 
 // OpenCV's adjustLocalExtrema: Newton steps on the 3x3 Hessian of the DoG (derivatives scaled by 1/255),
 // contrast and edge tests, keypoint fields in the octave numbering of the doubled image.
-__device__ bool refine(const Pyramid& P, int f, int o, int& layer, int& r, int& c, Cand* kp) {
+template <class L>
+__device__ bool refine(const L& P, int f, int o, int& layer, int& r, int& c, Cand* kp) {
   constexpr float img_scale = 1.f / 255.f, deriv_scale = img_scale * 0.5f, second_scale = img_scale,
                   cross_scale = img_scale * 0.25f;
-  const int w = P.w[o], h = P.h[o];
+  const int w = P.width(o, f), h = P.height(o, f);
   float xi = 0, xr = 0, xc = 0;
   int i = 0;
   for (; i < kMaxInterp; ++i) {
@@ -340,11 +485,12 @@ __device__ bool refine(const Pyramid& P, int f, int o, int& layer, int& r, int& 
 // Scale-space extrema of octave o: |DoG| > floor(0.5 * 0.04 / 3 * 255) = 1, not smaller (or not larger)
 // than all 26 neighbours, outside the 5-pixel border; refined survivors are appended to their frame's slab of
 // cand.  blockIdx.z = frame * kLayers + layer - 1.
-__global__ void sift_extrema_kernel(Pyramid P, int o, Cand* __restrict__ cand, int cap, int* __restrict__ counters) {
+template <class L>
+__global__ void sift_extrema_kernel(L P, int o, Cand* __restrict__ cand, int cap, int* __restrict__ counters) {
   const int c = kBorder + blockIdx.x * blockDim.x + threadIdx.x;
   const int r = kBorder + blockIdx.y * blockDim.y + threadIdx.y;
   const int f = blockIdx.z / kLayers, layer = 1 + blockIdx.z % kLayers;
-  if (c >= P.w[o] - kBorder || r >= P.h[o] - kBorder) return;
+  if (c >= P.width(o, f) - kBorder || r >= P.height(o, f) - kBorder) return;
   const float val = dog(P, f, o, layer, r, c);
   if (!(fabsf(val) > 1.f)) return;
   bool ext = true;
@@ -381,7 +527,8 @@ __global__ void sift_extrema_kernel(Pyramid P, int o, Cand* __restrict__ cand, i
 // OpenCV's calcOrientationHist + the peak loop of findScaleSpaceExtrema, one warp per candidate; blockIdx.y is
 // the frame whose slab the blocks walk.  Every keypoint is written to its frame's raw slab already moved to the
 // first octave -1 (octave byte - 1, pt and size halved).
-__global__ void __launch_bounds__(32 * kOriWarps) sift_orient_kernel(Pyramid P, const Cand* __restrict__ cand,
+template <class L>
+__global__ void __launch_bounds__(32 * kOriWarps) sift_orient_kernel(L P, const Cand* __restrict__ cand,
                                                                      int cap, int* __restrict__ counters,
                                                                      Kp* __restrict__ raw) {
   __shared__ float part[kOriWarps][32][kOriBins + 1];
@@ -391,9 +538,10 @@ __global__ void __launch_bounds__(32 * kOriWarps) sift_orient_kernel(Pyramid P, 
   const int n = min(fc[0], cap);
   for (int ci = blockIdx.x * kOriWarps + wib; ci < n; ci += gridDim.x * kOriWarps) {
     const Cand k = cand[(int64_t)blockIdx.y * cap + ci];
-    SOD_DCHECK(k.o >= 0 && k.o < P.n_oct && k.layer >= 1 && k.layer <= kLayers && k.frame == (int)blockIdx.y);
+    SOD_DCHECK(k.o >= 0 && k.o < P.octaves(k.frame) && k.layer >= 1 && k.layer <= kLayers &&
+               k.frame == (int)blockIdx.y);
     const float* img = P.level(k.o, k.layer, k.frame);
-    const int w = P.w[k.o], h = P.h[k.o];
+    const int w = P.width(k.o, k.frame), h = P.height(k.o, k.frame);
     const float scl = k.size * 0.5f / (float)(1 << k.o);
     const int radius = __float2int_rn(4.5f * scl);
     const float sigma = 1.5f * scl, expf_scale = -1.f / (2.f * sigma * sigma);
@@ -608,7 +756,8 @@ __global__ void sift_emit_kernel(const Kp* __restrict__ raw, int cap, int slots,
 // NULL) overrides n; frame (may be NULL = all 0) names each keypoint's pyramid.  A keypoint whose octave / layer
 // names no level of the pyramid gets a zero row and is counted in n_invalid (cv2 refuses such a keypoint).
 // 16 blocks an SM (32 registers): the grid below is 16 blocks an SM, one wave.
-__global__ void __launch_bounds__(128, 16) sift_descriptor_kernel(Pyramid P, const float* __restrict__ xy,
+template <class L>
+__global__ void __launch_bounds__(128, 16) sift_descriptor_kernel(L P, const float* __restrict__ xy,
                                                               const float* __restrict__ size,
                                                               const float* __restrict__ angle,
                                                               const int32_t* __restrict__ octave,
@@ -625,7 +774,9 @@ __global__ void __launch_bounds__(128, 16) sift_descriptor_kernel(Pyramid P, con
     const int layer = (packed >> 8) & 255;
     oct = oct < 128 ? oct : (-128 | oct);
     const int o = oct + 1;
-    if (o < 0 || o >= P.n_oct || layer > kLayers + 2) {
+    const int f = frame ? frame[q] : 0;
+    SOD_DCHECK(f >= 0);
+    if (o < 0 || o >= P.octaves(f) || layer > kLayers + 2) {
       des[q * 128 + tid] = 0;
       if (tid == 0 && n_invalid) atomicAdd(n_invalid, 1);
       continue;
@@ -635,10 +786,8 @@ __global__ void __launch_bounds__(128, 16) sift_descriptor_kernel(Pyramid P, con
     const float ptx = xy[2 * q] * scale, pty = xy[2 * q + 1] * scale;
     float ori = 360.f - angle[q];
     if (fabsf(ori - 360.f) < FLT_EPSILON) ori = 0.f;
-    const int f = frame ? frame[q] : 0;
-    SOD_DCHECK(f >= 0);
     const float* img = P.level(o, layer, f);
-    const int cols = P.w[o], rows = P.h[o];
+    const int cols = P.width(o, f), rows = P.height(o, f);
     const int px = __float2int_rn(ptx), py = __float2int_rn(pty);
     float cos_t = cosf(ori * (float)(3.14159265358979323846 / 180)),
           sin_t = sinf(ori * (float)(3.14159265358979323846 / 180));
@@ -709,8 +858,30 @@ __global__ void __launch_bounds__(128, 16) sift_descriptor_kernel(Pyramid P, con
 }
 
 // The Gaussian pyramids of `frames` images (frame_stride bytes apart) into the workspace, one launch per level.
-int build_pyramid(const uint8_t* gray, int width, int height, int64_t pitch, int64_t frame_stride, int frames,
-                  const Pyramid& P, cudaStream_t st) {
+// The arguments of each pyramid launch, for frames of one size (UniformSteps) or of any size (MixedSteps).
+struct UniformSteps {
+  const uint8_t* gray;
+  int width, height;
+  int64_t pitch, frame_stride;
+  Pyramid P;
+  UniformUpsample upsample() const {
+    return {gray, width, height, pitch, frame_stride, P.level(0, 1), P.fstride};
+  }
+  UniformStep step(int oi, int li, int oo, int lo) const {
+    return {P.level(oi, li), P.level(oo, lo), P.w[oi], P.h[oi], P.w[oo], P.h[oo], P.fstride};
+  }
+};
+
+struct MixedSteps {
+  Mixed M;
+  MixedStep upsample() const { return {M, -1, 0, 0, 1}; }
+  MixedStep step(int oi, int li, int oo, int lo) const { return {M, oi, li, oo, lo}; }
+};
+
+// The Gaussian pyramids of `frames` images into the workspace, one launch per level for all frames; grid holds
+// the launch sizes (per octave the largest frame's).
+template <class Steps>
+int build_pyramid(const Steps& s, const Pyramid& grid, int frames, cudaStream_t st) {
   double sig[kLevels];
   const double k = std::pow(2., 1. / kLayers);
   for (int i = 1; i < kLevels; ++i) {
@@ -725,29 +896,27 @@ int build_pyramid(const uint8_t* gray, int width, int height, int64_t pitch, int
   const dim3 pb(32, 8);
   auto pgrid = [&](int w, int h) { return dim3((w + 31) / 32, (h + 7) / 8, frames); };
   auto tgrid = [&](int w, int h) { return dim3((w + kTile - 1) / kTile, (h + kTile - 1) / kTile, frames); };
-  const int64_t fs = P.fstride;
+  const Pyramid& P = grid;
   // the doubled image goes to level 1's slot, blurred into level 0, and level 1 is then computed over it
-  sift_upsample_kernel<<<pgrid(P.w[0], P.h[0]), pb, 0, st>>>(gray, width, height, pitch, frame_stride, P.level(0, 1),
-                                                             fs);
-  sift_blur_kernel<<<tgrid(P.w[0], P.h[0]), 256, 0, st>>>(P.level(0, 1), P.level(0, 0), P.w[0], P.h[0], taps[0], fs);
+  sift_upsample_kernel<<<pgrid(P.w[0], P.h[0]), pb, 0, st>>>(s.upsample());
+  sift_blur_kernel<<<tgrid(P.w[0], P.h[0]), 256, 0, st>>>(s.step(0, 1, 0, 0), taps[0]);
   for (int o = 0; o < P.n_oct; ++o) {
-    if (o > 0)
-      sift_halve_kernel<<<pgrid(P.w[o], P.h[o]), pb, 0, st>>>(P.level(o - 1, kLayers), P.w[o - 1], P.level(o, 0),
-                                                            P.w[o], P.h[o], fs);
+    if (o > 0) sift_halve_kernel<<<pgrid(P.w[o], P.h[o]), pb, 0, st>>>(s.step(o - 1, kLayers, o, 0));
     for (int l = 1; l < kLevels; ++l)
-      sift_blur_kernel<<<tgrid(P.w[o], P.h[o]), 256, 0, st>>>(P.level(o, l - 1), P.level(o, l), P.w[o], P.h[o],
-                                                              taps[l], fs);
+      sift_blur_kernel<<<tgrid(P.w[o], P.h[o]), 256, 0, st>>>(s.step(o, l - 1, o, l), taps[l]);
   }
   SOD_CHECK_LAUNCH("sift pyramid");
   return SOD_OK;
 }
 
-// Detection, order, duplicate removal, rows and descriptors of p.frames images: the whole of sod_sift_extract and
-// sod_sift_extract_batch after their argument checks.  Never synchronises.
-int extract_frames(const uint8_t* gray, int width, int height, int64_t pitch, int64_t frame_stride, Plan& p,
-                   int64_t max_per_frame, const Rows& out, void* workspace, cudaStream_t st) {
+// Pyramids, detection, order, duplicate removal, rows and descriptors of p.frames images: the whole of
+// sod_sift_extract, sod_sift_extract_batch and sod_sift_extract_mixed after their argument checks (and, for a mixed
+// batch, its geometry table).  lay reads the pyramids, steps builds them, p.pyr sizes the launches.  Never
+// synchronises.
+template <class L, class Steps>
+int extract_frames(const L& lay, const Steps& steps, const Plan& p, int64_t max_per_frame, const Rows& out,
+                   void* workspace, cudaStream_t st) {
   char* ws = (char*)workspace;
-  p.pyr.base = (float*)ws;
   const int cap = (int)p.cap, frames = p.frames, slots = frames * cap;
   int32_t* counters = (int32_t*)(ws + p.counters);
   int32_t* batch = counters + kFrameInts * frames;
@@ -763,16 +932,16 @@ int extract_frames(const uint8_t* gray, int width, int height, int64_t pitch, in
   const int sms = device_sm_count();
   if (sms < 0) return SOD_ERR_CUDA;
   if (p.pyr.n_oct > 0) {
-    if (int rc = build_pyramid(gray, width, height, pitch, frame_stride, frames, p.pyr, st)) return rc;
+    if (int rc = build_pyramid(steps, p.pyr, frames, st)) return rc;
     for (int o = 0; o < p.pyr.n_oct; ++o) {
       const int iw = p.pyr.w[o] - 2 * kBorder, ih = p.pyr.h[o] - 2 * kBorder;
       if (iw <= 0 || ih <= 0) continue;
       sift_extrema_kernel<<<dim3((iw + 31) / 32, (ih + 7) / 8, kLayers * frames), dim3(32, 8), 0, st>>>(
-          p.pyr, o, cand, cap, counters);
+          lay, o, cand, cap, counters);
     }
     SOD_CHECK_LAUNCH("sift_extrema_kernel");
     // sms * 8 blocks in all, as for one frame, split over the frames' slabs
-    sift_orient_kernel<<<dim3((sms * 8 + frames - 1) / frames, frames), 32 * kOriWarps, 0, st>>>(p.pyr, cand, cap,
+    sift_orient_kernel<<<dim3((sms * 8 + frames - 1) / frames, frames), 32 * kOriWarps, 0, st>>>(lay, cand, cap,
                                                                                              counters, raw);
     SOD_CHECK_LAUNCH("sift_orient_kernel");
   }
@@ -804,11 +973,28 @@ int extract_frames(const uint8_t* gray, int width, int height, int64_t pitch, in
   sift_emit_kernel<<<blocks, 256, 0, st>>>(raw, cap, slots, vals, keep, pos, out);
   SOD_CHECK_LAUNCH("sift_emit_kernel");
   if (p.pyr.n_oct > 0) {
-    sift_descriptor_kernel<<<sms * 16, 128, 0, st>>>(p.pyr, out.xy, out.size, out.angle, out.octave, out.frame,
+    sift_descriptor_kernel<<<sms * 16, 128, 0, st>>>(lay, out.xy, out.size, out.angle, out.octave, out.frame,
                                                      out.cap_rows, batch, out.des, nullptr);
     SOD_CHECK_LAUNCH("sift_descriptor_kernel");
   }
   return SOD_OK;
+}
+
+// extract_frames of `frames` images of one size, image f at gray + f x frame_stride.
+int extract_uniform(const uint8_t* gray, int width, int height, int64_t pitch, int64_t frame_stride, Plan& p,
+                    int64_t max_per_frame, const Rows& out, void* workspace, cudaStream_t st) {
+  p.pyr.base = (float*)workspace;
+  return extract_frames(p.pyr, UniformSteps{gray, width, height, pitch, frame_stride, p.pyr}, p, max_per_frame, out,
+                        workspace, st);
+}
+
+// Copies the geometry table of a mixed batch from the kernel parameter into the workspace, so that the call
+// needs no host-to-device copy and stays capturable.  One block.
+__global__ void sift_mixed_setup_kernel(const __grid_constant__ MixedTable t, int frames, FrameGeom* __restrict__ g) {
+  static_assert(sizeof(FrameGeom) % sizeof(int) == 0, "FrameGeom is copied as ints");
+  const int n = frames * (int)(sizeof(FrameGeom) / sizeof(int));
+  const int* src = (const int*)t.f;
+  for (int i = threadIdx.x; i < n; i += blockDim.x) ((int*)g)[i] = src[i];
 }
 
 int check_image(const uint8_t* gray, int32_t width, int32_t height, int64_t pitch, const char* fn) {
@@ -817,6 +1003,25 @@ int check_image(const uint8_t* gray, int32_t width, int32_t height, int64_t pitc
   SOD_CHECK_ARG(pitch >= width, "%s: pitch %lld < width %d", fn, (long long)pitch, width);
   SOD_CHECK_ARG(gray != nullptr, "%s: null image", fn);
   return SOD_OK;
+}
+
+int check_batch_out(const sod_sift_batch_out* out, int32_t frames, const char* fn) {
+  SOD_CHECK_ARG(out != nullptr, "%s: null out", fn);
+  SOD_CHECK_ARG(out->cap_per_frame >= 1 && out->cap_per_frame <= SOD_SIFT_MAX_CAP &&
+                    frames * out->cap_per_frame <= SOD_SIFT_MAX_CAP,
+                "%s: cap_per_frame %lld out of range (1..%d / frames)", fn, (long long)out->cap_per_frame,
+                SOD_SIFT_MAX_CAP);
+  SOD_CHECK_ARG(out->cap_rows >= 1 && out->cap_rows <= SOD_SIFT_MAX_CAP, "%s: cap_rows %lld out of range (1..%d)",
+                fn, (long long)out->cap_rows, SOD_SIFT_MAX_CAP);
+  SOD_CHECK_ARG(out->xy && out->size && out->angle && out->response && out->octave && out->des && out->frame &&
+                    out->count && out->offset && out->overflow && out->rows_overflow,
+                "%s: null output array", fn);
+  return SOD_OK;
+}
+
+Rows batch_rows(const sod_sift_batch_out* out) {
+  return Rows{out->xy,    out->size,  out->angle,  out->response,   out->octave, out->des,
+              out->frame, out->count, out->offset, out->overflow, out->rows_overflow, out->cap_rows};
 }
 
 }  // namespace
@@ -871,7 +1076,7 @@ int sod_sift_extract(const uint8_t* gray, int32_t width, int32_t height, int64_t
   const Rows rows{out->xy,       out->size,         out->angle,  out->response,
                   out->octave,   out->des,          nullptr,     out->counters,
                   (int32_t*)((char*)workspace + p.offset), out->counters + 1, nullptr, out->cap};
-  return extract_frames(gray, width, height, pitch, (int64_t)pitch * height, p, 0, rows, workspace,
+  return extract_uniform(gray, width, height, pitch, (int64_t)pitch * height, p, 0, rows, workspace,
                         (cudaStream_t)stream);
 }
 
@@ -885,24 +1090,13 @@ int sod_sift_extract_batch(const uint8_t* gray, int32_t width, int32_t height, i
   SOD_CHECK_ARG(frame_stride >= pitch * height, "%s: frame_stride %lld < pitch x height %lld", fn,
                 (long long)frame_stride, (long long)(pitch * height));
   SOD_CHECK_ARG(max_per_frame >= 0, "%s: max_per_frame %lld < 0", fn, (long long)max_per_frame);
-  SOD_CHECK_ARG(out != nullptr, "%s: null out", fn);
-  SOD_CHECK_ARG(out->cap_per_frame >= 1 && out->cap_per_frame <= SOD_SIFT_MAX_CAP &&
-                    frames * out->cap_per_frame <= SOD_SIFT_MAX_CAP,
-                "%s: cap_per_frame %lld out of range (1..%d / frames)", fn, (long long)out->cap_per_frame,
-                SOD_SIFT_MAX_CAP);
-  SOD_CHECK_ARG(out->cap_rows >= 1 && out->cap_rows <= SOD_SIFT_MAX_CAP, "%s: cap_rows %lld out of range (1..%d)",
-                fn, (long long)out->cap_rows, SOD_SIFT_MAX_CAP);
-  SOD_CHECK_ARG(out->xy && out->size && out->angle && out->response && out->octave && out->des && out->frame &&
-                    out->count && out->offset && out->overflow && out->rows_overflow,
-                "%s: null output array", fn);
+  if (int rc = check_batch_out(out, frames, fn)) return rc;
   Plan p;
   SOD_CHECK_ARG(make_plan(width, height, frames, out->cap_per_frame, &p), "%s: too many octaves", fn);
   SOD_CHECK_ARG(workspace != nullptr && workspace_bytes >= p.total && ((uintptr_t)workspace & 255) == 0,
                 "%s: workspace of %zu bytes at %p; need %zu bytes, 256-byte aligned", fn, workspace_bytes, workspace,
                 p.total);
-  const Rows rows{out->xy,    out->size,  out->angle,  out->response,   out->octave, out->des,
-                  out->frame, out->count, out->offset, out->overflow, out->rows_overflow, out->cap_rows};
-  return extract_frames(gray, width, height, pitch, frame_stride, p, max_per_frame, rows, workspace,
+  return extract_uniform(gray, width, height, pitch, frame_stride, p, max_per_frame, batch_rows(out), workspace,
                         (cudaStream_t)stream);
 }
 
@@ -922,13 +1116,58 @@ int sod_sift_describe(const uint8_t* gray, int32_t width, int32_t height, int64_
   cudaStream_t st = (cudaStream_t)stream;
   p.pyr.base = (float*)workspace;
   if (p.pyr.n_oct > 0)
-    if (int rc = build_pyramid(gray, width, height, pitch, (int64_t)pitch * height, 1, p.pyr, st)) return rc;
+    if (int rc = build_pyramid(UniformSteps{gray, width, height, pitch, (int64_t)pitch * height, p.pyr}, p.pyr, 1, st))
+      return rc;
   const int sms = device_sm_count();
   if (sms < 0) return SOD_ERR_CUDA;
   sift_descriptor_kernel<<<sms * 16, 128, 0, st>>>(p.pyr, xy, size, angle, octave, nullptr, n, nullptr, des,
                                                    n_invalid);
   SOD_CHECK_LAUNCH("sift_descriptor_kernel");
   return SOD_OK;
+}
+
+size_t sod_sift_mixed_workspace_bytes(const int32_t* wh_host, int32_t frames, int64_t cap_per_frame) {
+  if (wh_host == nullptr || frames < 1 || frames > SOD_SIFT_MAX_MIXED_FRAMES || cap_per_frame < 0 ||
+      cap_per_frame > SOD_SIFT_MAX_CAP || frames * cap_per_frame > SOD_SIFT_MAX_CAP)
+    return 0;
+  for (int f = 0; f < frames; ++f)
+    if (wh_host[2 * f] < 1 || wh_host[2 * f + 1] < 1 || wh_host[2 * f] > kMaxSide || wh_host[2 * f + 1] > kMaxSide)
+      return 0;
+  Plan p;
+  MixedTable t;
+  return make_mixed_plan(wh_host, frames, cap_per_frame, &p, &t) ? p.total : 0;
+}
+
+int sod_sift_extract_mixed(const uint8_t* const* images_host, const int32_t* wh_host, const int64_t* pitch_host,
+                           int32_t frames, int64_t max_per_frame, const sod_sift_batch_out* out, void* workspace,
+                           size_t workspace_bytes, sod_stream_t stream) {
+  const char* fn = "sod_sift_extract_mixed";
+  SOD_CHECK_ARG(images_host && wh_host && pitch_host, "%s: null image, size or pitch array", fn);
+  SOD_CHECK_ARG(frames >= 1 && frames <= SOD_SIFT_MAX_MIXED_FRAMES, "%s: frames %d out of range (1..%d)", fn, frames,
+                SOD_SIFT_MAX_MIXED_FRAMES);
+  char what[64];
+  for (int f = 0; f < frames; ++f) {
+    snprintf(what, sizeof what, "%s: frame %d", fn, f);
+    if (int rc = check_image(images_host[f], wh_host[2 * f], wh_host[2 * f + 1], pitch_host[f], what)) return rc;
+  }
+  SOD_CHECK_ARG(max_per_frame >= 0, "%s: max_per_frame %lld < 0", fn, (long long)max_per_frame);
+  if (int rc = check_batch_out(out, frames, fn)) return rc;
+  Plan p;
+  MixedTable t;
+  SOD_CHECK_ARG(make_mixed_plan(wh_host, frames, out->cap_per_frame, &p, &t), "%s: too many octaves", fn);
+  SOD_CHECK_ARG(workspace != nullptr && workspace_bytes >= p.total && ((uintptr_t)workspace & 255) == 0,
+                "%s: workspace of %zu bytes at %p; need %zu bytes, 256-byte aligned", fn, workspace_bytes, workspace,
+                p.total);
+  for (int f = 0; f < frames; ++f) {
+    t.f[f].img = images_host[f];
+    t.f[f].pitch = pitch_host[f];
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  FrameGeom* g = (FrameGeom*)((char*)workspace + p.geom);
+  sift_mixed_setup_kernel<<<1, 256, 0, st>>>(t, frames, g);
+  SOD_CHECK_LAUNCH("sift_mixed_setup_kernel");
+  const Mixed M{(float*)workspace, g, frames};
+  return extract_frames(M, MixedSteps{M}, p, max_per_frame, batch_rows(out), workspace, st);
 }
 
 }  // extern "C"

@@ -144,7 +144,11 @@ _PROTOS = {
     "sod_sift_batch_workspace_bytes": (C.c_size_t, [_i32, _i32, _i32, _i64]),
     "sod_sift_extract_batch": (C.c_int, [_p, _i32, _i32, _i64, _i64, _i32, _i64, C.POINTER(SiftBatchOut), _p,
                                          C.c_size_t, _p]),
+    "sod_sift_mixed_workspace_bytes": (C.c_size_t, [_p, _i32, _i64]),
+    "sod_sift_extract_mixed": (C.c_int, [_p, _p, _p, _i32, _i64, C.POINTER(SiftBatchOut), _p, C.c_size_t, _p]),
 }
+
+SIFT_MAX_MIXED_FRAMES = 64
 
 
 def _bind() -> None:

@@ -7,12 +7,14 @@ and the reference; DESIGN.md 2 states how closely this one agrees with it.
 
 GpuSift.extract_batch runs many same-size frames in one pass (sod_sift_extract_batch) and leaves the result on the
 device, in the layout DetectionPipeline.load_queries takes; FrameStream uses it when the extractor has it.
+GpuSift.extract_mixed does the same for frames of different sizes (sod_sift_extract_mixed), such as the training
+images GenerateDatabaseInfo.build_database resizes to one width.
 """
 from __future__ import annotations
 
 import ctypes as C
 import threading
-from dataclasses import dataclass
+from dataclasses import dataclass, field
 
 import numpy as np
 
@@ -42,12 +44,13 @@ def _is_cuda(x) -> bool:
 
 @dataclass
 class SiftBatch:
-    """The keypoints of a batch of same-size frames, packed frame after frame on the device.
+    """The keypoints of a batch of frames, packed frame after frame on the device.
 
     des u8 [rows, 128], xy f32 [rows, 2], angle, size, response f32 [rows], octave, frame i32 [rows]: frame k's
     keypoints are rows offset[k]:offset[k] + count[k] (host arrays), in the order GpuSift.extract gives for that
-    frame alone.  The tensors are GpuSift's buffers: the next extract_batch of the same size, batch and slot
-    overwrites them."""
+    frame alone.  frame_size is the (w, h) of a same-size batch (None for a mixed one); frame_sizes (int [B, 2], None for a same-size
+    batch) gives each frame's own (w, h).  The tensors are GpuSift's buffers: the next extract_batch of the same
+    size, batch and slot, or the next extract_mixed of the same slot, overwrites them."""
     des: object
     xy: object
     angle: object
@@ -58,6 +61,7 @@ class SiftBatch:
     count: np.ndarray
     offset: np.ndarray
     frame_size: tuple
+    frame_sizes: np.ndarray | None = field(default=None)
 
     def __len__(self) -> int:
         return len(self.count)
@@ -71,8 +75,14 @@ class SiftBatch:
         lo, hi = int(self.offset[k]), int(self.offset[k] + self.count[k])
         out = {name: getattr(self, name)[lo:hi].cpu().numpy()
                for name in ("xy", "size", "angle", "response", "octave", "des")}
-        out["frame_size"] = self.frame_size
+        out["frame_size"] = self.size_of(k)
         return out
+
+    def size_of(self, k: int) -> tuple:
+        """Frame k's (w, h)."""
+        if self.frame_sizes is None:
+            return self.frame_size
+        return int(self.frame_sizes[k][0]), int(self.frame_sizes[k][1])
 
     def features(self, k: int) -> FrameFeatures:
         r = self.arrays(k)
@@ -111,6 +121,48 @@ class _BatchBuffers:
                                     fl[3 * f:].data_ptr(), r, self.capacity)
             self.outs[slot] = (t, st)
         return self.outs[slot]
+
+
+class _MixedBuffers:
+    """One output slot of extract_mixed: device workspace, device input arena, pinned staging and packed output
+    rows, each grown to the largest batch seen and reused for any mix that fits, whatever its sizes."""
+
+    def __init__(self, device):
+        self.device = device
+        self.ws = self.arena = self.host = self.t = self.out = self.flags = None
+        self.frames = 0
+
+    def _mk(self, shape, dt):
+        import torch
+        return torch.empty(shape, dtype=dt, device=self.device)
+
+    def fit(self, ws_bytes: int, arena_bytes: int, frames: int, capacity: int, max_keypoints: int | None) -> None:
+        import torch
+        if self.ws is None or self.ws.numel() < ws_bytes:
+            self.ws = None                    # release before allocating the larger one
+            self.ws = self._mk(ws_bytes, torch.uint8)
+        if arena_bytes and (self.arena is None or self.arena.numel() < arena_bytes):
+            self.arena = self.host = None
+            self.arena = self._mk(arena_bytes, torch.uint8)
+            self.host = torch.empty(arena_bytes, dtype=torch.uint8, pin_memory=True)
+        if frames > self.frames:
+            self.t = self.out = None
+            f, r = frames, frames * (capacity if max_keypoints is None else min(capacity, max(1, int(max_keypoints))))
+            mk = self._mk
+            t = dict(xy=mk((r, 2), torch.float32), size=mk(r, torch.float32), angle=mk(r, torch.float32),
+                     response=mk(r, torch.float32), octave=mk(r, torch.int32), des=mk((r, 128), torch.uint8),
+                     frame=mk(r, torch.int32), flags=mk(3 * f + 1, torch.int32))
+            fl = t["flags"]
+            self.out = _capi.SiftBatchOut(*(t[k].data_ptr() for k in ("xy", "size", "angle", "response", "octave",
+                                                                       "des", "frame")),
+                                          fl[:f].data_ptr(), fl[f:2 * f].data_ptr(), fl[2 * f:3 * f].data_ptr(),
+                                          fl[3 * f:].data_ptr(), r, capacity)
+            self.t, self.frames = t, frames
+            self.flags = torch.empty((3 * f + 1,), dtype=torch.int32, pin_memory=True)
+
+
+def _align256(n: int) -> int:
+    return (n + 255) & ~255
 
 
 class _Buffers:
@@ -157,6 +209,7 @@ class GpuSift:
         self._stream = None
         self._buffers: dict[tuple[int, int], _Buffers] = {}
         self._batch_buffers: dict[tuple[int, int, int], _BatchBuffers] = {}
+        self._mixed: list[_MixedBuffers | None] = [None, None]
 
     def _setup_stream(self) -> None:
         import torch
@@ -280,6 +333,95 @@ class GpuSift:
         rows = int(count.sum())
         return SiftBatch(t["des"][:rows], t["xy"][:rows], t["angle"][:rows], t["octave"][:rows], t["size"][:rows],
                          t["response"][:rows], t["frame"][:rows], count, offset, (w, h))
+
+    def extract_mixed(self, images, slot: int = 0) -> SiftBatch:
+        """SIFT of a batch of frames of any sizes in one pass (sod_sift_extract_mixed), the result left on the device.
+
+        images  a list of up to 64 frames, each a CUDA u8 [H, W] tensor (pitched or not) or a host image / path
+                (decoded and converted as extract does)
+        slot    0 or 1: which of two output sets to fill
+
+        Frame k's rows are those extract gives for it alone, in the same order; SiftBatch.frame_sizes holds each
+        frame's (w, h).  The buffers of a slot are grown to the largest batch seen, not kept per size.  Waits for
+        the batch; a frame with more than `capacity` keypoints raises SodError naming it."""
+        import torch
+        if slot not in (0, 1):
+            raise ValueError("slot must be 0 or 1")
+        frames = [self.prepare(im) for im in images]
+        n = len(frames)
+        if not 1 <= n <= _capi.SIFT_MAX_MIXED_FRAMES:
+            raise ValueError(f"extract_mixed takes 1..{_capi.SIFT_MAX_MIXED_FRAMES} frames, got {n}")
+        for k, f in enumerate(frames):
+            if f.ndim != 2 or (f.dtype != torch.uint8 if _is_cuda(f) else f.dtype != np.uint8):
+                raise ValueError(f"frame {k}: expected a u8 [H, W] image, got {f.dtype} {tuple(f.shape)}")
+        sizes = np.array([(f.shape[1], f.shape[0]) for f in frames], np.int32)
+        wh = (C.c_int32 * (2 * n))(*sizes.reshape(-1).tolist())
+        need = int(_capi.lib.sod_sift_mixed_workspace_bytes(C.cast(wh, C.c_void_p), n, self.capacity))
+        if need == 0:
+            raise ValueError(f"sod_sift: {n} frames of sizes {sizes.tolist()} with capacity {self.capacity} out of "
+                             "range")
+        # frames that need a copy (host images, CUDA tensors whose rows are not unit-stride) go to the arena,
+        # each at a 256-byte aligned offset with pitch = width
+        in_place = [_is_cuda(f) and f.stride(1) == 1 and f.stride(0) >= f.shape[1] for f in frames]
+        at, arena_off = 0, []
+        for f, keep in zip(frames, in_place):
+            arena_off.append(at)
+            if not keep:
+                at += _align256(f.shape[0] * f.shape[1])
+        with self._lock, torch.cuda.device(self._device or torch.cuda.current_device()):
+            self._setup_stream()
+            b = self._mixed[slot]
+            if b is None:
+                b = self._mixed[slot] = _MixedBuffers(self._device)
+            b.fit(need, at, n, self.capacity, self.max_keypoints)
+            if any(_is_cuda(f) for f in frames):
+                self._stream.wait_stream(torch.cuda.current_stream())
+            ptrs, pitches = [], []
+            try:
+                with torch.cuda.stream(self._stream):
+                    host = [k for k, f in enumerate(frames) if not _is_cuda(f)]
+                    for k in host:
+                        h, w = frames[k].shape
+                        b.host[arena_off[k]:arena_off[k] + h * w].copy_(torch.from_numpy(frames[k]).reshape(-1))
+                    if host:
+                        b.arena[:at].copy_(b.host[:at], non_blocking=True)
+                    for k, f in enumerate(frames):
+                        h, w = f.shape
+                        if _is_cuda(f) and f.device != b.ws.device:
+                            raise ValueError(f"frame {k} is on {f.device}, GpuSift on {b.ws.device}")
+                        if in_place[k]:
+                            ptrs.append(f.data_ptr())
+                            pitches.append(f.stride(0))
+                            continue
+                        if _is_cuda(f):
+                            b.arena[arena_off[k]:arena_off[k] + h * w].view(h, w).copy_(f)
+                        ptrs.append(b.arena[arena_off[k]:].data_ptr())
+                        pitches.append(w)
+                    mk = 0 if self.max_keypoints is None else max(1, int(self.max_keypoints))
+                    _capi.check(_capi.lib.sod_sift_extract_mixed(
+                        C.cast((C.c_void_p * n)(*ptrs), C.c_void_p), C.cast(wh, C.c_void_p),
+                        C.cast((C.c_int64 * n)(*pitches), C.c_void_p), n, mk, C.byref(b.out), b.ws.data_ptr(),
+                        b.ws.numel(), self._stream.cuda_stream), "sod_sift_extract_mixed")
+                    b.flags.copy_(b.t["flags"], non_blocking=True)
+            finally:
+                # as in extract_batch: once this returns the rows may be read on any stream and the buffers are
+                # free; also when a step above raised, since the pinned staging may still be in a copy
+                self._stream.synchronize()
+            fl, F = b.flags.numpy(), b.frames
+            count, offset = fl[:n].astype(np.int64), fl[F:F + n].astype(np.int64)
+            overflow, rows_overflow = fl[2 * F:2 * F + n].copy(), int(fl[3 * F])
+            t = b.t
+        bad = np.nonzero(overflow)[0]
+        if len(bad):
+            k = int(bad[0])
+            raise _capi.SodError(f"sod_sift_extract_mixed: more than capacity={self.capacity} keypoints in frame {k} "
+                                 f"({sizes[k][0]}x{sizes[k][1]}) of the batch; use a larger GpuSift(capacity=...)")
+        if rows_overflow:
+            raise _capi.SodError("sod_sift_extract_mixed: the packed rows exceed the output buffers")
+        rows = int(count.sum())
+        return SiftBatch(t["des"][:rows], t["xy"][:rows], t["angle"][:rows], t["octave"][:rows], t["size"][:rows],
+                         t["response"][:rows], t["frame"][:rows], count, offset, None,
+                         frame_sizes=sizes.astype(np.int64))
 
     def __call__(self, image) -> FrameFeatures:
         r = self.extract(image)

@@ -11,8 +11,14 @@ frame (144 MB) does not fit the 126 MB L2, smaller ones mostly do (stated per si
 
 Batch leg: device time per frame of sod_sift_extract_batch at B = 1, 4 and 16 distinct frames per size (input
 already on the device), and FrameStream frames/s through the batched device path.  With --parent-lib, the device
-time of sod_sift_extract of that library and of this tree's, each in its own process, alternated --ab-rounds
-times.
+time of sod_sift_extract and of sod_sift_extract_batch (16 frames) of that library and of this tree's, each in its
+own process, alternated --ab-rounds times.
+
+--mixed runs only the mixed-size legs (and the A/B with --parent-lib): device time per frame of 16 distinct frames
+of assorted sizes through sod_sift_extract_mixed, through sod_sift_extract one frame at a time and through
+sod_sift_extract_batch grouped by size; the same for a skewed mix (one 2000x1500 frame and fifteen 64x48 ones,
+where most blocks of the largest-frame grids are empty); and GenerateDatabaseInfo.build_database images/s on a
+folder of synthetic PNGs of distinct heights, GPU against cv2.
 """
 import argparse
 import ctypes as C
@@ -20,6 +26,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import time
 from pathlib import Path
 
@@ -137,6 +144,12 @@ def single_extract_ms(lib_path, reps):
     lib.sod_sift_extract.restype = C.c_int
     lib.sod_sift_extract.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.POINTER(_capi.SiftOut),
                                      C.c_void_p, C.c_size_t, C.c_void_p]
+    lib.sod_sift_batch_workspace_bytes.restype = C.c_size_t
+    lib.sod_sift_batch_workspace_bytes.argtypes = [C.c_int32, C.c_int32, C.c_int32, C.c_int64]
+    lib.sod_sift_extract_batch.restype = C.c_int
+    lib.sod_sift_extract_batch.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_int64, C.c_int32,
+                                           C.c_int64, C.POINTER(_capi.SiftBatchOut), C.c_void_p, C.c_size_t,
+                                           C.c_void_p]
     st, cap, out = torch.cuda.Stream(), 1 << 16, {}
     for (w, h) in SIZES:
         gray = imaging.textured(np.random.default_rng(w), w, h, shapes=200)
@@ -158,6 +171,34 @@ def single_extract_ms(lib_path, reps):
         n, overflow = (int(v) for v in arrays[-1].cpu())
         out[f"{w}x{h}_keypoints"] = n
         assert not overflow
+        del ws, arrays
+        # sod_sift_extract_batch of 16 distinct frames of this size, per frame
+        B, bcap = 16, 1 << 15
+        rng = np.random.default_rng(w + 1)
+        imgs = torch.from_numpy(np.stack([imaging.textured(rng, w, h, shapes=200) for _ in range(B)])).cuda()
+        nbytes = int(lib.sod_sift_batch_workspace_bytes(w, h, B, bcap))
+        ws = torch.empty(nbytes, dtype=torch.uint8, device="cuda")
+        rows = B * bcap
+        t = [torch.empty(s, dtype=dt, device="cuda") for s, dt in
+             (((rows, 2), torch.float32), (rows, torch.float32), (rows, torch.float32), (rows, torch.float32),
+              (rows, torch.int32), ((rows, 128), torch.uint8), (rows, torch.int32), (3 * B + 1, torch.int32))]
+        fl = t[-1]
+        bo = _capi.SiftBatchOut(*(x.data_ptr() for x in t[:7]), fl[:B].data_ptr(), fl[B:2 * B].data_ptr(),
+                                fl[2 * B:3 * B].data_ptr(), fl[3 * B:].data_ptr(), rows, bcap)
+        torch.cuda.synchronize()
+
+        def batch():
+            if lib.sod_sift_extract_batch(imgs.data_ptr(), w, h, w, w * h, B, 0, C.byref(bo), ws.data_ptr(), nbytes,
+                                          st.cuda_stream):
+                raise RuntimeError(f"sod_sift_extract_batch failed in {lib_path}")
+
+        device_ms(st, batch, 2)
+        out[f"batch16_{w}x{h}_per_frame"] = device_ms(st, batch, max(3, reps // 4)) / B
+        f = fl.cpu().numpy()
+        assert not f[2 * B:].any()
+        out[f"batch16_{w}x{h}_keypoints"] = int(f[:B].sum())
+        del ws, t, imgs
+        torch.cuda.empty_cache()
     return out
 
 
@@ -173,6 +214,100 @@ def ab_single(parent_lib, rounds, reps):
             runs[name].append(json.loads(r.stdout.strip().splitlines()[-1]))
     med = {name: {k: float(np.median([r[k] for r in v])) for k in v[0]} for name, v in runs.items()}
     return dict(rounds=runs, median_ms=med)
+
+
+MIXED_SIZES = ((640, 480), (640, 480), (640, 480), (640, 480), (800, 600), (800, 600), (800, 600), (1200, 900),
+               (1200, 900), (1200, 900), (480, 640), (480, 640), (1600, 1200), (1600, 1200), (2000, 1500),
+               (2000, 1500))
+SKEWED_SIZES = ((2000, 1500),) + ((64, 48),) * 15
+
+
+def mixed_per_frame(sizes, reps, seed):
+    """Device ms per frame of one mixed batch of these (distinct) frames: sod_sift_extract_mixed, sod_sift_extract
+    of each frame in turn, and sod_sift_extract_batch of the frames grouped by size.  Inputs on the device."""
+    lib = _capi.lib
+    rng = np.random.default_rng(seed)
+    frames = [imaging.textured(rng, w, h, shapes=200) for w, h in sizes]
+    dev = [torch.from_numpy(f).cuda() for f in frames]
+    n = len(frames)
+    gpu = GpuSift()
+    mb = gpu.extract_mixed(dev)
+    b = gpu._mixed[0]
+    st = gpu._stream
+    wh = (C.c_int32 * (2 * n))(*[v for s in sizes for v in s])
+    ptrs = (C.c_void_p * n)(*[d.data_ptr() for d in dev])
+    pitch = (C.c_int64 * n)(*[w for w, _ in sizes])
+
+    def mixed():
+        _capi.check(lib.sod_sift_extract_mixed(C.cast(ptrs, C.c_void_p), C.cast(wh, C.c_void_p),
+                                               C.cast(pitch, C.c_void_p), n, 0, C.byref(b.out), b.ws.data_ptr(),
+                                               b.ws.numel(), st.cuda_stream), "sod_sift_extract_mixed")
+
+    singles = []
+    for f in frames:
+        gpu.extract(f)
+    for d, (w, h) in zip(dev, sizes):
+        sb = gpu._buffers[(w, h)]
+        singles.append((d, w, h, sb))
+
+    def one_by_one():
+        for d, w, h, sb in singles:
+            _capi.check(lib.sod_sift_extract(d.data_ptr(), w, h, w, C.byref(sb.out), sb.ws.data_ptr(), sb.bytes,
+                                             st.cuda_stream), "sod_sift_extract")
+
+    groups = {}
+    for k, s in enumerate(sizes):
+        groups.setdefault(s, []).append(k)
+    grouped = []
+    for (w, h), ks in groups.items():
+        stacked = torch.stack([dev[k] for k in ks]).contiguous()
+        gpu.extract_batch(stacked)
+        bb = gpu._batch_buffers[(w, h, len(ks))]
+        grouped.append((stacked, w, h, len(ks), bb, bb.out(0)[1]))
+
+    def by_size():
+        for x, w, h, m, bb, so in grouped:
+            _capi.check(lib.sod_sift_extract_batch(x.data_ptr(), w, h, w, w * h, m, 0, C.byref(so), bb.ws.data_ptr(),
+                                                   bb.bytes, st.cuda_stream), "sod_sift_extract_batch")
+
+    torch.cuda.synchronize()
+    out = dict(frames=n, sizes=[list(s) for s in sizes], keypoints=int(mb.rows), size_groups=len(groups),
+               mixed_workspace_bytes=int(b.ws.numel()))
+    for name, fn in (("mixed", mixed), ("single_each", one_by_one), ("batch_by_size", by_size)):
+        device_ms(st, fn, 2)
+        out[f"{name}_device_ms_per_frame"] = device_ms(st, fn, reps) / n
+    out["mixed_speedup_vs_single_each"] = out["single_each_device_ms_per_frame"] / out["mixed_device_ms_per_frame"]
+    out["mixed_speedup_vs_batch_by_size"] = out["batch_by_size_device_ms_per_frame"] / out["mixed_device_ms_per_frame"]
+    del gpu
+    torch.cuda.empty_cache()
+    return out
+
+
+def builder_fps(n_images):
+    """GenerateDatabaseInfo.build_database images/s, GPU (GpuSift) against cv2, on PNGs of distinct heights."""
+    import GenerateDatabaseInfo as G
+    rng = np.random.default_rng(9)
+    out = {}
+    with tempfile.TemporaryDirectory() as d:
+        for i in range(n_images):
+            img = imaging.textured(rng, 600, 300 + 5 * i, shapes=150)
+            cv2.imwrite(os.path.join(d, f"img_{i:04d}.png"), cv2.cvtColor(img, cv2.COLOR_GRAY2BGR))
+        warm = os.path.join(d, "warm")
+        os.mkdir(warm)
+        for i in range(3):
+            cv2.imwrite(os.path.join(warm, f"w{i}.png"), cv2.imread(os.path.join(d, f"img_{i:04d}.png")))
+        gpu = GpuSift()
+        G.build_database(warm, os.path.join(d, "w.pkl"), extractor=gpu)
+        G.build_database(warm, os.path.join(d, "w.pkl"))
+        for name, ex in (("gpu", gpu), ("cv2", None)):
+            t = time.perf_counter()
+            rows = G.build_database(d, os.path.join(d, f"{name}.pkl"), extractor=ex)
+            dt = time.perf_counter() - t
+            out[name] = dict(images=len(rows), seconds=dt, images_per_s=len(rows) / dt,
+                             keypoints=int(sum(len(r[0]) for r in rows)))
+    out["heights_after_resize"] = [int(1500 * (300 + 5 * i) / 600) for i in (0, n_images - 1)]
+    out["gpu_speedup_vs_cv2"] = out["gpu"]["images_per_s"] / out["cv2"]["images_per_s"]
+    return out
 
 
 def stream_fps(n_frames, workers):
@@ -222,6 +357,8 @@ def main():
     ap.add_argument("--parent-lib", default=None, help="another build of libsod_b200.so to compare sod_sift_extract with")
     ap.add_argument("--ab-rounds", type=int, default=3)
     ap.add_argument("--single-lib", default=None, help=argparse.SUPPRESS)
+    ap.add_argument("--mixed", action="store_true", help="only the mixed-size legs (and the A/B with --parent-lib)")
+    ap.add_argument("--builder-images", type=int, default=64)
     a = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("bench_sift.py needs a CUDA device")
@@ -232,6 +369,20 @@ def main():
                        capture_output=True, text=True).stdout.strip().splitlines()
     rec = dict(device=torch.cuda.get_device_name(0), nvidia_smi=q[0] if q else None, host_cpus=os.cpu_count(),
                cv2_version=cv2.__version__, cv2_threads=cv2.getNumThreads(), frames=[])
+    if a.mixed:
+        del rec["frames"]
+        rec["mixed_assorted"] = mixed_per_frame(MIXED_SIZES, a.reps, 31)
+        print(json.dumps(rec["mixed_assorted"]), flush=True)
+        rec["mixed_skewed"] = mixed_per_frame(SKEWED_SIZES, a.reps, 32)
+        print(json.dumps(rec["mixed_skewed"]), flush=True)
+        rec["build_database"] = builder_fps(a.builder_images)
+        print(json.dumps(rec["build_database"]), flush=True)
+        if a.parent_lib:
+            rec["single_frame_ab"] = ab_single(a.parent_lib, a.ab_rounds, a.reps)
+            print(json.dumps(rec["single_frame_ab"]["median_ms"]), flush=True)
+        Path(a.out).parent.mkdir(parents=True, exist_ok=True)
+        Path(a.out).write_text(json.dumps(rec, indent=1) + "\n")
+        return
     gpu = GpuSift()
     for (w, h) in SIZES:
         rec["frames"].append(per_frame(gpu, w, h, a.reps, a.host_reps))
