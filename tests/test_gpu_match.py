@@ -4,6 +4,7 @@ import pytest
 import torch
 
 from conftest import sift_like
+from exact_top2 import direct_d2, exact_top2
 from oracle import sod_oracle as O
 
 pytestmark = pytest.mark.gpu
@@ -110,17 +111,6 @@ def test_pack_from_f32_rejects_non_integer():
         E.pack_descriptors(x)
 
 
-def _gpu_reference_top2(q, db):
-    """Exact top-2 on the GPU itself (fp64 matmul is exact for these magnitudes; ties -> lowest index
-    through an integer key), used where the numpy oracle would take minutes."""
-    qf, tf = q.double(), db.double()
-    d2 = (qf * qf).sum(1)[:, None] + (tf * tf).sum(1)[None, :] - 2.0 * (qf @ tf.T)
-    key = d2.round().long() * (1 << 32) + torch.arange(db.shape[0], device=q.device)[None, :]
-    best = torch.topk(key, min(2, db.shape[0]), dim=1, largest=False, sorted=True).values
-    idx = (best & 0xFFFFFFFF).int()
-    return idx, (best >> 32).int()
-
-
 def test_random_shapes_soak():
     """Many random shapes, including the few-queries / large-database ones whose segments share their
     thresholds through global memory, each run twice: results must be exact and repeatable."""
@@ -137,8 +127,9 @@ def test_random_shapes_soak():
         m = E.Matcher(E.prepare_db(db))
         idx1, d1 = m.top2(q)
         idx2, d2 = m.top2(q)
-        ridx, rd = _gpu_reference_top2(q, db)
-        assert torch.equal(idx1[:, :ridx.shape[1]], ridx) and torch.equal(d1[:, :rd.shape[1]], rd), (nq, ndb, hi)
+        ridx, rd = exact_top2(q, db)
+        assert torch.equal(idx1, ridx) and torch.equal(d1, rd), (nq, ndb, hi)
+        assert torch.equal(direct_d2(q, db, idx1), d1), (nq, ndb, hi)
         assert torch.equal(idx1, idx2) and torch.equal(d1, d2), (nq, ndb, hi)
 
 

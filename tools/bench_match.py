@@ -1,4 +1,5 @@
 """Dev tool: time sod_match_top2 alone on device-resident inputs (CUDA events)."""
+import hashlib
 import os
 import sys
 from pathlib import Path
@@ -19,8 +20,13 @@ def sift_like_gpu(n, g):
     return (x * 512).round_().clamp_(0, 255).to(torch.uint8)
 
 
-def run(nq, ndb, iters=10, kind="uniform"):
-    g = torch.Generator(device="cuda").manual_seed(1)
+KINDS = ("uniform", "sift", "selfmatch", "cluster", "dup", "noevent")
+
+
+def make_inputs(kind, nq, ndb, g):
+    """(q, db) u8 [n,128] on the GPU for one data kind, drawn from generator g.  The timed legs below and the
+    tests (tests/test_gpu_match_scale.py) build their inputs here, so the data that is timed is the data
+    that is checked."""
     if kind == "uniform":
         q = torch.randint(0, 256, (nq, 128), dtype=torch.uint8, device="cuda", generator=g)
         db = torch.randint(0, 256, (ndb, 128), dtype=torch.uint8, device="cuda", generator=g)
@@ -52,8 +58,24 @@ def run(nq, ndb, iters=10, kind="uniform"):
         q = torch.zeros((nq, 128), dtype=torch.uint8, device="cuda")
         db = sift_like_gpu(ndb, g)
         db[:2] = 0
-    else:
+    elif kind == "sift":
         q, db = sift_like_gpu(nq, g), sift_like_gpu(ndb, g)
+    else:
+        raise ValueError(f"unknown input kind {kind!r}: one of {', '.join(KINDS)}")
+    return q, db
+
+
+def input_hash(q, db):
+    """First 16 hex digits of the SHA-256 of q's and db's bytes: identifies a leg's exact inputs."""
+    h = hashlib.sha256()
+    for t in (q, db):
+        h.update(t.contiguous().cpu().numpy().tobytes())
+    return h.hexdigest()[:16]
+
+
+def run(nq, ndb, iters=10, kind="uniform"):
+    g = torch.Generator(device="cuda").manual_seed(1)
+    q, db = make_inputs(kind, nq, ndb, g)
     m = E.Matcher(E.prepare_db(db))
     for _ in range(3):
         m.top2(q)
@@ -68,7 +90,7 @@ def run(nq, ndb, iters=10, kind="uniform"):
     ms = float(np.median(ts))
     ops = 2.0 * nq * ndb * 128
     print(f"{kind:>8} nq={nq:>8} ndb={ndb:>8}  {ms:9.3f} ms (min {min(ts):.3f})  {ops / ms / 1e9:8.1f} TOPS  "
-          f"{nq / ms * 1e3 / 1e6:8.3f} Mq/s", flush=True)
+          f"{nq / ms * 1e3 / 1e6:8.3f} Mq/s  inputs {input_hash(q, db)}", flush=True)
 
 
 def run_float(nq, ndb, split, iters=10):
