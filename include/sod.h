@@ -283,6 +283,15 @@ size_t sod_compact_scratch_bytes(int64_t n_query);
 int sod_compact_matches(const int32_t* idx, const uint8_t* pass, int64_t n_query, int32_t t_lo,
                         int32_t t_hi, int32_t* match_q, int32_t* match_t, int32_t* n_out,
                         void* scratch, sod_stream_t stream);
+/* sod_compact_matches over the first *n_query_dev rows of n_query_cap, the row count read on the device: it
+ * replaces the host-side n_query where the count is only known on the device (a frame's SIFT output inside a
+ * captured CUDA graph), so the rows between the count and the capacity need no clearing - they are treated as
+ * not passing, whatever idx / pass hold there.  n_query_dev is a device int32; a value outside [0, n_query_cap]
+ * is clamped to that range (a -DSOD_DEVICE_CHECKS build traps on it).  Every pointer must be non-NULL;
+ * n_query_cap == 0 zeroes n_out.  scratch: sod_compact_scratch_bytes(n_query_cap). */
+int sod_compact_matches_dev(const int32_t* idx, const uint8_t* pass, int64_t n_query_cap,
+                            const int32_t* n_query_dev, int32_t t_lo, int32_t t_hi, int32_t* match_q,
+                            int32_t* match_t, int32_t* n_out, void* scratch, sod_stream_t stream);
 
 /* estimate_object_pose + calculate_bin_index only (HoughTransformHelperFunctions.py:4-72), no voting:
  * pose [n][4] and base_bin [n] as in sod_hough_out; near_edge may be NULL. */

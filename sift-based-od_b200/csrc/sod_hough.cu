@@ -874,12 +874,25 @@ __global__ void __launch_bounds__(kHugeThreads, 1) hough_finish_huge_kernel(cons
 // ------------------------------------------------------------------------------ compaction
 constexpr int kCompactThreads = 1024;
 
+// Rows a compaction covers: all n, or with kDevCount the first *n_dev of them (read on the device, so that a
+// captured graph can take the row count of the frame it replays), clamped to [0, n].
+template <bool kDevCount>
+__device__ __forceinline__ int64_t compact_rows(int64_t n, const int32_t* n_dev) {
+  if (!kDevCount) return n;
+  const int64_t v = *n_dev;
+  SOD_DCHECK(v >= 0 && v <= n);
+  return v < 0 ? 0 : (v > n ? n : v);
+}
+
+template <bool kDevCount>
 __global__ void __launch_bounds__(kCompactThreads)
 compact_count_kernel(const int32_t* __restrict__ idx, const uint8_t* __restrict__ pass, int64_t n,
-                     int32_t t_lo, int32_t t_hi, int32_t* __restrict__ block_counts) {
+                     const int32_t* __restrict__ n_dev, int32_t t_lo, int32_t t_hi,
+                     int32_t* __restrict__ block_counts) {
   __shared__ int s;
   if (threadIdx.x == 0) s = 0;
   __syncthreads();
+  n = compact_rows<kDevCount>(n, n_dev);
   const int64_t i = static_cast<int64_t>(blockIdx.x) * kCompactThreads + threadIdx.x;
   bool keep = i < n && pass[i];
   if (keep) {
@@ -892,12 +905,15 @@ compact_count_kernel(const int32_t* __restrict__ idx, const uint8_t* __restrict_
   if (threadIdx.x == 0) block_counts[blockIdx.x] = s;
 }
 
+template <bool kDevCount>
 __global__ void __launch_bounds__(kCompactThreads)
 compact_write_kernel(const int32_t* __restrict__ idx, const uint8_t* __restrict__ pass, int64_t n,
-                     int32_t t_lo, int32_t t_hi, const int32_t* __restrict__ block_off,
-                     int32_t* __restrict__ match_q, int32_t* __restrict__ match_t) {
+                     const int32_t* __restrict__ n_dev, int32_t t_lo, int32_t t_hi,
+                     const int32_t* __restrict__ block_off, int32_t* __restrict__ match_q,
+                     int32_t* __restrict__ match_t) {
   __shared__ int warp_base[kCompactThreads / 32];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  n = compact_rows<kDevCount>(n, n_dev);
   const int64_t i = static_cast<int64_t>(blockIdx.x) * kCompactThreads + threadIdx.x;
   bool keep = i < n && pass[i];
   int32_t t = 0;
@@ -919,6 +935,25 @@ compact_write_kernel(const int32_t* __restrict__ idx, const uint8_t* __restrict_
     match_q[pos] = static_cast<int32_t>(i);
     match_t[pos] = t;
   }
+}
+
+// count -> scan of the block counts -> write, over n rows (the first *n_dev of them with kDevCount).
+template <bool kDevCount>
+int launch_compact(const int32_t* idx, const uint8_t* pass, int64_t n, const int32_t* n_dev, int32_t t_lo,
+                   int32_t t_hi, int32_t* match_q, int32_t* match_t, int32_t* n_out, void* scratch,
+                   cudaStream_t st) {
+  const int64_t blocks = (n + kCompactThreads - 1) / kCompactThreads;
+  int32_t* counts = static_cast<int32_t*>(scratch);
+  int32_t* offs = counts + blocks + 1;
+  compact_count_kernel<kDevCount><<<static_cast<unsigned>(blocks), kCompactThreads, 0, st>>>(
+      idx, pass, n, n_dev, t_lo, t_hi, counts);
+  SOD_CHECK_LAUNCH("compact_count_kernel");
+  exclusive_scan_kernel<<<1, 1024, 0, st>>>(counts, blocks, offs, n_out, nullptr);
+  SOD_CHECK_LAUNCH("exclusive_scan_kernel");
+  compact_write_kernel<kDevCount><<<static_cast<unsigned>(blocks), kCompactThreads, 0, st>>>(
+      idx, pass, n, n_dev, t_lo, t_hi, offs, match_q, match_t);
+  SOD_CHECK_LAUNCH("compact_write_kernel");
+  return SOD_OK;
 }
 
 size_t align256(size_t x) { return (x + 255) & ~static_cast<size_t>(255); }
@@ -992,18 +1027,21 @@ int sod_compact_matches(const int32_t* idx, const uint8_t* pass, int64_t n_query
     return SOD_OK;
   }
   SOD_CHECK_ARG(idx && pass && match_q && match_t && scratch, "null pointer");
-  const int64_t blocks = (n_query + kCompactThreads - 1) / kCompactThreads;
-  int32_t* counts = static_cast<int32_t*>(scratch);
-  int32_t* offs = counts + blocks + 1;
-  compact_count_kernel<<<static_cast<unsigned>(blocks), kCompactThreads, 0, st>>>(idx, pass, n_query, t_lo,
-                                                                                  t_hi, counts);
-  SOD_CHECK_LAUNCH("compact_count_kernel");
-  exclusive_scan_kernel<<<1, 1024, 0, st>>>(counts, blocks, offs, n_out, nullptr);
-  SOD_CHECK_LAUNCH("exclusive_scan_kernel");
-  compact_write_kernel<<<static_cast<unsigned>(blocks), kCompactThreads, 0, st>>>(
-      idx, pass, n_query, t_lo, t_hi, offs, match_q, match_t);
-  SOD_CHECK_LAUNCH("compact_write_kernel");
-  return SOD_OK;
+  return launch_compact<false>(idx, pass, n_query, nullptr, t_lo, t_hi, match_q, match_t, n_out, scratch, st);
+}
+
+int sod_compact_matches_dev(const int32_t* idx, const uint8_t* pass, int64_t n_query_cap,
+                            const int32_t* n_query_dev, int32_t t_lo, int32_t t_hi, int32_t* match_q,
+                            int32_t* match_t, int32_t* n_out, void* scratch, sod_stream_t stream) {
+  SOD_CHECK_ARG(n_query_cap >= 0, "n_query_cap < 0");
+  SOD_CHECK_ARG(idx && pass && n_query_dev && match_q && match_t && n_out && scratch, "null pointer");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (n_query_cap == 0) {
+    SOD_CHECK_CUDA(cudaMemsetAsync(n_out, 0, 4, st));
+    return SOD_OK;
+  }
+  return launch_compact<true>(idx, pass, n_query_cap, n_query_dev, t_lo, t_hi, match_q, match_t, n_out, scratch,
+                              st);
 }
 
 int sod_estimate_pose(const sod_scene* scene, const int32_t* match_q, const int32_t* match_t,

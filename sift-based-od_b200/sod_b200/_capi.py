@@ -126,6 +126,7 @@ _PROTOS = {
     "sod_angle_adjacency": (C.c_int, [_p, _p, _i64, C.c_double, _p, _p, _p]),
     "sod_compact_scratch_bytes": (C.c_size_t, [_i64]),
     "sod_compact_matches": (C.c_int, [_p, _p, _i64, _i32, _i32, _p, _p, _p, _p, _p]),
+    "sod_compact_matches_dev": (C.c_int, [_p, _p, _i64, _p, _i32, _i32, _p, _p, _p, _p, _p]),
     "sod_estimate_pose": (C.c_int, [C.POINTER(Scene), _p, _p, _i64, _i32, _p, _p, _p, _p, _p]),
     "sod_pose_bin_index": (C.c_int, [_p, _i64, _i32, _i32, _i32, _p, _p, _p]),
     "sod_affine_residual_keep": (C.c_int, [_p, _p, _i64, _p, C.c_double, C.c_double, _p, _p]),

@@ -375,9 +375,11 @@ class SceneArrays:
             int(self.img_centroid.shape[0]), self.groups_per_frame)
 
 
-def compact_matches(idx: torch.Tensor, ok: torch.Tensor, t_lo: int = 0, t_hi: int = 2 ** 31 - 1):
+def compact_matches(idx: torch.Tensor, ok: torch.Tensor, t_lo: int = 0, t_hi: int = 2 ** 31 - 1,
+                    n_dev: torch.Tensor | None = None):
     """Ratio survivors (whose database row is in [t_lo, t_hi)) in query order ->
-    (match_q, match_t, n_dev); stays on the device."""
+    (match_q, match_t, n_dev); stays on the device.  n_dev (device int32 [1]): only the first n_dev[0] rows
+    count (sod_compact_matches_dev); the rows past it are ignored whatever they hold."""
     idx = _require_cuda(idx, torch.int32, "idx")
     ok = _require_cuda(ok, torch.uint8, "pass flags")
     nq = int(ok.shape[0])
@@ -386,8 +388,13 @@ def compact_matches(idx: torch.Tensor, ok: torch.Tensor, t_lo: int = 0, t_hi: in
     mt = torch.empty(max(nq, 1), dtype=torch.int32, device=dev)
     n = torch.zeros(1, dtype=torch.int32, device=dev)
     scratch = torch.empty(int(lib.sod_compact_scratch_bytes(nq)), dtype=torch.uint8, device=dev)
-    check(lib.sod_compact_matches(_ptr(idx), _ptr(ok), nq, int(t_lo), int(t_hi), _ptr(mq), _ptr(mt), _ptr(n),
-                                  _ptr(scratch), _stream()), "sod_compact_matches")
+    if n_dev is None:
+        check(lib.sod_compact_matches(_ptr(idx), _ptr(ok), nq, int(t_lo), int(t_hi), _ptr(mq), _ptr(mt), _ptr(n),
+                                      _ptr(scratch), _stream()), "sod_compact_matches")
+    else:
+        n_dev = _require_cuda(n_dev, torch.int32, "n_dev")
+        check(lib.sod_compact_matches_dev(_ptr(idx), _ptr(ok), nq, _ptr(n_dev), int(t_lo), int(t_hi), _ptr(mq),
+                                          _ptr(mt), _ptr(n), _ptr(scratch), _stream()), "sod_compact_matches_dev")
     return mq, mt, n
 
 

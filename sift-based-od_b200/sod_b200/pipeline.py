@@ -360,8 +360,11 @@ class DetectionPipeline:
         self._consumed[slot].record()
         return entry[1]
 
-    def detect_device(self, n: int, slot: int = 0, _events: bool = True):
-        """Run the path on the first n rows of query-buffer set `slot`; everything stays on the device."""
+    def detect_device(self, n: int, slot: int = 0, _events: bool = True, n_dev: torch.Tensor | None = None):
+        """Run the path on the first n rows of query-buffer set `slot`; everything stays on the device.
+        n_dev (device int32 [1], at most n): the true row count, read on the device.  The matcher and the ratio
+        merge then run on all n rows, and only the compaction reads n_dev: matches of rows past it are dropped,
+        so those rows may hold anything (a captured graph's previous frame)."""
         qs = self._qset(slot)
         if _events and self._loaded[slot] is not None:
             torch.cuda.current_stream(self.device).wait_event(self._loaded[slot])
@@ -392,7 +395,7 @@ class DetectionPipeline:
                 blocks = (n + QUERY_BLOCK - 1) // QUERY_BLOCK
                 idx, d2 = self.matcher.top2(q, None, thr, peer_table=self.peer_thr.table(0),
                                             block_rotation=blocks * self.rank // self.world)
-                return self._after_match(idx, d2, n, slot, _events, merge)
+                return self._after_match(idx, d2, n, slot, _events, merge, n_dev)
             thr = self.matcher.new_thresholds(n)       # (reached with a seed sample only: the NCCL form)
             if s_hi > s_lo:
                 self.seed_matcher.top2(q[s_lo:s_hi], None, thr[s_lo:])
@@ -415,9 +418,9 @@ class DetectionPipeline:
                 idx, d2, _, _ = E.merge_top2(torch.stack([p[0] for p in parts]), torch.stack([p[1] for p in parts]))
         else:
             idx, d2 = self.matcher.top2(q)
-        return self._after_match(idx, d2, n, slot, _events, merge)
+        return self._after_match(idx, d2, n, slot, _events, merge, n_dev)
 
-    def _after_match(self, idx, d2, n: int, slot: int, _events: bool, merge):
+    def _after_match(self, idx, d2, n: int, slot: int, _events: bool, merge, n_dev=None):
         """Exchange of the shard-local lists, compaction, Hough, affine (the rest of detect_device)."""
         if self.world > 1 and self.peer is not None and n <= self.peer.max_query:
             # The exchange through peer memory: two kernels, no collective call (sod_b200/peer.py).
@@ -443,7 +446,7 @@ class DetectionPipeline:
         else:
             idx, d2, dist_f, ok = merge(idx[None], d2[None])
         lo, hi = (self.row_lo, self.row_hi) if self.world > 1 else (0, 2 ** 31 - 1)
-        mq, mt, n_dev = E.compact_matches(idx, ok, lo, hi)
+        mq, mt, n_dev = E.compact_matches(idx, ok, lo, hi, n_dev=n_dev)
         if self._hough[slot] is None:
             self._hough[slot] = self.voter.new_result(self.max_queries)
             self._aff[slot] = E.AffineResult(self._hough[slot], self.vote_threshold, self.device)

@@ -7,7 +7,8 @@ and the reference; DESIGN.md 2 states how closely this one agrees with it.
 
 GpuSift.extract_batch runs many same-size frames in one pass (sod_sift_extract_batch) and leaves the result on the
 device, in the layout DetectionPipeline.load_queries takes; FrameStream uses it when the extractor has it.
-GpuSift.extract_mixed does the same for frames of different sizes (sod_sift_extract_mixed), such as the training
+GpuSift.enqueue_batch is the same pass without the wait, for callers that capture it in a CUDA graph
+(sod_b200.live.LiveDetector).  GpuSift.extract_mixed does the same for frames of different sizes (sod_sift_extract_mixed), such as the training
 images GenerateDatabaseInfo.build_database resizes to one width.
 """
 from __future__ import annotations
@@ -260,6 +261,49 @@ class GpuSift:
         it (decoded and converted on the host).  FrameStream's worker threads call this."""
         return image if _is_cuda(image) else _gray(image)
 
+    def _batch(self, w: int, h: int, n: int) -> _BatchBuffers:
+        b = self._batch_buffers.get((w, h, n))
+        if b is None:
+            b = self._batch_buffers[(w, h, n)] = _BatchBuffers(w, h, n, self.capacity, self.max_keypoints, self._device)
+        return b
+
+    def enqueue_batch(self, images, slot: int = 0) -> dict:
+        """sod_sift_extract_batch of a CUDA u8 [B, H, W] tensor (pitched or not), enqueued on the caller's current
+        stream; never waits, so it can be captured in a CUDA graph.
+
+        -> the output set's device tensors: des, xy, angle, size, response, octave, frame (the packed rows, at most
+        B x min(capacity, max_keypoints); frame k's are rows offset[k]:offset[k] + count[k]) and flags (int32
+        [3B + 1]: count[B], offset[B], overflow[B], then the rows-overflow flag).  Nothing is checked on the host:
+        the caller reads the flags once the stream has reached them.  The next call (or extract_batch) of the same
+        size, batch and slot overwrites the tensors."""
+        import torch
+        if slot not in (0, 1):
+            raise ValueError("slot must be 0 or 1")
+        if not _is_cuda(images) or images.dim() != 3 or images.dtype != torch.uint8:
+            raise ValueError(f"expected a CUDA u8 [B, H, W] tensor, got {getattr(images, 'dtype', type(images))} "
+                             f"{tuple(getattr(images, 'shape', ()))}")
+        with self._lock, torch.cuda.device(self._device or torch.cuda.current_device()):
+            self._setup_stream()
+            return self._enqueue(images, slot)
+
+    def _enqueue(self, images, slot: int) -> dict:
+        """enqueue_batch with the lock held, on the current stream."""
+        import torch
+        n, h, w = (int(v) for v in images.shape)
+        b = self._batch(w, h, n)
+        t, out = b.out(slot)
+        if images.device != b.img.device:
+            raise ValueError(f"images are on {images.device}, GpuSift on {b.img.device}")
+        src = images
+        if not (images.stride(2) == 1 and images.stride(1) >= w and images.stride(0) >= images.stride(1) * h):
+            b.img.copy_(images)
+            src = b.img
+        mk = 0 if self.max_keypoints is None else max(1, int(self.max_keypoints))
+        _capi.check(_capi.lib.sod_sift_extract_batch(src.data_ptr(), w, h, src.stride(1), src.stride(0), n, mk,
+                                                     C.byref(out), b.ws.data_ptr(), b.bytes,
+                                                     torch.cuda.current_stream().cuda_stream), "sod_sift_extract_batch")
+        return t
+
     def extract_batch(self, images, slot: int = 0) -> SiftBatch:
         """SIFT of a batch of same-size frames in one pass, the result left on the device.
 
@@ -269,7 +313,7 @@ class GpuSift:
                 extracted
 
         Waits for the batch (counts are read on the host); a frame with more than `capacity` keypoints raises
-        SodError naming it."""
+        SodError naming it.  enqueue_batch is the same pass without the wait."""
         import torch
         if slot not in (0, 1):
             raise ValueError("slot must be 0 or 1")
@@ -285,25 +329,13 @@ class GpuSift:
             raise ValueError(f"expected a u8 [B, H, W] tensor, got {images.dtype} {tuple(images.shape)}")
         with self._lock, torch.cuda.device(self._device or torch.cuda.current_device()):
             self._setup_stream()
-            b = self._batch_buffers.get((w, h, n))
-            if b is None:
-                b = self._batch_buffers[(w, h, n)] = _BatchBuffers(w, h, n, self.capacity, self.max_keypoints,
-                                                                   self._device)
-            t, out = b.out(slot)
-            src, pitch, fstride = b.img, w, w * h
+            b = self._batch(w, h, n)
             if dev_in or any(_is_cuda(f) for f in frames):
                 # CUDA inputs come from the caller's current stream; host inputs need no wait, so the SIFT can
                 # run beside the caller's other work (FrameStream's previous detection pass)
                 self._stream.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(self._stream):
-                if dev_in:
-                    if images.device != b.img.device:
-                        raise ValueError(f"images are on {images.device}, GpuSift on {b.img.device}")
-                    if images.stride(2) == 1 and images.stride(1) >= w and images.stride(0) >= images.stride(1) * h:
-                        src, pitch, fstride = images, images.stride(1), images.stride(0)
-                    else:
-                        b.img.copy_(images)
-                else:
+                if not dev_in:
                     on_host = [k for k, f in enumerate(frames) if not _is_cuda(f)]
                     if on_host and b.host is None:
                         b.host = torch.empty((n, h, w), dtype=torch.uint8, pin_memory=True)
@@ -314,10 +346,7 @@ class GpuSift:
                     else:
                         for k, f in enumerate(frames):
                             b.img[k].copy_(f if _is_cuda(f) else b.host[k], non_blocking=True)
-                mk = 0 if self.max_keypoints is None else max(1, int(self.max_keypoints))
-                _capi.check(_capi.lib.sod_sift_extract_batch(src.data_ptr(), w, h, pitch, fstride, n, mk,
-                                                             C.byref(out), b.ws.data_ptr(), b.bytes,
-                                                             self._stream.cuda_stream), "sod_sift_extract_batch")
+                t = self._enqueue(images if dev_in else b.img, slot)
                 b.flags.copy_(t["flags"], non_blocking=True)
             # the whole batch is done once this returns: its rows may be read on any stream, and the pinned
             # staging and the workspace are free for the next call

@@ -76,6 +76,26 @@ def plan_batches(counts: Iterable[int], max_frames: int, max_rows: int) -> list[
     return batches
 
 
+def split_frame(out: dict, poses: dict, spaces_per_frame: int, slot: int, lo: int, hi: int, **extra) -> dict:
+    """The part of a fetched batch result that belongs to frame `slot`, whose query rows are [lo, hi): match pairs
+    as (query keypoint index within the frame, database row), verified bins, final poses; `extra` (such as the
+    frame's FrameFeatures) is added as it is."""
+    ok = out["ok"][lo:hi].astype(bool)
+    gpf = spaces_per_frame
+    mine = (out["valid_group"] // gpf) == slot
+    return dict(match_q=np.nonzero(ok)[0].astype(np.int32), match_t=out["idx"][lo:hi, 0][ok],
+                n_descriptors=hi - lo, valid_group=out["valid_group"][mine] % gpf, valid_code=out["valid_code"][mine],
+                votes=out["votes"][mine], live=(out["status"][mine] & 1).astype(bool), params=out["params"][mine],
+                final_pose=poses.get(slot, []), **extra)
+
+
+def one_rank_error(who: str) -> str:
+    """Why a device-side SIFT path refuses a database-sharded pipeline of several ranks."""
+    return (f"{who} needs the whole batch on one rank: every rank of a database-sharded pipeline would need the "
+            "same query rows, and GPU SIFT descriptors may differ by 1 between runs; use "
+            "DetectionPipeline(shard='frames')")
+
+
 class _Staging:
     """One set of pinned host buffers for a batch (allocated lazily; torch only needed on the GPU side)."""
 
@@ -179,15 +199,8 @@ class FrameStream:
                 for k in range(len(feats))]
 
     def _split(self, out: dict, poses: dict, slot: int, lo: int, hi: int, feats: FrameFeatures | None) -> dict:
-        """The part of a batch result that belongs to frame `slot`, whose query rows are [lo, hi): match pairs as
-        (query keypoint index within the frame, database row), verified bins, final poses."""
-        ok = out["ok"][lo:hi].astype(bool)
-        gpf = self.pipeline.spaces_per_frame
-        mine = (out["valid_group"] // gpf) == slot
-        return dict(match_q=np.nonzero(ok)[0].astype(np.int32), match_t=out["idx"][lo:hi, 0][ok],
-                    n_descriptors=hi - lo, valid_group=out["valid_group"][mine] % gpf, valid_code=out["valid_code"][mine],
-                    votes=out["votes"][mine], live=(out["status"][mine] & 1).astype(bool), params=out["params"][mine],
-                    final_pose=poses.get(slot, []), **({"features": feats} if self.features else {}))
+        return split_frame(out, poses, self.pipeline.spaces_per_frame, slot, lo, hi,
+                           **({"features": feats} if self.features else {}))
 
     # -------------------------------------------------------------------------------- driver
     def run(self, frames: Iterable) -> Iterator[tuple[int, dict]]:
@@ -318,9 +331,7 @@ class FrameStream:
     def _run_device(self, frames: Iterable) -> Iterator[tuple[int, dict]]:
         p = self.pipeline
         if getattr(p, "world", 1) > 1 and getattr(p, "shard_mode", "db") == "db":
-            raise ValueError("FrameStream's device path needs the whole batch on one rank: every rank of a "
-                             "database-sharded pipeline would need the same query rows, and GPU SIFT descriptors "
-                             "may differ by 1 between runs; use DetectionPipeline(shard='frames')")
+            raise ValueError(one_rank_error("FrameStream's device path"))
         with ThreadPoolExecutor(self.workers) as pool:
             # Per pass: take the next pass (which may run the next SIFT batch, while the GPU still runs the
             # previous pass), read back the previous pass, enqueue this one, hand the previous frames over.
