@@ -395,6 +395,44 @@ int sod_pose_adjacency(const double* cx, const double* cy, const double* reach_x
 int sod_angle_adjacency(const double* angle, const int32_t* segment, int64_t n, double max_degrees,
                         uint32_t* adj, int32_t* label, sod_stream_t stream);
 
+/* Outputs of sod_final_poses (device), for up to cap bins; the first counters[0] clusters are written.
+ * Clusters are numbered by their lowest bin; bins are input positions (sod_final_poses_records: positions in the
+ * (group, order key) order of the live bins). */
+typedef struct {
+  int32_t* counters;       /* [2]: clusters, bins clustered */
+  int32_t* cluster_bins;   /* [cap]: cluster c is cluster_bins[cluster_offset[c] .. cluster_offset[c+1]), in its
+                            * group_position visiting order */
+  int32_t* cluster_offset; /* [cap + 1] */
+  int32_t* sub_bins;       /* [cap]: the same ranges, each cluster's bins in group_orientation visiting order */
+  int32_t* sub_first;      /* [cap]: 1 where a sub-cluster starts in sub_bins, else 0 */
+  double* pose;            /* [cap][6]: cx, cy, orientation, scale, w, h of get_final_pose */
+  int32_t* shape_bin;      /* [cap]: the bin whose (w, h) is the shape; -1 = (0, 0) */
+  int32_t* segment;        /* [cap]: the cluster's segment */
+  int64_t cap;
+} sod_poses_out;
+
+/* Bytes of workspace (256-byte aligned) for up to cap bins (about cap^2 / 8 of bit rows); 0 if cap is out of range. */
+size_t sod_final_poses_workspace_bytes(int64_t cap);
+
+/* Main.post_process (main.py:159-168): group_position -> group_orientation -> find_max_orientation ->
+ * get_final_pose (PostProcessing.py:4-112) on the device, bit-exact.  mean [n][6] = cx, cy, angle, scale, img_w,
+ * img_h of each bin (the PoseBin running means, sod_hough_out.bin_mean's layout).  segment (may be NULL) restricts
+ * position edges to bins of equal segment id; clusters are still numbered over the whole input.  n_dev (may be
+ * NULL): the count of bins to cluster, read on the device and clamped to 0..n (n is then the capacity).  The
+ * walks' visiting orders, the sums' order and the tie-breaks are the reference's; every fp64 operation is rounded
+ * on its own.  n <= SOD_MAX_CLUSTER_BINS; n = 0 does nothing.  No synchronisation, no allocation: capturable. */
+int sod_final_poses(const double* mean, const int32_t* segment, int64_t n, const int32_t* n_dev,
+                    const sod_poses_out* out, void* workspace, size_t workspace_bytes, sod_stream_t stream);
+
+/* sod_final_poses on the affine stage's records of up to cap verified bins, n_dev of them valid (clamped to cap):
+ * the bins with status bit 0 set, ordered by (group, order_key) as Main.post_process meets them, segment = group /
+ * groups_per_frame (the frame).  order_key int64 (sod_valid_bin_records' out_order), mean as sod_final_poses.
+ * Bin indices of out are positions in that order.  cap = 0 does nothing. */
+int sod_final_poses_records(const int32_t* status, const int32_t* group, const int64_t* order_key,
+                            const double* mean, int64_t cap, const int32_t* n_dev, int32_t groups_per_frame,
+                            const sod_poses_out* out, void* workspace, size_t workspace_bytes,
+                            sod_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------
  * SIFT extraction (in front of the path)
  * ---------------------------------------------------------------------------------------------- */

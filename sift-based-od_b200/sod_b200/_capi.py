@@ -57,6 +57,11 @@ class AffineOut(C.Structure):
                 ("member_keep", _p), ("cap_valid", _i64), ("cap_votes", _i64)]
 
 
+class PosesOut(C.Structure):
+    _fields_ = [("counters", _p), ("cluster_bins", _p), ("cluster_offset", _p), ("sub_bins", _p), ("sub_first", _p),
+                ("pose", _p), ("shape_bin", _p), ("segment", _p), ("cap", _i64)]
+
+
 class SiftOut(C.Structure):
     _fields_ = [("xy", _p), ("size", _p), ("angle", _p), ("response", _p), ("octave", _p), ("des", _p),
                 ("counters", _p), ("cap", _i64)]
@@ -87,6 +92,7 @@ def timing_read(stage: str) -> list[float]:
 SIGMA_LUT_MIN = -24
 SIGMA_LUT_LEN = 49
 MAX_BINS = 15
+MAX_CLUSTER_BINS = 65536
 
 _PROTOS = {
     "sod_version": (C.c_int, []),
@@ -124,6 +130,9 @@ _PROTOS = {
     "sod_top2_merge_f32": (C.c_int, [_p, _p, _i32, _i64, _p, _p, _p, _p, C.c_double, _p]),
     "sod_pose_adjacency": (C.c_int, [_p, _p, _p, _p, _p, _i64, _p, _p, _p]),
     "sod_angle_adjacency": (C.c_int, [_p, _p, _i64, C.c_double, _p, _p, _p]),
+    "sod_final_poses_workspace_bytes": (C.c_size_t, [_i64]),
+    "sod_final_poses": (C.c_int, [_p, _p, _i64, _p, C.POINTER(PosesOut), _p, C.c_size_t, _p]),
+    "sod_final_poses_records": (C.c_int, [_p, _p, _p, _p, _i64, _p, _i32, C.POINTER(PosesOut), _p, C.c_size_t, _p]),
     "sod_compact_scratch_bytes": (C.c_size_t, [_i64]),
     "sod_compact_matches": (C.c_int, [_p, _p, _i64, _i32, _i32, _p, _p, _p, _p, _p]),
     "sod_compact_matches_dev": (C.c_int, [_p, _p, _i64, _p, _i32, _i32, _p, _p, _p, _p, _p]),

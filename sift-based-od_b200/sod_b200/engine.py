@@ -313,7 +313,7 @@ def knn_match_ratio_float(q_f32: torch.Tensor, matcher: FloatMatcher, ratio: flo
 # ------------------------------------------------------------------------------------------------
 import math  # noqa: E402
 
-from ._capi import AffineOut, HoughOut, Keypoints, Scene  # noqa: E402
+from ._capi import AffineOut, HoughOut, Keypoints, PosesOut, Scene  # noqa: E402
 
 POS_FACTOR = 32          # main.py:141
 N_OCT = 4                # HoughTransformHelperFunctions.py:66
@@ -555,3 +555,65 @@ def affine_verify(scene: SceneArrays, match_q: torch.Tensor, match_t: torch.Tens
                                 float(factor if factor_y is None else factor_y), int(max_passes),
                                 C.byref(o), _stream()), "sod_affine_verify")
     return res
+
+
+class FinalPoses:
+    """sod_final_poses / sod_final_poses_records for up to `cap` bins, with the workspace and the outputs kept
+    across calls.  The outputs of a call on n bins are views of the first bytes of one device buffer, so one copy of
+    that many bytes reads all of them back; they are overwritten by the next call."""
+
+    _NAMES = ("counters", "cluster_offset", "cluster_bins", "sub_bins", "sub_first", "shape_bin", "segment")
+
+    def __init__(self, cap: int, device):
+        cap = int(cap)
+        if not 1 <= cap <= _capi.MAX_CLUSTER_BINS:
+            raise _capi.SodError(f"sod_final_poses: {cap} bins, the limit is {_capi.MAX_CLUSTER_BINS}")
+        self.cap, self.device = cap, torch.device(device)
+        self.ws = torch.empty(int(lib.sod_final_poses_workspace_bytes(cap)), dtype=torch.uint8, device=self.device)
+        self.buf = torch.empty(self._bytes(cap), dtype=torch.uint8, device=self.device)
+        v = self.views(cap)
+        self.pose, self.counters, self.shape_bin, self.segment = v["pose"], v["counters"], v["shape_bin"], v["segment"]
+
+    @staticmethod
+    def _bytes(n: int) -> int:
+        return n * 6 * 8 + (2 + (n + 1) + 5 * n) * 4
+
+    def views(self, n: int, buf=None) -> dict:
+        """The outputs of a call on n bins as views of buf (the device buffer, or a host copy of its first bytes)."""
+        buf = self.buf if buf is None else buf
+        tensor = isinstance(buf, torch.Tensor)
+        f8 = n * 6 * 8
+        pose = buf[:f8].view(torch.float64 if tensor else np.float64).reshape(n, 6)
+        iv = buf[f8:self._bytes(n)].view(torch.int32 if tensor else np.int32)
+        out, o = dict(pose=pose), 0
+        for name, size in zip(self._NAMES, (2, n + 1, n, n, n, n, n)):
+            out[name] = iv[o:o + size]
+            o += size
+        return out
+
+    def struct(self, n: int) -> PosesOut:
+        v = self.views(n)
+        return PosesOut(*(_ptr(v[name]) for name in ("counters", "cluster_bins", "cluster_offset", "sub_bins",
+                                                     "sub_first", "pose", "shape_bin", "segment")), n)
+
+    def run(self, mean: torch.Tensor, segment: torch.Tensor | None, n: int, n_dev: torch.Tensor | None = None):
+        """mean: device float64 [>= n][6] (cx, cy, angle, scale, img_w, img_h); segment: device int32 [>= n] or
+        None; n_dev: device int32 count (clamped to n), or None for n.  Outputs: views(n)."""
+        mean = _require_cuda(mean, torch.float64, "mean")
+        o = self.struct(int(n))
+        check(lib.sod_final_poses(_ptr(mean), _ptr(segment), int(n), _ptr(n_dev), C.byref(o), _ptr(self.ws),
+                                  self.ws.numel(), _stream()), "sod_final_poses")
+        return self
+
+    def run_records(self, status, group, order, mean, cap: int, n_dev: torch.Tensor, groups_per_frame: int):
+        """The live bins of the affine stage's first min(n_dev, cap) records, in (group, order key) order.
+        Outputs: views(cap)."""
+        o = self.struct(int(cap))
+        check(lib.sod_final_poses_records(_ptr(status), _ptr(group), _ptr(order), _ptr(mean), int(cap), _ptr(n_dev),
+                                          int(groups_per_frame), C.byref(o), _ptr(self.ws), self.ws.numel(),
+                                          _stream()), "sod_final_poses_records")
+        return self
+
+    def host(self, n: int) -> dict:
+        """The outputs of the last call on n bins, read back with one copy of their bytes (synchronises)."""
+        return self.views(n, self.buf[:self._bytes(n)].cpu().numpy())

@@ -11,9 +11,11 @@ frame, with one host synchronise per call:
 The graph holds the upload from pinned staging, the SIFT batch (GpuSift.enqueue_batch), the copies of its packed rows
 into the pipeline's query buffers (a fixed B x R rows), the true row total offset[B-1] + count[B-1] on the device, the
 detection pass on that capacity with the row count read by the compaction only (DetectionPipeline.detect_device's
-n_dev), and the device-to-host copies of the counters, the SIFT flags, idx / ok of the capacity rows and the records
-of up to max_bins verified bins.  The rows past the true count hold the previous frame's rows: they are matched and
-their matches are dropped by the compaction.
+n_dev), the final poses of the verified bins (DetectionPipeline.final_poses_device: Main.post_process on the device),
+and the device-to-host copies of the counters, the SIFT flags, idx / ok of the capacity rows, the records of up to
+max_bins verified bins and the poses.  The rows past the true count hold the previous frame's rows: they are matched
+and their matches are dropped by the compaction.  After the replay's one synchronise, detect only reads pinned
+memory.
 """
 from __future__ import annotations
 
@@ -37,7 +39,8 @@ class LiveDetector:
     sift        a GpuSift with max_keypoints set: a frame keeps cv2's first max_keypoints keypoints
     frame_size  (width, height) of every frame
     frames      B, frames per call
-    max_bins    verified bins read back per call; a call that verifies more raises
+    max_bins    verified bins read back per call (at most 65,536, the limit of the pose clustering); a call that
+                verifies more raises
     features    add each frame's FrameFeatures (its SIFT rows, read back from the device) to its result
 
     detect(frames) returns one dict per frame with the fields of a FrameStream frame result.  The graph is captured
@@ -113,16 +116,18 @@ class LiveDetector:
         n_dev = fl[B - 1:B] + fl[2 * B - 1:2 * B]            # offset[B-1] + count[B-1]: the rows of this call
         r = p.detect_device(R, 0, _events=False, n_dev=n_dev)
         a = r["affine"]
-        k = min(self.max_bins, a.cap_valid)
+        k = min(self.max_bins, a.cap_valid, _capi.MAX_CLUSTER_BINS)    # the poses are clustered on the device
         g, code, order, mean = r["records"]
         dev = dict(counters=r["counters"], flags=fl, idx=r["idx"][:R], ok=r["ok"][:R], valid_bin=a.valid_bin[:k],
                    params=a.params[:k], votes=a.votes[:k], status=a.status[:k], valid_group=g[:k], valid_code=code[:k],
                    valid_order=order[:k], valid_mean=mean[:k])
+        fp = p.final_poses_device(r, k)
+        dev.update(pose=fp["pose"], pose_frame=fp["frame"], pose_shape=fp["shape_bin"], pose_counters=fp["counters"])
         if host is None:
             host = {name: self._pinned(v) for name, v in dev.items()}
         for name, v in dev.items():
             host[name].copy_(v, non_blocking=True)
-        return dict(host=host, sift=t, n_dev=n_dev, k=k)
+        return dict(host=host, sift=t, n_dev=n_dev, k=k, poses=fp["poses"])
 
     def _graph(self, upload: bool):
         entry = self._graphs.get(upload)
@@ -143,7 +148,7 @@ class LiveDetector:
         # The workspaces the graph was captured with (allocated during the warm-up, outside its pool) stay alive
         # with it, even if another caller of the pipeline later grows them.
         state["keep"] = (p.matcher._ws, p.matcher._qn, p.voter._ws, p._hough[0], p._aff[0], p.scene.frame_wh,
-                         p._qset(0), self.sift._batch_buffers[(*self.frame_size, self.frames)])
+                         p._qset(0), self.sift._batch_buffers[(*self.frame_size, self.frames)], state["poses"])
         entry = self._graphs[upload] = (graph, state)
         return entry
 
@@ -182,7 +187,12 @@ class LiveDetector:
         out.update({name: hv[name][:n_valid].copy() for name in _BIN_FIELDS})
         out.update(row_lo=0, n_matches=n_m, n_bins=n_bins, n_votes=n_votes, n_near_edge=n_edge,
                    n_unresolved_edge=n_open, n_valid=n_valid, n_singular=n_singular, n_residual_edge=n_res_edge)
-        poses = p.final_poses(out)
+        n_clusters = int(hv["pose_counters"][0])
+        poses: dict[int, list] = {}
+        for pose, frame, shape in zip(hv["pose"][:n_clusters], hv["pose_frame"][:n_clusters].tolist(),
+                                      hv["pose_shape"][:n_clusters].tolist()):
+            cx, cy, ori, scale = pose[:4].tolist()
+            poses.setdefault(frame, []).append(((cx, cy), ori, scale, (pose[4], pose[5]) if shape >= 0 else (0, 0)))
         sb = None
         if self.features:
             t = state["sift"]

@@ -259,6 +259,7 @@ class DetectionPipeline:
                     torch.from_numpy(np.ascontiguousarray(np.asarray(db.des)[rows]))
                 self.seed_matcher = E.Matcher(E.prepare_db(sample.to(self.device).contiguous(), index_base=0))
         self._graphs: dict = {}
+        self._poses: dict = {}           # capacity -> engine.FinalPoses of final_poses_device
         if world > 1 and (self.float_path or self.exchange == "gather"):
             self._gather_idx = torch.empty((world, self.max_queries, 2), dtype=torch.int32, device=dev)
             self._gather_d2 = torch.empty((world, self.max_queries, 2),
@@ -556,6 +557,25 @@ class DetectionPipeline:
         for cl, pose in zip(clusters, final):
             poses.setdefault(int(frame[cl[0]]), []).append(pose)
         return poses
+
+    def final_poses_device(self, r: dict, cap: int | None = None) -> dict:
+        """final_poses of a detect_device result on the device, with no host step (sod_final_poses_records):
+        the live bins of the first min(n_valid, cap) verified bins (cap: the affine output capacity by default,
+        at most 65,536) -> device tensors pose float64 [cap][6] (cx, cy, orientation, scale, w, h), frame int32
+        [cap], shape_bin int32 [cap] (-1: the reference's (0, 0) shape) and counters int32 [2] (clusters, live
+        bins); the first counters[0] rows are the clusters, numbered as final_poses meets them.  The tensors
+        belong to `poses` (an engine.FinalPoses kept per capacity) and are overwritten by its next call."""
+        if self._local_spaces != self.spaces_per_frame:
+            raise ValueError("final_poses_device needs every Hough space of a frame on this rank; a database-sharded "
+                             "run with per-object spaces numbers them per rank (use fetch and final_poses)")
+        a = r["affine"]
+        g, _, order, mean = r["records"]
+        k = min(a.cap_valid if cap is None else int(cap), a.cap_valid, E._capi.MAX_CLUSTER_BINS)
+        fp = self._poses.get(k)
+        if fp is None:
+            fp = self._poses[k] = E.FinalPoses(k, self.device)
+        fp.run_records(a.status, g, order, mean, k, a.counters[:1], self.spaces_per_frame)
+        return dict(pose=fp.pose, frame=fp.segment, shape_bin=fp.shape_bin, counters=fp.counters, poses=fp)
 
     @staticmethod
     def fetched_bytes(out: dict) -> int:

@@ -1,21 +1,27 @@
 """Pose clustering after the affine stage (SURVEY.md §8f N1) on arrays.
 
-The O(V^2) neighbour tests of group_position / group_orientation (PostProcessing.py:14-63) run on
-the GPU (csrc/sod_cluster.cu: bit-matrix adjacency + union-find labels); the reference's depth-first
-visiting order - which fixes the order of its float sums, the order of the clusters and the
-tie-break of find_max_orientation - is recovered here from the bit rows with integer bitsets
-(V steps of V/64-word operations), so results are identical to the reference's and there is no
-recursion limit (SURVEY Q12).
+post_process_arrays runs all four steps of Main.post_process on the device (csrc/sod_cluster.cu,
+sod_final_poses): one upload, one call, one read-back.  The walks there follow the reference's depth-first
+visiting order - which fixes the order of its float sums, the order of the clusters and the tie-break of
+find_max_orientation - so results are identical to the reference's and there is no recursion limit
+(SURVEY Q12).
+
+The step-by-step functions (cluster_positions, orientation_subclusters) serve the drop-in's group_position /
+group_orientation on caller-built lists: the O(V^2) neighbour tests run on the GPU (bit-matrix adjacency +
+union-find labels) and the visiting order is recovered here from the bit rows with integer bitsets (V steps of
+V/64-word operations).
 """
 from __future__ import annotations
-
-import math
 
 import numpy as np
 import torch
 
+from . import _capi
 from ._capi import check, lib
-from .engine import _ptr, _stream
+from .engine import FinalPoses, _ptr, _stream
+
+_final: dict = {}      # device -> FinalPoses kept for later calls (up to _KEEP_BINS bins)
+_KEEP_BINS = 4096      # workspace about 2.4 MB; larger calls get a FinalPoses of their own, freed after the call
 
 
 def _graph(kind: str, arrays, segment, n: int, device, limit: float = 1.0):
@@ -104,31 +110,51 @@ def cluster_orientations(angle, clusters, device="cuda", max_degrees: float = 1.
     return [[[cl[p] for p in comp] for comp in comps] for cl, comps in zip(clusters, pos)]
 
 
+def _final_poses(n: int, device) -> FinalPoses:
+    device = torch.device(device)
+    if device.type == "cuda" and device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    if n > _KEEP_BINS:
+        return FinalPoses(n, device)
+    fp = _final.get(device)
+    if fp is None or fp.cap < n:
+        fp = _final[device] = FinalPoses(max(n, 256), device)
+    return fp
+
+
 def post_process_arrays(cx, cy, scale, angle, img_w, img_h, segment=None, device="cuda"):
     """The four reference steps on arrays -> (clusters, sub_clusters, orientations, final) with
-    final[c] = ((cx, cy), orientation, scale, (w, h)) exactly as get_final_pose returns it."""
-    clusters, label = cluster_positions(cx, cy, scale, img_w, img_h, segment, device)
-    subs = cluster_orientations(angle, clusters, device)
-    orientations, final = [], []
-    for cl, sc in zip(clusters, subs):
-        best, ori = 0, 0
-        for sub in sc:                      # later sub-clusters win ties (PostProcessing.py:65-82)
-            if len(sub) >= best:
-                best = len(sub)
-                ori = 0
-                for i in sub:
-                    ori += float(angle[i])
-                ori = ori / len(sub)
-        orientations.append(ori)
-        sx = sy = ss = 0
-        min_area, shape = math.inf, (0, 0)
-        for i in cl:                        # PostProcessing.py:86-112
-            sx += float(cx[i])
-            sy += float(cy[i])
-            ss += float(scale[i])
-            area = (img_w[i] * float(scale[i])) * (img_h[i] * float(scale[i]))
-            if area < min_area:
-                min_area, shape = area, (img_w[i], img_h[i])
-        m = len(cl)
-        final.append(((sx / m, sy / m), ori, ss / m, shape))
+    final[c] = ((cx, cy), orientation, scale, (w, h)) exactly as get_final_pose returns it.  segment (one id
+    per bin, e.g. its frame) keeps bins of different segments apart."""
+    n = len(cx)
+    if n == 0:
+        return [], [], [], []
+    if n > _capi.MAX_CLUSTER_BINS:
+        raise _capi.SodError(f"sod_final_poses: n = {n}, the limit is {_capi.MAX_CLUSTER_BINS}")
+    # one upload: the means [n][6] (the sod_hough_out.bin_mean layout) and the segment ids behind them
+    host = np.empty(n * 52, np.uint8)
+    mean = host[:n * 48].view(np.float64).reshape(n, 6)
+    for f, a in enumerate((cx, cy, angle, scale, img_w, img_h)):
+        mean[:, f] = np.asarray(a, np.float64)
+    host[n * 48:].view(np.int32)[:] = 0 if segment is None else np.asarray(segment, np.int32)
+    fp = _final_poses(n, device)
+    with torch.cuda.device(fp.device):
+        dev = torch.from_numpy(host).to(fp.device)
+        fp.run(dev[:n * 48].view(torch.float64), dev[n * 48:].view(torch.int32) if segment is not None else None, n)
+        h = fp.host(n)
+    nc = int(h["counters"][0])
+    off = h["cluster_offset"][:nc + 1].tolist()
+    bins, sub_bins = h["cluster_bins"][:n].tolist(), h["sub_bins"][:n].tolist()
+    starts = np.flatnonzero(h["sub_first"][:n])
+    per_cluster = np.diff(np.searchsorted(starts, off)).tolist()     # sub-clusters per cluster
+    bounds = starts.tolist() + [n]
+    clusters = [bins[off[c]:off[c + 1]] for c in range(nc)]
+    subs, s = [], 0
+    for m in per_cluster:
+        subs.append([sub_bins[bounds[u]:bounds[u + 1]] for u in range(s, s + m)])
+        s += m
+    pose = h["pose"][:nc].tolist()
+    orientations = [p[2] for p in pose]
+    final = [((p[0], p[1]), p[2], p[3], (img_w[k], img_h[k]) if k >= 0 else (0, 0))
+             for p, k in zip(pose, h["shape_bin"][:nc].tolist())]
     return clusters, subs, orientations, final
