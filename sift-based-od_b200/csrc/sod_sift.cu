@@ -22,6 +22,9 @@
 // followed, for B > 1, by a stable sort by frame, so each frame's slab ends up in the order one frame alone
 // gets.  sod_sift_extract is the batch of one.  sod_sift_extract_mixed runs frames of different sizes through the
 // same kernels: each reads a frame's geometry through the layout it is instantiated for (Pyramid or Mixed, below).
+// Its pyramid launches are flattened when the largest frame's grid would be mostly idle: a launch's blocks are then
+// the sum of every frame's own tiles of that level, not the largest frame's tiles times the frames, and each block
+// finds its frame and tile in the launch's table of per-frame tile starts (Flat).
 #include <cub/block/block_scan.cuh>
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
@@ -53,10 +56,18 @@ constexpr int kTile = 32;              // blur output tile
 constexpr int kMaxRadius = 13;         // largest blur radius of the default parameters (sigma 3.09, 27 taps)
 constexpr int kOriWarps = 4;
 
+// The block of a pyramid launch that a kernel works on: frame f, tile column x and row y of that frame's level
+// (unsigned as blockIdx is, so that the largest-frame grids compile to the same code as when they read blockIdx).
+struct Tile {
+  int f;
+  unsigned x, y;
+};
+
 // The kernels read a frame's geometry through one accessor, templated on the layout: Pyramid (frames of one size,
 // fstride elements apart) or Mixed (a per-frame table, frames of any size).  Both give level(o, l, f), the size
 // width / height(o, f) of octave o of frame f and octaves(f); the pyramid kernels take a step view of either
-// (UniformUpsample / UniformStep or MixedStep: where frame f reads and writes one level).
+// (UniformUpsample / UniformStep or MixedStep: where frame f reads and writes one level), which also gives tile():
+// which block this is (for frames of one size, blockIdx itself).
 struct Pyramid {
   float* base;
   int64_t off[kMaxOct];                // element offset of octave o's first level
@@ -100,6 +111,33 @@ struct Mixed {
   }
 };
 
+// The blocks of one mixed pyramid launch, flattened: frame f owns blocks start[f] .. start[f + 1] - 1, its tiles of
+// 32 columns in row-major order; a frame without the launch's octave owns none.  The table travels in the launch's
+// parameters, so a captured graph holds it.  Tile counts fit an int: a frame's doubled image has at most 2^32
+// pixels, 2^24 tiles of 32 x 8, and a launch covers at most 64 frames.
+struct Flat {
+  int start[SOD_SIFT_MAX_MIXED_FRAMES + 1];
+  int frames;
+  // the frame that owns this block: the last one whose tiles start at or before it
+  __device__ int frame() const {
+    const int b = blockIdx.x;
+    int lo = 0, hi = frames - 1;
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (start[mid] <= b) lo = mid;
+      else hi = mid - 1;
+    }
+    SOD_DCHECK(lo >= 0 && lo < frames && start[lo] <= b && b < start[lo + 1]);
+    return lo;
+  }
+  // this block's tile in frame f, whose level is w pixels wide
+  __device__ Tile tile(int f, int w) const {
+    const int cols = (w + 31) / 32, t = blockIdx.x - start[f];
+    SOD_DCHECK(cols > 0);
+    return {f, (unsigned)(t % cols), (unsigned)(t / cols)};
+  }
+};
+
 struct Plane {                         // one level of one frame; w = h = 0 when the frame has no such octave
   float* p;
   int w, h;
@@ -120,6 +158,7 @@ struct UniformUpsample {
   int64_t dst_stride;
   __device__ Image image(int f) const { return {src + f * frame_stride, sw, sh, pitch}; }
   __device__ Plane out(int f) const { return {dst + f * dst_stride, 2 * sw, 2 * sh}; }
+  __device__ Tile tile() const { return {(int)blockIdx.z, blockIdx.x, blockIdx.y}; }
 };
 
 struct UniformStep {
@@ -130,14 +169,16 @@ struct UniformStep {
   int64_t fstride;
   __device__ Plane in(int f) const { return {const_cast<float*>(src) + f * fstride, sw, sh}; }
   __device__ Plane out(int f) const { return {dst + f * fstride, dw, dh}; }
+  __device__ Tile tile() const { return {(int)blockIdx.z, blockIdx.x, blockIdx.y}; }
 };
 
 // Frames of any size: level (oi, li) -> level (oo, lo) of each frame (oi = -1: its u8 image).  Grids cover the
-// largest frame; blocks outside their frame's level return at once.
+// largest frame (blockIdx.z = frame); blocks outside their frame's level return at once.
 struct MixedStep {
   static constexpr bool kRagged = true;
   Mixed P;
   int oi, li, oo, lo;
+  __device__ Tile tile() const { return {(int)blockIdx.z, blockIdx.x, blockIdx.y}; }
   __device__ Image image(int f) const {
     SOD_DCHECK(f >= 0 && f < P.frames);
     const FrameGeom& g = P.g[f];
@@ -149,6 +190,15 @@ struct MixedStep {
   }
   __device__ Plane in(int f) const { return plane(oi, li, f); }
   __device__ Plane out(int f) const { return plane(oo, lo, f); }
+};
+
+// MixedStep over each frame's own tiles of level (oo, lo), flattened.
+struct FlatStep : MixedStep {
+  Flat tiles;
+  __device__ Tile tile() const {
+    const int f = tiles.frame();
+    return tiles.tile(f, P.width(oo, f));
+  }
 };
 
 struct Taps {
@@ -259,8 +309,8 @@ void plan_slabs(int frames, int64_t cap, size_t at, Plan* p) {
 
 // A mixed batch: frame f's pyramid at the sum of the pyramids of frames 0..f-1 (each as plan_pyramid sizes it),
 // then the slabs as for a uniform batch, then the geometry table (p->geom, frames x FrameGeom).  p->pyr holds the
-// launch grids: per octave the largest size any frame has, and the largest octave count.  Sizes are the caller's
-// check (1..kMaxSide a side).
+// extrema launch grids: per octave the largest size any frame has, and the largest octave count.  Sizes are the
+// caller's check (1..kMaxSide a side).
 bool make_mixed_plan(const int32_t* wh, int frames, int64_t cap, Plan* p, MixedTable* t) {
   Pyramid& grid = p->pyr;
   grid = Pyramid{};
@@ -336,12 +386,12 @@ __device__ __forceinline__ float fast_atan2(float y, float x) {
 }
 
 // cv::resize(INTER_LINEAR) to exactly twice the size: source coordinate (d + 0.5) / 2 - 0.5, clamped.
-// blockIdx.z = frame.
 template <class S>
 __global__ void sift_upsample_kernel(S s) {
-  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
-  const Image im = s.image(blockIdx.z);
-  const Plane d = s.out(blockIdx.z);
+  const Tile t = s.tile();
+  const int x = t.x * blockDim.x + threadIdx.x, y = t.y * blockDim.y + threadIdx.y;
+  const Image im = s.image(t.f);
+  const Plane d = s.out(t.f);
   const int sw = im.w, sh = im.h, dw = d.w, dh = d.h;
   const int64_t pitch = im.pitch;
   if (x >= dw || y >= dh) return;
@@ -365,17 +415,18 @@ __global__ void sift_upsample_kernel(S s) {
 
 // cv::GaussianBlur on a float image: horizontal pass into shared memory, then the vertical pass, both in the
 // symmetric form of OpenCV's row / column filters (centre tap, then pairs outwards), BORDER_REFLECT_101.
-// blockIdx.z = frame; source and destination have the same size.
+// Source and destination have the same size.
 template <class S>
 __global__ void __launch_bounds__(256) sift_blur_kernel(S s, Taps t) {
   __shared__ float in[kTile + 2 * kMaxRadius][kTile + 2 * kMaxRadius + 1];
   __shared__ float mid[kTile + 2 * kMaxRadius][kTile + 1];
   __shared__ float k[2 * kMaxRadius + 1];
-  const Plane a = s.in(blockIdx.z);
-  const int w = a.w, h = a.h, r = t.r, x0 = blockIdx.x * kTile, y0 = blockIdx.y * kTile, span = kTile + 2 * r;
+  const Tile b = s.tile();
+  const Plane a = s.in(b.f);
+  const int w = a.w, h = a.h, r = t.r, x0 = b.x * kTile, y0 = b.y * kTile, span = kTile + 2 * r;
   if (S::kRagged && (x0 >= w || y0 >= h)) return;
   const float* __restrict__ src = a.p;
-  float* __restrict__ dst = s.out(blockIdx.z).p;
+  float* __restrict__ dst = s.out(b.f).p;
   if (threadIdx.x < 2 * r + 1) k[threadIdx.x] = t.k[threadIdx.x];
   for (int i = threadIdx.x; i < span * span; i += blockDim.x) {
     const int ty = i / span, tx = i - ty * span;
@@ -401,13 +452,14 @@ __global__ void __launch_bounds__(256) sift_blur_kernel(S s, Taps t) {
   }
 }
 
-// cv::resize(INTER_NEAREST) to half size: every other pixel.  blockIdx.z = frame.
+// cv::resize(INTER_NEAREST) to half size: every other pixel.
 template <class S>
 __global__ void sift_halve_kernel(S s) {
-  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
-  const Plane d = s.out(blockIdx.z);
+  const Tile t = s.tile();
+  const int x = t.x * blockDim.x + threadIdx.x, y = t.y * blockDim.y + threadIdx.y;
+  const Plane d = s.out(t.f);
   if (x >= d.w || y >= d.h) return;
-  const Plane a = s.in(blockIdx.z);
+  const Plane a = s.in(t.f);
   d.p[(int64_t)y * d.w + x] = a.p[(int64_t)(2 * y) * a.w + 2 * x];
 }
 
@@ -857,31 +909,78 @@ __global__ void __launch_bounds__(128, 16) sift_descriptor_kernel(L P, const flo
   }
 }
 
-// The Gaussian pyramids of `frames` images (frame_stride bytes apart) into the workspace, one launch per level.
-// The arguments of each pyramid launch, for frames of one size (UniformSteps) or of any size (MixedSteps).
+// Each pyramid launch with its argument and grid, for frames of one size (UniformSteps: frames x one frame's tiles)
+// or of any size (MixedSteps: the largest frame's tiles x frames, or each frame's own tiles, flattened).  th is the
+// launch's tile height in pixels (its tiles are 32 pixels wide).
 struct UniformSteps {
   const uint8_t* gray;
   int width, height;
   int64_t pitch, frame_stride;
   Pyramid P;
-  UniformUpsample upsample() const {
-    return {gray, width, height, pitch, frame_stride, P.level(0, 1), P.fstride};
+  int frames;
+  dim3 grid(int o, int th) const { return dim3((P.w[o] + 31) / 32, (P.h[o] + th - 1) / th, frames); }
+  template <class Launch>
+  void upsample(int th, Launch&& kernel) const {
+    kernel(grid(0, th), UniformUpsample{gray, width, height, pitch, frame_stride, P.level(0, 1), P.fstride});
   }
-  UniformStep step(int oi, int li, int oo, int lo) const {
-    return {P.level(oi, li), P.level(oo, lo), P.w[oi], P.h[oi], P.w[oo], P.h[oo], P.fstride};
+  template <class Launch>
+  void launch(int oi, int li, int oo, int lo, int th, Launch&& kernel) const {
+    kernel(grid(oo, th), UniformStep{P.level(oi, li), P.level(oo, lo), P.w[oi], P.h[oi], P.w[oo], P.h[oo], P.fstride});
   }
 };
+
+// A mixed launch is flattened when its frames' own tiles are at most 1 / kFlatShare of the largest frame's grid
+// times the frames.  Measured on a B200 (DESIGN.md 4): one 2000x1500 frame with fifteen 64x48 ones (6 % of the grid
+// is real) is 13 % faster flattened; 16 frames of six sizes from 640x480 to 2000x1500 (34 % real) are 0.4-0.7 % slower.
+// SOD_SIFT_FLAT_SHARE overrides it in experiment builds (python -m sod_b200.build --variant ...; 1 flattens every
+// launch).
+#ifndef SOD_SIFT_FLAT_SHARE
+#define SOD_SIFT_FLAT_SHARE 4
+#endif
+constexpr int kFlatShare = SOD_SIFT_FLAT_SHARE;
 
 struct MixedSteps {
   Mixed M;
-  MixedStep upsample() const { return {M, -1, 0, 0, 1}; }
-  MixedStep step(int oi, int li, int oo, int lo) const { return {M, oi, li, oo, lo}; }
+  const MixedTable* t;                 // the host copy of the geometry table
+  const Pyramid* G;                    // per octave the largest size any frame has
+  // each frame's tiles of th rows over octave o
+  Flat flat(int o, int th) const {
+    Flat s;
+    s.frames = M.frames;
+    int at = 0;
+    for (int f = 0; f < M.frames; ++f) {
+      const FrameGeom& g = t->f[f];
+      const int w = o < g.n_oct ? (2 * g.width) >> o : 0, h = o < g.n_oct ? (2 * g.height) >> o : 0;
+      s.start[f] = at;
+      at += ((w + 31) / 32) * ((h + th - 1) / th);
+    }
+    s.start[M.frames] = at;
+    return s;
+  }
+  // Launches kernel(grid, argument) of level (oi, li) -> (oo, lo) with tiles of th rows: flattened (FlatStep) when
+  // the frames' own tiles are at most 1 / kFlatShare of the largest frame's grid, else over that grid (MixedStep).
+  template <class Launch>
+  void launch(int oi, int li, int oo, int lo, int th, Launch&& kernel) const {
+    const MixedStep m{M, oi, li, oo, lo};
+    const Flat f = flat(oo, th);
+    const int64_t largest = (int64_t)((G->w[oo] + 31) / 32) * ((G->h[oo] + th - 1) / th) * M.frames;
+    if ((int64_t)f.start[M.frames] * kFlatShare <= largest) {
+      FlatStep x;
+      static_cast<MixedStep&>(x) = m;
+      x.tiles = f;
+      kernel(dim3(f.start[M.frames], 1, 1), x);
+    } else {
+      kernel(dim3((G->w[oo] + 31) / 32, (G->h[oo] + th - 1) / th, M.frames), m);
+    }
+  }
+  template <class Launch>
+  void upsample(int th, Launch&& kernel) const { launch(-1, 0, 0, 1, th, kernel); }
 };
 
-// The Gaussian pyramids of `frames` images into the workspace, one launch per level for all frames; grid holds
-// the launch sizes (per octave the largest frame's).
+// The Gaussian pyramids of the frames into the workspace, one launch per level for all frames, over octaves
+// 0 .. n_oct - 1 (the largest octave count of any frame).
 template <class Steps>
-int build_pyramid(const Steps& s, const Pyramid& grid, int frames, cudaStream_t st) {
+int build_pyramid(const Steps& s, int n_oct, cudaStream_t st) {
   double sig[kLevels];
   const double k = std::pow(2., 1. / kLayers);
   for (int i = 1; i < kLevels; ++i) {
@@ -894,16 +993,16 @@ int build_pyramid(const Steps& s, const Pyramid& grid, int frames, cudaStream_t 
   for (int i = 1; i < kLevels; ++i)
     if (!gaussian_taps(sig[i], &taps[i])) return SOD_ERR_UNSUPPORTED;
   const dim3 pb(32, 8);
-  auto pgrid = [&](int w, int h) { return dim3((w + 31) / 32, (h + 7) / 8, frames); };
-  auto tgrid = [&](int w, int h) { return dim3((w + kTile - 1) / kTile, (h + kTile - 1) / kTile, frames); };
-  const Pyramid& P = grid;
+  static_assert(kTile == 32, "blur tiles are as wide as the pixel kernels' blocks");
   // the doubled image goes to level 1's slot, blurred into level 0, and level 1 is then computed over it
-  sift_upsample_kernel<<<pgrid(P.w[0], P.h[0]), pb, 0, st>>>(s.upsample());
-  sift_blur_kernel<<<tgrid(P.w[0], P.h[0]), 256, 0, st>>>(s.step(0, 1, 0, 0), taps[0]);
-  for (int o = 0; o < P.n_oct; ++o) {
-    if (o > 0) sift_halve_kernel<<<pgrid(P.w[o], P.h[o]), pb, 0, st>>>(s.step(o - 1, kLayers, o, 0));
-    for (int l = 1; l < kLevels; ++l)
-      sift_blur_kernel<<<tgrid(P.w[o], P.h[o]), 256, 0, st>>>(s.step(o, l - 1, o, l), taps[l]);
+  auto upsample = [&](dim3 g, const auto& a) { sift_upsample_kernel<<<g, pb, 0, st>>>(a); };
+  auto halve = [&](dim3 g, const auto& a) { sift_halve_kernel<<<g, pb, 0, st>>>(a); };
+  auto blur = [&](int l) { return [&, l](dim3 g, const auto& a) { sift_blur_kernel<<<g, 256, 0, st>>>(a, taps[l]); }; };
+  s.upsample(8, upsample);
+  s.launch(0, 1, 0, 0, kTile, blur(0));
+  for (int o = 0; o < n_oct; ++o) {
+    if (o > 0) s.launch(o - 1, kLayers, o, 0, 8, halve);
+    for (int l = 1; l < kLevels; ++l) s.launch(o, l - 1, o, l, kTile, blur(l));
   }
   SOD_CHECK_LAUNCH("sift pyramid");
   return SOD_OK;
@@ -911,8 +1010,8 @@ int build_pyramid(const Steps& s, const Pyramid& grid, int frames, cudaStream_t 
 
 // Pyramids, detection, order, duplicate removal, rows and descriptors of p.frames images: the whole of
 // sod_sift_extract, sod_sift_extract_batch and sod_sift_extract_mixed after their argument checks (and, for a mixed
-// batch, its geometry table).  lay reads the pyramids, steps builds them, p.pyr sizes the launches.  Never
-// synchronises.
+// batch, its geometry table).  lay reads the pyramids, steps builds them and sizes their launches, p.pyr sizes the
+// extrema launches (per octave the largest frame's).  Never synchronises.
 template <class L, class Steps>
 int extract_frames(const L& lay, const Steps& steps, const Plan& p, int64_t max_per_frame, const Rows& out,
                    void* workspace, cudaStream_t st) {
@@ -932,7 +1031,7 @@ int extract_frames(const L& lay, const Steps& steps, const Plan& p, int64_t max_
   const int sms = device_sm_count();
   if (sms < 0) return SOD_ERR_CUDA;
   if (p.pyr.n_oct > 0) {
-    if (int rc = build_pyramid(steps, p.pyr, frames, st)) return rc;
+    if (int rc = build_pyramid(steps, p.pyr.n_oct, st)) return rc;
     for (int o = 0; o < p.pyr.n_oct; ++o) {
       const int iw = p.pyr.w[o] - 2 * kBorder, ih = p.pyr.h[o] - 2 * kBorder;
       if (iw <= 0 || ih <= 0) continue;
@@ -984,8 +1083,8 @@ int extract_frames(const L& lay, const Steps& steps, const Plan& p, int64_t max_
 int extract_uniform(const uint8_t* gray, int width, int height, int64_t pitch, int64_t frame_stride, Plan& p,
                     int64_t max_per_frame, const Rows& out, void* workspace, cudaStream_t st) {
   p.pyr.base = (float*)workspace;
-  return extract_frames(p.pyr, UniformSteps{gray, width, height, pitch, frame_stride, p.pyr}, p, max_per_frame, out,
-                        workspace, st);
+  return extract_frames(p.pyr, UniformSteps{gray, width, height, pitch, frame_stride, p.pyr, p.frames}, p,
+                        max_per_frame, out, workspace, st);
 }
 
 // Copies the geometry table of a mixed batch from the kernel parameter into the workspace, so that the call
@@ -1116,7 +1215,8 @@ int sod_sift_describe(const uint8_t* gray, int32_t width, int32_t height, int64_
   cudaStream_t st = (cudaStream_t)stream;
   p.pyr.base = (float*)workspace;
   if (p.pyr.n_oct > 0)
-    if (int rc = build_pyramid(UniformSteps{gray, width, height, pitch, (int64_t)pitch * height, p.pyr}, p.pyr, 1, st))
+    if (int rc = build_pyramid(UniformSteps{gray, width, height, pitch, (int64_t)pitch * height, p.pyr, 1}, p.pyr.n_oct,
+                               st))
       return rc;
   const int sms = device_sm_count();
   if (sms < 0) return SOD_ERR_CUDA;
@@ -1167,7 +1267,7 @@ int sod_sift_extract_mixed(const uint8_t* const* images_host, const int32_t* wh_
   sift_mixed_setup_kernel<<<1, 256, 0, st>>>(t, frames, g);
   SOD_CHECK_LAUNCH("sift_mixed_setup_kernel");
   const Mixed M{(float*)workspace, g, frames};
-  return extract_frames(M, MixedSteps{M}, p, max_per_frame, batch_rows(out), workspace, st);
+  return extract_frames(M, MixedSteps{M, &t, &p.pyr}, p, max_per_frame, batch_rows(out), workspace, st);
 }
 
 }  // extern "C"

@@ -9,7 +9,8 @@ GpuSift.extract_batch runs many same-size frames in one pass (sod_sift_extract_b
 device, in the layout DetectionPipeline.load_queries takes; FrameStream uses it when the extractor has it.
 GpuSift.enqueue_batch is the same pass without the wait, for callers that capture it in a CUDA graph
 (sod_b200.live.LiveDetector).  GpuSift.extract_mixed does the same for frames of different sizes (sod_sift_extract_mixed), such as the training
-images GenerateDatabaseInfo.build_database resizes to one width.
+images GenerateDatabaseInfo.build_database resizes to one width, and GpuSift.enqueue_mixed is its pass without the
+wait (LiveDetector over a camera rig).
 """
 from __future__ import annotations
 
@@ -164,6 +165,19 @@ class _MixedBuffers:
 
 def _align256(n: int) -> int:
     return (n + 255) & ~255
+
+
+def mixed_workspace_bytes(sizes: np.ndarray, capacity: int) -> int:
+    """sod_sift_mixed_workspace_bytes of frames of these (w, h) (int [B, 2]) and `capacity` keypoints a frame, a host
+    computation; raises ValueError where the pass would refuse them (a side above 32768, frames x capacity above
+    2^24)."""
+    n = len(sizes)
+    wh = (C.c_int32 * (2 * n))(*np.asarray(sizes, np.int64).reshape(-1).tolist())
+    need = int(_capi.lib.sod_sift_mixed_workspace_bytes(C.cast(wh, C.c_void_p), n, int(capacity)))
+    if need == 0:
+        raise ValueError(f"sod_sift: {n} frames of sizes {np.asarray(sizes).tolist()} with capacity {capacity} out "
+                         "of range")
+    return need
 
 
 class _Buffers:
@@ -363,6 +377,85 @@ class GpuSift:
         return SiftBatch(t["des"][:rows], t["xy"][:rows], t["angle"][:rows], t["octave"][:rows], t["size"][:rows],
                          t["response"][:rows], t["frame"][:rows], count, offset, (w, h))
 
+    @staticmethod
+    def _mixed_layout(frames, who: str = "extract_mixed") -> tuple:
+        """Sizes (int32 [B, 2]) of a mixed batch's frames, which of them the pass reads in place (CUDA tensors with
+        unit-stride rows), the arena offset of every other one (256-byte aligned, pitch = width) and the arena's
+        bytes."""
+        import torch
+        n = len(frames)
+        if not 1 <= n <= _capi.SIFT_MAX_MIXED_FRAMES:
+            raise ValueError(f"{who} takes 1..{_capi.SIFT_MAX_MIXED_FRAMES} frames, got {n}")
+        for k, f in enumerate(frames):
+            if f.ndim != 2 or (f.dtype != torch.uint8 if _is_cuda(f) else f.dtype != np.uint8):
+                raise ValueError(f"frame {k}: expected a u8 [H, W] image, got {f.dtype} {tuple(f.shape)}")
+        sizes = np.array([(f.shape[1], f.shape[0]) for f in frames], np.int32)
+        in_place = [_is_cuda(f) and f.stride(1) == 1 and f.stride(0) >= f.shape[1] for f in frames]
+        at, arena_off = 0, []
+        for f, keep in zip(frames, in_place):
+            arena_off.append(at)
+            if not keep:
+                at += _align256(f.shape[0] * f.shape[1])
+        return sizes, in_place, arena_off, at
+
+    def _mixed_slot(self, slot: int) -> _MixedBuffers:
+        b = self._mixed[slot]
+        if b is None:
+            b = self._mixed[slot] = _MixedBuffers(self._device)
+        return b
+
+    def _enqueue_mixed(self, b: _MixedBuffers, frames, layout) -> dict:
+        """sod_sift_extract_mixed of `frames` into the buffers b (fitted to them), on the current stream: CUDA frames
+        that are not read in place are copied into b's arena first; host frames must already be there."""
+        import torch
+        sizes, in_place, arena_off, _ = layout
+        ptrs, pitches = [], []
+        for k, f in enumerate(frames):
+            h, w = f.shape
+            if _is_cuda(f) and f.device != b.ws.device:
+                raise ValueError(f"frame {k} is on {f.device}, GpuSift on {b.ws.device}")
+            if in_place[k]:
+                ptrs.append(f.data_ptr())
+                pitches.append(f.stride(0))
+                continue
+            if _is_cuda(f):
+                b.arena[arena_off[k]:arena_off[k] + h * w].view(h, w).copy_(f)
+            ptrs.append(b.arena[arena_off[k]:].data_ptr())
+            pitches.append(w)
+        n = len(frames)
+        wh = (C.c_int32 * (2 * n))(*sizes.reshape(-1).tolist())
+        mk = 0 if self.max_keypoints is None else max(1, int(self.max_keypoints))
+        _capi.check(_capi.lib.sod_sift_extract_mixed(
+            C.cast((C.c_void_p * n)(*ptrs), C.c_void_p), C.cast(wh, C.c_void_p),
+            C.cast((C.c_int64 * n)(*pitches), C.c_void_p), n, mk, C.byref(b.out), b.ws.data_ptr(), b.ws.numel(),
+            torch.cuda.current_stream().cuda_stream), "sod_sift_extract_mixed")
+        return b.t
+
+    def enqueue_mixed(self, frames, slot: int = 0) -> dict:
+        """sod_sift_extract_mixed of a list of up to 64 CUDA u8 [H, W] tensors of any sizes (pitched or not),
+        enqueued on the caller's current stream; never waits, so it can be captured in a CUDA graph.
+
+        -> the output set's device tensors: des, xy, angle, size, response, octave, frame (the packed rows; frame
+        k's are rows offset[k]:offset[k] + count[k]) and flags (int32 [3F + 1], F >= B the frames the slot is sized
+        for: count at [0:B], offset at [F:F + B], overflow at [2F:2F + B], the rows-overflow flag at [3F]).  Nothing
+        is checked on the host.  Frames whose rows are not unit-stride are copied into the slot's arena first.  The
+        slot's buffers are those of extract_mixed: the next call of either on the same slot overwrites them, and one
+        of a larger batch may replace them."""
+        if slot not in (0, 1):
+            raise ValueError("slot must be 0 or 1")
+        frames = list(frames)
+        for k, f in enumerate(frames):
+            if not _is_cuda(f):
+                raise ValueError(f"frame {k}: expected a CUDA u8 [H, W] tensor, got {type(f).__name__}")
+        layout = self._mixed_layout(frames, "enqueue_mixed")
+        need = mixed_workspace_bytes(layout[0], self.capacity)
+        import torch
+        with self._lock, torch.cuda.device(self._device or torch.cuda.current_device()):
+            self._setup_stream()
+            b = self._mixed_slot(slot)
+            b.fit(need, layout[3], len(frames), self.capacity, self.max_keypoints)
+            return self._enqueue_mixed(b, frames, layout)
+
     def extract_mixed(self, images, slot: int = 0) -> SiftBatch:
         """SIFT of a batch of frames of any sizes in one pass (sod_sift_extract_mixed), the result left on the device.
 
@@ -372,40 +465,22 @@ class GpuSift:
 
         Frame k's rows are those extract gives for it alone, in the same order; SiftBatch.frame_sizes holds each
         frame's (w, h).  The buffers of a slot are grown to the largest batch seen, not kept per size.  Waits for
-        the batch; a frame with more than `capacity` keypoints raises SodError naming it."""
+        the batch; a frame with more than `capacity` keypoints raises SodError naming it.  enqueue_mixed is the same
+        pass without the wait."""
         import torch
         if slot not in (0, 1):
             raise ValueError("slot must be 0 or 1")
         frames = [self.prepare(im) for im in images]
         n = len(frames)
-        if not 1 <= n <= _capi.SIFT_MAX_MIXED_FRAMES:
-            raise ValueError(f"extract_mixed takes 1..{_capi.SIFT_MAX_MIXED_FRAMES} frames, got {n}")
-        for k, f in enumerate(frames):
-            if f.ndim != 2 or (f.dtype != torch.uint8 if _is_cuda(f) else f.dtype != np.uint8):
-                raise ValueError(f"frame {k}: expected a u8 [H, W] image, got {f.dtype} {tuple(f.shape)}")
-        sizes = np.array([(f.shape[1], f.shape[0]) for f in frames], np.int32)
-        wh = (C.c_int32 * (2 * n))(*sizes.reshape(-1).tolist())
-        need = int(_capi.lib.sod_sift_mixed_workspace_bytes(C.cast(wh, C.c_void_p), n, self.capacity))
-        if need == 0:
-            raise ValueError(f"sod_sift: {n} frames of sizes {sizes.tolist()} with capacity {self.capacity} out of "
-                             "range")
-        # frames that need a copy (host images, CUDA tensors whose rows are not unit-stride) go to the arena,
-        # each at a 256-byte aligned offset with pitch = width
-        in_place = [_is_cuda(f) and f.stride(1) == 1 and f.stride(0) >= f.shape[1] for f in frames]
-        at, arena_off = 0, []
-        for f, keep in zip(frames, in_place):
-            arena_off.append(at)
-            if not keep:
-                at += _align256(f.shape[0] * f.shape[1])
+        layout = self._mixed_layout(frames)
+        sizes, _, arena_off, at = layout
+        need = mixed_workspace_bytes(sizes, self.capacity)
         with self._lock, torch.cuda.device(self._device or torch.cuda.current_device()):
             self._setup_stream()
-            b = self._mixed[slot]
-            if b is None:
-                b = self._mixed[slot] = _MixedBuffers(self._device)
+            b = self._mixed_slot(slot)
             b.fit(need, at, n, self.capacity, self.max_keypoints)
             if any(_is_cuda(f) for f in frames):
                 self._stream.wait_stream(torch.cuda.current_stream())
-            ptrs, pitches = [], []
             try:
                 with torch.cuda.stream(self._stream):
                     host = [k for k, f in enumerate(frames) if not _is_cuda(f)]
@@ -414,24 +489,8 @@ class GpuSift:
                         b.host[arena_off[k]:arena_off[k] + h * w].copy_(torch.from_numpy(frames[k]).reshape(-1))
                     if host:
                         b.arena[:at].copy_(b.host[:at], non_blocking=True)
-                    for k, f in enumerate(frames):
-                        h, w = f.shape
-                        if _is_cuda(f) and f.device != b.ws.device:
-                            raise ValueError(f"frame {k} is on {f.device}, GpuSift on {b.ws.device}")
-                        if in_place[k]:
-                            ptrs.append(f.data_ptr())
-                            pitches.append(f.stride(0))
-                            continue
-                        if _is_cuda(f):
-                            b.arena[arena_off[k]:arena_off[k] + h * w].view(h, w).copy_(f)
-                        ptrs.append(b.arena[arena_off[k]:].data_ptr())
-                        pitches.append(w)
-                    mk = 0 if self.max_keypoints is None else max(1, int(self.max_keypoints))
-                    _capi.check(_capi.lib.sod_sift_extract_mixed(
-                        C.cast((C.c_void_p * n)(*ptrs), C.c_void_p), C.cast(wh, C.c_void_p),
-                        C.cast((C.c_int64 * n)(*pitches), C.c_void_p), n, mk, C.byref(b.out), b.ws.data_ptr(),
-                        b.ws.numel(), self._stream.cuda_stream), "sod_sift_extract_mixed")
-                    b.flags.copy_(b.t["flags"], non_blocking=True)
+                    t = self._enqueue_mixed(b, frames, layout)
+                    b.flags.copy_(t["flags"], non_blocking=True)
             finally:
                 # as in extract_batch: once this returns the rows may be read on any stream and the buffers are
                 # free; also when a step above raised, since the pinned staging may still be in a copy
@@ -439,7 +498,6 @@ class GpuSift:
             fl, F = b.flags.numpy(), b.frames
             count, offset = fl[:n].astype(np.int64), fl[F:F + n].astype(np.int64)
             overflow, rows_overflow = fl[2 * F:2 * F + n].copy(), int(fl[3 * F])
-            t = b.t
         bad = np.nonzero(overflow)[0]
         if len(bad):
             k = int(bad[0])

@@ -13,6 +13,13 @@ Databases: the benchmark's 1,000 objects x 1,000 rows (bench.make_workload, synt
 the frames) and a 3-object database built with cv2 SIFT from textured images that are planted in the frames.
 
     python tools/bench_live.py --out profiles/r10_live_bench.json
+
+--rig 1920x1080,1280x720,640x480,640x480 times a camera rig instead: one call takes one frame per camera, host frames
+to the final poses of all of them, through three routes alternated call by call:
+  rig         one LiveDetector over the rig's sizes: one replay
+  per_camera  one LiveDetector per size, called camera after camera (one replay and one synchronise each)
+  eager       GpuSift.extract_mixed + DetectionPipeline.load_queries / detect_device / fetch / final_poses
+Reported with the host times: the device time of the rig's replay and the sum of the per-camera replays.
 """
 from __future__ import annotations
 
@@ -142,6 +149,48 @@ def run(db_name, mdb, sizes, frames_by_size, args):
     return out
 
 
+def run_rig(db_name, mdb, sizes, pool, args):
+    R, B = args.max_keypoints, len(sizes)
+    pipe = DetectionPipeline(mdb, max_queries=B * R, frame_wh=np.zeros((B, 2), np.int32))
+    sift = GpuSift(max_keypoints=R)
+    rig = LiveDetector(pipe, sift, sizes)
+    cams = {s: LiveDetector(pipe, sift, s) for s in sizes}
+
+    def eager(frames):
+        sb = sift.extract_mixed(frames)
+        if sb.rows == 0:
+            return {}
+        pipe.scene.frame_wh[:B].copy_(torch.from_numpy(sb.frame_sizes.astype(np.int32)))
+        pipe.load_queries(sb.des, sb.xy, sb.angle, sb.octave, sb.frame)
+        return pipe.final_poses(pipe.fetch(pipe.detect_device(sb.rows)))
+
+    routes = {
+        "rig": lambda fr: [r["final_pose"] for r in rig.detect(fr)],
+        "per_camera": lambda fr: [cams[s].detect([f])[0]["final_pose"] for s, f in zip(sizes, fr)],
+        "eager": eager,
+    }
+    times = {k: [] for k in routes}
+    for i in range(args.warmup + args.frames):
+        fr = pool[i % len(pool)]
+        for name in (list(routes) if i % 2 == 0 else list(routes)[::-1]):
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            routes[name](fr)
+            t1 = time.perf_counter()
+            if i >= args.warmup:
+                times[name].append((t1 - t0) * 1e3)
+    rig_replay = device_ms(rig._graph(True)[0].replay, 50)
+    cam_replay = {f"{w}x{h}": device_ms(cams[(w, h)]._graph(True)[0].replay, 50) for w, h in cams}
+    per_camera = sum(cam_replay[f"{w}x{h}"] for w, h in sizes)
+    rows = [int(c) for c in sift.extract_mixed(pool[0]).count]
+    rec = dict(sizes=[list(s) for s in sizes], capacity_rows_per_frame=R, rows_first_call=rows,
+               host_ms={k: stats(v) for k, v in times.items()},
+               replay_device_ms=dict(rig=rig_replay, per_camera_sum=per_camera, per_size=cam_replay))
+    print(db_name, "rig", json.dumps({k: round(v["median_ms"], 3) for k, v in rec["host_ms"].items()}),
+          f"replay {rig_replay:.3f} ms, per-camera replays {per_camera:.3f} ms", flush=True)
+    return rec
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--frames", type=int, default=500)
@@ -149,6 +198,7 @@ def main():
     ap.add_argument("--max-keypoints", type=int, default=4000)
     ap.add_argument("--pool", type=int, default=8, help="distinct frames per size, cycled")
     ap.add_argument("--sizes", default="640x480,1200x900,2000x1500")
+    ap.add_argument("--rig", default=None, help="camera sizes of a rig, e.g. 1920x1080,1280x720,640x480,640x480")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     if not torch.cuda.is_available():
@@ -159,6 +209,18 @@ def main():
     sizes = [tuple(int(v) for v in s.split("x")) for s in args.sizes.split(",")]
     rng = np.random.default_rng(11)
     small, objs = small_database(rng)
+    if args.rig:
+        rig = [tuple(int(v) for v in s.split("x")) for s in args.rig.split(",")]
+        by_size = {s: scene_frames(rng, objs, *s, args.pool) for s in set(rig)}
+        pool = [[by_size[s][(i + k) % args.pool] for k, s in enumerate(rig)] for i in range(args.pool)]
+        result = dict(card=card[0] if card else None, frames=args.frames, warmup=args.warmup,
+                      max_keypoints=args.max_keypoints, rig={})
+        result["rig"]["3 objects"] = run_rig("3 objects", small, rig, pool, args)
+        result["rig"]["1000 objects x 1000 rows"] = run_rig("1000 x 1000", big_database(), rig, pool, args)
+        if args.out:
+            Path(args.out).parent.mkdir(parents=True, exist_ok=True)
+            Path(args.out).write_text(json.dumps(result, indent=1))
+        return
     frames = {s: scene_frames(rng, objs, *s, args.pool) for s in sizes}
     result = dict(card=card[0] if card else None, frames=args.frames, warmup=args.warmup,
                   max_keypoints=args.max_keypoints, databases={})

@@ -17,8 +17,9 @@ own process, alternated --ab-rounds times.
 --mixed runs only the mixed-size legs (and the A/B with --parent-lib): device time per frame of 16 distinct frames
 of assorted sizes through sod_sift_extract_mixed, through sod_sift_extract one frame at a time and through
 sod_sift_extract_batch grouped by size; the same for a skewed mix (one 2000x1500 frame and fifteen 64x48 ones,
-where most blocks of the largest-frame grids are empty); and GenerateDatabaseInfo.build_database images/s on a
-folder of synthetic PNGs of distinct heights, GPU against cv2.
+where a launch sized for the largest frame would leave most blocks empty); and GenerateDatabaseInfo.build_database
+images/s on a folder of synthetic PNGs of distinct heights, GPU against cv2.  With --parent-lib, both mixes also run
+through that library and through this tree's, each in its own process (SOD_B200_LIB), alternated --ab-rounds times.
 """
 import argparse
 import ctypes as C
@@ -283,6 +284,29 @@ def mixed_per_frame(sizes, reps, seed):
     return out
 
 
+def mixed_legs():
+    return dict(assorted=mixed_per_frame(MIXED_SIZES, 20, 31), skewed=mixed_per_frame(SKEWED_SIZES, 20, 32))
+
+
+def ab_mixed(parent_lib, rounds):
+    """Both mixes with the parent library and with this tree's, alternated, each run in a fresh process."""
+    runs = {"parent": [], "this_tree": []}
+    for _ in range(rounds):
+        for name, lib in (("parent", parent_lib), ("this_tree", str(_capi._LIB_PATH))):
+            r = subprocess.run([sys.executable, __file__, "--out", "-", "--mixed-legs"],
+                               env=dict(os.environ, SOD_B200_LIB=lib), capture_output=True, text=True)
+            if r.returncode:
+                raise RuntimeError(f"mixed run of {lib} failed:\n{r.stderr}")
+            runs[name].append(json.loads(r.stdout.strip().splitlines()[-1]))
+    keys = ("mixed_device_ms_per_frame", "single_each_device_ms_per_frame", "batch_by_size_device_ms_per_frame")
+    med = {name: {f"{mix}.{k}": float(np.median([r[mix][k] for r in v])) for mix in ("assorted", "skewed")
+                  for k in keys} for name, v in runs.items()}
+    spread = {name: {f"{mix}.mixed": [min(r[mix]["mixed_device_ms_per_frame"] for r in v),
+                                      max(r[mix]["mixed_device_ms_per_frame"] for r in v)]
+                     for mix in ("assorted", "skewed")} for name, v in runs.items()}
+    return dict(rounds=runs, median_ms_per_frame=med, min_max_mixed_ms_per_frame=spread)
+
+
 def builder_fps(n_images):
     """GenerateDatabaseInfo.build_database images/s, GPU (GpuSift) against cv2, on PNGs of distinct heights."""
     import GenerateDatabaseInfo as G
@@ -357,6 +381,7 @@ def main():
     ap.add_argument("--parent-lib", default=None, help="another build of libsod_b200.so to compare sod_sift_extract with")
     ap.add_argument("--ab-rounds", type=int, default=3)
     ap.add_argument("--single-lib", default=None, help=argparse.SUPPRESS)
+    ap.add_argument("--mixed-legs", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--mixed", action="store_true", help="only the mixed-size legs (and the A/B with --parent-lib)")
     ap.add_argument("--builder-images", type=int, default=64)
     a = ap.parse_args()
@@ -364,6 +389,9 @@ def main():
         raise SystemExit("bench_sift.py needs a CUDA device")
     if a.single_lib:
         print(json.dumps(single_extract_ms(a.single_lib, a.reps)))
+        return
+    if a.mixed_legs:
+        print(json.dumps(mixed_legs()))
         return
     q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
                        capture_output=True, text=True).stdout.strip().splitlines()
@@ -378,6 +406,8 @@ def main():
         rec["build_database"] = builder_fps(a.builder_images)
         print(json.dumps(rec["build_database"]), flush=True)
         if a.parent_lib:
+            rec["mixed_ab"] = ab_mixed(a.parent_lib, a.ab_rounds)
+            print(json.dumps(rec["mixed_ab"]["median_ms_per_frame"]), flush=True)
             rec["single_frame_ab"] = ab_single(a.parent_lib, a.ab_rounds, a.reps)
             print(json.dumps(rec["single_frame_ab"]["median_ms"]), flush=True)
         Path(a.out).parent.mkdir(parents=True, exist_ok=True)
